@@ -2,6 +2,7 @@
 """Headline benchmark: log_prob + sample throughput (samples/s, inverse/forward + log-det) of the flow hot path.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl product|reference] [--workload c2|c3] [--no-also]
+                    [--dump-outputs DIR]
 
 Workload at every N (weak scaling: fixed rows per GPU, no data-path collective -- rows are independent):
   c2 (default, BASELINE.json configs[1]): 8 SplineCouplingLayers, data_dim=2, hidden 64, 8 RQ-spline bins,
@@ -339,7 +340,7 @@ def measure(wl, args, N, dev, world, rank, barrier, steps, warmup, precision="fp
         xs, ld2 = model.forward(z)
         if ev:
             ev[2].record()
-        return lp, xs
+        return lp, xs, ld2
 
     # end-to-end arm: the same step through the public modules from pinned HOST buffers.  Three input/output buffer
     # sets and three streams (H2D, compute, D2H) let the copy engines run under the kernels, as a serving loop would;
@@ -392,12 +393,17 @@ def measure(wl, args, N, dev, world, rank, barrier, steps, warmup, precision="fp
         t0 = time.time()
         e_start, e_end = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e_start.record()
-        for i in range(steps):
+        # only the last step's outputs are kept (for --dump-outputs): holding every step's outputs into the next step
+        # changes what the caching allocator has to map inside the timed window
+        for i in range(steps - 1):
             step_resident(i, evs[i])
+        last = step_resident(steps - 1, evs[steps - 1])
         e_end.record()
         barrier()
         t1 = time.time()
         launches = N._lib.launch_count() - launches0
+        outputs = dict(zip(("log_prob", "sample", "sample_log_det"), (t.float().cpu() for t in last)))
+        del last
         ms_total = e_start.elapsed_time(e_end)
         clk = clocks.stop(t0, t1) if clocks else None
         # ---- end-to-end through the public API from pinned host buffers ----------------------
@@ -435,10 +441,25 @@ def measure(wl, args, N, dev, world, rank, barrier, steps, warmup, precision="fp
                 "h2d_bytes_per_step": 2 * rows * D * 4, "d2h_bytes_per_step": rows * 4 + rows * D * 4,
                 "ms_per_step_runs": [t / steps for t in e2e_runs], "reported": "median of 7 regions of K steps (this rank)"},
         "gpu_launches": int(launches), "ms_log_prob": ms_lp, "ms_sample": ms_fwd, "clocks": clk, "config": config,
-        "precision": precision, "dev_sets": dev_sets,
+        "precision": precision, "dev_sets": dev_sets, "outputs": outputs,
     }
     N.set_gemm_precision("fp32")
     return res
+
+
+DUMP_ARRAY_BYTES = 8 << 20
+
+
+def dump_outputs(out_dir, prefix, outputs):
+    """Write the outputs of the last timed step as <out_dir>/<prefix>_<name>.npy (float32).  An array larger than 8 MB
+    keeps a fixed, seeded sample of its rows (the same rows in every run), so a default run writes at most 36 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        if t.numel() * t.element_size() > DUMP_ARRAY_BYTES:
+            keep = DUMP_ARRAY_BYTES // (t[0].numel() * t.element_size())
+            rows = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            t = t[rows]
+        np.save(os.path.join(out_dir, f"{prefix}_{name}.npy"), t.numpy())
 
 
 def roofline_for(wl, r, precision):
@@ -510,6 +531,8 @@ def run_product(args):
     wl = args.workload
     steps, warmup = args.steps, max(args.warmup, 3)
     r = measure(wl, args, N, dev, world, rank, barrier, steps, warmup)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, wl, r["outputs"])
     out = {
         "metric": METRIC, "value": r["value"], "unit": UNIT, "n_gpus": world, "steps": steps, "warmup": warmup,
         "ms_per_step": r["ms_per_step"], "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
@@ -528,12 +551,14 @@ def run_product(args):
         modes = ["fp32"] + (["bf16"] if "bf16" in getattr(N, "GEMM_PRECISIONS", ()) and not os.environ.get("NF_SKIP_BF16") else [])
         for mode in modes:
             try:
-                a = measure("c3", args, N, dev, world, rank, barrier, min(steps, 10), 3, precision=mode, with_clocks=False)
+                a = measure("c3", args, N, dev, world, rank, barrier, steps, 3, precision=mode, with_clocks=False)
             except Exception as e:
                 also["c3_" + mode] = {"unavailable": f"{type(e).__name__}: {str(e)[:160]}"}
                 continue
+            if args.dump_outputs and rank == 0:
+                dump_outputs(args.dump_outputs, "c3" if mode == "fp32" else "c3_" + mode, a["outputs"])
             blk = {"workload": WORKLOADS["c3"]["name"], "gemm_precision": mode, "value": a["value"], "unit": UNIT,
-                   "steps": min(steps, 10), "ms_per_step": a["ms_per_step"], "e2e": a["e2e"], "gpu_launches": a["gpu_launches"],
+                   "steps": steps, "ms_per_step": a["ms_per_step"], "e2e": a["e2e"], "gpu_launches": a["gpu_launches"],
                    "ms_per_launch": {"log_prob": a["ms_log_prob"], "sample": a["ms_sample"]},
                    "roofline": roofline_for("c3", a, mode)}
             if mode == "fp32" and rank == 0 and world == 1 and not args.no_cpu:
@@ -566,6 +591,9 @@ def main():
     ap.add_argument("--workload", default="c2", choices=list(WORKLOADS))
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline and eager_cuda legs")
     ap.add_argument("--no-also", action="store_true", help="skip the c3 block of the default run")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the log_prob, sample and sample log-det of the last timed step of each product "
+                         "workload as DIR/<workload>[_<mode>]_<name>.npy, float32")
     args = ap.parse_args()
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if world == 1 and args.gpus > 1 and args.impl == "product":

@@ -1,9 +1,12 @@
 """Host-side pieces of bench.py that need no GPU: the roofline block of the JSON line (algorithmic FLOPs over the measured
-launch time against the measured peak, traffic read from the committed cold-cache capture of the same precision mode) and
-the bounded CPU sample sizes."""
+launch time against the measured peak, traffic read from the committed cold-cache capture of the same precision mode),
+the bounded CPU sample sizes and the writer of --dump-outputs."""
 import importlib.util
 import os
 import sys
+
+import numpy as np
+import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -41,3 +44,22 @@ def test_cpu_sample_is_bounded():
     b = _bench()
     for wl in b.WORKLOADS:
         assert 0 < b.cpu_sample_rows(wl) <= b.WORKLOADS[wl]["rows"]
+
+
+def test_dump_outputs_writes_whole_small_arrays_and_a_fixed_sample_of_large_ones(tmp_path):
+    b = _bench()
+    rows, D = b.WORKLOADS["c3"]["rows"], b.WORKLOADS["c3"]["D"]
+    g = torch.Generator().manual_seed(3)
+    sample = torch.randn(rows, D, generator=g)
+    sample[:, 0] = torch.arange(rows)                   # each row carries its index
+    outputs = {"log_prob": torch.randn(rows, generator=g), "sample": sample}
+    for d in ("a", "b"):
+        b.dump_outputs(str(tmp_path / d), "c3", outputs)
+    lp = np.load(tmp_path / "a" / "c3_log_prob.npy")
+    assert lp.dtype == np.float32 and np.array_equal(lp, outputs["log_prob"].numpy())
+    xs = np.load(tmp_path / "a" / "c3_sample.npy")
+    assert xs.dtype == np.float32 and xs.nbytes == b.DUMP_ARRAY_BYTES and xs.shape[1] == D
+    assert np.array_equal(xs, np.load(tmp_path / "b" / "c3_sample.npy"))
+    # the sample is whole rows of the output, in order
+    src = xs[:, 0].astype(np.int64)
+    assert np.all(np.diff(src) > 0) and np.array_equal(xs, sample.numpy()[src])

@@ -56,16 +56,10 @@ NF_API const char* nf_status_string(int status);
 NF_API const char* nf_last_cuda_error(void);
 /* number of kernel launches issued by this library since load (bench.py's gpu_launches) */
 NF_API int64_t nf_launch_count(void);
-/* library options for A/B measurements: key 1 = fused spline stack variant (0: one warpgroup per CTA, 1: two, default);
- * key 2 = nf_linear_wgrad_tc: longest TMEM accumulation chain in 32-row blocks (default 64);
- * key 3 = nf_ar_blocked_forward in-block kernel (0: CTA-barrier version, 1: warp-private tiles, default);
- * key 5 = nf_linear_tc*: 0 = one TMEM accumulation chain per output tile (gemm_tc.cu), 1 = chains of 2 K blocks folded into
- *         registers with round-to-nearest adds (gemm_tc2.cu, default);
- * key 6 = nf_linear_tc*: K <= 128 through gemm_tc2.cu's persistent direct variant (1, default) or gemm_tc.cu (0);
+/* library options (0 = accepted; any other key than 7, 10 and 11 is refused with NF_ERR_UNSUPPORTED):
  * key 7 = nf_linear_tc* and nf_linear_wgrad_tc*: tensor-core passes per product.  3 = 3xTF32 (fp32 parity, default);
  *         1 = one TF32 pass, operands rounded to the nearest TF32 (the reduced-precision conditioner-GEMM mode the
  *         reference reaches with autocast, optimization/mixed_precision.py:89-105; w_lo is not read);
- * key 9 = nf_linear_tc* (K > 128): TMEM split of gemm_tc2.cu, 3 chain accumulators + 2 A stages (default) or 2 + 4;
  * key 10 = nf_linear_tc* in the one-pass mode: 1 = A operand straight from shared memory (x truncated to TF32 by the tensor
  *         core instead of rounded by the converter warps); default 0;
  * key 11 = nf_spline_transform_* (float32, compact layout, 8 / 10 bins): 1 = TMA-staged kernels (spline_stream.cu,
@@ -283,7 +277,7 @@ NF_API int nf_made_stack_tc_forward(const void* packed, const void* hdr_host, in
 NF_API int64_t nf_made_stack_tc_block_words(int D);
 
 /* ---- a8/a10 and the conditioner MLPs on the tensor cores: y[M,N] = relu?(x[M,K] * W[N,K]^T + bias) ---------
- * fp32 in / fp32 out, 3xTF32 on tcgen05 (fp32-accurate), TMA-fed, accumulators in TMEM (csrc/gemm_tc.cu).
+ * fp32 in / fp32 out, 3xTF32 on tcgen05 (fp32-accurate), TMA-fed, accumulators in TMEM (csrc/gemm_tc2.cu).
  * w_hi / w_lo: the split of W produced by nf_split_tf32 (K contiguous).  ldx / ldw / ldy: row pitches in elements
  * (sub-matrices of larger arrays are addressed by pointer offset + pitch).  k_extent as in nf_gemm.  Requires
  * 16-byte aligned x / w_hi / w_lo and ldx % 4 == 0, ldw % 4 == 0 (NF_ERR_UNSUPPORTED otherwise: use nf_gemm). */

@@ -538,6 +538,8 @@ ar_block_warp_kernel(const float* __restrict__ vin, float* __restrict__ xcur, co
 //     reference's loop, masked_autoregressive_flow.py:46-78), so the noise v stays in registers and the x tile starts at 0.
 // ------------------------------------------------------------------------------------------------------------------
 constexpr int kMmaMaxTiles = 16;     // 8-unit tiles per block (8 degrees of <= 16 units)
+constexpr int kMmaRows = 16;         // rows per warp: one m16 tile
+constexpr int kMmaMaxWarps = 16;
 constexpr int kSxPitch = 12;         // x tile: 8 dims + 4
 constexpr int kH3Pitch = 20;         // layer-3 scratch: 2 tiles + 4
 
@@ -567,38 +569,25 @@ static inline MmaBlockGeom mma_block_geom(const int32_t* gstart, int g0, int g1)
     return m;
 }
 
-// A fragments of the warp's m16 tiles from a row-major tile, split hi / lo: p0 = the lane's element (row rq, column q) of
-// m-tile 0 in the k-tile, p8 = 8 * pitch
-template <int MT>
-__device__ __forceinline__ void mma_load_a(const float* __restrict__ p0, int p8, uint32_t (&ah)[MT][4], uint32_t (&al)[MT][4]) {
-    float x[MT][4];
+// A fragment of the warp's m16 tile from a row-major tile, split hi / lo: p0 = the lane's element (row rq, column q) in
+// the k-tile, p8 = 8 * pitch
+__device__ __forceinline__ void mma_load_a(const float* __restrict__ p0, int p8, uint32_t (&ah)[4], uint32_t (&al)[4]) {
+    float x[4];
+    x[0] = p0[0]; x[1] = p0[p8]; x[2] = p0[4]; x[3] = p0[p8 + 4];
 #pragma unroll
-    for (int mt = 0; mt < MT; ++mt) {
-        const float* p = p0 + mt * 2 * p8;
-        x[mt][0] = p[0]; x[mt][1] = p[p8]; x[mt][2] = p[4]; x[mt][3] = p[p8 + 4];
-    }
-#pragma unroll
-    for (int mt = 0; mt < MT; ++mt)
-#pragma unroll
-        for (int i = 0; i < 4; ++i) split_tf32_reg(x[mt][i], ah[mt][i], al[mt][i]);
+    for (int i = 0; i < 4; ++i) split_tf32_reg(x[i], ah[i], al[i]);
 }
-// acc (main / correction) += A (k-tile) x B fragment, 3xTF32, both m16 tiles
-template <int MT>
-__device__ __forceinline__ void mma_step(float (&am)[MT][4], float (&ac)[MT][4], const uint32_t (&ah)[MT][4], const uint32_t (&al)[MT][4],
-                                         float2 b) {
+// acc (main / correction) += A (k-tile) x B fragment, 3xTF32
+__device__ __forceinline__ void mma_step(float (&am)[4], float (&ac)[4], const uint32_t (&ah)[4], const uint32_t (&al)[4], float2 b) {
     uint32_t bh0, bl0, bh1, bl1;
     split_tf32_reg(b.x, bh0, bl0);
     split_tf32_reg(b.y, bh1, bl1);
-#pragma unroll
-    for (int mt = 0; mt < MT; ++mt) mma_tf32_16x8x8(ac[mt], al[mt], bh0, bh1);
-#pragma unroll
-    for (int mt = 0; mt < MT; ++mt) mma_tf32_16x8x8(am[mt], ah[mt], bh0, bh1);
-#pragma unroll
-    for (int mt = 0; mt < MT; ++mt) mma_tf32_16x8x8(ac[mt], ah[mt], bl0, bl1);
+    mma_tf32_16x8x8(ac, al, bh0, bh1);
+    mma_tf32_16x8x8(am, ah, bh0, bh1);
+    mma_tf32_16x8x8(ac, ah, bl0, bl1);
 }
 
-template <int MT>
-__global__ void __launch_bounds__(MT == 1 ? 512 : 256)
+__global__ void __launch_bounds__(32 * kMmaMaxWarps)
 ar_block_mma_kernel(const float* __restrict__ vin, float* __restrict__ xcur, const float* __restrict__ pre1,
                     const float* __restrict__ pre2, const float* __restrict__ pre3, const float* __restrict__ preo,
                     float* __restrict__ act1, float* __restrict__ act2, float* __restrict__ act3,
@@ -608,7 +597,7 @@ ar_block_mma_kernel(const float* __restrict__ vin, float* __restrict__ xcur, con
                     float* __restrict__ ldacc, int* __restrict__ bad, int64_t B, int D, int H, int g0, int g1, int u0,
                     int mode, int NT, int P) {
     extern __shared__ __align__(16) float sm[];
-    constexpr int R = 16 * MT;                                   // rows per warp
+    constexpr int R = kMmaRows;                                  // rows per warp
     const int nd = g1 - g0, NU8 = NT * 8, AP = NU8 + 4;
     float2* Bf0 = reinterpret_cast<float2*>(sm);                 // [NT][32]       input layer: k-tile = the block's dims
     float2* Bf1 = Bf0 + NT * 32;                                 // [P][32]        hidden -> hidden
@@ -676,7 +665,7 @@ ar_block_mma_kernel(const float* __restrict__ vin, float* __restrict__ xcur, con
     float* a1 = sx + R * kSxPitch;
     float* a2 = a1 + R * AP;
     float* h3s = a2 + R * AP;
-    // the lane's A-fragment origins (row rq, column q) in both m16 tiles of each tile array
+    // the lane's A-fragment origins (row rq, column q) in the m16 tile of each tile array
     const float* sx0 = sx + rq * kSxPitch + q;
     const float* a10 = a1 + rq * AP + q;
     const float* a20 = a2 + rq * AP + q;
@@ -705,27 +694,25 @@ ar_block_mma_kernel(const float* __restrict__ vin, float* __restrict__ xcur, con
             }
         }
         asm volatile("cp.async.commit_group;\n" ::);
-        // ---- per-lane row state: rows mt * 16 + rq + 8 * h; the quad's lane q owns dims q and q + 4 of the block
-        float vreg[MT][2][2], par[MT][2][4], ldv[MT][2];
-        int pois[MT][2];
+        // ---- per-lane row state: rows rq + 8 * h; the quad's lane q owns dims q and q + 4 of the block
+        float vreg[2][2], par[2][4], ldv[2];
+        int pois[2];
 #pragma unroll
-        for (int mt = 0; mt < MT; ++mt)
+        for (int h = 0; h < 2; ++h) {
+            const int r = rq + 8 * h;
+            const bool ok = r < nrow;
+            const float* vr = vin + (r0 + r) * (int64_t)D + g0;
+            vreg[h][0] = (ok && q < nd) ? vr[q] : 0.f;
+            vreg[h][1] = (ok && q + 4 < nd) ? vr[q + 4] : 0.f;
+            const float* prow = preo + (r0 + r) * 2 * (int64_t)D + 2 * g0;
 #pragma unroll
-            for (int h = 0; h < 2; ++h) {
-                const int r = mt * 16 + rq + 8 * h;
-                const bool ok = r < nrow;
-                const float* vr = vin + (r0 + r) * (int64_t)D + g0;
-                vreg[mt][h][0] = (ok && q < nd) ? vr[q] : 0.f;
-                vreg[mt][h][1] = (ok && q + 4 < nd) ? vr[q + 4] : 0.f;
-                const float* prow = preo + (r0 + r) * 2 * (int64_t)D + 2 * g0;
-#pragma unroll
-                for (int n2 = 0; n2 < 2; ++n2) {
-                    const float2 pv = (preo && ok && n2 * 4 + q < nd) ? *reinterpret_cast<const float2*>(prow + 2 * (n2 * 4 + q)) : make_float2(0.f, 0.f);
-                    par[mt][n2][2 * h] = pv.x; par[mt][n2][2 * h + 1] = pv.y;
-                }
-                ldv[mt][h] = (!first && ok && q == 0) ? ldacc[r0 + r] : 0.f;
-                pois[mt][h] = (!first && ok) ? bad[r0 + r] : 0;
+            for (int n2 = 0; n2 < 2; ++n2) {
+                const float2 pv = (preo && ok && n2 * 4 + q < nd) ? *reinterpret_cast<const float2*>(prow + 2 * (n2 * 4 + q)) : make_float2(0.f, 0.f);
+                par[n2][2 * h] = pv.x; par[n2][2 * h + 1] = pv.y;
             }
+            ldv[h] = (!first && ok && q == 0) ? ldacc[r0 + r] : 0.f;
+            pois[h] = (!first && ok) ? bad[r0 + r] : 0;
+        }
         asm volatile("cp.async.wait_group 0;\n" ::: "memory");
         __syncwarp();
 
@@ -736,106 +723,96 @@ ar_block_mma_kernel(const float* __restrict__ vin, float* __restrict__ xcur, con
                 const bool owner = (q == (gi & 3));
                 const float bmu = b3s[2 * gi], bal = b3s[2 * gi + 1];
 #pragma unroll
-                for (int mt = 0; mt < MT; ++mt)
-#pragma unroll
-                    for (int h = 0; h < 2; ++h) {
-                        const float pm = (gi & 4) ? par[mt][1][2 * h] : par[mt][0][2 * h];
-                        const float pa = (gi & 4) ? par[mt][1][2 * h + 1] : par[mt][0][2 * h + 1];
-                        const float xv = (gi & 4) ? vreg[mt][h][1] : vreg[mt][h][0];
-                        float o, t;
-                        affine_ar_elem<float>(mode, xv, bmu + pm, bal + pa, o, t);
-                        if (pois[mt][h]) { o = __int_as_float(0x7fc00000); t = o; }
-                        int nb = is_finite(o) ? 0 : 1;
-                        nb = __shfl_sync(0xffffffffu, nb, (lane & ~3) | (gi & 3));
-                        if (owner) { sx[(mt * 16 + rq + 8 * h) * kSxPitch + gi] = o; ldv[mt][h] += t; }
-                        pois[mt][h] |= nb;           // 0 * NaN of the dense reference poisons every later dim
-                    }
+                for (int h = 0; h < 2; ++h) {
+                    const float pm = (gi & 4) ? par[1][2 * h] : par[0][2 * h];
+                    const float pa = (gi & 4) ? par[1][2 * h + 1] : par[0][2 * h + 1];
+                    const float xv = (gi & 4) ? vreg[h][1] : vreg[h][0];
+                    float o, t;
+                    affine_ar_elem<float>(mode, xv, bmu + pm, bal + pa, o, t);
+                    if (pois[h]) { o = __int_as_float(0x7fc00000); t = o; }
+                    int nb = is_finite(o) ? 0 : 1;
+                    nb = __shfl_sync(0xffffffffu, nb, (lane & ~3) | (gi & 3));
+                    if (owner) { sx[(rq + 8 * h) * kSxPitch + gi] = o; ldv[h] += t; }
+                    pois[h] |= nb;           // 0 * NaN of the dense reference poisons every later dim
+                }
             }
             if (g == D - 1) break;
             __syncwarp();
             const int t0 = Tt[gi], t1 = Tt[gi + 1], cg = cnt[gi];
-            uint32_t ah[MT][4], al[MT][4];
+            uint32_t ah[4], al[4];
             // previous blocks' share of this degree's layer-3 pre-activations: requested now, used two layers later (in the
             // layer-3 loop the load sat on the critical path of every step: 6 % of the stall samples, profiles/r02as)
-            float2 pv3[2][MT][2];
+            float2 pv3[2][2];
 #pragma unroll
             for (int tt = 0; tt < 2; ++tt)
 #pragma unroll
-                for (int mt = 0; mt < MT; ++mt)
-#pragma unroll
-                    for (int h = 0; h < 2; ++h) {
-                        const int r = mt * 16 + rq + 8 * h, j = tt * 8 + 2 * q;
-                        pv3[tt][mt][h] = (pre3 && (tt == 0 || t1 - t0 > 1) && j < cg && r < nrow) ? *reinterpret_cast<const float2*>(pre3 + (r0 + r) * (int64_t)H + u0 + gsl[gi] + j)
-                                                                       : make_float2(0.f, 0.f);
-                    }
+                for (int h = 0; h < 2; ++h) {
+                    const int r = rq + 8 * h, j = tt * 8 + 2 * q;
+                    pv3[tt][h] = (pre3 && (tt == 0 || t1 - t0 > 1) && j < cg && r < nrow) ? *reinterpret_cast<const float2*>(pre3 + (r0 + r) * (int64_t)H + u0 + gsl[gi] + j)
+                                                                   : make_float2(0.f, 0.f);
+                }
             // (B) hidden units of degree g, layer by layer
             for (int nt = t0; nt < t1; ++nt) {               // layer 1: one k-tile (the block's dims; later dims are still zero)
-                float am[MT][4] = {}, ac[MT][4] = {};
-                mma_load_a<MT>(sx0, 8 * kSxPitch, ah, al);
-                mma_step<MT>(am, ac, ah, al, Bf0[nt * 32 + lane]);
+                float am[4] = {}, ac[4] = {};
+                mma_load_a(sx0, 8 * kSxPitch, ah, al);
+                mma_step(am, ac, ah, al, Bf0[nt * 32 + lane]);
                 const int j = (nt - t0) * 8 + 2 * q;
                 const bool live = j < cg;
                 const float2 bb = *reinterpret_cast<const float2*>(bs + nt * 8 + 2 * q);
 #pragma unroll
-                for (int mt = 0; mt < MT; ++mt)
-#pragma unroll
-                    for (int h = 0; h < 2; ++h) {
-                        float2* dst = reinterpret_cast<float2*>(a1 + (mt * 16 + rq + 8 * h) * AP + nt * 8 + 2 * q);
-                        const float2 pv = *dst;
-                        *dst = live ? make_float2(relu_nan(pv.x + bb.x + (am[mt][2 * h] + ac[mt][2 * h])),
-                                                  relu_nan(pv.y + bb.y + (am[mt][2 * h + 1] + ac[mt][2 * h + 1]))) : make_float2(0.f, 0.f);
-                    }
+                for (int h = 0; h < 2; ++h) {
+                    float2* dst = reinterpret_cast<float2*>(a1 + (rq + 8 * h) * AP + nt * 8 + 2 * q);
+                    const float2 pv = *dst;
+                    *dst = live ? make_float2(relu_nan(pv.x + bb.x + (am[2 * h] + ac[2 * h])),
+                                              relu_nan(pv.y + bb.y + (am[2 * h + 1] + ac[2 * h + 1]))) : make_float2(0.f, 0.f);
+                }
             }
             __syncwarp();
             for (int nt = t0; nt < t1; ++nt) {               // layer 2
-                float am[MT][4] = {}, ac[MT][4] = {};
+                float am[4] = {}, ac[4] = {};
                 const float2* bp = Bf1 + pb[nt] * 32 + lane;
                 const int nk = kmax[nt];
                 for (int kt = 0; kt < nk; ++kt) {
-                    mma_load_a<MT>(a10 + kt * 8, 8 * AP, ah, al);
-                    mma_step<MT>(am, ac, ah, al, bp[kt * 32]);
+                    mma_load_a(a10 + kt * 8, 8 * AP, ah, al);
+                    mma_step(am, ac, ah, al, bp[kt * 32]);
                 }
                 const int j = (nt - t0) * 8 + 2 * q;
                 const bool live = j < cg;
                 const float2 bb = *reinterpret_cast<const float2*>(bs + NU8 + nt * 8 + 2 * q);
 #pragma unroll
-                for (int mt = 0; mt < MT; ++mt)
-#pragma unroll
-                    for (int h = 0; h < 2; ++h) {
-                        float2* dst = reinterpret_cast<float2*>(a2 + (mt * 16 + rq + 8 * h) * AP + nt * 8 + 2 * q);
-                        const float2 pv = *dst;
-                        *dst = live ? make_float2(relu_nan(pv.x + bb.x + (am[mt][2 * h] + ac[mt][2 * h])),
-                                                  relu_nan(pv.y + bb.y + (am[mt][2 * h + 1] + ac[mt][2 * h + 1]))) : make_float2(0.f, 0.f);
-                    }
+                for (int h = 0; h < 2; ++h) {
+                    float2* dst = reinterpret_cast<float2*>(a2 + (rq + 8 * h) * AP + nt * 8 + 2 * q);
+                    const float2 pv = *dst;
+                    *dst = live ? make_float2(relu_nan(pv.x + bb.x + (am[2 * h] + ac[2 * h])),
+                                              relu_nan(pv.y + bb.y + (am[2 * h + 1] + ac[2 * h + 1]))) : make_float2(0.f, 0.f);
+                }
             }
             __syncwarp();
             for (int nt = t0; nt < t1; ++nt) {               // layer 3: to global memory and the push scratch, never to a tile
                 const int j = (nt - t0) * 8 + 2 * q;
                 const bool live = j < cg;
-                float am[MT][4] = {}, ac[MT][4] = {};
+                float am[4] = {}, ac[4] = {};
                 const float2* bp = Bf2 + pb[nt] * 32 + lane;
                 const int nk = kmax[nt];
                 for (int kt = 0; kt < nk; ++kt) {
-                    mma_load_a<MT>(a20 + kt * 8, 8 * AP, ah, al);
-                    mma_step<MT>(am, ac, ah, al, bp[kt * 32]);
+                    mma_load_a(a20 + kt * 8, 8 * AP, ah, al);
+                    mma_step(am, ac, ah, al, bp[kt * 32]);
                 }
                 const float2 bb = *reinterpret_cast<const float2*>(bs + 2 * NU8 + nt * 8 + 2 * q);
 #pragma unroll
-                for (int mt = 0; mt < MT; ++mt)
-#pragma unroll
-                    for (int h = 0; h < 2; ++h) {
-                        const int r = mt * 16 + rq + 8 * h;
-                        const float2 pvv = (nt == t0) ? pv3[0][mt][h] : pv3[1][mt][h];
-                        const float2 hv = live ? make_float2(relu_nan(pvv.x + bb.x + (am[mt][2 * h] + ac[mt][2 * h])),
-                                                             relu_nan(pvv.y + bb.y + (am[mt][2 * h + 1] + ac[mt][2 * h + 1]))) : make_float2(0.f, 0.f);
-                        *reinterpret_cast<float2*>(h3s + r * kH3Pitch + j) = hv;
-                        if (g1 < D && live && r < nrow) *reinterpret_cast<float2*>(act3 + (r0 + r) * (int64_t)H + u0 + gsl[gi] + j) = hv;
-                    }
+                for (int h = 0; h < 2; ++h) {
+                    const int r = rq + 8 * h;
+                    const float2 pvv = (nt == t0) ? pv3[0][h] : pv3[1][h];
+                    const float2 hv = live ? make_float2(relu_nan(pvv.x + bb.x + (am[2 * h] + ac[2 * h])),
+                                                         relu_nan(pvv.y + bb.y + (am[2 * h + 1] + ac[2 * h + 1]))) : make_float2(0.f, 0.f);
+                    *reinterpret_cast<float2*>(h3s + r * kH3Pitch + j) = hv;
+                    if (g1 < D && live && r < nrow) *reinterpret_cast<float2*>(act3 + (r0 + r) * (int64_t)H + u0 + gsl[gi] + j) = hv;
+                }
             }
             __syncwarp();
             if (gi + 1 < nd) {                               // push into the parameters of the block's later dims
                 for (int kt = 0; kt < t1 - t0; ++kt) {
-                    mma_load_a<MT>(h30 + kt * 8, 8 * kH3Pitch, ah, al);
+                    mma_load_a(h30 + kt * 8, 8 * kH3Pitch, ah, al);
 #pragma unroll
                     for (int n2 = 0; n2 < 2; ++n2) {
                         if (n2 * 4 + 3 <= gi || n2 * 4 >= nd) continue;          // all four dims of this half are done / beyond the block
@@ -843,12 +820,9 @@ ar_block_mma_kernel(const float* __restrict__ vin, float* __restrict__ xcur, con
                         uint32_t bh0, bl0, bh1, bl1;
                         split_tf32_reg(b.x, bh0, bl0);
                         split_tf32_reg(b.y, bh1, bl1);
-#pragma unroll
-                        for (int mt = 0; mt < MT; ++mt) {
-                            mma_tf32_16x8x8(par[mt][n2], al[mt], bh0, bh1);
-                            mma_tf32_16x8x8(par[mt][n2], ah[mt], bl0, bl1);
-                            mma_tf32_16x8x8(par[mt][n2], ah[mt], bh0, bh1);
-                        }
+                        mma_tf32_16x8x8(par[n2], al, bh0, bh1);
+                        mma_tf32_16x8x8(par[n2], ah, bl0, bl1);
+                        mma_tf32_16x8x8(par[n2], ah, bh0, bh1);
                     }
                 }
                 __syncwarp();                                // the scratch is rewritten by the next step's layer 3
@@ -869,22 +843,16 @@ ar_block_mma_kernel(const float* __restrict__ vin, float* __restrict__ xcur, con
             }
         }
 #pragma unroll
-        for (int mt = 0; mt < MT; ++mt)
-#pragma unroll
-            for (int h = 0; h < 2; ++h) {
-                float s = ldv[mt][h];
-                s += __shfl_xor_sync(0xffffffffu, s, 1);
-                s += __shfl_xor_sync(0xffffffffu, s, 2);
-                const int r = mt * 16 + rq + 8 * h;
-                if (q == 0 && r < nrow) { ldacc[r0 + r] = s; bad[r0 + r] = pois[mt][h]; }
-            }
+        for (int h = 0; h < 2; ++h) {
+            float s = ldv[h];
+            s += __shfl_xor_sync(0xffffffffu, s, 1);
+            s += __shfl_xor_sync(0xffffffffu, s, 2);
+            const int r = rq + 8 * h;
+            if (q == 0 && r < nrow) { ldacc[r0 + r] = s; bad[r0 + r] = pois[h]; }
+        }
         __syncwarp();                                // the drain's reads of the tiles are done before the next fill lands
     }
 }
-
-int g_ar_block_variant = 3;          // nf_set_option(3, v): 0 = first in-block kernel (CTA barriers), 1 = warp-private tiles (FP32 pipe),
-                                     // 2 / 3 = tensor-core in-block steps (mma.sync 3xTF32) with 32 / 16 rows per warp; they fall back
-                                     // to 1 where the layout does not allow them.  Measured at C3: 4.97 / 4.65 / 4.39 ms per pass (1 / 2 / 3)
 
 }  // namespace nf
 
@@ -948,48 +916,41 @@ extern "C" int nf_ar_blocked_forward(const void* v, const void* const* w, const 
         const bool hp = prev && u0 > 0;
         const bool have_preo = pushed;               // some earlier block pushed into preo (it covers every later dim)
         bool launched = false;
-        if (g_ar_block_variant >= 2 && nu > 0 && nd <= kBlkMaxDeg && (nd % 4) == 0) {
-            // tensor-core variant (mma.sync): every degree of the block 4-aligned (per-degree padded layout) and <= 16 units
+        if (nu > 0 && nd <= kBlkMaxDeg && (nd % 4) == 0) {
+            // tensor-core kernel (mma.sync): every degree of the block 4-aligned (per-degree padded layout) and <= 16 units
             bool ok = true;
             for (int g = g0; g < g1; ++g)
                 if ((gstart_host[g] % 4) != 0 || gstart_host[g + 1] - gstart_host[g] > 16) ok = false;
             const MmaBlockGeom mg = mma_block_geom(gstart_host, g0, g1);
             const int NU8 = mg.NT * 8, AP = NU8 + 4;
             const size_t wfl = (size_t)mg.NT * 64 + 2 * (size_t)mg.P * 64 + (size_t)mg.NT * 128 + 3 * (size_t)NU8 + 16 + 60 + NU8 + NU8 / 2;
-            const int MT = g_ar_block_variant == 3 ? 1 : 2;                             // m16 tiles (16 rows) per warp
-            const int R = 16 * MT, maxw = MT == 1 ? 16 : 8;
-            const size_t tfl = (size_t)R * (size_t)(kSxPitch + 2 * AP + kH3Pitch);
+            const size_t tfl = (size_t)kMmaRows * (size_t)(kSxPitch + 2 * AP + kH3Pitch);
             int nw = (ok && mg.NT >= 1 && mg.NT <= kMmaMaxTiles && wfl * sizeof(float) < 180 * 1024)
                          ? (int)((226 * 1024 / sizeof(float) - wfl) / tfl) : 0;
-            if (nw > maxw) nw = maxw;
+            if (nw > kMmaMaxWarps) nw = kMmaMaxWarps;
             if (nw >= 2) {
                 const size_t smem2 = sizeof(float) * (wfl + (size_t)nw * tfl);
-                const int64_t ctas = cdiv(cdiv(B, (int64_t)R), (int64_t)nw);
+                const int64_t ctas = cdiv(cdiv(B, (int64_t)kMmaRows), (int64_t)nw);
                 const int grid2 = (int)(ctas < kNumSMs ? ctas : kNumSMs);              // persistent: one CTA per SM
-#define NF_ABM(MTV)                                                                                                           \
-                do {                                                                                                          \
-                    NF_CUDA(cudaFuncSetAttribute(ar_block_mma_kernel<MTV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2)); \
-                    ar_block_mma_kernel<MTV><<<grid2, 32 * nw, smem2, st>>>(                                                   \
-                        (const float*)v, xcur, prev ? pre1 : nullptr, hp ? pre2 : nullptr, hp ? pre3 : nullptr,                \
-                        have_preo ? preo : nullptr, act1, act2, act3, w0, (const float*)b[0], w1, (const float*)b[1], w2,      \
-                        (const float*)b[2], w3, (const float*)b[3], gstart_dev, ldacc, bad, B, D, H, g0, g1, u0, mode, mg.NT, mg.P); \
-                } while (0)
-                if (MT == 1) NF_ABM(1); else NF_ABM(2);
-#undef NF_ABM
+                NF_CUDA(cudaFuncSetAttribute(ar_block_mma_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem2));
+                ar_block_mma_kernel<<<grid2, 32 * nw, smem2, st>>>(
+                    (const float*)v, xcur, prev ? pre1 : nullptr, hp ? pre2 : nullptr, hp ? pre3 : nullptr,
+                    have_preo ? preo : nullptr, act1, act2, act3, w0, (const float*)b[0], w1, (const float*)b[1], w2,
+                    (const float*)b[2], w3, (const float*)b[3], gstart_dev, ldacc, bad, B, D, H, g0, g1, u0, mode, mg.NT, mg.P);
                 count_launch();
                 NF_LAUNCH_CHECK();
                 launched = true;
             }
         }
         if (!launched) {
-            // warp-private variant: shared transposed weights + one tile per warp; as many warps as fit in 220 KB
+            // warp-private kernel (FP32 pipe): shared transposed weights + one tile per warp; as many warps as fit in 220 KB
             const int need = ((nu + 3) & ~3) + 4 * kWarpChunks;
             const int nup = need <= 48 ? 48 : (need <= 80 ? 80 : (need <= 96 ? 96 : 160));   // compile-time pitches of ar_block_warp_kernel
             const size_t wfl = (size_t)(nd + 2 * nu) * nup + (size_t)nu * 2 * kBlkMaxDeg + ((3 * nu + 3) & ~3) + 2 * kBlkMaxDeg + 16;
             const size_t tfl = (size_t)(nd + 2 * nu) * kBlkPad;
             int nw = wfl * sizeof(float) < 200 * 1024 ? (int)((220 * 1024 / sizeof(float) - wfl) / tfl) : 0;
             if (nw > 8) nw = 8;
-            if (g_ar_block_variant >= 1 && nw >= 2 && need <= 160 && nd <= kBlkMaxDeg && (nd % 4) == 0) {
+            if (nw >= 2 && need <= 160 && nd <= kBlkMaxDeg && (nd % 4) == 0) {
                 const size_t smem2 = sizeof(float) * (wfl + (size_t)nw * tfl);
                 const int64_t ctas = cdiv(cdiv(B, (int64_t)kBlkRows), (int64_t)nw);
                 const int grid2 = (int)(ctas < kNumSMs ? ctas : kNumSMs);              // persistent: one CTA per SM

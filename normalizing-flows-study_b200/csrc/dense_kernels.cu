@@ -4,7 +4,7 @@
 //   nf_mul_rows, nf_relu_backward, nf_col_sum     small elementwise / reduction helpers
 //   nf_batchnorm_*       nn.BatchNorm1d (+ReLU) of the coupling conditioners (coupling_layer.py:20-24)
 // fp32 accumulate in fp32 FFMA (bit-level parity class of the reference's sgemm); fp64 for gradcheck.
-// The tcgen05 GEMMs for the large shapes live in gemm_tc2.cu / gemm_tc.cu / wgrad_tc.cu, the streaming kernels for
+// The tcgen05 GEMMs for the large shapes live in gemm_tc2.cu / wgrad_tc.cu, the streaming kernels for
 // shapes with one tiny dimension in skinny_kernels.cu; this kernel is the exact-fp32 fallback
 // for every shape and the only path for fp64.
 #include "nf_common.cuh"

@@ -1,6 +1,7 @@
-// gemm_tc2.cu -- second tensor-core dense layer:  Y[M,N] = act(X[M,K] * W[N,K]^T + bias), 3xTF32 on tcgen05 with
-// SHORT accumulation chains.  (F.linear of MaskedLinear / MADE and of the coupling / spline conditioners; same contract
-// as gemm_tc.cu's nf_linear_tc_range.)
+// gemm_tc2.cu -- dense layer on the 5th-gen tensor cores:  Y[M,N] = act(X[M,K] * W[N,K]^T + bias), 3xTF32 on tcgen05
+// with SHORT accumulation chains (nf_linear_tc / nf_linear_tc_range; W pre-split into W_hi / W_lo by nf_split_tf32).
+//   (F.linear of MaskedLinear / MADE, masked_linear.py:14-18, made.py:136-140, and of the coupling / spline
+//    conditioner MLPs, coupling_layer.py:18-35, spline_coupling_layer.py:55-62)
 //
 // Why: the tensor core truncates its fp32 accumulator on every MMA, so the error of a TMEM accumulation chain grows
 // linearly with its length (DESIGN.md: K = 1024 -> 384 MMAs -> rms 7e-6 of rms(y), 12x an FFMA GEMM, and a coherent
@@ -33,21 +34,19 @@ constexpr int k2MaxStages = 6;
 constexpr int k2Threads = 320;
 constexpr int k2ThreadsDirect = 448;          // two drainer groups
 constexpr int k2ChainKB = 2;                  // K blocks per TMEM accumulation chain
-constexpr int k2NAcc = 3;                     // chain accumulators in flight by default (drain latency hides behind two chains)
+constexpr int k2NAcc = 3;                     // chain accumulators in flight (drain latency hides behind two chains)
+constexpr int k2AStages = 2;                  // TMEM A stages (hi 32 + lo 32 columns each)
 constexpr int k2TmemCols = 512;               // D0: 0 | D1: 128 | D2: 256 | A stage 0: 384 (hi 32 + lo 32) | A stage 1: 448
-// TMEM split, template parameter NACC: 3 accumulators + 2 A stages (default) or 2 accumulators + 4 A stages
-// (nf_set_option(9, 2): the converters may run three K blocks ahead of the MMAs instead of one)
-int g_gemm_tc2_nacc = 3;
+constexpr int k2ColA = k2NAcc * 128;
+static_assert(k2ColA + k2AStages * 64 == k2TmemCols, "TMEM split");
 // nf_set_option(10, 1), one-pass mode only: feed the X tile to the MMA straight from shared memory (SS form; the tensor
-// core then TRUNCATES x to TF32 instead of the converters' round-to-nearest) -- no converter work at all.  A/B option.
+// core then TRUNCATES x to TF32 instead of the converters' round-to-nearest) -- no converter work at all.
 int g_gemm_tc2_ss = 0;
 constexpr uint32_t k2XBytes = k2BM * k2BK * 4, k2WBytes = k2BN * k2BK * 4;
 constexpr uint32_t k2StageBytes = k2XBytes + 2 * k2WBytes;
 // per drainer group: two 128-float bias tiles (aligned outputs) OR four per-warp [32][33] transpose buffers (unaligned ones)
 constexpr uint32_t k2TbufBytes = 4 * 32 * 33 * 4;
 
-int g_gemm_tc_variant = 1;                    // nf_set_option(5, v): 0 = gemm_tc.cu (one chain per tile), 1 = this kernel
-int g_gemm_tc_small_k = 1;                    // nf_set_option(6, v): K <= 128 through the persistent DIRECT variant (1) or gemm_tc.cu (0)
 // nf_set_option(7, v): tensor-core passes per product.  3 = 3xTF32 (fp32 parity, default); 1 = one TF32 pass (operands
 // rounded to nearest TF32, 10-bit mantissa: the documented reduced-precision mode for the conditioner GEMMs -- three
 // more mantissa bits than bf16, no W_lo traffic, no lo conversions; chains of k2ChainKBFast K blocks = the same 24 MMAs)
@@ -89,10 +88,10 @@ __device__ __forceinline__ void tile_k_range(int n0, int N, int K, const int32_t
 
 // DIRECT = true: contractions of at most 128 (<= 4 K blocks = one short chain per tile).  No register accumulation is
 // needed, so the drainers write each tile straight from TMEM and there are two drainer groups (warps 6-9 and 10-13)
-// taking alternate tiles: for small K the tile's epilogue (64 KB of output) is longer than its main loop, and the
-// non-persistent kernel in gemm_tc.cu pays launch, TMEM allocation and pipeline fill per tile (measured at
-// 2^20 x 64 x 64: 0.22 ms = 2.4 TB/s of a 0.08 ms HBM floor).
-template <bool DIRECT, int NACC>
+// taking alternate tiles: for small K the tile's epilogue (64 KB of output) is longer than its main loop, and a
+// non-persistent kernel pays launch, TMEM allocation and pipeline fill per tile (measured with the first, one-chain-per-
+// tile kernel at 2^20 x 64 x 64: 0.22 ms = 2.4 TB/s of a 0.08 ms HBM floor).
+template <bool DIRECT>
 __global__ void __launch_bounds__(DIRECT ? k2ThreadsDirect : k2Threads, 1)
 gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUtensorMap tm_wh,
                 const __grid_constant__ CUtensorMap tm_wl, float* __restrict__ Y, const float* __restrict__ bias,
@@ -108,23 +107,19 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant_
     uint64_t* bars = reinterpret_cast<uint64_t*>(tbuf_base + (DIRECT ? 2 : 1) * k2TbufBytes);
     uint64_t* full = bars;                         // [S] TMA landed
     uint64_t* empty = full + k2MaxStages;          // [S] stage consumed (MMA commit)
-    constexpr int kAStages = (k2TmemCols - NACC * 128) / 64;      // 64 columns (hi 32 + lo 32) per A stage: 2 or 4
-    constexpr int kAShift = kAStages == 4 ? 2 : 1;
-    constexpr int kColA = NACC * 128;
-    static_assert(kAStages == 2 || kAStages == 4, "TMEM split");
-    uint64_t* a_full = empty + k2MaxStages;        // [<= 4] converters wrote the TMEM A stage
-    uint64_t* a_empty = a_full + 4;                // [<= 4] MMAs consumed the TMEM A stage
-    uint64_t* d_full = a_empty + 4;                // [<= 3] chain accumulator complete
-    uint64_t* d_empty = d_full + 3;                // [<= 3] drainers read the chain accumulator
-    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(d_empty + 3);
+    uint64_t* a_full = empty + k2MaxStages;        // [A] converters wrote the TMEM A stage
+    uint64_t* a_empty = a_full + k2AStages;        // [A] MMAs consumed the TMEM A stage
+    uint64_t* d_full = a_empty + k2AStages;        // [NAcc] chain accumulator complete
+    uint64_t* d_empty = d_full + k2NAcc;           // [NAcc] drainers read the chain accumulator
+    uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(d_empty + k2NAcc);
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int n_tiles = (N + k2BN - 1) / k2BN;
 
     if (warp == 0 && lane == 0) {
         for (int i = 0; i < k2MaxStages; ++i) { tc::mbar_init(&full[i], 1); tc::mbar_init(&empty[i], 1); }
-        for (int i = 0; i < kAStages; ++i) { tc::mbar_init(&a_full[i], 128); tc::mbar_init(&a_empty[i], 1); }
-        for (int i = 0; i < NACC; ++i) { tc::mbar_init(&d_full[i], 1); tc::mbar_init(&d_empty[i], 128); }
+        for (int i = 0; i < k2AStages; ++i) { tc::mbar_init(&a_full[i], 128); tc::mbar_init(&a_empty[i], 1); }
+        for (int i = 0; i < k2NAcc; ++i) { tc::mbar_init(&d_full[i], 1); tc::mbar_init(&d_empty[i], 128); }
         tc::fence_mbar_init();
     }
     if (warp == 1) tc::tmem_alloc(tmem_slot, k2TmemCols);
@@ -174,14 +169,14 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant_
             // rounded up to the instruction's N granularity of 16 -- its cost is proportional to N
             const uint32_t idesc = tc::idesc_tf32_m128((uint32_t)((min(k2BN, N - n0) + 15) & ~15));
             for (int kb = 0; kb < nkb; ++kb, ++it) {
-                const int a = it & (kAStages - 1);
+                const int a = it & (k2AStages - 1);
                 if (ic == 0 && !first_acc_round) tc::mbar_wait(&d_empty[cb], dph ^ 1u);
                 tc::mbar_wait(&full[s], ph);
-                if (!ss) tc::mbar_wait(&a_full[a], (it >> kAShift) & 1);
+                if (!ss) tc::mbar_wait(&a_full[a], (it >> 1) & 1);
                 tc::fence_after_sync();
                 const uint32_t st = tc::smem_u32(smem + s * stage_bytes);
                 const uint64_t d_hi = tc::smem_desc_k_sw128(st + k2XBytes), d_lo = tc::smem_desc_k_sw128(st + k2XBytes + k2WBytes);
-                const uint32_t a_hi = tb + kColA + a * 64, a_lo = a_hi + 32;
+                const uint32_t a_hi = tb + k2ColA + a * 64, a_lo = a_hi + 32;
                 const uint32_t dcol = tb + cb * 128;
                 if (ss) {
                     const uint64_t d_x = tc::smem_desc_k_sw128(st);          // the X tile as landed by TMA: K-major SWIZZLE_128B
@@ -211,7 +206,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant_
                 if (++s == n_stages) { s = 0; ph ^= 1u; }
                 if (chain_end) {
                     ic = 0;
-                    if (++cb == NACC) { cb = 0; dph ^= 1u; first_acc_round = false; }
+                    if (++cb == k2NAcc) { cb = 0; dph ^= 1u; first_acc_round = false; }
                 } else {
                     ++ic;
                 }
@@ -231,9 +226,9 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant_
             int kb_first, nkb;
             tile_k_range(n0, N, K, k_extent, k_begin, kb_first, nkb);
             for (int kb = 0; kb < nkb; ++kb, ++it) {
-                const int a = it & (kAStages - 1);
+                const int a = it & (k2AStages - 1);
                 tc::mbar_wait(&full[s], ph);
-                if (it >= kAStages) tc::mbar_wait(&a_empty[a], ((it >> kAShift) - 1) & 1);
+                if (it >= k2AStages) tc::mbar_wait(&a_empty[a], ((it >> 1) - 1) & 1);
                 tc::fence_after_sync();
                 const uint8_t* xrow = smem + s * stage_bytes + (r >> 3) * 1024 + (r & 7) * 128;
                 uint32_t hi[32], lo[32];
@@ -245,7 +240,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant_
                     tc::split_tf32(v.z, hi[4 * c + 2], lo[4 * c + 2]);
                     tc::split_tf32(v.w, hi[4 * c + 3], lo[4 * c + 3]);
                 }
-                const uint32_t a_hi = lane_addr + kColA + a * 64, a_lo = a_hi + 32;
+                const uint32_t a_hi = lane_addr + k2ColA + a * 64, a_lo = a_hi + 32;
                 {
                     uint32_t t0[16], t1[16];
 #pragma unroll
@@ -276,7 +271,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant_
             const int my_cc = cc;
             if (nkb > 0) ++cc;                                   // one chain per non-empty tile, counted by both groups
             if ((ti & 1) != grp) continue;
-            const int cb = my_cc % NACC;
+            const int cb = my_cc % k2NAcc;
             // aligned outputs: bias tile -> shared memory (two buffers per group, alternating with the group's tiles);
             // unaligned outputs: the same memory is the warps' transpose buffers
             float* grp_mem = reinterpret_cast<float*>(tbuf_base) + grp * (k2TbufBytes / 4);
@@ -284,7 +279,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant_
             float* tbuf = grp_mem + (size_t)(warp - 6 - 4 * grp) * 32 * 33;
             if (vec) tc::stage_bias_tile(bias_s, bias, n0, N, (warp - 6 - 4 * grp) * 32 + lane, 1 + grp);
             if (nkb > 0) {
-                tc::mbar_wait(&d_full[cb], (my_cc / NACC) & 1);
+                tc::mbar_wait(&d_full[cb], (my_cc / k2NAcc) & 1);
                 tc::fence_after_sync();
             }
             const int row = m0 + q * 32 + lane;
@@ -381,7 +376,7 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant_
                 }
                 tc::fence_before_sync();
                 tc::mbar_arrive(&d_empty[cb]);
-                if (++cb == NACC) { cb = 0; dph ^= 1u; }
+                if (++cb == k2NAcc) { cb = 0; dph ^= 1u; }
             }
             // epilogue from registers: the thread owns row m0 + 32q + lane; ReLU + one 256-bit store per 8 columns
             const int row = m0 + q * 32 + lane;
@@ -412,26 +407,19 @@ gemm_tc2_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant_
     if (warp == 1) tc::tmem_dealloc(tb, k2TmemCols);
 }
 
-typedef CUresult (*Encode2Fn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                              const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                              CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static Encode2Fn encode2_fn() {
-    static Encode2Fn fn = nullptr;
-    static bool tried = false;
-    if (!tried) {
-        tried = true;
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
-            qres == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<Encode2Fn>(p);
+// W ~= hi + lo: hi = W rounded to the nearest TF32, lo = (W - hi) rounded to the nearest TF32 (|W - hi - lo| <= 2^-24 |W|)
+__global__ void split_tf32_kernel(const float* __restrict__ w, float* __restrict__ hi, float* __restrict__ lo, int64_t n) {
+    const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        uint32_t h, l;
+        tc::split_tf32_weight(w[i], h, l);
+        hi[i] = __uint_as_float(h);
+        lo[i] = __uint_as_float(l);
     }
-    return fn;
 }
 
 static bool make_map2(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int64_t ld, int box_rows) {
-    Encode2Fn fn = encode2_fn();
+    const tc::EncodeTiledFn fn = tc::encode_tiled_fn();
     if (!fn) return false;
     cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
     cuuint64_t strides[1] = {(cuuint64_t)ld * 4};
@@ -442,7 +430,8 @@ static bool make_map2(CUtensorMap* m, const void* base, int64_t rows, int64_t co
               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-// returns NF_OK when launched; NF_ERR_UNSUPPORTED when the caller should use gemm_tc.cu
+// returns NF_OK when launched; NF_ERR_UNSUPPORTED when a tensor map cannot be encoded or `accumulate` is asked for
+// outside its conditions
 int gemm_tc2_launch(const void* x, const void* w_hi, const void* w_lo, const void* bias, void* y, int64_t M, int64_t N, int64_t K,
                     int64_t ldx, int64_t ldw, int64_t ldy, int relu, const int32_t* k_begin, const int32_t* k_extent,
                     cudaStream_t st, int accumulate) {
@@ -462,22 +451,52 @@ int gemm_tc2_launch(const void* x, const void* w_hi, const void* w_lo, const voi
     if (accumulate && (K > 4 * k2BK || !vec || bias != nullptr || relu)) return NF_ERR_UNSUPPORTED;
     if (K <= 4 * k2BK) {
         const size_t smem = (size_t)k2Stages * k2StageBytes + 2 * k2TbufBytes + 256;
-        NF_CUDA(cudaFuncSetAttribute(gemm_tc2_kernel<true, k2NAcc>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        gemm_tc2_kernel<true, k2NAcc><<<grid, k2ThreadsDirect, smem, st>>>(tx, twh, twl, (float*)y, (const float*)bias, (int)M, (int)N, (int)K,
-                                                                   ldy, relu, k_extent, k_begin, (int)tiles, g_tc_passes, vec, ss, accumulate, wbox);
+        NF_CUDA(cudaFuncSetAttribute(gemm_tc2_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        gemm_tc2_kernel<true><<<grid, k2ThreadsDirect, smem, st>>>(tx, twh, twl, (float*)y, (const float*)bias, (int)M, (int)N, (int)K,
+                                                           ldy, relu, k_extent, k_begin, (int)tiles, g_tc_passes, vec, ss, accumulate, wbox);
     } else {
         const size_t smem = (size_t)k2Stages * k2StageBytes + k2TbufBytes + 256;
-        if (g_gemm_tc2_nacc == 2) {
-            NF_CUDA(cudaFuncSetAttribute(gemm_tc2_kernel<false, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            gemm_tc2_kernel<false, 2><<<grid, k2Threads, smem, st>>>((tx), twh, twl, (float*)y, (const float*)bias, (int)M, (int)N, (int)K, ldy,
-                                                                     relu, k_extent, k_begin, (int)tiles, g_tc_passes, vec, ss, accumulate, wbox);
-        } else {
-            NF_CUDA(cudaFuncSetAttribute(gemm_tc2_kernel<false, k2NAcc>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            gemm_tc2_kernel<false, k2NAcc><<<grid, k2Threads, smem, st>>>(tx, twh, twl, (float*)y, (const float*)bias, (int)M, (int)N, (int)K, ldy,
-                                                                          relu, k_extent, k_begin, (int)tiles, g_tc_passes, vec, ss, accumulate, wbox);
-        }
+        NF_CUDA(cudaFuncSetAttribute(gemm_tc2_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        gemm_tc2_kernel<false><<<grid, k2Threads, smem, st>>>(tx, twh, twl, (float*)y, (const float*)bias, (int)M, (int)N, (int)K, ldy,
+                                                              relu, k_extent, k_begin, (int)tiles, g_tc_passes, vec, ss, accumulate, wbox);
     }
     return NF_OK;
 }
 
 }  // namespace nf
+
+using namespace nf;
+#define NF_REQ(p) do { if ((p) == nullptr) return NF_ERR_NULL; } while (0)
+
+extern "C" int nf_split_tf32(const void* w, void* w_hi, void* w_lo, int64_t n, nf_stream_t stream) {
+    if (n < 0) return NF_ERR_BAD_SHAPE;
+    if (n == 0) return NF_OK;
+    NF_REQ(w); NF_REQ(w_hi); NF_REQ(w_lo);
+    int64_t need = cdiv(n, 256), cap = (int64_t)kNumSMs * 8;
+    split_tf32_kernel<<<(int)(need < cap ? need : cap), 256, 0, (cudaStream_t)stream>>>((const float*)w, (float*)w_hi, (float*)w_lo, n);
+    count_launch();
+    NF_LAUNCH_CHECK();
+    return NF_OK;
+}
+
+extern "C" int nf_linear_tc_range(const void* x, const void* w_hi, const void* w_lo, const void* bias, void* y, int64_t M,
+                                  int64_t N, int64_t K, int64_t ldx, int64_t ldw, int64_t ldy, int relu,
+                                  const int32_t* k_begin, const int32_t* k_extent, nf_stream_t stream) {
+    if (M < 0 || N < 1 || K < 1 || ldx < K || ldw < K || ldy < N) return NF_ERR_BAD_SHAPE;
+    if (M == 0) return NF_OK;
+    NF_REQ(x); NF_REQ(w_hi); NF_REQ(w_lo); NF_REQ(y);
+    // TMA: 16-byte aligned bases and row pitches
+    if (!aligned16(x) || !aligned16(w_hi) || !aligned16(w_lo) || (ldx % 4) != 0 || (ldw % 4) != 0) return NF_ERR_UNSUPPORTED;
+    if (M > 2147483647LL - 128 || N > 2147483647LL - 128 || K > 2147483647LL - 64) return NF_ERR_BAD_SHAPE;
+    const int rc = gemm_tc2_launch(x, w_hi, w_lo, bias, y, M, N, K, ldx, ldw, ldy, relu, k_begin, k_extent, (cudaStream_t)stream, 0);
+    if (rc != NF_OK) return rc;
+    count_launch();
+    NF_LAUNCH_CHECK();
+    return NF_OK;
+}
+
+extern "C" int nf_linear_tc(const void* x, const void* w_hi, const void* w_lo, const void* bias, void* y, int64_t M,
+                            int64_t N, int64_t K, int64_t ldx, int64_t ldw, int64_t ldy, int relu,
+                            const int32_t* k_extent, nf_stream_t stream) {
+    return nf_linear_tc_range(x, w_hi, w_lo, bias, y, M, N, K, ldx, ldw, ldy, relu, nullptr, k_extent, stream);
+}

@@ -383,27 +383,9 @@ made_chain_bf16_kernel(const __grid_constant__ CUtensorMap tm_w0, const __grid_c
     if (warp == 1) tc::tmem_dealloc(tb, kMcTmemCols);
 }
 
-typedef CUresult (*McEncodeFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                               const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                               CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static McEncodeFn mc_encode_fn() {
-    static McEncodeFn fn = nullptr;
-    static bool tried = false;
-    if (!tried) {
-        tried = true;
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
-            qres == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<McEncodeFn>(p);
-    }
-    return fn;
-}
-
 // bf16 weight [rows, K] row-major (K % 64 == 0, rows % 128 == 0): boxes of [128 rows x 64 k] = one SWIZZLE_128B atom block
 static bool mc_make_map(CUtensorMap* m, const void* base, int64_t rows, int64_t K) {
-    McEncodeFn fn = mc_encode_fn();
+    const tc::EncodeTiledFn fn = tc::encode_tiled_fn();
     if (!fn) return false;
     cuuint64_t dims[2] = {(cuuint64_t)K, (cuuint64_t)rows};
     cuuint64_t strides[1] = {(cuuint64_t)K * 2};

@@ -3,7 +3,8 @@
 //   nf_coupling_stack_tc_forward   L x CouplingLayer in eval mode (conditioner BatchNorm folded at pack time)
 // (spline_coupling_layer.py:96-309, coupling_layer.py:40-96, normalizing_flow_model.py:25-128)
 //
-// Mapping.  CTA = 128 threads; thread t owns row t of a 128-row sub-tile and keeps its x / log-det in registers for
+// Mapping.  Warpgroup = 128 threads (one per CTA; two independent ones in the spline stack kernel, see there); thread t
+// owns row t of a 128-row sub-tile and keeps its x / log-det in registers for
 // the whole stack (a row is 8..32 bytes: HBM traffic is 4D in + 4D+4 out).  Per layer and sub-tile:
 //   (a) layer 1 (K = data_dim <= 8) on the FP32 pipe, ReLU, 3xTF32 split, written by the owning thread straight
 //       into TMEM as the A operand (lane = row, column = k) with tcgen05.st          -- no activation in smem
@@ -22,10 +23,6 @@
 
 namespace nf {
 
-#ifdef NF_TC_PROFILE
-__device__ long long g_tc_prof[8];
-#endif
-static int g_tc_two_warpgroups = 1;      // nf_set_option(1, v): spline stack kernel variant (1 = two warpgroups per CTA)
 constexpr int kTcThreads = 128;
 constexpr int kTcSub = 4;            // sub-tiles (of 128 rows) per weight staging
 constexpr int kColAhi = 0, kColAlo = 64, kColD2 = 128, kColD3 = 192;
@@ -139,36 +136,9 @@ __device__ __forceinline__ void hidden2_to_tmem(const float* __restrict__ sb2, u
     }
 }
 
-
 // named barriers (ids 1..15; id 0 is __syncthreads): sub-block synchronisation of the two-warpgroup kernel
 __device__ __forceinline__ void named_sync(int id, int nthreads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
 __device__ __forceinline__ void named_arrive(int id, int nthreads) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
-
-// (c) with two 16-column loads in flight per wait (register budget of the 256-thread kernel: 128 per thread)
-__device__ __forceinline__ void hidden2_to_tmem_2x(const float* __restrict__ sb2, uint32_t lane_addr) {
-#pragma unroll
-    for (int cc = 0; cc < 2; ++cc) {
-        uint32_t v[2][16];
-        tc::tmem_ld16(lane_addr + kColD2 + (2 * cc) * 16, v[0]);
-        tc::tmem_ld16(lane_addr + kColD2 + (2 * cc + 1) * 16, v[1]);
-        tc::wait_ld();
-#pragma unroll
-        for (int h = 0; h < 2; ++h) {
-            const int c = 2 * cc + h;
-            uint32_t hi[16], lo[16];
-#pragma unroll
-            for (int j4 = 0; j4 < 4; ++j4) {
-                const float4 b = *reinterpret_cast<const float4*>(sb2 + c * 16 + j4 * 4);
-                tc::split_tf32(relu_keepnan(__uint_as_float(v[h][j4 * 4 + 0]) + b.x), hi[j4 * 4 + 0], lo[j4 * 4 + 0]);
-                tc::split_tf32(relu_keepnan(__uint_as_float(v[h][j4 * 4 + 1]) + b.y), hi[j4 * 4 + 1], lo[j4 * 4 + 1]);
-                tc::split_tf32(relu_keepnan(__uint_as_float(v[h][j4 * 4 + 2]) + b.z), hi[j4 * 4 + 2], lo[j4 * 4 + 2]);
-                tc::split_tf32(relu_keepnan(__uint_as_float(v[h][j4 * 4 + 3]) + b.w), hi[j4 * 4 + 3], lo[j4 * 4 + 3]);
-            }
-            tc::tmem_st16(lane_addr + kColAhi + c * 16, hi);
-            tc::tmem_st16(lane_addr + kColAlo + c * 16, lo);
-        }
-    }
-}
 
 // layout of one layer block in shared memory (words)
 struct BlkOff { int w1k, b2, b3, w2hi, w2lo, w3hi, w3lo, net_words; };
@@ -186,213 +156,7 @@ __host__ __device__ inline BlkOff blk_offsets(int W1S, int NO3, int HP = 64) {
 }
 
 // ------------------------------------------------------------------------------------------------
-// spline stack
-// ------------------------------------------------------------------------------------------------
-// KS > 0: num_bins known at compile time (== KMAX), every per-bin guard folds away; KS == 0: runtime num_bins <= KMAX
-template <int DM, int KMAX, int KS>
-__global__ void __launch_bounds__(kTcThreads, 2)
-spline_stack_tc_kernel(const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
-                       float* __restrict__ ld, int64_t B, int flags) {
-    const int inverse = flags & NF_STACK_INVERSE;
-    // dynamic shared memory only (no static __shared__), so its base is the CTA's 1024-byte aligned window start:
-    // [2 x layer block | row state | mbarrier | tmem base]
-    extern __shared__ __align__(1024) float sbuf[];
-    const TcHdr hd = read_tc_hdr(packed);
-    const int D = hd.D, K = (KS > 0) ? KS : hd.K, L = hd.L, W1S = hd.W1S, NO3 = hd.NO3, BW = hd.blk_words;
-    float* sx = sbuf + (size_t)2 * BW;                         // [kTcSub][DM+1][128] row state
-    uint64_t* bars = reinterpret_cast<uint64_t*>(sx + kTcSub * (DM + 1) * kTcThreads);
-    uint64_t& bar = bars[0];                                   // MMA completion
-    uint64_t* wbar = bars + 1;                                 // [2] weight-block arrival
-    uint32_t& tmem_base_s = *reinterpret_cast<uint32_t*>(bars + 3);
-    const BlkOff off = blk_offsets(W1S, NO3);
-
-    RqsCfg<float> cfg;
-    cfg.lo = -hd.bound; cfg.hi = hd.bound; cfg.span = 2.0f * hd.bound; cfg.eps = 1e-8f;
-    cfg.min_w = hd.min_w; cfg.min_h = hd.min_h; cfg.min_d = hd.min_d; cfg.scale_w = hd.scale_w; cfg.scale_h = hd.scale_h;
-
-    const int tid = threadIdx.x, warp = tid >> 5;
-    if (warp == 0) tc::tmem_alloc(&tmem_base_s, kTmemCols);
-    if (tid == 0) { tc::mbar_init(&bar, 1); tc::mbar_init(&wbar[0], 1); tc::mbar_init(&wbar[1], 1); tc::fence_mbar_init(); }
-    tc::fence_before_sync();
-    __syncthreads();
-    tc::fence_after_sync();
-    const uint32_t tb = tmem_base_s;
-    const uint32_t lane_addr = tb + ((uint32_t)(warp * 32) << 16);
-    uint32_t phase = 0;
-#ifdef NF_TC_PROFILE
-    long long pt[6] = {0, 0, 0, 0, 0, 0}, pt0 = clock64(), ptk = clock64();
-#define NF_TICK(i) do { long long n__ = clock64(); pt[i] += n__ - pt0; pt0 = n__; } while (0)
-#else
-#define NF_TICK(i) do { } while (0)
-#endif
-
-    constexpr int ROWS = kTcThreads * kTcSub;
-    const int64_t ntiles = (B + ROWS - 1) / ROWS;
-    const float* layers = packed + NF_STACK_HDR;
-
-    // layer blocks travel through the TMA unit (cp.async.bulk, async proxy): thread 0 issues one bulk copy per block,
-    // completion is signalled on wbar[buffer]; the first layer of the first tile is requested here
-    int buf = 0;
-    uint32_t wphase = 0u;                       // bit b = parity to wait for on wbar[b]
-    if (tid == 0 && (int64_t)blockIdx.x < ntiles) {
-        tc::mbar_arrive_expect_tx(&wbar[0], (uint32_t)BW * 4u);
-        tc::bulk_g2s(sbuf, layers + (size_t)(inverse ? L - 1 : 0) * BW, (uint32_t)BW * 4u, &wbar[0]);
-    }
-    for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
-        // per-row state (x, running log-det) of the kTcSub sub-tiles: one shared-memory column per thread
-#pragma unroll
-        for (int s = 0; s < kTcSub; ++s) {
-            const int64_t r = tile * ROWS + s * kTcThreads + tid;
-#pragma unroll
-            for (int d = 0; d < DM; ++d) sx[(s * (DM + 1) + d) * kTcThreads + tid] = (d < D && r < B) ? ld_stream(x + r * D + d) : 0.f;
-            sx[(s * (DM + 1) + DM) * kTcThreads + tid] = 0.f;
-        }
-        for (int li = 0; li < L; ++li) {
-            // everyone is done with the other buffer (previous layer) -> request the next layer into it, then wait
-            // for this layer's block
-            tc::fence_proxy_async_smem();
-            __syncthreads();
-            if (tid == 0) {
-                const bool last = (li == L - 1);
-                if (!last || (tile + gridDim.x < ntiles)) {
-                    const int nli = last ? 0 : li + 1;
-                    tc::mbar_arrive_expect_tx(&wbar[buf ^ 1], (uint32_t)BW * 4u);
-                    tc::bulk_g2s(sbuf + (size_t)(buf ^ 1) * BW, layers + (size_t)(inverse ? L - 1 - nli : nli) * BW,
-                                 (uint32_t)BW * 4u, &wbar[buf ^ 1]);
-                }
-            }
-            tc::mbar_wait(&wbar[buf], (wphase >> buf) & 1u);
-            wphase ^= (1u << buf);
-            const float* sL = sbuf + (size_t)buf * BW;
-            const float* net = sL + NF_LAYER_HDR;
-            const int* meta = reinterpret_cast<const int*>(sL + 16);
-            const bool rescale = meta[1] != 0, bn_on = meta[2] != 0;
-            const float* mask = sL;
-            const uint32_t w2hi = tc::smem_u32(net + off.w2hi), w2lo = tc::smem_u32(net + off.w2lo);
-            const uint32_t w3hi = tc::smem_u32(net + off.w3hi), w3lo = tc::smem_u32(net + off.w3lo);
-
-#pragma unroll 1
-            for (int s = 0; s < kTcSub; ++s) {
-                float xv[DM], tot;
-#pragma unroll
-                for (int d = 0; d < DM; ++d) xv[d] = sx[(s * (DM + 1) + d) * kTcThreads + tid];
-                tot = sx[(s * (DM + 1) + DM) * kTcThreads + tid];
-                if (inverse && bn_on) bn_between_tc<DM>(sL, D, true, xv, tot);
-                float xs[DM], xa[DM];
-#pragma unroll
-                for (int d = 0; d < DM; ++d) {
-                    float v = xv[d];
-                    if (rescale && d < D) v = sL[24 + d] * (v - sL[32 + d]) - hd.bound;
-                    xs[d] = v;
-                    xa[d] = (d < D) ? v * mask[d] : 0.f;
-                }
-                NF_TICK(5);
-                layer1_to_tmem<DM>(net + off.w1k, W1S, xa, lane_addr);
-                tc::wait_st();
-                tc::fence_before_sync();
-                __syncthreads();
-                NF_TICK(0);
-                if (warp == 0) { tc::fence_after_sync(); tc::warp_issue_gemm_k64_3xtf32(tb, kColD2, kColAhi, kColAlo, w2hi, w2lo, 64u, &bar); }
-                tc::mbar_wait(&bar, phase); phase ^= 1;
-                tc::fence_after_sync();
-                NF_TICK(1);
-                hidden2_to_tmem<64>(net + off.b2, lane_addr);
-                tc::wait_st();
-                tc::fence_before_sync();
-                __syncthreads();
-                NF_TICK(2);
-                if (warp == 0) { tc::fence_after_sync(); tc::warp_issue_gemm_k64_3xtf32(tb, kColD3, kColAhi, kColAlo, w3hi, w3lo, (uint32_t)NO3, &bar); }
-                tc::mbar_wait(&bar, phase); phase ^= 1;
-                tc::fence_after_sync();
-                NF_TICK(3);
-
-                // (e) this row's spline parameters: 32 columns per transformed dim
-                float lsum = 0.f;
-                int t = 0;
-#pragma unroll
-                for (int d = 0; d < DM; ++d) {
-                    if (d < D && mask[d] == 0.f) {
-                        uint32_t p0[16], p1[16];
-                        tc::tmem_ld16(lane_addr + kColD3 + t * 32, p0);
-                        if constexpr (3 * KMAX - 1 <= 24) {
-                            uint32_t q[8];
-                            tc::tmem_ld8(lane_addr + kColD3 + t * 32 + 16, q);
-#pragma unroll
-                            for (int j = 0; j < 8; ++j) p1[j] = q[j];
-#pragma unroll
-                            for (int j = 8; j < 16; ++j) p1[j] = 0u;
-                        } else {
-                            tc::tmem_ld16(lane_addr + kColD3 + t * 32 + 16, p1);
-                        }
-                        tc::wait_ld();
-                        const float* b3 = net + off.b3 + t * 32;
-                        float prm[32];
-#pragma unroll
-                        for (int j = 0; j < 16; j += 4) {             // packed fp32 bias adds (FADD2), bias fetched 16 bytes at a time
-                            const float4 ba = *reinterpret_cast<const float4*>(b3 + j), bb = *reinterpret_cast<const float4*>(b3 + 16 + j);
-                            const float2 s0 = __fadd2_rn(make_float2(__uint_as_float(p0[j]), __uint_as_float(p0[j + 1])), make_float2(ba.x, ba.y));
-                            const float2 s1 = __fadd2_rn(make_float2(__uint_as_float(p0[j + 2]), __uint_as_float(p0[j + 3])), make_float2(ba.z, ba.w));
-                            const float2 s2 = __fadd2_rn(make_float2(__uint_as_float(p1[j]), __uint_as_float(p1[j + 1])), make_float2(bb.x, bb.y));
-                            const float2 s3 = __fadd2_rn(make_float2(__uint_as_float(p1[j + 2]), __uint_as_float(p1[j + 3])), make_float2(bb.z, bb.w));
-                            prm[j] = s0.x; prm[j + 1] = s0.y; prm[j + 2] = s1.x; prm[j + 3] = s1.y;
-                            prm[16 + j] = s2.x; prm[16 + j + 1] = s2.y; prm[16 + j + 2] = s3.x; prm[16 + j + 3] = s3.y;
-                        }
-                        // columns of one transformed dim: [uw: KMAX slots | uh: KMAX slots | ud: KMAX-1 slots] (host packing)
-                        float uw[KMAX], uh[KMAX], ud[KMAX];
-#pragma unroll
-                        for (int j = 0; j < KMAX; ++j) {
-                            uw[j] = prm[j];
-                            uh[j] = prm[KMAX + j];
-                            ud[j] = (j < KMAX - 1) ? prm[2 * KMAX + j] : 0.f;
-                        }
-                        float out, lad;
-                        rqs_eval<float, KMAX, true>(xs[d], uw, uh, ud, K, inverse != 0, cfg, out, lad);
-                        if (rescale) out = (out + hd.bound) * sL[40 + d] + sL[32 + d];
-                        xv[d] = out;
-                        lsum += lad;
-                        ++t;
-                    }
-                }
-#pragma unroll
-                for (int d = 0; d < DM; ++d) xv[d] = scrub0(xv[d]);      // layer-level scrub (:130-135)
-                tot += scrub0(lsum);
-                if (!inverse && bn_on) bn_between_tc<DM>(sL, D, false, xv, tot);
-#pragma unroll
-                for (int d = 0; d < DM; ++d) sx[(s * (DM + 1) + d) * kTcThreads + tid] = xv[d];
-                sx[(s * (DM + 1) + DM) * kTcThreads + tid] = tot;
-                NF_TICK(4);
-            }
-            buf ^= 1;
-        }
-#pragma unroll
-        for (int s = 0; s < kTcSub; ++s) {
-            const int64_t r = tile * ROWS + s * kTcThreads + tid;
-            if (r < B) {
-                float zr[DM];
-#pragma unroll
-                for (int d = 0; d < DM; ++d) zr[d] = sx[(s * (DM + 1) + d) * kTcThreads + tid];
-                if (!(flags & NF_STACK_SKIP_Y)) {
-#pragma unroll
-                    for (int d = 0; d < DM; ++d) if (d < D) st_stream(y + r * D + d, zr[d]);
-                }
-                const float tot = sx[(s * (DM + 1) + DM) * kTcThreads + tid];
-                st_stream(ld + r, (flags & NF_STACK_LOG_PROB_HEAD) ? nf_stack_row_head<DM>(zr, D, tot) : tot);
-            }
-        }
-    }
-    tc::fence_before_sync();
-    __syncthreads();
-    if (warp == 0) tc::tmem_dealloc(tb, kTmemCols);
-#ifdef NF_TC_PROFILE
-    if (blockIdx.x == 0 && tid == 0) {
-        for (int i = 0; i < 6; ++i) g_tc_prof[i] = pt[i];
-        g_tc_prof[6] = (long long)clock64() - ptk;
-    }
-#endif
-}
-
-// ------------------------------------------------------------------------------------------------
-// spline stack, two independent warpgroups per CTA (256 threads), half-K staging.
+// spline stack: two independent warpgroups per CTA (256 threads), half-K staging.
 // Each warpgroup owns 128 TMEM columns: A_hi 32 | A_lo 32 | D 64.  A K=64 contraction is fed in two halves of 32
 // (st half 1 -> 12 MMAs -> st half 2 -> 12 accumulating MMAs), the second half being computed on the FP32 pipe while
 // the first half's MMAs run; the head accumulator aliases D2 (read out to registers first).  Halving the A footprint
@@ -441,6 +205,7 @@ __device__ __forceinline__ void hidden2_chunk(const uint32_t (&v)[16], const flo
     }
 }
 
+// KS > 0: num_bins known at compile time (== KMAX), every per-bin guard folds away; KS == 0: runtime num_bins <= KMAX
 template <int DM, int KMAX, int KS>
 __global__ void __launch_bounds__(kTc2Threads, 2)
 spline_stack_tc2_kernel(const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
@@ -1032,32 +797,19 @@ extern "C" int nf_spline_stack_tc_forward(const void* packed, const void* hdr_ho
     if (smem > 227 * 1024) return NF_ERR_UNSUPPORTED;
     const int rows = kTcThreads * kTcSub;
     const int64_t ntiles = cdiv(B, rows);
-    const bool two_wg = g_tc_two_warpgroups && NO3 <= 64;
+    int per_sm = (int)((227 * 1024) / (smem + 1024));
+    if (per_sm < 1) return NF_ERR_UNSUPPORTED;
+    if (per_sm > 512 / kTmemCols) per_sm = 512 / kTmemCols;   // TMEM: 512 columns per SM
+    const int64_t cap = (int64_t)kNumSMs * per_sm;
+    const int grid = (int)(ntiles < cap ? ntiles : cap);
 #define NF_TC(DMv, KMv, KSv)                                                                                         \
     do {                                                                                                             \
-        if (two_wg) {                                                                                                \
-            auto kern2 = spline_stack_tc2_kernel<DMv, KMv, KSv>;                                                     \
-            NF_CUDA(cudaFuncSetAttribute(kern2, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));            \
-            NF_CUDA(cudaFuncSetAttribute(kern2, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)); \
-            int per_sm2 = (int)((227 * 1024) / (smem + 1024));                                                       \
-            if (per_sm2 < 1) return NF_ERR_UNSUPPORTED;                                                              \
-            if (per_sm2 > 512 / kTmemCols) per_sm2 = 512 / kTmemCols;                                                \
-            const int64_t cap2 = (int64_t)kNumSMs * per_sm2;                                                         \
-            const int grid2 = (int)(ntiles < cap2 ? ntiles : cap2);                                                  \
-            kern2<<<grid2, kTc2Threads, smem, st>>>((const float*)packed, (const float*)x, (float*)y, (float*)ld, B, inverse); \
-            break;                                                                                                   \
-        }                                                                                                            \
-        auto kern = spline_stack_tc_kernel<DMv, KMv, KSv>;                                                           \
+        auto kern = spline_stack_tc2_kernel<DMv, KMv, KSv>;                                                          \
         NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                 \
         /* ask for the largest shared-memory carveout: with the default preference the driver sizes the SM for ONE   \
            CTA of this kernel and the second co-resident CTA (the latency hiding of this design) never arrives */    \
         NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)); \
-        int per_sm = (int)((227 * 1024) / (smem + 1024));                                                            \
-        if (per_sm < 1) return NF_ERR_UNSUPPORTED;                                                                   \
-        if (per_sm > 512 / kTmemCols) per_sm = 512 / kTmemCols;   /* TMEM: 512 columns per SM */                     \
-        const int64_t cap = (int64_t)kNumSMs * per_sm;                                                               \
-        const int grid = (int)(ntiles < cap ? ntiles : cap);                                                         \
-        kern<<<grid, kTcThreads, smem, st>>>((const float*)packed, (const float*)x, (float*)y, (float*)ld, B, inverse); \
+        kern<<<grid, kTc2Threads, smem, st>>>((const float*)packed, (const float*)x, (float*)y, (float*)ld, B, inverse); \
     } while (0)
 #define NF_TC_K(DMv)                                      \
     do {                                                  \
@@ -1075,13 +827,6 @@ extern "C" int nf_spline_stack_tc_forward(const void* packed, const void* hdr_ho
     NF_LAUNCH_CHECK();
     return NF_OK;
 }
-
-#ifdef NF_TC_PROFILE
-// debug builds only (-DNF_TC_PROFILE): per-phase cycle counters of CTA 0 / thread 0 of the last launch
-extern "C" __attribute__((visibility("default"))) int nf_debug_tc_profile(long long* out) {
-    return cudaMemcpyFromSymbol(out, nf::g_tc_prof, sizeof(long long) * 8) == cudaSuccess ? 0 : -4;
-}
-#endif
 
 extern "C" int64_t nf_coupling_stack_tc_block_words(int D) {
     if (D < 1 || D > NF_STACK_DMAX) return -1;
@@ -1182,22 +927,15 @@ extern "C" int nf_made_stack_tc_forward(const void* packed, const void* hdr_host
     return NF_OK;
 }
 
-// library options (debugging / A-B measurements): key 1 = spline stack kernel variant (0: one warpgroup, 1: two);
-// key 2 = weight-gradient kernel: maximum number of 32-row K blocks accumulated in TMEM per split (wgrad_tc.cu);
-// key 3 = in-block kernel of the blocked sequential direction (ar_blocked.cu): 0 = CTA-barrier version, 1 = warp-private tiles
-// key 5 / 6 = dense-layer kernel selection (gemm_tc2.cu); key 7 = tensor-core passes per product of the dense-layer and
-// weight-gradient kernels: 3 = 3xTF32 (fp32 parity, default), 1 = one TF32 pass (reduced-precision mode);
-// key 11 = compact spline transform: 1 = TMA-staged kernels of spline_stream.cu (default), 0 = first-version kernels
-namespace nf { int g_wgrad_max_kb = 64; extern int g_ar_block_variant; extern int g_gemm_tc_variant; extern int g_gemm_tc_small_k; extern int g_tc_passes; extern int g_gemm_tc2_nacc; extern int g_gemm_tc2_ss; extern int g_spline_stream; }
+// library options: key 7 = tensor-core passes per product of the dense-layer and weight-gradient kernels: 3 = 3xTF32
+// (fp32 parity, default), 1 = one TF32 pass (reduced-precision mode, set_gemm_precision("tf32"));
+// key 10 = one-pass mode only: the dense layer reads its X operand straight from shared memory (SS form, gemm_tc2.cu;
+// set_gemm_precision("bf16") turns it on); key 11 = compact spline transform: 1 = TMA-staged kernels of spline_stream.cu
+// (default), 0 = first-version kernels (the bit-identical reference).  Any other key is refused.
+namespace nf { extern int g_tc_passes; extern int g_gemm_tc2_ss; extern int g_spline_stream; }
 extern "C" int nf_set_option(int key, int value) {
-    if (key == 1) { nf::g_tc_two_warpgroups = value != 0; return NF_OK; }
-    if (key == 2) { if (value < 1) return NF_ERR_BAD_SHAPE; nf::g_wgrad_max_kb = value; return NF_OK; }
-    if (key == 3) { if (value < 0 || value > 3) return NF_ERR_UNSUPPORTED; nf::g_ar_block_variant = value; return NF_OK; }
-    if (key == 5) { nf::g_gemm_tc_variant = value != 0; return NF_OK; }
-    if (key == 6) { nf::g_gemm_tc_small_k = value != 0; return NF_OK; }
-    if (key == 10) { nf::g_gemm_tc2_ss = value != 0; return NF_OK; }
-    if (key == 9) { if (value != 2 && value != 3) return NF_ERR_BAD_SHAPE; nf::g_gemm_tc2_nacc = value; return NF_OK; }
-    if (key == 11) { nf::g_spline_stream = value != 0; return NF_OK; }
     if (key == 7) { if (value != 1 && value != 3) return NF_ERR_BAD_SHAPE; nf::g_tc_passes = value; return NF_OK; }
+    if (key == 10) { nf::g_gemm_tc2_ss = value != 0; return NF_OK; }
+    if (key == 11) { nf::g_spline_stream = value != 0; return NF_OK; }
     return NF_ERR_UNSUPPORTED;
 }

@@ -1,5 +1,6 @@
 // tc_common.cuh -- sm_100a tensor-core plumbing shared by the tcgen05 kernels: mbarrier, TMEM allocation,
-// tcgen05.mma (kind::tf32, A from TMEM or shared memory, B from shared memory), tcgen05.ld/st, descriptors.
+// tcgen05.mma (kind::tf32, A from TMEM or shared memory, B from shared memory), tcgen05.ld/st, descriptors, and
+// the host-side lookup of the TMA tensor-map encoder.
 //
 // Conventions used by every kernel here:
 //   * operands are fp32 containers read as TF32 by the tensor core; fp32 accuracy comes from the 3xTF32 split
@@ -10,6 +11,7 @@
 //     (n/8)*1024 + (n%8)*128 and its eight 16-byte chunks are XOR-swizzled with (n%8); the host packs that image;
 //   * A (activations) is written by its owning thread into TMEM: lane = tile row, column = k (M = 128).
 #pragma once
+#include <cuda.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 
@@ -283,6 +285,24 @@ __device__ __forceinline__ void stage_bias_tile(float* bias_s, const float* __re
 // byte offset of element (n, k) inside a K-major SWIZZLE_128B image of an [rows][K] fp32 matrix (K % 32 == 0, rows % 8 == 0)
 __host__ __device__ constexpr uint32_t sw128_offset(uint32_t n, uint32_t k, uint32_t rows) {
     return (k >> 5) * (rows * 128u) + (n >> 3) * 1024u + (n & 7u) * 128u + ((((k & 31u) >> 2) ^ (n & 7u)) << 4) + (k & 3u) * 4u;
+}
+
+// ---- host: TMA tensor maps -----------------------------------------------------------------------------
+// cuTensorMapEncodeTiled through the runtime's driver entry point (the library does not link libcuda); nullptr when
+// the driver does not provide it.  Each caller builds its own maps: box, swizzle and element type differ per kernel.
+typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
+                                  const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
+                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
+
+inline EncodeTiledFn encode_tiled_fn() {
+    static const EncodeTiledFn fn = [] {
+        void* p = nullptr;
+        cudaDriverEntryPointQueryResult qres;
+        const bool ok = cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
+                        qres == cudaDriverEntryPointSuccess;
+        return ok ? reinterpret_cast<EncodeTiledFn>(p) : nullptr;
+    }();
+    return fn;
 }
 
 }  // namespace tc

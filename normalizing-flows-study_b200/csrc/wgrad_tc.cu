@@ -14,7 +14,7 @@
 // 3xTF32: D += A_hi*B_hi + A_lo*B_hi + A_hi*B_lo with fp32 accumulation in TMEM.
 // Few output tiles, very long reduction => split over the batch: grid = tiles x splits, every split writes its
 // partial tile to the caller's workspace and wgrad_reduce_kernel sums the partials in a fixed order (deterministic,
-// no atomics).  Warp roles as in gemm_tc.cu: warp 0 TMA producer, warp 1 MMA issuer, warps 2-5 converters + epilogue.
+// no atomics).  Warp roles: warp 0 TMA producer, warp 1 MMA issuer, warps 2-5 converters + epilogue.
 #include <cuda.h>
 #include "nf_common.cuh"
 #include "tc_common.cuh"
@@ -287,27 +287,9 @@ wgrad_reduce_wide_kernel(const float* __restrict__ part, float* __restrict__ dw,
     }
 }
 
-typedef CUresult (*WgEncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*, const cuuint64_t*,
-                                    const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                    CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static WgEncodeTiledFn wg_encode_fn() {
-    static WgEncodeTiledFn fn = nullptr;
-    static bool tried = false;
-    if (!tried) {
-        tried = true;
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
-            qres == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<WgEncodeTiledFn>(p);
-    }
-    return fn;
-}
-
 // row-major fp32 [rows, cols] with pitch ld: box = 32 rows x 32 floats (one 128-byte swizzle span wide), zero OOB fill
 static bool wg_make_map(CUtensorMap* m, const void* base, int64_t rows, int64_t cols, int64_t ld, CUtensorMapSwizzle swz) {
-    WgEncodeTiledFn fn = wg_encode_fn();
+    const tc::EncodeTiledFn fn = tc::encode_tiled_fn();
     if (!fn) return false;
     cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
     cuuint64_t strides[1] = {(cuuint64_t)ld * 4};
@@ -318,12 +300,12 @@ static bool wg_make_map(CUtensorMap* m, const void* base, int64_t rows, int64_t 
               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-extern int g_wgrad_max_kb;     // nf_set_option(2, v)
-extern int g_tc_passes;        // nf_set_option(7, v)
+constexpr int kWgradMaxKB = 64;    // K blocks per TMEM accumulation chain at most (see wg_plan)
+extern int g_tc_passes;             // nf_set_option(7, v)
 
 // Number of batch splits.  (1) Fill two CTAs per SM, with at least 8 K blocks (256 rows) per split.  (2) The tensor
 // core's fp32 accumulation truncates (measured: the error of a TMEM accumulation chain grows linearly, ~2^-24 of the
-// running sum per MMA, 12 MMAs per K block), so a chain is at most g_wgrad_max_kb K blocks long; the partials are then
+// running sum per MMA, 12 MMAs per K block), so a chain is at most kWgradMaxKB K blocks long; the partials are then
 // summed with round-to-nearest fp32 adds by wgrad_reduce_kernel.
 static void wg_plan(int64_t B, int64_t N, int64_t K, int* splits, int* kb_per_split, int* nkb_out) {
     const int64_t tiles = cdiv(N, kWgBM) * cdiv(K, kWgBN);
@@ -332,7 +314,7 @@ static void wg_plan(int64_t B, int64_t N, int64_t K, int* splits, int* kb_per_sp
     if (s < 1) s = 1;
     const int64_t smax = nkb / 8 > 1 ? nkb / 8 : 1;
     if (s > smax) s = smax;
-    const int64_t smin = cdiv(nkb, (int64_t)g_wgrad_max_kb);
+    const int64_t smin = cdiv(nkb, (int64_t)kWgradMaxKB);
     if (s < smin) s = smin;
     const int64_t per = cdiv(nkb, s);
     s = cdiv(nkb, per);

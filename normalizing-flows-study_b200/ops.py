@@ -847,7 +847,7 @@ def _ptr_array(tensors):
 
 
 def ar_sequential_blocked(v, folded, mode):
-    """MAF.forward / IAF.inverse, blocked: previous-block contributions on tcgen05, in-block steps in ar_block_warp_kernel.
+    """MAF.forward / IAF.inverse, blocked: previous-block contributions on tcgen05, in-block steps in ar_blocked.cu.
     Returns None when the configuration is not taken (no TF32 splits, D not a multiple of 4)."""
     if folded.w_split is None or v.dtype != torch.float32 or folded.D % 4 or AR_BLOCK_DEGREES % 4:
         return None

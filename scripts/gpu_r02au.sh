@@ -1,5 +1,5 @@
 #!/bin/bash
-# pass au: mma.sync in-block kernel as the default of the blocked sequential direction: route tests (all variants), full-size
+# pass au: mma.sync in-block kernel as the default of the blocked sequential direction: route tests, full-size
 # C3 comparisons, sampler timing in both precision modes.  usage: <tag>
 set -u
 TAG=${1:-r02au}
@@ -9,4 +9,3 @@ timeout 600 python -m pytest tests -q -m gpu -p no:cacheprovider --timeout=300 -
 for prec in fp32 bf16; do
   timeout 120 python scripts/sampler_target.py --precision $prec --reps 10 > gpurun_out/sampler_${TAG}_$prec.json 2> gpurun_out/sampler_${TAG}_$prec.err; echo "sampler $prec rc=$?"; cat gpurun_out/sampler_${TAG}_$prec.json
 done
-timeout 120 python scripts/sampler_target.py --variant 1 --reps 10 > gpurun_out/sampler_${TAG}_v1.json 2>/dev/null; cat gpurun_out/sampler_${TAG}_v1.json

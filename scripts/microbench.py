@@ -213,17 +213,6 @@ def bench_gemm():
                 ms = timeit(lambda: ops.linear_tc(a, hi, lo, bias, relu=True), reps=3, inner=4)
                 N.set_gemm_precision("fp32")
                 report(f"nf_linear_tc 1xTF32 (reduced precision) {name} [{M}x{Nn}x{K}]", ms, None, 2.0 * M * Nn * K)
-                if K > 128:
-                    N._lib.call("nf_set_option", 9, 2)
-                    try:
-                        ms = timeit(lambda: ops.linear_tc(a, hi, lo, bias, relu=True), reps=3, inner=4)
-                        report(f"nf_linear_tc 3xTF32, 2 accumulators + 4 A stages {name} [{M}x{Nn}x{K}]", ms, None, 2.0 * M * Nn * K)
-                        N.set_gemm_precision("tf32")
-                        ms = timeit(lambda: ops.linear_tc(a, hi, lo, bias, relu=True), reps=3, inner=4)
-                        report(f"nf_linear_tc 1xTF32, 2 accumulators + 4 A stages {name} [{M}x{Nn}x{K}]", ms, None, 2.0 * M * Nn * K)
-                    finally:
-                        N.set_gemm_precision("fp32")
-                        N._lib.call("nf_set_option", 9, 3)
 
 
 def bench_stacks():

@@ -9,12 +9,9 @@ ap = argparse.ArgumentParser()
 ap.add_argument("--reps", type=int, default=10)
 ap.add_argument("--rows", type=int, default=262144)
 ap.add_argument("--precision", default="fp32")
-ap.add_argument("--variant", type=int, default=-1, help="nf_set_option(3, v): in-block kernel of the blocked route (1 = FP32 pipe, 2 = mma.sync)")
 a = ap.parse_args()
 torch.manual_seed(0)
 N.set_gemm_precision(a.precision)
-if a.variant >= 0:
-    assert N._lib.lib().nf_set_option(3, a.variant) == 0
 m = N.MaskedAutoregressiveFlow(64, 512).cuda().eval()
 with torch.no_grad():
     for p in m.parameters():
@@ -31,13 +28,6 @@ with torch.no_grad():
     e1.record(); torch.cuda.synchronize()
     ms = e0.elapsed_time(e1) / a.reps
     zz, ld2 = m.inverse(x)
-    cmp = {}
-    if a.variant >= 0 and a.variant != 1:             # against the FP32-pipe in-block kernel on the same input
-        N._lib.lib().nf_set_option(3, 1)
-        x1, ld1 = m.forward(z)
-        N._lib.lib().nf_set_option(3, a.variant)
-        cmp = {"vs_variant1_x_max_abs": float((x - x1).abs().max()), "vs_variant1_ld_max_abs": float((ld - ld1).abs().max()),
-               "x_absmax": float(x1.abs().max())}
-    print(json.dumps({"what": "MAF(64,512).forward", "rows": a.rows, "precision": a.precision, "variant": a.variant, "ms": ms, **cmp,
+    print(json.dumps({"what": "MAF(64,512).forward", "rows": a.rows, "precision": a.precision, "ms": ms,
                       "launches_per_pass": (N._lib.launch_count() - before) / a.reps,
                       "roundtrip_max_abs": float((zz - z).abs().max()), "ld_sum_abs": float((ld + ld2).abs().max())}))

@@ -4,6 +4,7 @@
 Tolerances (north_star): z within 1e-5*max(1,|z|), row log-det within 1e-4 absolute; written at each assert."""
 import json
 import os
+import re
 
 import pytest
 import torch
@@ -334,11 +335,22 @@ def test_spline_transform_large_batch(D, K, B, compact):
                 lambda: noise()[1].reshape(B, Dt).sum(1), terms=Dt)
 
 
+# the in-block kernel each layout reaches (ar_blocked.cu picks it from the block layout alone): whole 8-unit tiles of at
+# most 16 units per degree -> mma.sync; degrees not padded to multiples of 4 (the padding would cost > 10 % more units)
+# -> warp-private FP32 tiles; blocks of more than ~148 units (~34 per degree at MAF(16, 512)) -> CTA barriers
+_IN_BLOCK_KERNEL = {(64, 512): "ar_block_mma_kernel", (32, 256): "ar_block_mma_kernel", (20, 128): "ar_block_warp_kernel",
+                    (36, 288): "ar_block_mma_kernel", (12, 96): "ar_block_warp_kernel", (16, 512): "ar_block_kernel"}
+# shapes the module's own blocked route takes, with a launch count the route exceeds (in-block kernels, pull and push
+# products, finish; MAF(16, 512) has two blocks: 7 launches) and the one-launch kernel does not
+_MODULE_BLOCKED_LAUNCHES = {(64, 512): 8, (32, 256): 8, (20, 128): 8, (16, 512): 6}
+
+
 @pytest.mark.parametrize("kind,D,H,B", [("maf", 64, 512, 2048), ("iaf", 32, 256, 1500), ("maf", 20, 128, 1024),
-                                       ("maf", 36, 288, 1001), ("iaf", 12, 96, 777)])     # last block of 4 degrees; ragged row tiles
+                                       ("maf", 36, 288, 1001), ("iaf", 12, 96, 777),      # last block of 4 degrees; ragged row tiles
+                                       ("maf", 16, 512, 1024)])
 def test_blocked_sequential_direction_matches_oracle(kind, D, H, B):
     """MAF.forward / IAF.inverse through the blocked tensor-core evaluation (ar_blocked.cu) against the oracle's
-    D-step loop and against the one-launch incremental kernel."""
+    D-step loop and against the one-launch incremental kernel; the profiler confirms which in-block kernel ran."""
     sd = O.init_made_sd(D, H, seed=D + H, sigma=0.03, prefix="conditioner.")
     cls = N.MaskedAutoregressiveFlow if kind == "maf" else N.InverseAutoregressiveFlow
     m = cls(D, H)
@@ -352,29 +364,23 @@ def test_blocked_sequential_direction_matches_oracle(kind, D, H, B):
         ref_y, ref_ld = O.maf_forward(sd, "", v) if kind == "maf" else O.iaf_inverse(sd, "", v)
         folded = m.conditioner.folded()
         mode = N._lib.AR_MAF_FORWARD if kind == "maf" else N._lib.AR_IAF_INVERSE
-        blocked = N.ops.ar_sequential_blocked(v.to(_dev()), folded, mode)
+        with torch.profiler.profile(activities=[torch.profiler.ProfilerActivity.CUDA]) as prof:
+            blocked = N.ops.ar_sequential_blocked(v.to(_dev()), folded, mode)
+            torch.cuda.synchronize()
         assert blocked is not None
+        in_block = {hit.group(1) for e in prof.events()
+                    for hit in [re.search(r"\b(ar_block(?:_mma|_warp)?_kernel)\b", e.name)] if hit}
+        assert in_block == {_IN_BLOCK_KERNEL[(D, H)]}, in_block
         sd64 = {k: (t.double() if t.is_floating_point() else t) for k, t in sd.items()}
         y64, ld64 = (O.maf_forward(sd64, "", v.double())) if kind == "maf" else O.iaf_inverse(sd64, "", v.double())
         _within(blocked[0].cpu(), ref_y, y64, Z_ATOL, Z_RTOL, f"blocked {kind} z")
         _within(blocked[1].cpu(), ref_ld, ld64, LD_ATOL, LD_RTOL, f"blocked {kind} ld")
-        # the in-block kernel's other variants (nf_set_option(3, v): 1 = FP32 pipe, 2 = mma.sync with 32 rows per warp;
-        # the default, 3, is mma.sync with 16 rows per warp) compute the same recurrence
-        try:
-            for variant in (1, 2):
-                assert N._lib.lib().nf_set_option(3, variant) == 0
-                alt = N.ops.ar_sequential_blocked(v.to(_dev()), folded, mode)
-                _within(alt[0].cpu(), ref_y, y64, Z_ATOL, Z_RTOL, f"blocked {kind} z, in-block variant {variant}")
-                _within(alt[1].cpu(), ref_ld, ld64, LD_ATOL, LD_RTOL, f"blocked {kind} ld, in-block variant {variant}")
-                assert torch.equal(torch.isnan(alt[0]), torch.isnan(blocked[0]))
-        finally:
-            assert N._lib.lib().nf_set_option(3, 3) == 0
         # module entry point takes the blocked route at this size
         before = N._lib.launch_count()
         y2, ld2 = m.forward(v.to(_dev())) if kind == "maf" else m.inverse(v.to(_dev()))
         assert torch.equal(torch.isnan(y2), torch.isnan(blocked[0]))
-        if (D, H) in ((64, 512), (32, 256), (20, 128)):
-            assert N._lib.launch_count() - before > 8
+        if (D, H) in _MODULE_BLOCKED_LAUNCHES:
+            assert N._lib.launch_count() - before > _MODULE_BLOCKED_LAUNCHES[(D, H)]
             assert torch.allclose(y2.nan_to_num(), blocked[0].nan_to_num())
         else:                          # the added shapes are too small for the module's blocked route: the one-launch kernel
             _within(y2.cpu(), ref_y, y64, Z_ATOL, Z_RTOL, f"module route {kind} z")

@@ -111,15 +111,20 @@ def test_product_does_not_import_oracle():
 
 def test_library_options_from_the_environment():
     """NFB200_OPTIONS="key:value,..." (the A/B knob of the measurement scripts) is applied through nf_set_option when the
-    library is loaded; a refused value fails the load loudly.  The in-block kernel selector (key 3) takes 0..3."""
+    library is loaded; a refused value fails the load loudly.  Only keys 7, 10 and 11 exist: the keys of the retired
+    kernel variants (1, 2, 3, 5, 6, 9) are refused, so a script that still sets one fails instead of measuring the default."""
     import subprocess, sys
-    code = "import nfb200; l = nfb200._lib.lib(); print(l.nf_set_option(3, 3), l.nf_set_option(3, 4))"
-    env = dict(os.environ, NFB200_OPTIONS="3:1,7:3")
+    code = "import nfb200; l = nfb200._lib.lib(); print(l.nf_set_option(11, 1), l.nf_set_option(7, 2))"
+    env = dict(os.environ, NFB200_OPTIONS="11:0,7:3")
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=env, cwd=ROOT)
-    assert r.returncode == 0 and r.stdout.split() == ["0", str(N._lib.lib().nf_set_option(3, 4))], r.stderr[-400:]
-    assert N._lib.lib().nf_set_option(3, 4) != 0 and N._lib.lib().nf_set_option(3, 3) == 0
-    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=dict(os.environ, NFB200_OPTIONS="3:9"), cwd=ROOT)
-    assert r.returncode != 0 and "refused" in r.stderr
+    out = r.stdout.split()
+    assert r.returncode == 0 and out[0] == "0" and out[1] != "0", r.stderr[-400:]
+    for key in (1, 2, 3, 5, 6, 9):
+        for value in (0, 1, 2, 3, 64):
+            assert N._lib.lib().nf_set_option(key, value) != 0, (key, value)
+    for opts in ("7:2", "3:3"):
+        r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, env=dict(os.environ, NFB200_OPTIONS=opts), cwd=ROOT)
+        assert r.returncode != 0 and "refused" in r.stderr, opts
 
 
 def test_gemm_precision_switch_is_host_only_and_validated():

@@ -251,6 +251,33 @@ NF_API int nf_std_normal_log_prob_forward(const void* z, const void* ld, void* l
 NF_API int nf_std_normal_log_prob_backward(const void* z, const void* glp, void* gz, int64_t B, int D, int dtype,
                                     nf_stream_t stream);
 
+/* ---- sample_and_log_prob with a standard-normal base: z ~ N(0, I), (x, log_det) = forward(z), log_q = log N(z) - log_det
+ * The base stream (csrc/nf_rng.cuh) is Philox4x32-10 keyed by (lo32(seed) ^ 0x6E666232, hi32(seed)), counter
+ * (j, row, lo32(offset/4), hi32(offset/4)) for dims 4j..4j+3 of a row, Box-Muller on the two word pairs; every route draws
+ * the same bits for the same (seed, offset), and a row does not depend on B.  B >= 2^32 is refused (NF_ERR_BAD_SHAPE).
+ * nf_std_normal_draw: z [B,D] <- the draw (NF_F64 widens the float32 normals; float32 with D % 4 == 0 needs a 16-byte
+ * aligned z).  log-q head: lq[b] = sum_d(-z[b,d]^2/2) - D/2*log(2*pi) - ld[b]; backward: gz = -z*glq[b] and
+ * gld = -glq (either output may be NULL, then it is not written). */
+NF_API int nf_std_normal_draw(uint64_t seed, uint64_t offset, void* z, int64_t B, int D, int dtype, nf_stream_t stream);
+NF_API int nf_std_normal_log_q_forward(const void* z, const void* ld, void* lq, int64_t B, int D, int dtype,
+                                       nf_stream_t stream);
+NF_API int nf_std_normal_log_q_backward(const void* z, const void* glq, void* gz, void* gld, int64_t B, int D, int dtype,
+                                        nf_stream_t stream);
+/* The fused stacks with the draw in the kernel: the row load of nf_*_stack*_forward becomes the draw above, the stack runs
+ * in the sampling direction, x (may be NULL) receives the rows and log_q the per-row log N(z) - log_det; one launch, no
+ * input tensor.  Same packed layouts, headers and NF_ERR_UNSUPPORTED envelopes as the forward entry points. */
+NF_API int nf_spline_stack_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, uint64_t seed,
+                                  uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream);
+NF_API int nf_spline_stack_tc_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, uint64_t seed,
+                                     uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream);
+NF_API int nf_coupling_stack_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, uint64_t seed,
+                                    uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream);
+NF_API int nf_coupling_stack_tc_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, uint64_t seed,
+                                       uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream);
+/* mode: NF_AR_IAF_FORWARD (any data_dim <= 8) or NF_AR_MAF_FORWARD (data_dim == 2) */
+NF_API int nf_made_stack_tc_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, int mode, uint64_t seed,
+                                   uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream);
+
 /* ---- fused inference stacks on the tensor cores (tcgen05 + TMEM, 3xTF32 = fp32-accurate): same contract as
  * nf_spline_stack_forward, for hidden_dim <= 64, num_bins <= 10 and at most 2 transformed dims per layer; `packed`
  * follows the tensor-core layout (csrc/stack_tc.cu; magic 'NFS2').  NF_ERR_UNSUPPORTED otherwise. */
@@ -347,7 +374,8 @@ NF_API int64_t nf_ar_blocked_workspace_floats(int64_t B, int D, int H);
  * rows, others zero): bf16, row-major, mask folded, hidden units sorted by degree; b0..b2 [H], b3 [128] (same row layout
  * as w3): fp32.  kext16_host: HOST int32[16] = [layer][128-column block] number of 16-wide k-steps holding non-zero
  * weights (the rest is skipped).  flags: bit 1 (2) = ld receives log N(out; 0, I) + log_det (Flow.log_prob head, flow.py:56-73);
- * bit 2 (4) = out is not stored (may be NULL).  mode: NF_AR_MAF_INVERSE or NF_AR_IAF_FORWARD.
+ * bit 2 (4) = out is not stored (may be NULL); bit 3 (NF_STACK_SAMPLE_LOG_Q = 8, NF_AR_IAF_FORWARD only) = ld receives
+ * log N(x; 0, I) - log_det of the INPUT row, the sample_and_log_prob head when x is the N(0, I) draw.  mode: NF_AR_MAF_INVERSE or NF_AR_IAF_FORWARD.
  * NF_ERR_UNSUPPORTED unless D <= 64, D % 4 == 0, H % 128 == 0, H <= 512. */
 NF_API int nf_made_chain_bf16_forward(const void* x, const void* w0, const void* w1, const void* w2, const void* w3,
                                const void* b0, const void* b1, const void* b2, const void* b3, const int32_t* kext16_host,

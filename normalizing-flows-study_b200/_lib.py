@@ -20,7 +20,7 @@ NF_ERR_UNSUPPORTED = -2
 AR_MAF_INVERSE, AR_IAF_FORWARD, AR_MAF_FORWARD, AR_IAF_INVERSE = 0, 1, 2, 3
 
 _c = ctypes
-_P, _I, _L, _D = _c.c_void_p, _c.c_int, _c.c_int64, _c.c_double
+_P, _I, _L, _D, _U = _c.c_void_p, _c.c_int, _c.c_int64, _c.c_double, _c.c_uint64
 
 # name -> argtypes (restype is int unless listed in _RESTYPES); mirrors include/nfb200.h one to one
 _SIGNATURES = {
@@ -59,6 +59,14 @@ _SIGNATURES = {
     "nf_ar_finish_backward": [_P] * 7 + [_L, _I, _I, _I, _P],
     "nf_std_normal_log_prob_forward": [_P] * 3 + [_L, _I, _I, _P],
     "nf_std_normal_log_prob_backward": [_P] * 3 + [_L, _I, _I, _P],
+    "nf_std_normal_draw": [_U, _U, _P, _L, _I, _I, _P],
+    "nf_std_normal_log_q_forward": [_P] * 3 + [_L, _I, _I, _P],
+    "nf_std_normal_log_q_backward": [_P] * 4 + [_L, _I, _I, _P],
+    "nf_spline_stack_sample": [_P, _P, _L, _U, _U, _P, _P, _L, _P],
+    "nf_spline_stack_tc_sample": [_P, _P, _L, _U, _U, _P, _P, _L, _P],
+    "nf_coupling_stack_sample": [_P, _P, _L, _U, _U, _P, _P, _L, _P],
+    "nf_coupling_stack_tc_sample": [_P, _P, _L, _U, _U, _P, _P, _L, _P],
+    "nf_made_stack_tc_sample": [_P, _P, _L, _I, _U, _U, _P, _P, _L, _P],
     "nf_debug_tc_gemm128": [_P, _P, _P, _I, _I, _P, _I, _P],
     "nf_linear_tc": [_P, _P, _P, _P, _P, _L, _L, _L, _L, _L, _L, _I, _P, _P],
     "nf_linear_tc_range": [_P, _P, _P, _P, _P, _L, _L, _L, _L, _L, _L, _I, _P, _P, _P],
@@ -149,12 +157,15 @@ def dtype_code(t: torch.Tensor) -> int:
     raise TypeError(f"libnfb200 computes in float32/float64, got {t.dtype}")
 
 
+NO_CPU_PATH = "libnfb200 has no CPU path: tensors (and modules) must live on a CUDA device"
+
+
 def ptr(t):
     """Device pointer of a contiguous CUDA tensor (None -> NULL)."""
     if t is None:
         return None
     if not t.is_cuda:
-        raise RuntimeError("libnfb200 has no CPU path: tensors (and modules) must live on a CUDA device")
+        raise RuntimeError(NO_CPU_PATH)
     if not t.is_contiguous():
         raise RuntimeError("internal error: non-contiguous tensor passed to libnfb200")
     return t.data_ptr()

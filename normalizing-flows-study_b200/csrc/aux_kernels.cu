@@ -9,6 +9,7 @@
 //   nf_ar_finish_*        the NaN/Inf scrubs and log-det clamp that close that loop (:69-76 / :93-101)
 // All are streaming, HBM-bound kernels; reductions over rows accumulate in double.
 #include "nf_common.cuh"
+#include "nf_rng.cuh"
 
 namespace nf {
 
@@ -314,7 +315,8 @@ ar_finish_bwd_kernel(const T* __restrict__ cur, const T* __restrict__ ld_sum, co
 // ------------------------------------------------------------------------------------------------
 // Flow.log_prob head for a standard-normal base (flow.py:56-73): lp = sum_d(-z^2/2) - D/2 log(2 pi) + log_det
 // ------------------------------------------------------------------------------------------------
-template <typename T, int G>
+// LOG_Q: the sample_and_log_prob head log N(z; 0, I) - ld instead (ld required)
+template <typename T, int G, bool LOG_Q = false>
 __global__ void __launch_bounds__(256)
 std_normal_log_prob_fwd_kernel(const T* __restrict__ z, const T* __restrict__ ld, T* __restrict__ lp, int64_t B, int D,
                                T norm_const) {
@@ -330,7 +332,7 @@ std_normal_log_prob_fwd_kernel(const T* __restrict__ z, const T* __restrict__ ld
         if (valid)
             for (int d = g; d < D; d += G) { const T v = ld_stream(z + row * D + d); acc += T(-0.5) * v * v; }
         acc = group_sum<T, G>(acc);
-        if (valid && g == 0) lp[row] = acc - norm_const + (ld ? ld[row] : T(0));
+        if (valid && g == 0) lp[row] = LOG_Q ? acc - norm_const - ld[row] : acc - norm_const + (ld ? ld[row] : T(0));
     }
 }
 
@@ -392,6 +394,40 @@ std_normal_log_prob_d2_kernel(const float* __restrict__ z, const float* __restri
         float a = 0.f;
         a += -0.5f * z[2 * r] * z[2 * r]; a += -0.5f * z[2 * r + 1] * z[2 * r + 1];
         lp[r] = a - norm_const + (ld ? ld[r] : 0.f);
+    }
+}
+
+// backward of log N(z; 0, I) - ld: gz = -z * g (skipped when gz is NULL: a drawn z is a constant), gld = -g
+template <typename T>
+__global__ void __launch_bounds__(256)
+std_normal_log_q_bwd_kernel(const T* __restrict__ z, const T* __restrict__ g, T* __restrict__ gz, T* __restrict__ gld,
+                            int64_t B, int D) {
+    const int64_t n = gz ? B * D : B, stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        if (gz) gz[i] = -z[i] * g[i / D];
+        if (gld && i < B) gld[i] = -g[i];
+    }
+}
+
+// the N(0, I) base draw of nf_rng.cuh: one thread per group of four dims of a row; float64 widens the fp32 normals
+template <typename T>
+__global__ void __launch_bounds__(256)
+std_normal_draw_kernel(uint64_t seed, uint64_t offset, T* __restrict__ z, int64_t B, int D) {
+    const int J = (D + 3) >> 2;
+    const int64_t n = B * J, stride = (int64_t)gridDim.x * blockDim.x;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
+        const int64_t r = i / J;
+        const int j = (int)(i - r * J);
+        float q[4];
+        nf_std_normal4(seed, offset, (uint32_t)r, (uint32_t)j, q);
+        T* p = z + r * D + 4 * j;
+        if (sizeof(T) == 4 && (D & 3) == 0) {
+            __stcs(reinterpret_cast<float4*>(p), make_float4(q[0], q[1], q[2], q[3]));
+        } else {
+            const int m = D - 4 * j < 4 ? D - 4 * j : 4;
+#pragma unroll
+            for (int k = 0; k < 4; ++k) if (k < m) st_stream(p + k, (T)q[k]);
+        }
     }
 }
 
@@ -643,6 +679,58 @@ extern "C" int nf_std_normal_log_prob_backward(const void* z, const void* glp, v
     NF_DISPATCH(
         (std_normal_log_prob_bwd_kernel<float><<<grid, 256, 0, st>>>((const float*)z, (const float*)glp, (float*)gz, B, D)),
         (std_normal_log_prob_bwd_kernel<double><<<grid, 256, 0, st>>>((const double*)z, (const double*)glp, (double*)gz, B, D)));
+    count_launch();
+    NF_LAUNCH_CHECK();
+    return NF_OK;
+}
+
+extern "C" int nf_std_normal_draw(uint64_t seed, uint64_t offset, void* z, int64_t B, int D, int dtype, nf_stream_t stream) {
+    if (B < 0 || B > (int64_t)0xFFFFFFFFLL || D < 1) return NF_ERR_BAD_SHAPE;
+    if (B == 0) return NF_OK;
+    NF_REQ(z);
+    if (dtype == NF_F32 && (D & 3) == 0 && !aligned16(z)) return NF_ERR_MISALIGNED;
+    cudaStream_t st = (cudaStream_t)stream;
+    const int grid = ew_grid(B * ((D + 3) / 4));
+    NF_DISPATCH(
+        (std_normal_draw_kernel<float><<<grid, 256, 0, st>>>(seed, offset, (float*)z, B, D)),
+        (std_normal_draw_kernel<double><<<grid, 256, 0, st>>>(seed, offset, (double*)z, B, D)));
+    count_launch();
+    NF_LAUNCH_CHECK();
+    return NF_OK;
+}
+
+extern "C" int nf_std_normal_log_q_forward(const void* z, const void* ld, void* lq, int64_t B, int D, int dtype,
+                                           nf_stream_t stream) {
+    if (B < 0 || D < 1) return NF_ERR_BAD_SHAPE;
+    if (B == 0) return NF_OK;
+    NF_REQ(z); NF_REQ(ld); NF_REQ(lq);
+    cudaStream_t st = (cudaStream_t)stream;
+    const double nc = 0.5 * (double)D * 1.8378770664093453;   // D/2 * log(2 pi)
+    int G = 1; while (G < D && G < 32) G <<= 1;
+    int64_t need = cdiv(cdiv(B, 32 / G), 8), cap = (int64_t)kNumSMs * 32;
+    const int grid = (int)(need < 1 ? 1 : (need < cap ? need : cap));
+#define NF_LQ(T, GG) std_normal_log_prob_fwd_kernel<T, GG, true><<<grid, 256, 0, st>>>((const T*)z, (const T*)ld, (T*)lq, B, D, (T)nc)
+#define NF_LQ_G(T) switch (G) { case 1: NF_LQ(T, 1); break; case 2: NF_LQ(T, 2); break; case 4: NF_LQ(T, 4); break; \
+                                case 8: NF_LQ(T, 8); break; case 16: NF_LQ(T, 16); break; default: NF_LQ(T, 32); break; }
+    NF_DISPATCH(NF_LQ_G(float), NF_LQ_G(double));
+#undef NF_LQ_G
+#undef NF_LQ
+    count_launch();
+    NF_LAUNCH_CHECK();
+    return NF_OK;
+}
+
+extern "C" int nf_std_normal_log_q_backward(const void* z, const void* glq, void* gz, void* gld, int64_t B, int D, int dtype,
+                                            nf_stream_t stream) {
+    if (B < 0 || D < 1) return NF_ERR_BAD_SHAPE;
+    if (B == 0 || (!gz && !gld)) return NF_OK;
+    NF_REQ(glq);
+    if (gz) NF_REQ(z);
+    cudaStream_t st = (cudaStream_t)stream;
+    const int grid = ew_grid(gz ? B * D : B);
+    NF_DISPATCH(
+        (std_normal_log_q_bwd_kernel<float><<<grid, 256, 0, st>>>((const float*)z, (const float*)glq, (float*)gz, (float*)gld, B, D)),
+        (std_normal_log_q_bwd_kernel<double><<<grid, 256, 0, st>>>((const double*)z, (const double*)glq, (double*)gz, (double*)gld, B, D)));
     count_launch();
     NF_LAUNCH_CHECK();
     return NF_OK;

@@ -63,7 +63,7 @@ struct McParams {
     int KA;                 // K atoms of the hidden layers (H / 64)
     int D;                  // data_dim (<= 64, multiple of 4)
     int mode;               // NF_AR_MAF_INVERSE / NF_AR_IAF_FORWARD
-    int flags;              // NF_STACK_LOG_PROB_HEAD | NF_STACK_SKIP_Y semantics (bits 1, 2)
+    int flags;              // NF_STACK_LOG_PROB_HEAD | NF_STACK_SKIP_Y | NF_STACK_SAMPLE_LOG_Q semantics (bits 1, 2, 3)
     int64_t B;
     int num_tiles;
 };
@@ -348,7 +348,8 @@ made_chain_bf16_kernel(const __grid_constant__ CUtensorMap tm_w0, const __grid_c
                         affine_ar_elem<float>(P.mode, xc[i], mu, al, ov, tt);
                         if (!is_finite(ov)) ov = iaf ? xc[i] : 0.f;          // IAF scrubs to the input (:53)
                         lsum += tt;
-                        sq += -0.5f * ov * ov;
+                        const float hv = (P.flags & NF_STACK_SAMPLE_LOG_Q) ? xc[i] : ov;     // head on the input row
+                        sq += -0.5f * hv * hv;
                     }
                     o16[i] = ov;
                 }
@@ -366,9 +367,11 @@ made_chain_bf16_kernel(const __grid_constant__ CUtensorMap tm_w0, const __grid_c
                 if (cq == 0 && row < P.B) {
                     const float tot = clamp_mm(scrub0(((lsum + part[r]) + part[256 + r]) + part[512 + r]), -lim, lim);
                     float res = tot;
-                    if (P.flags & NF_STACK_LOG_PROB_HEAD)
-                        res = (((sq + part[128 + r]) + part[256 + 128 + r]) + part[512 + 128 + r]) -
-                              (float)(0.5 * (double)D * 1.8378770664093453) + tot;
+                    if (P.flags & (NF_STACK_LOG_PROB_HEAD | NF_STACK_SAMPLE_LOG_Q)) {
+                        const float lz = (((sq + part[128 + r]) + part[256 + 128 + r]) + part[512 + 128 + r]) -
+                                         (float)(0.5 * (double)D * 1.8378770664093453);
+                        res = (P.flags & NF_STACK_SAMPLE_LOG_Q) ? lz - tot : lz + tot;
+                    }
                     __stcs(ld_out + row, res);
                 }
             }
@@ -413,6 +416,7 @@ extern "C" int nf_made_chain_bf16_forward(const void* x, const void* w0, const v
                                           int flags, nf_stream_t stream) {
     if (B < 0 || D < 1 || H < 1) return NF_ERR_BAD_SHAPE;
     if (mode != NF_AR_MAF_INVERSE && mode != NF_AR_IAF_FORWARD) return NF_ERR_UNSUPPORTED;
+    if ((flags & NF_STACK_SAMPLE_LOG_Q) && (mode != NF_AR_IAF_FORWARD || (flags & NF_STACK_LOG_PROB_HEAD))) return NF_ERR_UNSUPPORTED;
     if (D > 64 || (D % 4) != 0 || (H % 128) != 0 || H > kMcMaxKA * kMcAtom) return NF_ERR_UNSUPPORTED;
     NF_REQ(kext16_host);
     if (B == 0) return NF_OK;

@@ -15,6 +15,7 @@
 //     registers.  No activation ever touches HBM.
 #include "nf_common.cuh"
 #include "stack_small.cuh"
+#include "nf_rng.cuh"
 
 namespace nf {
 
@@ -142,10 +143,12 @@ __device__ __forceinline__ void bn_between(const float* __restrict__ sL, int D, 
 // ------------------------------------------------------------------------------------------------
 // spline stack
 // ------------------------------------------------------------------------------------------------
-template <int HP, int R, int DM, int KMAX>
+// SAMPLE (both kernels, nf_*_stack_sample): the row is the N(0, I) draw of nf_rng.cuh instead of a load, tot starts at
+// -log N(z) and the epilogue stores -tot = log N(z) - log_det (sample_and_log_prob)
+template <int HP, int R, int DM, int KMAX, bool SAMPLE = false>
 __global__ void __launch_bounds__(kStackThreads)
 spline_stack_kernel(const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
-                    float* __restrict__ ld, int64_t B, int flags, int layer_words_pad) {
+                    float* __restrict__ ld, int64_t B, int flags, int layer_words_pad, uint64_t seed, uint64_t offset) {
     const int inverse = flags & NF_STACK_INVERSE;
     extern __shared__ __align__(16) float smem[];
     const StackHdr hd = read_hdr(packed);
@@ -171,6 +174,10 @@ spline_stack_kernel(const float* __restrict__ packed, const float* __restrict__ 
 #pragma unroll
         for (int i = 0; i < R; ++i) {
             row[i] = tile * ROWS + i * kStackThreads + tid;
+            if constexpr (SAMPLE) {
+                tot[i] = -nf_std_normal_row<DM>(seed, offset, (uint32_t)row[i], D, xv[i]);
+                continue;
+            }
             tot[i] = 0.f;
 #pragma unroll
             for (int d = 0; d < DM; ++d) xv[i][d] = (d < D && row[i] < B) ? ld_stream(x + row[i] * D + d) : 0.f;
@@ -252,7 +259,7 @@ spline_stack_kernel(const float* __restrict__ packed, const float* __restrict__ 
 #pragma unroll
                     for (int d = 0; d < DM; ++d) if (d < D) st_stream(y + row[i] * D + d, xv[i][d]);
                 }
-                st_stream(ld + row[i], (flags & NF_STACK_LOG_PROB_HEAD) ? nf_stack_row_head<DM>(xv[i], D, tot[i]) : tot[i]);
+                st_stream(ld + row[i], SAMPLE ? -tot[i] : (flags & NF_STACK_LOG_PROB_HEAD) ? nf_stack_row_head<DM>(xv[i], D, tot[i]) : tot[i]);
             }
         }
     }
@@ -261,10 +268,10 @@ spline_stack_kernel(const float* __restrict__ packed, const float* __restrict__ 
 // ------------------------------------------------------------------------------------------------
 // affine coupling stack (eval mode)
 // ------------------------------------------------------------------------------------------------
-template <int HP, int R, int DM>
+template <int HP, int R, int DM, bool SAMPLE = false>
 __global__ void __launch_bounds__(kStackThreads)
 coupling_stack_kernel(const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
-                      float* __restrict__ ld, int64_t B, int flags) {
+                      float* __restrict__ ld, int64_t B, int flags, uint64_t seed, uint64_t offset) {
     const int inverse = flags & NF_STACK_INVERSE;
     extern __shared__ __align__(16) float smem[];
     const StackHdr hd = read_hdr(packed);
@@ -282,6 +289,10 @@ coupling_stack_kernel(const float* __restrict__ packed, const float* __restrict_
 #pragma unroll
         for (int i = 0; i < R; ++i) {
             row[i] = tile * ROWS + i * kStackThreads + tid;
+            if constexpr (SAMPLE) {
+                tot[i] = -nf_std_normal_row<DM>(seed, offset, (uint32_t)row[i], D, xv[i]);
+                continue;
+            }
             tot[i] = 0.f;
 #pragma unroll
             for (int d = 0; d < DM; ++d) xv[i][d] = (d < D && row[i] < B) ? ld_stream(x + row[i] * D + d) : 0.f;
@@ -344,7 +355,7 @@ coupling_stack_kernel(const float* __restrict__ packed, const float* __restrict_
 #pragma unroll
                     for (int d = 0; d < DM; ++d) if (d < D) st_stream(y + row[i] * D + d, xv[i][d]);
                 }
-                st_stream(ld + row[i], (flags & NF_STACK_LOG_PROB_HEAD) ? nf_stack_row_head<DM>(xv[i], D, tot[i]) : tot[i]);
+                st_stream(ld + row[i], SAMPLE ? -tot[i] : (flags & NF_STACK_LOG_PROB_HEAD) ? nf_stack_row_head<DM>(xv[i], D, tot[i]) : tot[i]);
             }
         }
     }
@@ -355,7 +366,8 @@ coupling_stack_kernel(const float* __restrict__ packed, const float* __restrict_
 // ------------------------------------------------------------------------------------------------
 template <typename Kern>
 static int launch_stack(Kern kern, size_t smem_bytes, int rows_per_cta, const void* packed, const void* x, void* y,
-                        void* ld, int64_t B, int inverse, int extra, bool has_extra, cudaStream_t st) {
+                        void* ld, int64_t B, int inverse, int extra, bool has_extra, uint64_t seed, uint64_t offset,
+                        cudaStream_t st) {
     if (smem_bytes > 227 * 1024) return NF_ERR_UNSUPPORTED;
     NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
     NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
@@ -365,9 +377,11 @@ static int launch_stack(Kern kern, size_t smem_bytes, int rows_per_cta, const vo
     const int64_t ntiles = cdiv(B, rows_per_cta);
     const int64_t cap = (int64_t)kNumSMs * per_sm;
     const int grid = (int)(ntiles < cap ? ntiles : cap);
-    (void)extra; (void)has_extra;
-    void* args_s[] = {(void*)&packed, (void*)&x, (void*)&y, (void*)&ld, (void*)&B, (void*)&inverse, (void*)&extra};
-    NF_CUDA(cudaLaunchKernel((const void*)kern, dim3(grid), dim3(kStackThreads), args_s, smem_bytes, st));
+    void* args_s[] = {(void*)&packed, (void*)&x, (void*)&y, (void*)&ld, (void*)&B, (void*)&inverse, (void*)&extra,
+                      (void*)&seed, (void*)&offset};
+    void* args_n[] = {(void*)&packed, (void*)&x, (void*)&y, (void*)&ld, (void*)&B, (void*)&inverse, (void*)&seed,
+                      (void*)&offset};
+    NF_CUDA(cudaLaunchKernel((const void*)kern, dim3(grid), dim3(kStackThreads), has_extra ? args_s : args_n, smem_bytes, st));
     count_launch();
     return NF_OK;
 }
@@ -400,12 +414,15 @@ static int check_hdr(const int32_t* h, int magic) {
     return NF_OK;
 }
 
-extern "C" int nf_spline_stack_forward(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
-                                       void* y, void* ld, int64_t B, int inverse, nf_stream_t stream) {
-    if (B < 0) return NF_ERR_BAD_SHAPE;
+// sample: the SAMPLE kernel draws the rows from (seed, offset); x is not read
+static int spline_stack_launch(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x, void* y,
+                               void* ld, int64_t B, int inverse, bool sample, uint64_t seed, uint64_t offset,
+                               nf_stream_t stream) {
+    if (B < 0 || (sample && B > (int64_t)0xFFFFFFFFLL)) return NF_ERR_BAD_SHAPE;
     NF_REQ(hdr_host);
     if (B == 0) return NF_OK;
-    NF_REQ(packed); NF_REQ(x); NF_REQ(ld);
+    NF_REQ(packed); NF_REQ(ld);
+    if (!sample) NF_REQ(x);
     if (!(inverse & NF_STACK_SKIP_Y)) NF_REQ(y);
     if (!aligned16(packed)) return NF_ERR_MISALIGNED;
     const int32_t* h = (const int32_t*)hdr_host;
@@ -418,8 +435,9 @@ extern "C" int nf_spline_stack_forward(const void* packed, const void* hdr_host,
     const int R = (HP == 64) ? 2 : 1;
     const int rows = kStackThreads * R;
     const size_t smem = sizeof(float) * ((size_t)stride + (size_t)NO * rows);
-#define NF_SS(HPv, Rv, DMv, KMv) \
-    return launch_stack(spline_stack_kernel<HPv, Rv, DMv, KMv>, smem, rows, packed, x, y, ld, B, inverse, stride, true, st)
+#define NF_SS(HPv, Rv, DMv, KMv)                                                                                     \
+    return launch_stack(sample ? spline_stack_kernel<HPv, Rv, DMv, KMv, true> : spline_stack_kernel<HPv, Rv, DMv, KMv>,   \
+                        smem, rows, packed, x, y, ld, B, inverse, stride, true, seed, offset, st)
     if (HP == 64) {
         if (D <= 3) { if (K <= 8) NF_SS(64, 2, 4, 8); else NF_SS(64, 2, 4, 16); }
         else        { if (K <= 8) NF_SS(64, 2, 8, 8); else NF_SS(64, 2, 8, 16); }
@@ -430,13 +448,25 @@ extern "C" int nf_spline_stack_forward(const void* packed, const void* hdr_host,
 #undef NF_SS
 }
 
-extern "C" int nf_coupling_stack_forward(const void* packed, const void* hdr_host, int64_t packed_bytes,
-                                         const void* x, void* y, void* ld, int64_t B, int inverse,
-                                         nf_stream_t stream) {
-    if (B < 0) return NF_ERR_BAD_SHAPE;
+extern "C" int nf_spline_stack_forward(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
+                                       void* y, void* ld, int64_t B, int inverse, nf_stream_t stream) {
+    return spline_stack_launch(packed, hdr_host, packed_bytes, x, y, ld, B, inverse, false, 0, 0, stream);
+}
+
+extern "C" int nf_spline_stack_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, uint64_t seed,
+                                      uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream) {
+    return spline_stack_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true, seed,
+                               offset, stream);
+}
+
+static int coupling_stack_launch(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x, void* y,
+                                 void* ld, int64_t B, int inverse, bool sample, uint64_t seed, uint64_t offset,
+                                 nf_stream_t stream) {
+    if (B < 0 || (sample && B > (int64_t)0xFFFFFFFFLL)) return NF_ERR_BAD_SHAPE;
     NF_REQ(hdr_host);
     if (B == 0) return NF_OK;
-    NF_REQ(packed); NF_REQ(x); NF_REQ(ld);
+    NF_REQ(packed); NF_REQ(ld);
+    if (!sample) NF_REQ(x);
     if (!(inverse & NF_STACK_SKIP_Y)) NF_REQ(y);
     if (!aligned16(packed)) return NF_ERR_MISALIGNED;
     const int32_t* h = (const int32_t*)hdr_host;
@@ -449,9 +479,22 @@ extern "C" int nf_coupling_stack_forward(const void* packed, const void* hdr_hos
     const int R = (HP == 64) ? 2 : 1;
     const int rows = kStackThreads * R;
     const size_t smem = sizeof(float) * (size_t)stride;
-#define NF_CS(HPv, Rv, DMv) \
-    return launch_stack(coupling_stack_kernel<HPv, Rv, DMv>, smem, rows, packed, x, y, ld, B, inverse, 0, false, st)
+#define NF_CS(HPv, Rv, DMv)                                                                                          \
+    return launch_stack(sample ? coupling_stack_kernel<HPv, Rv, DMv, true> : coupling_stack_kernel<HPv, Rv, DMv>, smem, \
+                        rows, packed, x, y, ld, B, inverse, 0, false, seed, offset, st)
     if (HP == 64) { if (D <= 3) NF_CS(64, 2, 4); else NF_CS(64, 2, 8); }
     else          { if (D <= 3) NF_CS(128, 1, 4); else NF_CS(128, 1, 8); }
 #undef NF_CS
+}
+
+extern "C" int nf_coupling_stack_forward(const void* packed, const void* hdr_host, int64_t packed_bytes,
+                                         const void* x, void* y, void* ld, int64_t B, int inverse,
+                                         nf_stream_t stream) {
+    return coupling_stack_launch(packed, hdr_host, packed_bytes, x, y, ld, B, inverse, false, 0, 0, stream);
+}
+
+extern "C" int nf_coupling_stack_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, uint64_t seed,
+                                        uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream) {
+    return coupling_stack_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true, seed,
+                                 offset, stream);
 }

@@ -35,9 +35,12 @@
 //   bit 1  log-prob head: the per-row output is log N(z; 0, I) + log_det (Flow.log_prob, flow.py:56-73) instead of
 //          log_det -- the standard-normal head evaluated on the row while it is still in registers
 //   bit 2  do not store the transformed rows (y may be NULL): Flow.log_prob only returns the per-row value
+//   bit 3  (nf_made_chain_bf16_forward, IAF.forward only) the per-row output is log N(x_in; 0, I) - log_det of the INPUT
+//          row: the sample_and_log_prob head when the input is the N(0, I) draw
 #define NF_STACK_INVERSE 1
 #define NF_STACK_LOG_PROB_HEAD 2
 #define NF_STACK_SKIP_Y 4
+#define NF_STACK_SAMPLE_LOG_Q 8
 
 static inline int nf_stack_hp(int H) { return H <= 64 ? 64 : 128; }
 static inline int nf_stack_w1s(int D) { return D <= 3 ? 4 : 12; }

@@ -18,6 +18,7 @@
 // one CTA's tensor phase with the other's FP32 phase.  TMEM: A_hi | A_lo | D2 | D3 = 64+64+64+<=64 columns.
 #include <stdio.h>
 #include "nf_common.cuh"
+#include "nf_rng.cuh"
 #include "stack_small.cuh"
 #include "tc_common.cuh"
 
@@ -47,6 +48,17 @@ __device__ __forceinline__ float relu_keepnan(float x) {      // torch.relu: NaN
     float r;
     asm("max.NaN.f32 %0, %1, 0f00000000;" : "=f"(r) : "f"(x));
     return r;
+}
+
+// SAMPLE variants of the stack kernels (nf_*_sample): the row is the N(0, I) draw of nf_rng.cuh instead of a load, and
+// its log-det slot starts at -log N(z) -- the epilogue stores the negated sum, log N(z) - log_det (sample_and_log_prob)
+template <int DM>
+__device__ __forceinline__ void draw_row_tc(float* srow, int64_t r, int64_t B, int D, uint64_t seed, uint64_t offset) {
+    float z[DM];
+    const float lz = nf_std_normal_row<DM>(seed, offset, (uint32_t)r, D, z);
+#pragma unroll
+    for (int d = 0; d < DM; ++d) srow[d * kTcThreads] = (r < B) ? z[d] : 0.f;
+    srow[DM * kTcThreads] = -lz;
 }
 
 // between-layer BatchNorm as an invertible affine on running stats (normalizing_flow_model.py:67-128)
@@ -206,10 +218,10 @@ __device__ __forceinline__ void hidden2_chunk(const uint32_t (&v)[16], const flo
 }
 
 // KS > 0: num_bins known at compile time (== KMAX), every per-bin guard folds away; KS == 0: runtime num_bins <= KMAX
-template <int DM, int KMAX, int KS>
+template <int DM, int KMAX, int KS, bool SAMPLE = false>
 __global__ void __launch_bounds__(kTc2Threads, 2)
 spline_stack_tc2_kernel(const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
-                        float* __restrict__ ld, int64_t B, int flags) {
+                        float* __restrict__ ld, int64_t B, int flags, uint64_t seed, uint64_t offset) {
     const int inverse = flags & NF_STACK_INVERSE;
     extern __shared__ __align__(1024) float sbuf[];
     const TcHdr hd = read_tc_hdr(packed);
@@ -251,6 +263,10 @@ spline_stack_tc2_kernel(const float* __restrict__ packed, const float* __restric
     for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         for (int s = wg; s < kTcSub; s += 2) {
             const int64_t r = tile * ROWS + s * kTcThreads + wtid;
+            if constexpr (SAMPLE) {
+                draw_row_tc<DM>(sx + s * (DM + 1) * kTcThreads + wtid, r, B, D, seed, offset);
+                continue;
+            }
 #pragma unroll
             for (int d = 0; d < DM; ++d) sx[(s * (DM + 1) + d) * kTcThreads + wtid] = (d < D && r < B) ? ld_stream(x + r * D + d) : 0.f;
             sx[(s * (DM + 1) + DM) * kTcThreads + wtid] = 0.f;
@@ -414,7 +430,7 @@ spline_stack_tc2_kernel(const float* __restrict__ packed, const float* __restric
                     for (int d = 0; d < DM; ++d) if (d < D) st_stream(y + r * D + d, zr[d]);
                 }
                 const float tot = sx[(s * (DM + 1) + DM) * kTcThreads + wtid];
-                st_stream(ld + r, (flags & NF_STACK_LOG_PROB_HEAD) ? nf_stack_row_head<DM>(zr, D, tot) : tot);
+                st_stream(ld + r, SAMPLE ? -tot : (flags & NF_STACK_LOG_PROB_HEAD) ? nf_stack_row_head<DM>(zr, D, tot) : tot);
             }
         }
     }
@@ -433,10 +449,10 @@ spline_stack_tc2_kernel(const float* __restrict__ packed, const float* __restric
 //   D2 128, D3 16 = all 512 columns of the SM, so ONE CTA per SM; a net block is ~151 KB (W2 hi / lo images alone 128 KB)
 //   and is single buffered -- the next block is requested when every thread is done with the current one (~1 us of a
 //   ~16 us net pass per tile).  Same code otherwise: K = 128 is 16 k-steps per pass, the head reads 4 K atoms.
-template <int DM, int HP>
+template <int DM, int HP, bool SAMPLE = false>
 __global__ void __launch_bounds__(kTcThreads, HP == 64 ? 2 : 1)
 coupling_stack_tc_kernel(const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
-                         float* __restrict__ ld, int64_t B, int flags, int nsub) {     // nsub <= kTcSub sub-tiles per weight staging
+                         float* __restrict__ ld, int64_t B, int flags, int nsub, uint64_t seed, uint64_t offset) {     // nsub <= kTcSub sub-tiles per weight staging
     constexpr int NBUF = (HP == 64) ? 2 : 1;
     constexpr int kColAhi = 0, kColAlo = HP, kColD2 = 2 * HP, kColD3 = 3 * HP;
     constexpr int kTmemCols = (HP == 64) ? 256 : 512;
@@ -477,6 +493,10 @@ coupling_stack_tc_kernel(const float* __restrict__ packed, const float* __restri
     for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         for (int s = 0; s < nsub; ++s) {
             const int64_t r = tile * ROWS + s * kTcThreads + tid;
+            if constexpr (SAMPLE) {
+                draw_row_tc<DM>(sx + s * (DM + 1) * kTcThreads + tid, r, B, D, seed, offset);
+                continue;
+            }
 #pragma unroll
             for (int d = 0; d < DM; ++d) sx[(s * (DM + 1) + d) * kTcThreads + tid] = (d < D && r < B) ? ld_stream(x + r * D + d) : 0.f;
             sx[(s * (DM + 1) + DM) * kTcThreads + tid] = 0.f;
@@ -585,7 +605,7 @@ coupling_stack_tc_kernel(const float* __restrict__ packed, const float* __restri
                     for (int d = 0; d < DM; ++d) if (d < D) st_stream(y + r * D + d, zr[d]);
                 }
                 const float tot = sx[(s * (DM + 1) + DM) * kTcThreads + tid];
-                st_stream(ld + r, (flags & NF_STACK_LOG_PROB_HEAD) ? nf_stack_row_head<DM>(zr, D, tot) : tot);
+                st_stream(ld + r, SAMPLE ? -tot : (flags & NF_STACK_LOG_PROB_HEAD) ? nf_stack_row_head<DM>(zr, D, tot) : tot);
             }
         }
     }
@@ -618,10 +638,10 @@ __host__ __device__ inline MadeBlkOff made_blk_offsets(int W1S) {
     return o;
 }
 
-template <int DM>
+template <int DM, bool SAMPLE = false>
 __global__ void __launch_bounds__(kTcThreads, 2)
 made_stack_tc_kernel(const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
-                     float* __restrict__ ld, int64_t B, int flags, int nsub, int mode) {
+                     float* __restrict__ ld, int64_t B, int flags, int nsub, int mode, uint64_t seed, uint64_t offset) {
     const int inverse = flags & NF_STACK_INVERSE;
     extern __shared__ __align__(1024) float sbuf[];
     const TcHdr hd = read_tc_hdr(packed);
@@ -652,6 +672,10 @@ made_stack_tc_kernel(const float* __restrict__ packed, const float* __restrict__
     for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         for (int s = 0; s < nsub; ++s) {
             const int64_t r = tile * ROWS + s * kTcThreads + tid;
+            if constexpr (SAMPLE) {
+                draw_row_tc<DM>(sx + s * (DM + 1) * kTcThreads + tid, r, B, D, seed, offset);
+                continue;
+            }
 #pragma unroll
             for (int d = 0; d < DM; ++d) sx[(s * (DM + 1) + d) * kTcThreads + tid] = (d < D && r < B) ? ld_stream(x + r * D + d) : 0.f;
             sx[(s * (DM + 1) + DM) * kTcThreads + tid] = 0.f;
@@ -756,7 +780,7 @@ made_stack_tc_kernel(const float* __restrict__ packed, const float* __restrict__
                     for (int d = 0; d < DM; ++d) if (d < D) st_stream(y + r * D + d, zr[d]);
                 }
                 const float tot = sx[(s * (DM + 1) + DM) * kTcThreads + tid];
-                st_stream(ld + r, (flags & NF_STACK_LOG_PROB_HEAD) ? nf_stack_row_head<DM>(zr, D, tot) : tot);
+                st_stream(ld + r, SAMPLE ? -tot : (flags & NF_STACK_LOG_PROB_HEAD) ? nf_stack_row_head<DM>(zr, D, tot) : tot);
             }
         }
     }
@@ -776,12 +800,15 @@ extern "C" int64_t nf_spline_stack_tc_block_words(int D, int K, int max_dt) {
     return NF_LAYER_HDR + blk_offsets(W1S, NO3).net_words;
 }
 
-extern "C" int nf_spline_stack_tc_forward(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
-                                          void* y, void* ld, int64_t B, int inverse, nf_stream_t stream) {
-    if (B < 0) return NF_ERR_BAD_SHAPE;
+// sample: the SAMPLE kernel draws the rows from (seed, offset); x is not read
+static int spline_stack_tc_launch(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x, void* y,
+                                  void* ld, int64_t B, int inverse, bool sample, uint64_t seed, uint64_t offset,
+                                  nf_stream_t stream) {
+    if (B < 0 || (sample && B > (int64_t)0xFFFFFFFFLL)) return NF_ERR_BAD_SHAPE;
     NF_REQ(hdr_host);
     if (B == 0) return NF_OK;
-    NF_REQ(packed); NF_REQ(x); NF_REQ(ld);
+    NF_REQ(packed); NF_REQ(ld);
+    if (!sample) NF_REQ(x);
     if (!(inverse & NF_STACK_SKIP_Y)) NF_REQ(y);
     if (!aligned16(packed)) return NF_ERR_MISALIGNED;
     const int32_t* h = (const int32_t*)hdr_host;
@@ -804,12 +831,13 @@ extern "C" int nf_spline_stack_tc_forward(const void* packed, const void* hdr_ho
     const int grid = (int)(ntiles < cap ? ntiles : cap);
 #define NF_TC(DMv, KMv, KSv)                                                                                         \
     do {                                                                                                             \
-        auto kern = spline_stack_tc2_kernel<DMv, KMv, KSv>;                                                          \
+        auto kern = sample ? spline_stack_tc2_kernel<DMv, KMv, KSv, true> : spline_stack_tc2_kernel<DMv, KMv, KSv>; \
         NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                 \
         /* ask for the largest shared-memory carveout: with the default preference the driver sizes the SM for ONE   \
            CTA of this kernel and the second co-resident CTA (the latency hiding of this design) never arrives */    \
         NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)); \
-        kern<<<grid, kTc2Threads, smem, st>>>((const float*)packed, (const float*)x, (float*)y, (float*)ld, B, inverse); \
+        kern<<<grid, kTc2Threads, smem, st>>>((const float*)packed, (const float*)x, (float*)y, (float*)ld, B, inverse, \
+                                              seed, offset);                                                         \
     } while (0)
 #define NF_TC_K(DMv)                                      \
     do {                                                  \
@@ -828,6 +856,17 @@ extern "C" int nf_spline_stack_tc_forward(const void* packed, const void* hdr_ho
     return NF_OK;
 }
 
+extern "C" int nf_spline_stack_tc_forward(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
+                                          void* y, void* ld, int64_t B, int inverse, nf_stream_t stream) {
+    return spline_stack_tc_launch(packed, hdr_host, packed_bytes, x, y, ld, B, inverse, false, 0, 0, stream);
+}
+
+extern "C" int nf_spline_stack_tc_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, uint64_t seed,
+                                         uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream) {
+    return spline_stack_tc_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true,
+                                  seed, offset, stream);
+}
+
 extern "C" int64_t nf_coupling_stack_tc_block_words(int D) {
     if (D < 1 || D > NF_STACK_DMAX) return -1;
     return NF_LAYER_HDR + blk_offsets(nf_stack_w1s(D), 16).net_words;      // words per NET block (2 per layer)
@@ -837,12 +876,14 @@ extern "C" int64_t nf_coupling_stack_tc_block_words_hidden(int D, int H) {  // h
     return NF_LAYER_HDR + blk_offsets(nf_stack_w1s(D), 16, H <= 64 ? 64 : 128).net_words;
 }
 
-extern "C" int nf_coupling_stack_tc_forward(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
-                                            void* y, void* ld, int64_t B, int inverse, nf_stream_t stream) {
-    if (B < 0) return NF_ERR_BAD_SHAPE;
+static int coupling_stack_tc_launch(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
+                                    void* y, void* ld, int64_t B, int inverse, bool sample, uint64_t seed, uint64_t offset,
+                                    nf_stream_t stream) {
+    if (B < 0 || (sample && B > (int64_t)0xFFFFFFFFLL)) return NF_ERR_BAD_SHAPE;
     NF_REQ(hdr_host);
     if (B == 0) return NF_OK;
-    NF_REQ(packed); NF_REQ(x); NF_REQ(ld);
+    NF_REQ(packed); NF_REQ(ld);
+    if (!sample) NF_REQ(x);
     if (!(inverse & NF_STACK_SKIP_Y)) NF_REQ(y);
     if (!aligned16(packed)) return NF_ERR_MISALIGNED;
     const int32_t* h = (const int32_t*)hdr_host;
@@ -865,7 +906,7 @@ extern "C" int nf_coupling_stack_tc_forward(const void* packed, const void* hdr_
     const int64_t ntiles = cdiv(B, kTcThreads * nsub);
 #define NF_CTC(DMv, HPv)                                                                                                  \
     do {                                                                                                             \
-        auto kern = coupling_stack_tc_kernel<DMv, HPv>;                                                                   \
+        auto kern = sample ? coupling_stack_tc_kernel<DMv, HPv, true> : coupling_stack_tc_kernel<DMv, HPv>;            \
         NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                 \
         NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)); \
         int per_sm = (int)((227 * 1024) / (smem + 1024));                                                            \
@@ -873,7 +914,8 @@ extern "C" int nf_coupling_stack_tc_forward(const void* packed, const void* hdr_
         if (per_sm > 512 / tmem_cols) per_sm = 512 / tmem_cols;                                                      \
         const int64_t cap = (int64_t)kNumSMs * per_sm;                                                               \
         const int grid = (int)(ntiles < cap ? ntiles : cap);                                                         \
-        kern<<<grid, kTcThreads, smem, st>>>((const float*)packed, (const float*)x, (float*)y, (float*)ld, B, inverse, nsub); \
+        kern<<<grid, kTcThreads, smem, st>>>((const float*)packed, (const float*)x, (float*)y, (float*)ld, B, inverse, nsub, \
+                                             seed, offset);                                                          \
     } while (0)
     if (HP == 64) { if (D <= 2) NF_CTC(2, 64); else if (D <= 3) NF_CTC(4, 64); else NF_CTC(8, 64); }
     else          { if (D <= 2) NF_CTC(2, 128); else if (D <= 3) NF_CTC(4, 128); else NF_CTC(8, 128); }
@@ -883,17 +925,30 @@ extern "C" int nf_coupling_stack_tc_forward(const void* packed, const void* hdr_
     return NF_OK;
 }
 
+extern "C" int nf_coupling_stack_tc_forward(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
+                                            void* y, void* ld, int64_t B, int inverse, nf_stream_t stream) {
+    return coupling_stack_tc_launch(packed, hdr_host, packed_bytes, x, y, ld, B, inverse, false, 0, 0, stream);
+}
+
+extern "C" int nf_coupling_stack_tc_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, uint64_t seed,
+                                           uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream) {
+    return coupling_stack_tc_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true,
+                                    seed, offset, stream);
+}
+
 extern "C" int64_t nf_made_stack_tc_block_words(int D) {
     if (D < 1 || D > NF_STACK_DMAX) return -1;
     return NF_LAYER_HDR + made_blk_offsets(nf_stack_w1s(D)).words;           // words per layer block
 }
 
-extern "C" int nf_made_stack_tc_forward(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
-                                        void* y, void* ld, int64_t B, int flags, int mode, nf_stream_t stream) {
-    if (B < 0) return NF_ERR_BAD_SHAPE;
+static int made_stack_tc_launch(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x, void* y,
+                                void* ld, int64_t B, int flags, int mode, bool sample, uint64_t seed, uint64_t offset,
+                                nf_stream_t stream) {
+    if (B < 0 || (sample && B > (int64_t)0xFFFFFFFFLL)) return NF_ERR_BAD_SHAPE;
     NF_REQ(hdr_host);
     if (B == 0) return NF_OK;
-    NF_REQ(packed); NF_REQ(x); NF_REQ(ld);
+    NF_REQ(packed); NF_REQ(ld);
+    if (!sample) NF_REQ(x);
     if (!(flags & NF_STACK_SKIP_Y)) NF_REQ(y);
     if (!aligned16(packed)) return NF_ERR_MISALIGNED;
     const int32_t* h = (const int32_t*)hdr_host;
@@ -915,16 +970,29 @@ extern "C" int nf_made_stack_tc_forward(const void* packed, const void* hdr_host
     const int grid = (int)(ntiles < res_ctas ? ntiles : res_ctas);
 #define NF_MTC(DMv)                                                                                                  \
     do {                                                                                                             \
-        auto kern = made_stack_tc_kernel<DMv>;                                                                       \
+        auto kern = sample ? made_stack_tc_kernel<DMv, true> : made_stack_tc_kernel<DMv>;                            \
         NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                 \
         NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)); \
-        kern<<<grid, kTcThreads, smem, st>>>((const float*)packed, (const float*)x, (float*)y, (float*)ld, B, flags, nsub, mode); \
+        kern<<<grid, kTcThreads, smem, st>>>((const float*)packed, (const float*)x, (float*)y, (float*)ld, B, flags, nsub, mode, \
+                                             seed, offset);                                                          \
     } while (0)
     if (D <= 2) NF_MTC(2); else if (D <= 3) NF_MTC(4); else NF_MTC(8);
 #undef NF_MTC
     count_launch();
     NF_LAUNCH_CHECK();
     return NF_OK;
+}
+
+extern "C" int nf_made_stack_tc_forward(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
+                                        void* y, void* ld, int64_t B, int flags, int mode, nf_stream_t stream) {
+    return made_stack_tc_launch(packed, hdr_host, packed_bytes, x, y, ld, B, flags, mode, false, 0, 0, stream);
+}
+
+extern "C" int nf_made_stack_tc_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, int mode, uint64_t seed,
+                                       uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream) {
+    if (mode != NF_AR_IAF_FORWARD && mode != NF_AR_MAF_FORWARD) return NF_ERR_UNSUPPORTED;     // the sampling directions
+    return made_stack_tc_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, mode, true,
+                                seed, offset, stream);
 }
 
 // library options: key 7 = tensor-core passes per product of the dense-layer and weight-gradient kernels: 3 = 3xTF32

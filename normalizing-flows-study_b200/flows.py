@@ -126,6 +126,72 @@ def flow_log_prob(flow, x, base_dist, fused_head=None):
     return log_p_z + log_det_inv
 
 
+def _event_dim(flow):
+    """data_dim of a flow or container (SequentialFlow and the models take it from their first layer)."""
+    d = getattr(flow, "data_dim", None)
+    if d is None:
+        flows = getattr(flow, "flows", None)
+        if flows is None and hasattr(flow, "flow"):
+            flows = flow.flow.flows
+        if flows:
+            d = _event_dim(flows[0])
+    return d
+
+
+def _draw_state(generator, device):
+    """(seed, offset) of one N(0, I) draw: the torch CUDA generator's seed and Philox offset, after which the offset
+    moves on by 4 (torch keeps offsets a multiple of 4) -- torch.manual_seed makes a call reproducible, and consecutive
+    calls draw new samples."""
+    if torch.cuda.is_current_stream_capturing():
+        raise RuntimeError("sample_and_log_prob cannot be captured in a CUDA graph: the seed and offset of the draw are "
+                           "read on the host, so every replay would repeat the same samples")
+    gen = generator
+    if gen is None:
+        torch.cuda.init()
+        gen = torch.cuda.default_generators[device.index if device.index is not None else torch.cuda.current_device()]
+    seed, offset = int(gen.initial_seed()), int(gen.get_offset())
+    gen.set_offset(offset + 4)
+    return seed, offset
+
+
+def flow_sample_and_log_prob(flow, num_samples, base_dist=None, device=None, generator=None):
+    """(x, log_q): z ~ base, (x, log_det) = flow.forward(z), log_q = log p_base(z) - log_det (summed over the event axis
+    as in Flow.log_prob), without materialising z where the route allows it.
+
+    A standard-normal base (None, or any base is_std_normal accepts) is drawn on the device from the counter-based
+    stream of csrc/nf_rng.cuh, seeded from `generator` (default: torch's default CUDA generator of `device`); float64
+    models widen its float32 normals.  A fused stack draws inside its one launch and evaluates log N(z) - log_det in the
+    last layer's epilogue (`_sample_fused`); every other route draws z with nf_std_normal_draw, runs forward(z) -- with
+    its autograd graph when parameters require grad, the reparameterised gradient -- and the log-q head kernel.  Any
+    other base is sampled by torch (rsample where it has one) and cannot take a generator."""
+    p = next(flow.parameters(), None)
+    device = torch.device(device if device is not None else (p.device if p is not None else "cpu"))
+    dtype = p.dtype if p is not None else torch.float32
+    D = _event_dim(flow)
+    n = int(num_samples)
+    if base_dist is not None and not is_std_normal(base_dist, D):
+        if generator is not None:
+            raise ValueError("generator= seeds the on-device N(0, I) draw only; torch distributions cannot take a generator")
+        z = (base_dist.rsample if base_dist.has_rsample else base_dist.sample)((n,)).to(device)
+        x, log_det = flow.forward(z)
+        log_p_z = base_dist.log_prob(z)
+        if log_p_z.dim() > 1:
+            log_p_z = log_p_z.sum(dim=1)
+        return x, log_p_z - log_det
+    if device.type != "cuda":
+        raise RuntimeError(L.NO_CPU_PATH)
+    with torch.cuda.device(device):
+        seed, offset = _draw_state(generator, device)
+        fused = getattr(flow, "_sample_fused", None)
+        if fused is not None and not wants_grad(flow):
+            out = fused(torch.empty((n, D), dtype=dtype, device=device), (seed, offset))
+            if out is not None:
+                return out
+        z = ops.std_normal_draw(seed, offset, n, D, dtype, device)
+        x, log_det = flow.forward(z)
+        return x, ops.std_normal_log_q(z, log_det)
+
+
 def _module_tensors(module: nn.Module):
     return list(module.parameters()) + list(module.buffers())
 
@@ -218,6 +284,14 @@ class Flow(nn.Module):
         A standard-normal base is detected (is_std_normal) and evaluated by the fused head kernels."""
         return flow_log_prob(self, x, base_dist, getattr(self, "_log_prob_fused", None))
 
+    def sample_and_log_prob(self, num_samples, base_dist=None, device=None, generator=None):
+        """Samples and their log-density in one pass: z ~ base, (x, log_det) = forward(z), log_q = log p_base(z) - log_det.
+        device=None: the parameters' device; dtype: the parameters'.  A standard-normal base (None or N(0, I)) is drawn on
+        the GPU from `generator` (torch.Generator on that device; None = torch's default CUDA generator, so
+        torch.manual_seed makes the call reproducible); float64 models widen the float32 draw.  Raises RuntimeError under
+        CUDA-graph capture, ValueError for a generator with any other base.  See flow_sample_and_log_prob."""
+        return flow_sample_and_log_prob(self, num_samples, base_dist, device, generator)
+
 
 class SequentialFlow(Flow):
     """Flows applied in order; inverse walks them backwards (sequential_flow.py:5-34)."""
@@ -232,6 +306,9 @@ class SequentialFlow(Flow):
     def _log_prob_fused(self, x):
         out = self._chain.run(self.flows, None, self.training, x, True, head=True)
         return None if out is None else out[1]
+
+    def _sample_fused(self, x, draw):
+        return self._chain.run(self.flows, None, self.training, x, False, sample=draw)
 
     @on_input_device
     def _run(self, v, inverse):
@@ -322,6 +399,12 @@ class CouplingLayer(Flow):
         s_raw = self._conditioner(self.s_net, v)
         b_raw = self._conditioner(self.b_net, v)
         return ops.affine_coupling(v, s_raw, b_raw, self.mask, inverse)
+
+    def _sample_fused(self, x, draw):
+        """The layer's own fused route of forward (one launch), drawing its input in the kernel."""
+        if self.fusable(x):
+            return run_coupling_stack(self._pack, self._pack.tensors_of([self]), [self], None, x, False, sample=draw)
+        return None
 
     def _fold_wide(self):
         with torch.no_grad():
@@ -419,6 +502,11 @@ class SplineCouplingLayer(Flow):
         params = ops.linear(h, w4, b4)
         return ops.spline_transform(v, params, self.mask, tidx, self.num_bins, inverse, self.bound, self._mins,
                                     rescale, compact=True)
+
+    def _sample_fused(self, x, draw):
+        if self.fusable(x):
+            return run_spline_stack(self._pack, self._pack.tensors_of([self]), [self], None, x, False, sample=draw)
+        return None
 
     def _fold_wide(self, tlist):
         """Mask-folded first Linear, compact head, TF32 splits: cached per weight version for the no-grad route."""
@@ -641,6 +729,17 @@ class InverseAutoregressiveFlow(_AffineAutoregressive):
     def inverse(self, x):
         return self._sequential(x)
 
+    def _sample_fused(self, x, draw):
+        """bf16 fused-chain mode (the route forward takes there): the draw, then one chain launch whose epilogue evaluates
+        log N(z) - log_det on the input row."""
+        if (not ops.MADE_CHAIN_BF16 or not ops.USE_TENSOR_CORE_GEMM or x.shape[0] < 128
+                or (self.conditioner.use_batch_norm and self.training)):
+            return None
+        f = self.conditioner.folded()
+        if f is None or f.w[0].dtype != x.dtype:
+            return None
+        return ops.made_chain_bf16(x, f, self._mode_parallel, draw=draw)
+
 
 class ARQS(Flow):
     """Autoregressive rational-quadratic-spline flow (src/flows/spline/arqs.py:7-114): a MADE conditioner with 3K-1
@@ -693,8 +792,9 @@ class ARQS(Flow):
 USE_TENSOR_CORES = True      # tcgen05 stack kernels (3xTF32, fp32-accurate); False forces the FP32-pipe kernels
 
 
-def run_spline_stack(cache: _PackCache, tensors, flows, bns, v, inverse, head=False):
-    """Spline-coupling stack in one launch: tcgen05 kernel when the configuration fits it, FP32-pipe kernel otherwise."""
+def run_spline_stack(cache: _PackCache, tensors, flows, bns, v, inverse, head=False, sample=None):
+    """Spline-coupling stack in one launch: tcgen05 kernel when the configuration fits it, FP32-pipe kernel otherwise.
+    sample=(seed, offset): the in-kernel N(0, I) draw into v, returning (x, log_q) (see ops._stack)."""
     def build():
         tcp = packing.pack_spline_stack_tc(flows, bns) if USE_TENSOR_CORES else None
         return ("tc", tcp) if tcp is not None else ("simt", packing.pack_spline_stack(flows, bns))
@@ -702,15 +802,15 @@ def run_spline_stack(cache: _PackCache, tensors, flows, bns, v, inverse, head=Fa
     if pk is None:
         return None
     if kind == "tc":
-        out = ops.spline_stack_tc(pk[0], pk[1], v, inverse, head)
+        out = ops.spline_stack_tc(pk[0], pk[1], v, inverse, head, sample)
         if out is not None:
             return out
         pk = packing.pack_spline_stack(flows, bns)
-        return None if pk is None else ops.spline_stack(pk[0], pk[1], v, inverse, head)
-    return ops.spline_stack(pk[0], pk[1], v, inverse, head)
+        return None if pk is None else ops.spline_stack(pk[0], pk[1], v, inverse, head, sample)
+    return ops.spline_stack(pk[0], pk[1], v, inverse, head, sample)
 
 
-def run_coupling_stack(cache: _PackCache, tensors, flows, bns, v, inverse, head=False):
+def run_coupling_stack(cache: _PackCache, tensors, flows, bns, v, inverse, head=False, sample=None):
     """Eval-mode affine coupling stack in one launch: tcgen05 kernel when hidden_dim <= 64, FP32-pipe kernel otherwise."""
     def build():
         tcp = packing.pack_coupling_stack_tc(flows, bns) if USE_TENSOR_CORES else None
@@ -719,12 +819,12 @@ def run_coupling_stack(cache: _PackCache, tensors, flows, bns, v, inverse, head=
     if pk is None:
         return None
     if kind == "tc":
-        out = ops.coupling_stack_tc(pk[0], pk[1], v, inverse, head)
+        out = ops.coupling_stack_tc(pk[0], pk[1], v, inverse, head, sample)
         if out is not None:
             return out
         pk = packing.pack_coupling_stack(flows, bns)
-        return None if pk is None else ops.coupling_stack(pk[0], pk[1], v, inverse, head)
-    return ops.coupling_stack(pk[0], pk[1], v, inverse, head)
+        return None if pk is None else ops.coupling_stack(pk[0], pk[1], v, inverse, head, sample)
+    return ops.coupling_stack(pk[0], pk[1], v, inverse, head, sample)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -738,10 +838,12 @@ class ChainPlan:
     def __init__(self):
         self._pack = _PackCache()
 
-    def run(self, flows, bns, training, v, inverse, head=False):
+    def run(self, flows, bns, training, v, inverse, head=False, sample=None):
         """(y, log_det) from one fused launch, or None when the chain must be walked layer by layer.
         head=True (inverse only): (None, log_prob) with the standard-normal Flow.log_prob head evaluated in the last
-        layer's epilogue -- z is never written."""
+        layer's epilogue -- z is never written.
+        sample=(seed, offset) (forward only): the sampling twin of the head -- v is the [n, D] output buffer, the rows are
+        the N(0, I) draw of csrc/nf_rng.cuh made in the kernel, and the result is (x, log N(z) - log_det)."""
         flows = list(flows)
         v = compute_input(v)
         if not flows or not v.is_cuda or v.dim() != 2:
@@ -750,7 +852,7 @@ class ChainPlan:
             return None
         kind = type(flows[0])
         if kind in (MaskedAutoregressiveFlow, InverseAutoregressiveFlow):
-            return self._run_made_stack(flows, bns, v, inverse, head)
+            return self._run_made_stack(flows, bns, v, inverse, head, sample)
         if kind not in (CouplingLayer, SplineCouplingLayer) or any(type(f) is not kind for f in flows):
             return None
         if not all(f.fusable(v) for f in flows):
@@ -760,10 +862,10 @@ class ChainPlan:
         if torch.is_grad_enabled() and (v.requires_grad or any(t.requires_grad for t in tensors)):
             return None
         if kind is CouplingLayer:
-            return run_coupling_stack(self._pack, tensors, flows, bns, v, inverse, head)
-        return run_spline_stack(self._pack, tensors, flows, bns, v, inverse, head)
+            return run_coupling_stack(self._pack, tensors, flows, bns, v, inverse, head, sample)
+        return run_spline_stack(self._pack, tensors, flows, bns, v, inverse, head, sample)
 
-    def _run_made_stack(self, flows, bns, v, inverse, head):
+    def _run_made_stack(self, flows, bns, v, inverse, head, sample):
         """Homogeneous MAF / IAF stack, hidden_dim <= 64, data_dim <= 8 (the sequential direction: data_dim == 2):
         one tcgen05 launch (made_stack_tc_kernel).  None -> the layers run one by one."""
         kind = type(flows[0])
@@ -789,4 +891,4 @@ class ChainPlan:
         if pk is None:
             return None
         mode = f0._mode_parallel if parallel else f0._mode_sequential
-        return ops.made_stack_tc(pk[0], pk[1], v, inverse, mode, head)
+        return ops.made_stack_tc(pk[0], pk[1], v, inverse, mode, head, sample)

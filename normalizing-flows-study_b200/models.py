@@ -10,7 +10,8 @@ import torch
 import torch.nn as nn
 
 from . import ops
-from .flows import ChainPlan, CouplingLayer, SplineCouplingLayer, _default_base, flow_log_prob, on_input_device
+from .flows import (ChainPlan, CouplingLayer, SplineCouplingLayer, _default_base, flow_log_prob, flow_sample_and_log_prob,
+                    on_input_device)
 
 
 class _DensityAPI:
@@ -33,6 +34,11 @@ class _DensityAPI:
         z = base_dist.sample((num_samples,)).to(device)
         x, _ = self.forward(z)
         return x
+
+    def sample_and_log_prob(self, num_samples, base_dist=None, device=None, generator=None):
+        """(x, log_q) with z ~ base, (x, log_det) = forward(z), log_q = log p_base(z) - log_det: Flow.sample_and_log_prob.
+        A standard-normal base is drawn on the GPU (one launch for a fused stack, z never written)."""
+        return flow_sample_and_log_prob(self, num_samples, base_dist, device, generator)
 
 
 class NormalizingFlowModel(_DensityAPI, nn.Module):
@@ -81,6 +87,9 @@ class NormalizingFlowModel(_DensityAPI, nn.Module):
     def _log_prob_fused(self, x):
         out = self._chain.run(self.flows, self._bns(), self.training, x, True, head=True)
         return None if out is None else out[1]
+
+    def _sample_fused(self, x, draw):
+        return self._chain.run(self.flows, self._bns(), self.training, x, False, sample=draw)
 
     @on_input_device
     def forward(self, z):
@@ -135,6 +144,9 @@ class RealNVP(_DensityAPI, nn.Module):
     def _log_prob_fused(self, x):
         return self.flow._log_prob_fused(x)
 
+    def _sample_fused(self, x, draw):
+        return self.flow._sample_fused(x, draw)
+
     def forward(self, z):
         return self.flow.forward(z)
 
@@ -151,6 +163,9 @@ class RealNVPSpline(_DensityAPI, nn.Module):
 
     def _log_prob_fused(self, x):
         return self.flow._log_prob_fused(x)
+
+    def _sample_fused(self, x, draw):
+        return self.flow._sample_fused(x, draw)
 
     def forward(self, z):
         return self.flow.forward(z)

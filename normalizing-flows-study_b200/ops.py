@@ -684,10 +684,46 @@ def std_normal_log_prob(z, log_det=None):
     return _StdNormalLogProbFn.apply(z, log_det)
 
 
+def std_normal_draw(seed, offset, B, D, dtype, device):
+    """z [B, D] ~ N(0, I) from the counter-based stream of csrc/nf_rng.cuh at (seed, offset): the same bits as the
+    in-kernel draw of the fused stacks.  float64 widens the float32 normals."""
+    z = torch.empty((B, D), dtype=dtype, device=device)
+    call("nf_std_normal_draw", seed, offset, ptr(z), B, D, L.dtype_code(z), stream())
+    return z
+
+
+class _StdNormalLogQFn(Function):
+    @staticmethod
+    def forward(ctx, z, ld):
+        z, ld = _c(z), _c(ld)
+        B, D = z.shape
+        lq = torch.empty(B, dtype=z.dtype, device=z.device)
+        call("nf_std_normal_log_q_forward", ptr(z), ptr(ld), ptr(lq), B, D, L.dtype_code(z), stream())
+        ctx.save_for_backward(z)
+        return lq
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, glq):
+        z, = ctx.saved_tensors
+        B, D = z.shape
+        gz = torch.empty_like(z) if ctx.needs_input_grad[0] else None
+        gld = torch.empty(B, dtype=z.dtype, device=z.device) if ctx.needs_input_grad[1] else None
+        call("nf_std_normal_log_q_backward", ptr(z), ptr(_c(glq)), ptr(gz), ptr(gld), B, D, L.dtype_code(z), stream())
+        return gz, gld
+
+
+def std_normal_log_q(z, log_det):
+    """log N(z; 0, I) - log_det per row: the sample_and_log_prob head for a standard-normal base."""
+    if log_det.dtype != z.dtype:
+        log_det = log_det.to(z.dtype)
+    return _StdNormalLogQFn.apply(z, log_det)
+
+
 # --------------------------------------------------------------------------------------------
 # fused inference launches
 # --------------------------------------------------------------------------------------------
-STACK_INVERSE, STACK_LOG_PROB_HEAD, STACK_SKIP_Y = 1, 2, 4      # csrc/stack_small.cuh
+STACK_INVERSE, STACK_LOG_PROB_HEAD, STACK_SKIP_Y, STACK_SAMPLE_LOG_Q = 1, 2, 4, 8      # csrc/stack_small.cuh
 
 
 def _stack_flags(inverse, head):
@@ -696,67 +732,57 @@ def _stack_flags(inverse, head):
     return (STACK_INVERSE if inverse else 0) | ((STACK_LOG_PROB_HEAD | STACK_SKIP_Y) if head else 0)
 
 
-def spline_stack(packed, hdr_host, x, inverse, head=False):
+def _stack(name, packed, hdr_host, x, inverse, head, sample, mode=()):
+    """One fused-stack launch; returns None if the configuration is unsupported.  sample=(seed, offset): the `_sample`
+    entry point instead -- x is the output buffer of the rows, drawn from N(0, I) in the kernel and run forward, and the
+    per-row output is log N(z) - log_det (sample_and_log_prob)."""
+    x = _c(x)
+    B = x.shape[0]
+    ld = torch.empty(B, dtype=x.dtype, device=x.device)
+    hdr, nbytes = hdr_host.ctypes.data, packed.numel() * 4
+    if sample is not None:
+        ok = L.try_call(name + "_sample", ptr(packed), hdr, nbytes, *mode, sample[0], sample[1], ptr(x), ptr(ld), B,
+                        stream())
+        return (x, ld) if ok else None
+    y = None if head else torch.empty_like(x)
+    ok = L.try_call(name + "_forward", ptr(packed), hdr, nbytes, ptr(x), ptr(y), ptr(ld), B, _stack_flags(inverse, head),
+                    *mode, stream())
+    return (y, ld) if ok else None
+
+
+def spline_stack(packed, hdr_host, x, inverse, head=False, sample=None):
     """Whole spline-coupling stack in one launch; returns None if the configuration is unsupported."""
-    x = _c(x)
-    B, D = x.shape
-    y = None if head else torch.empty_like(x)
-    ld = torch.empty(B, dtype=x.dtype, device=x.device)
-    ok = L.try_call("nf_spline_stack_forward", ptr(packed), hdr_host.ctypes.data, packed.numel() * 4, ptr(x), ptr(y),
-                    ptr(ld), B, _stack_flags(inverse, head), stream())
-    return (y, ld) if ok else None
+    return _stack("nf_spline_stack", packed, hdr_host, x, inverse, head, sample)
 
 
-def spline_stack_tc(packed, hdr_host, x, inverse, head=False):
+def spline_stack_tc(packed, hdr_host, x, inverse, head=False, sample=None):
     """Tensor-core (tcgen05) variant of spline_stack; returns None if the configuration is unsupported."""
-    x = _c(x)
-    B, D = x.shape
-    y = None if head else torch.empty_like(x)
-    ld = torch.empty(B, dtype=x.dtype, device=x.device)
-    ok = L.try_call("nf_spline_stack_tc_forward", ptr(packed), hdr_host.ctypes.data, packed.numel() * 4, ptr(x), ptr(y),
-                    ptr(ld), B, _stack_flags(inverse, head), stream())
-    return (y, ld) if ok else None
+    return _stack("nf_spline_stack_tc", packed, hdr_host, x, inverse, head, sample)
 
 
-def coupling_stack_tc(packed, hdr_host, x, inverse, head=False):
+def coupling_stack_tc(packed, hdr_host, x, inverse, head=False, sample=None):
     """Tensor-core (tcgen05) variant of coupling_stack; returns None if the configuration is unsupported."""
-    x = _c(x)
-    B, D = x.shape
-    y = None if head else torch.empty_like(x)
-    ld = torch.empty(B, dtype=x.dtype, device=x.device)
-    ok = L.try_call("nf_coupling_stack_tc_forward", ptr(packed), hdr_host.ctypes.data, packed.numel() * 4, ptr(x), ptr(y),
-                    ptr(ld), B, _stack_flags(inverse, head), stream())
-    return (y, ld) if ok else None
+    return _stack("nf_coupling_stack_tc", packed, hdr_host, x, inverse, head, sample)
 
 
-def made_stack_tc(packed, hdr_host, x, inverse, mode, head=False):
+def made_stack_tc(packed, hdr_host, x, inverse, mode, head=False, sample=None):
     """Whole MAF / IAF stack in one tcgen05 launch (csrc/stack_tc.cu: made_stack_tc_kernel); None if unsupported."""
-    x = _c(x)
-    B, D = x.shape
-    y = None if head else torch.empty_like(x)
-    ld = torch.empty(B, dtype=x.dtype, device=x.device)
-    ok = L.try_call("nf_made_stack_tc_forward", ptr(packed), hdr_host.ctypes.data, packed.numel() * 4, ptr(x), ptr(y),
-                    ptr(ld), B, _stack_flags(inverse, head), mode, stream())
-    return (y, ld) if ok else None
+    return _stack("nf_made_stack_tc", packed, hdr_host, x, inverse, head, sample, (mode,))
 
 
-def coupling_stack(packed, hdr_host, x, inverse, head=False):
-    x = _c(x)
-    B, D = x.shape
-    y = None if head else torch.empty_like(x)
-    ld = torch.empty(B, dtype=x.dtype, device=x.device)
-    ok = L.try_call("nf_coupling_stack_forward", ptr(packed), hdr_host.ctypes.data, packed.numel() * 4, ptr(x),
-                    ptr(y), ptr(ld), B, _stack_flags(inverse, head), stream())
-    return (y, ld) if ok else None
+def coupling_stack(packed, hdr_host, x, inverse, head=False, sample=None):
+    return _stack("nf_coupling_stack", packed, hdr_host, x, inverse, head, sample)
 
 
 MADE_CHAIN_BF16 = False          # set by nfb200.set_gemm_precision("bf16"): the fused bf16 chain kernel for MAF / IAF
 
 
-def made_chain_bf16(v, folded, mode, head=False):
+def made_chain_bf16(v, folded, mode, head=False, draw=None):
     """Whole parallel direction in ONE launch on bf16 tensor cores (csrc/made_chain_bf16.cu); None when the shape is
     outside the kernel's envelope (data_dim <= 64 and a multiple of 4, hidden_dim a multiple of 128 and <= 512).
-    head=True: returns (None, log N(z;0,I) + log_det) without storing z."""
+    head=True: returns (None, log N(z;0,I) + log_det) without storing z.
+    draw=(seed, offset) (IAF.forward): v only gives the shape; the input is the N(0, I) draw at (seed, offset), made by
+    nf_std_normal_draw once the shape is known to fit, and the result is (x, log N(z) - log_det)."""
     from . import packing
     if v.dtype != torch.float32:
         return None
@@ -765,13 +791,17 @@ def made_chain_bf16(v, folded, mode, head=False):
     pk = folded.bf16
     if pk is False:
         return None
-    v = _c(v)
     B, D = v.shape
+    flags = (STACK_LOG_PROB_HEAD | STACK_SKIP_Y) if head else 0
+    if draw is not None:
+        v = std_normal_draw(draw[0], draw[1], B, D, v.dtype, v.device)
+        flags = STACK_SAMPLE_LOG_Q
+    v = _c(v)
     out = None if head else torch.empty_like(v)
     ld = torch.empty(B, dtype=v.dtype, device=v.device)
     ok = L.try_call("nf_made_chain_bf16_forward", ptr(v), ptr(pk.w[0]), ptr(pk.w[1]), ptr(pk.w[2]), ptr(pk.w[3]),
                     ptr(pk.b[0]), ptr(pk.b[1]), ptr(pk.b[2]), ptr(pk.b[3]), pk.kext16_host.ctypes.data, ptr(out), ptr(ld),
-                    B, D, folded.H, mode, (STACK_LOG_PROB_HEAD | STACK_SKIP_Y) if head else 0, stream())
+                    B, D, folded.H, mode, flags, stream())
     return (out, ld) if ok else None
 
 

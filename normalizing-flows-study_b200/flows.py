@@ -811,7 +811,8 @@ def run_spline_stack(cache: _PackCache, tensors, flows, bns, v, inverse, head=Fa
 
 
 def run_coupling_stack(cache: _PackCache, tensors, flows, bns, v, inverse, head=False, sample=None):
-    """Eval-mode affine coupling stack in one launch: tcgen05 kernel when hidden_dim <= 64, FP32-pipe kernel otherwise."""
+    """Eval-mode affine coupling stack in one launch: the tcgen05 kernel (hidden_dim <= 128), or the FP32-pipe kernel
+    when USE_TENSOR_CORES is False."""
     def build():
         tcp = packing.pack_coupling_stack_tc(flows, bns) if USE_TENSOR_CORES else None
         return ("tc", tcp) if tcp is not None else ("simt", packing.pack_coupling_stack(flows, bns))

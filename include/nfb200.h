@@ -277,6 +277,29 @@ NF_API int nf_coupling_stack_tc_sample(const void* packed, const void* hdr_host,
 /* mode: NF_AR_IAF_FORWARD (any data_dim <= 8) or NF_AR_MAF_FORWARD (data_dim == 2) */
 NF_API int nf_made_stack_tc_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, int mode, uint64_t seed,
                                    uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream);
+/* Device-resident generator state (CUDA-graph safe drawing): the *_state twins of nf_std_normal_draw and the five
+ * nf_*_sample entry points take `rng_state`, caller-owned device memory holding uint64[4] = {seed, offset, ticket,
+ * reserved} (8-byte aligned), ticket 0 between calls.  The call draws with the key (seed, offset) it reads from the state,
+ * the same bits as the entry point above with that seed and offset, and the same launch advances the state: once the
+ * call completes, offset has moved on by 4 and ticket is 0 (the last CTA to read the key stores them).  Nothing is read
+ * or advanced on the host, so a captured call draws new samples on every replay.  B == 0 launches a one-thread kernel
+ * that only advances the state; a refused call (any error code) launches nothing and leaves the state as it was.
+ * A device-state launch of a tcgen05 stack needs 16 bytes more shared memory (the key) and the FP32-pipe sampling kernels
+ * hold it in both forms; no configuration inside the envelopes comes within 16 bytes of a shared-memory limit (the closest
+ * leaves 1.8 KB), so both forms accept the same configurations and the bit equality holds wherever either runs.
+ * Stream-ordered: one state must not be used by two streams at once.  The library neither allocates nor synchronises;
+ * the state is caller memory. */
+NF_API int nf_std_normal_draw_state(void* rng_state, void* z, int64_t B, int D, int dtype, nf_stream_t stream);
+NF_API int nf_spline_stack_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes, void* rng_state,
+                                        void* x, void* log_q, int64_t B, nf_stream_t stream);
+NF_API int nf_spline_stack_tc_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes, void* rng_state,
+                                           void* x, void* log_q, int64_t B, nf_stream_t stream);
+NF_API int nf_coupling_stack_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes, void* rng_state,
+                                          void* x, void* log_q, int64_t B, nf_stream_t stream);
+NF_API int nf_coupling_stack_tc_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes,
+                                             void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream);
+NF_API int nf_made_stack_tc_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes, int mode,
+                                         void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream);
 
 /* ---- fused inference stacks on the tensor cores (tcgen05 + TMEM, 3xTF32 = fp32-accurate): same contract as
  * nf_spline_stack_forward, for hidden_dim <= 64, num_bins <= 10 and at most 2 transformed dims per layer; `packed`

@@ -6,14 +6,14 @@ The directory name is not a Python identifier; import it through the `nfb200` al
 """
 from . import _lib, ops, packing, parallel, graphs  # noqa: F401
 from .flows import (Flow, SequentialFlow, CouplingLayer, SplineCouplingLayer, rational_quadratic_spline,  # noqa: F401
-                    MaskedLinear, MADE, MaskedAutoregressiveFlow, InverseAutoregressiveFlow, ARQS)
+                    MaskedLinear, MADE, MaskedAutoregressiveFlow, InverseAutoregressiveFlow, ARQS, DeviceGenerator)
 from .models import NormalizingFlowModel, RealNVP, RealNVPSpline  # noqa: F401
 from .packing import invalidate_caches  # noqa: F401
 
 __all__ = ["Flow", "SequentialFlow", "CouplingLayer", "SplineCouplingLayer", "rational_quadratic_spline",
            "MaskedLinear", "MADE", "MaskedAutoregressiveFlow", "InverseAutoregressiveFlow", "ARQS",
            "NormalizingFlowModel", "RealNVP", "RealNVPSpline", "set_strict_fp32", "set_gemm_precision",
-           "get_gemm_precision", "invalidate_caches"]
+           "get_gemm_precision", "invalidate_caches", "DeviceGenerator"]
 
 
 def set_strict_fp32(flag: bool = True) -> None:

@@ -67,6 +67,12 @@ _SIGNATURES = {
     "nf_coupling_stack_sample": [_P, _P, _L, _U, _U, _P, _P, _L, _P],
     "nf_coupling_stack_tc_sample": [_P, _P, _L, _U, _U, _P, _P, _L, _P],
     "nf_made_stack_tc_sample": [_P, _P, _L, _I, _U, _U, _P, _P, _L, _P],
+    "nf_std_normal_draw_state": [_P, _P, _L, _I, _I, _P],
+    "nf_spline_stack_sample_state": [_P, _P, _L, _P, _P, _P, _L, _P],
+    "nf_spline_stack_tc_sample_state": [_P, _P, _L, _P, _P, _P, _L, _P],
+    "nf_coupling_stack_sample_state": [_P, _P, _L, _P, _P, _P, _L, _P],
+    "nf_coupling_stack_tc_sample_state": [_P, _P, _L, _P, _P, _P, _L, _P],
+    "nf_made_stack_tc_sample_state": [_P, _P, _L, _I, _P, _P, _P, _L, _P],
     "nf_debug_tc_gemm128": [_P, _P, _P, _I, _I, _P, _I, _P],
     "nf_linear_tc": [_P, _P, _P, _P, _P, _L, _L, _L, _L, _L, _L, _I, _P, _P],
     "nf_linear_tc_range": [_P, _P, _P, _P, _P, _L, _L, _L, _L, _L, _L, _I, _P, _P, _P],

@@ -409,10 +409,18 @@ std_normal_log_q_bwd_kernel(const T* __restrict__ z, const T* __restrict__ g, T*
     }
 }
 
-// the N(0, I) base draw of nf_rng.cuh: one thread per group of four dims of a row; float64 widens the fp32 normals
+// the N(0, I) base draw of nf_rng.cuh: one thread per group of four dims of a row; float64 widens the fp32 normals.
+// rng_state != NULL: the key is read from, and advanced in, the device-resident state (nf_rng_state_take)
 template <typename T>
 __global__ void __launch_bounds__(256)
-std_normal_draw_kernel(uint64_t seed, uint64_t offset, T* __restrict__ z, int64_t B, int D) {
+std_normal_draw_kernel(uint64_t seed, uint64_t offset, unsigned long long* rng_state, T* __restrict__ z, int64_t B, int D) {
+    if (rng_state) {
+        const unsigned long long* key = nf_rng_key_static();
+        nf_rng_state_take(rng_state, nf_rng_key_static());
+        __syncthreads();
+        seed = key[0];
+        offset = key[1];
+    }
     const int J = (D + 3) >> 2;
     const int64_t n = B * J, stride = (int64_t)gridDim.x * blockDim.x;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += stride) {
@@ -429,6 +437,18 @@ std_normal_draw_kernel(uint64_t seed, uint64_t offset, T* __restrict__ z, int64_
             for (int k = 0; k < 4; ++k) if (k < m) st_stream(p + k, (T)q[k]);
         }
     }
+}
+
+// B == 0 under a device-resident state: the call draws nothing but still moves the offset on by 4
+__global__ void __launch_bounds__(1) rng_state_advance_kernel(unsigned long long* rng_state) {
+    nf_rng_state_take(rng_state, nf_rng_key_static());
+}
+
+int nf_rng_state_advance(unsigned long long* state, cudaStream_t st) {
+    rng_state_advance_kernel<<<1, 1, 0, st>>>(state);
+    count_launch();
+    NF_LAUNCH_CHECK();
+    return NF_OK;
 }
 
 template <typename T>
@@ -684,19 +704,32 @@ extern "C" int nf_std_normal_log_prob_backward(const void* z, const void* glp, v
     return NF_OK;
 }
 
-extern "C" int nf_std_normal_draw(uint64_t seed, uint64_t offset, void* z, int64_t B, int D, int dtype, nf_stream_t stream) {
+// rng_state == NULL: the key (seed, offset) given by the caller; otherwise the device-resident state
+static int std_normal_draw_launch(uint64_t seed, uint64_t offset, unsigned long long* rng_state, void* z, int64_t B,
+                                  int D, int dtype, nf_stream_t stream) {
     if (B < 0 || B > (int64_t)0xFFFFFFFFLL || D < 1) return NF_ERR_BAD_SHAPE;
-    if (B == 0) return NF_OK;
+    if (rng_state && dtype != NF_F32 && dtype != NF_F64) return NF_ERR_UNSUPPORTED;    // refused: the state stays put
+    cudaStream_t st = (cudaStream_t)stream;
+    if (B == 0) return rng_state ? nf_rng_state_advance(rng_state, st) : NF_OK;
     NF_REQ(z);
     if (dtype == NF_F32 && (D & 3) == 0 && !aligned16(z)) return NF_ERR_MISALIGNED;
-    cudaStream_t st = (cudaStream_t)stream;
     const int grid = ew_grid(B * ((D + 3) / 4));
     NF_DISPATCH(
-        (std_normal_draw_kernel<float><<<grid, 256, 0, st>>>(seed, offset, (float*)z, B, D)),
-        (std_normal_draw_kernel<double><<<grid, 256, 0, st>>>(seed, offset, (double*)z, B, D)));
+        (std_normal_draw_kernel<float><<<grid, 256, 0, st>>>(seed, offset, rng_state, (float*)z, B, D)),
+        (std_normal_draw_kernel<double><<<grid, 256, 0, st>>>(seed, offset, rng_state, (double*)z, B, D)));
     count_launch();
     NF_LAUNCH_CHECK();
     return NF_OK;
+}
+
+extern "C" int nf_std_normal_draw(uint64_t seed, uint64_t offset, void* z, int64_t B, int D, int dtype, nf_stream_t stream) {
+    return std_normal_draw_launch(seed, offset, nullptr, z, B, D, dtype, stream);
+}
+
+extern "C" int nf_std_normal_draw_state(void* rng_state, void* z, int64_t B, int D, int dtype, nf_stream_t stream) {
+    const int rc = nf_rng_state_check(rng_state);
+    if (rc != NF_OK) return rc;
+    return std_normal_draw_launch(0, 0, (unsigned long long*)rng_state, z, B, D, dtype, stream);
 }
 
 extern "C" int nf_std_normal_log_q_forward(const void* z, const void* ld, void* lq, int64_t B, int D, int dtype,

@@ -93,6 +93,44 @@ NF_RNG_HD float nf_std_normal_row(uint64_t seed, uint64_t offset, uint32_t row, 
     return acc - (float)(0.5 * (double)D * 1.8378770664093453);
 }
 
+#ifdef __CUDACC__
+// Device-resident generator state (nf_*_sample_state, nf_std_normal_draw_state): uint64[4] = {seed, offset, ticket,
+// reserved} in caller memory, ticket 0 between calls.  A launch draws with the key (seed, offset) it reads there and
+// moves offset on by 4 in the same launch, so a CUDA-graph replay draws new samples.  Ticket protocol: every CTA of the
+// grid calls this exactly once, before any early exit or role split; thread 0 reads (seed, offset) into key[0..1]
+// (shared memory), fences, and takes a ticket.  The CTA that takes ticket gridDim.x - 1 knows every CTA has read the
+// key, so it stores offset + 4 and ticket = 0.  key[] is valid for the CTA after the caller's next __syncthreads(); the
+// kernels read it where they draw, so the key costs no registers across the kernel.
+__device__ __forceinline__ void nf_rng_state_take(unsigned long long* state, unsigned long long* key) {
+    if (threadIdx.x == 0) {
+        const unsigned long long seed = __ldcg(state), offset = __ldcg(state + 1);
+        key[0] = seed;
+        key[1] = offset;
+        __threadfence();
+        if (atomicAdd(state + 2, 1ull) == (unsigned long long)gridDim.x - 1) {
+            __threadfence();
+            state[1] = offset + 4;
+            state[2] = 0;
+        }
+    }
+}
+
+// the key slot of kernels without a spare dynamic shared-memory word (one per kernel: a function-scope static)
+__device__ __forceinline__ unsigned long long* nf_rng_key_static() {
+    __shared__ unsigned long long key[2];
+    return key;
+}
+
+// entry-point check of a caller's state pointer (64-bit atomics need 8-byte alignment)
+inline int nf_rng_state_check(const void* state) {
+    if (state == nullptr) return NF_ERR_NULL;
+    return (reinterpret_cast<uintptr_t>(state) & 7) ? NF_ERR_MISALIGNED : NF_OK;
+}
+
+// B == 0: the sampling entry points launch nothing else, but a call still advances the state (aux_kernels.cu)
+int nf_rng_state_advance(unsigned long long* state, cudaStream_t st);
+#endif
+
 }  // namespace nf
 
 #undef NF_RNG_HD

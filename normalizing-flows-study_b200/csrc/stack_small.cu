@@ -144,11 +144,14 @@ __device__ __forceinline__ void bn_between(const float* __restrict__ sL, int D, 
 // spline stack
 // ------------------------------------------------------------------------------------------------
 // SAMPLE (both kernels, nf_*_stack_sample): the row is the N(0, I) draw of nf_rng.cuh instead of a load, tot starts at
-// -log N(z) and the epilogue stores -tot = log N(z) - log_det (sample_and_log_prob)
+// -log N(z) and the epilogue stores -tot = log N(z) - log_det (sample_and_log_prob).  rng_state != NULL
+// (nf_*_stack_sample_state): the key comes from the device-resident state, which the launch advances; otherwise from
+// the seed / offset arguments.  Non-SAMPLE instantiations ignore all three.
 template <int HP, int R, int DM, int KMAX, bool SAMPLE = false>
 __global__ void __launch_bounds__(kStackThreads)
 spline_stack_kernel(const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
-                    float* __restrict__ ld, int64_t B, int flags, int layer_words_pad, uint64_t seed, uint64_t offset) {
+                    float* __restrict__ ld, int64_t B, int flags, int layer_words_pad, uint64_t seed, uint64_t offset,
+                    unsigned long long* rng_state) {
     const int inverse = flags & NF_STACK_INVERSE;
     extern __shared__ __align__(16) float smem[];
     const StackHdr hd = read_hdr(packed);
@@ -167,6 +170,12 @@ spline_stack_kernel(const float* __restrict__ packed, const float* __restrict__ 
     cfg.min_w = hd.min_w; cfg.min_h = hd.min_h; cfg.min_d = hd.min_d; cfg.scale_w = hd.scale_w; cfg.scale_h = hd.scale_h;
 
     const int tid = threadIdx.x;
+    if constexpr (SAMPLE) {
+        if (rng_state) {                        // every CTA, before the tile loop (a CTA may find no tile)
+            nf_rng_state_take(rng_state, nf_rng_key_static());
+            __syncthreads();
+        }
+    }
     const int64_t ntiles = (B + ROWS - 1) / ROWS;
     for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         float xv[R][DM], tot[R];
@@ -175,7 +184,9 @@ spline_stack_kernel(const float* __restrict__ packed, const float* __restrict__ 
         for (int i = 0; i < R; ++i) {
             row[i] = tile * ROWS + i * kStackThreads + tid;
             if constexpr (SAMPLE) {
-                tot[i] = -nf_std_normal_row<DM>(seed, offset, (uint32_t)row[i], D, xv[i]);
+                const unsigned long long* key = nf_rng_key_static();
+                tot[i] = -nf_std_normal_row<DM>(rng_state ? key[0] : seed, rng_state ? key[1] : offset, (uint32_t)row[i],
+                                                D, xv[i]);
                 continue;
             }
             tot[i] = 0.f;
@@ -271,7 +282,8 @@ spline_stack_kernel(const float* __restrict__ packed, const float* __restrict__ 
 template <int HP, int R, int DM, bool SAMPLE = false>
 __global__ void __launch_bounds__(kStackThreads)
 coupling_stack_kernel(const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
-                      float* __restrict__ ld, int64_t B, int flags, uint64_t seed, uint64_t offset) {
+                      float* __restrict__ ld, int64_t B, int flags, uint64_t seed, uint64_t offset,
+                      unsigned long long* rng_state) {
     const int inverse = flags & NF_STACK_INVERSE;
     extern __shared__ __align__(16) float smem[];
     const StackHdr hd = read_hdr(packed);
@@ -282,6 +294,12 @@ coupling_stack_kernel(const float* __restrict__ packed, const float* __restrict_
     const int net_words = HP * W1S + HP * HP + HP + NO * HP + NO;
 
     const int tid = threadIdx.x;
+    if constexpr (SAMPLE) {
+        if (rng_state) {                        // every CTA, before the tile loop (a CTA may find no tile)
+            nf_rng_state_take(rng_state, nf_rng_key_static());
+            __syncthreads();
+        }
+    }
     const int64_t ntiles = (B + ROWS - 1) / ROWS;
     for (int64_t tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
         float xv[R][DM], tot[R];
@@ -290,7 +308,9 @@ coupling_stack_kernel(const float* __restrict__ packed, const float* __restrict_
         for (int i = 0; i < R; ++i) {
             row[i] = tile * ROWS + i * kStackThreads + tid;
             if constexpr (SAMPLE) {
-                tot[i] = -nf_std_normal_row<DM>(seed, offset, (uint32_t)row[i], D, xv[i]);
+                const unsigned long long* key = nf_rng_key_static();
+                tot[i] = -nf_std_normal_row<DM>(rng_state ? key[0] : seed, rng_state ? key[1] : offset, (uint32_t)row[i],
+                                                D, xv[i]);
                 continue;
             }
             tot[i] = 0.f;
@@ -366,9 +386,10 @@ coupling_stack_kernel(const float* __restrict__ packed, const float* __restrict_
 // ------------------------------------------------------------------------------------------------
 template <typename Kern>
 static int launch_stack(Kern kern, size_t smem_bytes, int rows_per_cta, const void* packed, const void* x, void* y,
-                        void* ld, int64_t B, int inverse, int extra, bool has_extra, uint64_t seed, uint64_t offset,
-                        cudaStream_t st) {
-    if (smem_bytes > 227 * 1024) return NF_ERR_UNSUPPORTED;
+                        void* ld, int64_t B, int inverse, int extra, bool has_extra, bool sample, uint64_t seed,
+                        uint64_t offset, unsigned long long* rng_state, cudaStream_t st) {
+    // the SAMPLE twins hold the 16-byte key of nf_rng_state_take in static shared memory
+    if (smem_bytes + (sample ? 16 : 0) > 227 * 1024) return NF_ERR_UNSUPPORTED;
     NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
     NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     int per_sm = 0;
@@ -378,9 +399,9 @@ static int launch_stack(Kern kern, size_t smem_bytes, int rows_per_cta, const vo
     const int64_t cap = (int64_t)kNumSMs * per_sm;
     const int grid = (int)(ntiles < cap ? ntiles : cap);
     void* args_s[] = {(void*)&packed, (void*)&x, (void*)&y, (void*)&ld, (void*)&B, (void*)&inverse, (void*)&extra,
-                      (void*)&seed, (void*)&offset};
+                      (void*)&seed, (void*)&offset, (void*)&rng_state};
     void* args_n[] = {(void*)&packed, (void*)&x, (void*)&y, (void*)&ld, (void*)&B, (void*)&inverse, (void*)&seed,
-                      (void*)&offset};
+                      (void*)&offset, (void*)&rng_state};
     NF_CUDA(cudaLaunchKernel((const void*)kern, dim3(grid), dim3(kStackThreads), has_extra ? args_s : args_n, smem_bytes, st));
     count_launch();
     return NF_OK;
@@ -417,10 +438,10 @@ static int check_hdr(const int32_t* h, int magic) {
 // sample: the SAMPLE kernel draws the rows from (seed, offset); x is not read
 static int spline_stack_launch(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x, void* y,
                                void* ld, int64_t B, int inverse, bool sample, uint64_t seed, uint64_t offset,
-                               nf_stream_t stream) {
+                               unsigned long long* rng_state, nf_stream_t stream) {
     if (B < 0 || (sample && B > (int64_t)0xFFFFFFFFLL)) return NF_ERR_BAD_SHAPE;
     NF_REQ(hdr_host);
-    if (B == 0) return NF_OK;
+    if (B == 0) return rng_state ? nf_rng_state_advance(rng_state, (cudaStream_t)stream) : NF_OK;
     NF_REQ(packed); NF_REQ(ld);
     if (!sample) NF_REQ(x);
     if (!(inverse & NF_STACK_SKIP_Y)) NF_REQ(y);
@@ -437,7 +458,7 @@ static int spline_stack_launch(const void* packed, const void* hdr_host, int64_t
     const size_t smem = sizeof(float) * ((size_t)stride + (size_t)NO * rows);
 #define NF_SS(HPv, Rv, DMv, KMv)                                                                                     \
     return launch_stack(sample ? spline_stack_kernel<HPv, Rv, DMv, KMv, true> : spline_stack_kernel<HPv, Rv, DMv, KMv>,   \
-                        smem, rows, packed, x, y, ld, B, inverse, stride, true, seed, offset, st)
+                        smem, rows, packed, x, y, ld, B, inverse, stride, true, sample, seed, offset, rng_state, st)
     if (HP == 64) {
         if (D <= 3) { if (K <= 8) NF_SS(64, 2, 4, 8); else NF_SS(64, 2, 4, 16); }
         else        { if (K <= 8) NF_SS(64, 2, 8, 8); else NF_SS(64, 2, 8, 16); }
@@ -450,21 +471,29 @@ static int spline_stack_launch(const void* packed, const void* hdr_host, int64_t
 
 extern "C" int nf_spline_stack_forward(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
                                        void* y, void* ld, int64_t B, int inverse, nf_stream_t stream) {
-    return spline_stack_launch(packed, hdr_host, packed_bytes, x, y, ld, B, inverse, false, 0, 0, stream);
+    return spline_stack_launch(packed, hdr_host, packed_bytes, x, y, ld, B, inverse, false, 0, 0, nullptr, stream);
 }
 
 extern "C" int nf_spline_stack_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, uint64_t seed,
                                       uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream) {
     return spline_stack_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true, seed,
-                               offset, stream);
+                               offset, nullptr, stream);
+}
+
+extern "C" int nf_spline_stack_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes,
+                                            void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream) {
+    const int rc = nf_rng_state_check(rng_state);
+    if (rc != NF_OK) return rc;
+    return spline_stack_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true, 0, 0,
+                               (unsigned long long*)rng_state, stream);
 }
 
 static int coupling_stack_launch(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x, void* y,
                                  void* ld, int64_t B, int inverse, bool sample, uint64_t seed, uint64_t offset,
-                                 nf_stream_t stream) {
+                                 unsigned long long* rng_state, nf_stream_t stream) {
     if (B < 0 || (sample && B > (int64_t)0xFFFFFFFFLL)) return NF_ERR_BAD_SHAPE;
     NF_REQ(hdr_host);
-    if (B == 0) return NF_OK;
+    if (B == 0) return rng_state ? nf_rng_state_advance(rng_state, (cudaStream_t)stream) : NF_OK;
     NF_REQ(packed); NF_REQ(ld);
     if (!sample) NF_REQ(x);
     if (!(inverse & NF_STACK_SKIP_Y)) NF_REQ(y);
@@ -481,7 +510,7 @@ static int coupling_stack_launch(const void* packed, const void* hdr_host, int64
     const size_t smem = sizeof(float) * (size_t)stride;
 #define NF_CS(HPv, Rv, DMv)                                                                                          \
     return launch_stack(sample ? coupling_stack_kernel<HPv, Rv, DMv, true> : coupling_stack_kernel<HPv, Rv, DMv>, smem, \
-                        rows, packed, x, y, ld, B, inverse, 0, false, seed, offset, st)
+                        rows, packed, x, y, ld, B, inverse, 0, false, sample, seed, offset, rng_state, st)
     if (HP == 64) { if (D <= 3) NF_CS(64, 2, 4); else NF_CS(64, 2, 8); }
     else          { if (D <= 3) NF_CS(128, 1, 4); else NF_CS(128, 1, 8); }
 #undef NF_CS
@@ -490,11 +519,19 @@ static int coupling_stack_launch(const void* packed, const void* hdr_host, int64
 extern "C" int nf_coupling_stack_forward(const void* packed, const void* hdr_host, int64_t packed_bytes,
                                          const void* x, void* y, void* ld, int64_t B, int inverse,
                                          nf_stream_t stream) {
-    return coupling_stack_launch(packed, hdr_host, packed_bytes, x, y, ld, B, inverse, false, 0, 0, stream);
+    return coupling_stack_launch(packed, hdr_host, packed_bytes, x, y, ld, B, inverse, false, 0, 0, nullptr, stream);
 }
 
 extern "C" int nf_coupling_stack_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, uint64_t seed,
                                         uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream) {
     return coupling_stack_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true, seed,
-                                 offset, stream);
+                                 offset, nullptr, stream);
+}
+
+extern "C" int nf_coupling_stack_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes,
+                                              void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream) {
+    const int rc = nf_rng_state_check(rng_state);
+    if (rc != NF_OK) return rc;
+    return coupling_stack_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true, 0, 0,
+                                 (unsigned long long*)rng_state, stream);
 }

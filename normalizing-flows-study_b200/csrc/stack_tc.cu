@@ -51,9 +51,17 @@ __device__ __forceinline__ float relu_keepnan(float x) {      // torch.relu: NaN
 }
 
 // SAMPLE variants of the stack kernels (nf_*_sample): the row is the N(0, I) draw of nf_rng.cuh instead of a load, and
-// its log-det slot starts at -log N(z) -- the epilogue stores the negated sum, log N(z) - log_det (sample_and_log_prob)
+// its log-det slot starts at -log N(z) -- the epilogue stores the negated sum, log N(z) - log_det (sample_and_log_prob).
+// rng_state != NULL (nf_*_sample_state): the key comes from the device-resident state, taken by every CTA before the
+// setup barrier into two words after the barriers (the launch adds 16 bytes of shared memory for them) and advanced by
+// the launch; otherwise from the seed / offset arguments.  Non-SAMPLE kernels ignore it.  The coupling and MADE kernels
+// read the key where they draw (it then holds no registers across the kernel), the spline kernel once after its setup
+// barrier: each is the form with the lower register and spill counts.
+// rng_key: the key slot of nf_rng_state_take when the launch has a device-resident state, NULL otherwise
 template <int DM>
-__device__ __forceinline__ void draw_row_tc(float* srow, int64_t r, int64_t B, int D, uint64_t seed, uint64_t offset) {
+__device__ __forceinline__ void draw_row_tc(float* srow, int64_t r, int64_t B, int D, uint64_t seed, uint64_t offset,
+                                            const unsigned long long* rng_key) {
+    if (rng_key) { seed = rng_key[0]; offset = rng_key[1]; }
     float z[DM];
     const float lz = nf_std_normal_row<DM>(seed, offset, (uint32_t)r, D, z);
 #pragma unroll
@@ -221,7 +229,8 @@ __device__ __forceinline__ void hidden2_chunk(const uint32_t (&v)[16], const flo
 template <int DM, int KMAX, int KS, bool SAMPLE = false>
 __global__ void __launch_bounds__(kTc2Threads, 2)
 spline_stack_tc2_kernel(const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
-                        float* __restrict__ ld, int64_t B, int flags, uint64_t seed, uint64_t offset) {
+                        float* __restrict__ ld, int64_t B, int flags, uint64_t seed, uint64_t offset,
+                        unsigned long long* rng_state) {
     const int inverse = flags & NF_STACK_INVERSE;
     extern __shared__ __align__(1024) float sbuf[];
     const TcHdr hd = read_tc_hdr(packed);
@@ -240,6 +249,8 @@ spline_stack_tc2_kernel(const float* __restrict__ packed, const float* __restric
     const int tid = threadIdx.x, warp = tid >> 5, wg = tid >> 7, wtid = tid & 127, wwarp = warp & 3;
     const int bar_local = 1 + wg;
     if (warp == 0) tc::tmem_alloc(&tmem_base_s, kTmemCols);
+    unsigned long long* rng_key = reinterpret_cast<unsigned long long*>(bars + 5);   // SAMPLE + device state: every
+    if constexpr (SAMPLE) if (rng_state) nf_rng_state_take(rng_state, rng_key);   // CTA, before the role split / tiles
     if (tid == 0) {
         tc::mbar_init(&mbar[0], 1); tc::mbar_init(&mbar[1], 1); tc::mbar_init(&wbar[0], 1); tc::mbar_init(&wbar[1], 1);
         tc::fence_mbar_init();
@@ -247,6 +258,9 @@ spline_stack_tc2_kernel(const float* __restrict__ packed, const float* __restric
     tc::fence_before_sync();
     __syncthreads();
     tc::fence_after_sync();
+    // this kernel takes the key into the seed / offset registers once (reading it at each draw, as the coupling and MADE
+    // kernels do, makes ptxas spill in the DM = 4 twins); the draw below is then the host-key code unchanged
+    if constexpr (SAMPLE) if (rng_state) { seed = rng_key[0]; offset = rng_key[1]; }
     const uint32_t tb = tmem_base_s + (uint32_t)(wg * kWgCols);           // this warpgroup's 128 columns
     const uint32_t lane_addr = tb + ((uint32_t)(wwarp * 32) << 16);
     uint64_t* mb = &mbar[wg];
@@ -264,7 +278,7 @@ spline_stack_tc2_kernel(const float* __restrict__ packed, const float* __restric
         for (int s = wg; s < kTcSub; s += 2) {
             const int64_t r = tile * ROWS + s * kTcThreads + wtid;
             if constexpr (SAMPLE) {
-                draw_row_tc<DM>(sx + s * (DM + 1) * kTcThreads + wtid, r, B, D, seed, offset);
+                draw_row_tc<DM>(sx + s * (DM + 1) * kTcThreads + wtid, r, B, D, seed, offset, nullptr);
                 continue;
             }
 #pragma unroll
@@ -452,7 +466,8 @@ spline_stack_tc2_kernel(const float* __restrict__ packed, const float* __restric
 template <int DM, int HP, bool SAMPLE = false>
 __global__ void __launch_bounds__(kTcThreads, HP == 64 ? 2 : 1)
 coupling_stack_tc_kernel(const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
-                         float* __restrict__ ld, int64_t B, int flags, int nsub, uint64_t seed, uint64_t offset) {     // nsub <= kTcSub sub-tiles per weight staging
+                         float* __restrict__ ld, int64_t B, int flags, int nsub, uint64_t seed, uint64_t offset,
+                         unsigned long long* rng_state) {     // nsub <= kTcSub sub-tiles per weight staging
     constexpr int NBUF = (HP == 64) ? 2 : 1;
     constexpr int kColAhi = 0, kColAlo = HP, kColD2 = 2 * HP, kColD3 = 3 * HP;
     constexpr int kTmemCols = (HP == 64) ? 256 : 512;
@@ -471,6 +486,8 @@ coupling_stack_tc_kernel(const float* __restrict__ packed, const float* __restri
 
     const int tid = threadIdx.x, warp = tid >> 5;
     if (warp == 0) tc::tmem_alloc(&tmem_base_s, kTmemCols);
+    unsigned long long* rng_key = reinterpret_cast<unsigned long long*>(bars + 4);   // SAMPLE + device state: every
+    if constexpr (SAMPLE) if (rng_state) nf_rng_state_take(rng_state, rng_key);   // CTA, before the role split / tiles
     if (tid == 0) { tc::mbar_init(&bar, 1); tc::mbar_init(&wbar[0], 1); tc::mbar_init(&wbar[1], 1); tc::fence_mbar_init(); }
     tc::fence_before_sync();
     __syncthreads();
@@ -494,7 +511,7 @@ coupling_stack_tc_kernel(const float* __restrict__ packed, const float* __restri
         for (int s = 0; s < nsub; ++s) {
             const int64_t r = tile * ROWS + s * kTcThreads + tid;
             if constexpr (SAMPLE) {
-                draw_row_tc<DM>(sx + s * (DM + 1) * kTcThreads + tid, r, B, D, seed, offset);
+                draw_row_tc<DM>(sx + s * (DM + 1) * kTcThreads + tid, r, B, D, seed, offset, rng_state ? rng_key : nullptr);
                 continue;
             }
 #pragma unroll
@@ -641,7 +658,8 @@ __host__ __device__ inline MadeBlkOff made_blk_offsets(int W1S) {
 template <int DM, bool SAMPLE = false>
 __global__ void __launch_bounds__(kTcThreads, 2)
 made_stack_tc_kernel(const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
-                     float* __restrict__ ld, int64_t B, int flags, int nsub, int mode, uint64_t seed, uint64_t offset) {
+                     float* __restrict__ ld, int64_t B, int flags, int nsub, int mode, uint64_t seed, uint64_t offset,
+                     unsigned long long* rng_state) {
     const int inverse = flags & NF_STACK_INVERSE;
     extern __shared__ __align__(1024) float sbuf[];
     const TcHdr hd = read_tc_hdr(packed);
@@ -658,6 +676,8 @@ made_stack_tc_kernel(const float* __restrict__ packed, const float* __restrict__
 
     const int tid = threadIdx.x, warp = tid >> 5;
     if (warp == 0) tc::tmem_alloc(&tmem_base_s, kTmemCols);
+    unsigned long long* rng_key = reinterpret_cast<unsigned long long*>(bars + 3);   // SAMPLE + device state: every
+    if constexpr (SAMPLE) if (rng_state) nf_rng_state_take(rng_state, rng_key);   // CTA, before the role split / tiles
     if (tid == 0) { tc::mbar_init(&bar, 1); tc::mbar_init(&wbar, 1); tc::fence_mbar_init(); }
     tc::fence_before_sync();
     __syncthreads();
@@ -673,7 +693,7 @@ made_stack_tc_kernel(const float* __restrict__ packed, const float* __restrict__
         for (int s = 0; s < nsub; ++s) {
             const int64_t r = tile * ROWS + s * kTcThreads + tid;
             if constexpr (SAMPLE) {
-                draw_row_tc<DM>(sx + s * (DM + 1) * kTcThreads + tid, r, B, D, seed, offset);
+                draw_row_tc<DM>(sx + s * (DM + 1) * kTcThreads + tid, r, B, D, seed, offset, rng_state ? rng_key : nullptr);
                 continue;
             }
 #pragma unroll
@@ -803,10 +823,10 @@ extern "C" int64_t nf_spline_stack_tc_block_words(int D, int K, int max_dt) {
 // sample: the SAMPLE kernel draws the rows from (seed, offset); x is not read
 static int spline_stack_tc_launch(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x, void* y,
                                   void* ld, int64_t B, int inverse, bool sample, uint64_t seed, uint64_t offset,
-                                  nf_stream_t stream) {
+                                  unsigned long long* rng_state, nf_stream_t stream) {
     if (B < 0 || (sample && B > (int64_t)0xFFFFFFFFLL)) return NF_ERR_BAD_SHAPE;
     NF_REQ(hdr_host);
-    if (B == 0) return NF_OK;
+    if (B == 0) return rng_state ? nf_rng_state_advance(rng_state, (cudaStream_t)stream) : NF_OK;
     NF_REQ(packed); NF_REQ(ld);
     if (!sample) NF_REQ(x);
     if (!(inverse & NF_STACK_SKIP_Y)) NF_REQ(y);
@@ -820,7 +840,7 @@ static int spline_stack_tc_launch(const void* packed, const void* hdr_host, int6
     if (packed_bytes < (int64_t)sizeof(float) * (NF_STACK_HDR + (int64_t)L * BW)) return NF_ERR_WORKSPACE;
     cudaStream_t st = (cudaStream_t)stream;
     const int DMh = D <= 2 ? 2 : (D <= 3 ? 4 : 8);
-    const size_t smem = sizeof(float) * ((size_t)2 * BW + (size_t)kTcSub * (DMh + 1) * kTcThreads + 12);
+    const size_t smem = sizeof(float) * ((size_t)2 * BW + (size_t)kTcSub * (DMh + 1) * kTcThreads + 12 + (rng_state ? 4 : 0));
     if (smem > 227 * 1024) return NF_ERR_UNSUPPORTED;
     const int rows = kTcThreads * kTcSub;
     const int64_t ntiles = cdiv(B, rows);
@@ -837,7 +857,7 @@ static int spline_stack_tc_launch(const void* packed, const void* hdr_host, int6
            CTA of this kernel and the second co-resident CTA (the latency hiding of this design) never arrives */    \
         NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)); \
         kern<<<grid, kTc2Threads, smem, st>>>((const float*)packed, (const float*)x, (float*)y, (float*)ld, B, inverse, \
-                                              seed, offset);                                                         \
+                                              seed, offset, rng_state);                                              \
     } while (0)
 #define NF_TC_K(DMv)                                      \
     do {                                                  \
@@ -858,13 +878,21 @@ static int spline_stack_tc_launch(const void* packed, const void* hdr_host, int6
 
 extern "C" int nf_spline_stack_tc_forward(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
                                           void* y, void* ld, int64_t B, int inverse, nf_stream_t stream) {
-    return spline_stack_tc_launch(packed, hdr_host, packed_bytes, x, y, ld, B, inverse, false, 0, 0, stream);
+    return spline_stack_tc_launch(packed, hdr_host, packed_bytes, x, y, ld, B, inverse, false, 0, 0, nullptr, stream);
 }
 
 extern "C" int nf_spline_stack_tc_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, uint64_t seed,
                                          uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream) {
     return spline_stack_tc_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true,
-                                  seed, offset, stream);
+                                  seed, offset, nullptr, stream);
+}
+
+extern "C" int nf_spline_stack_tc_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes,
+                                               void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream) {
+    const int rc = nf_rng_state_check(rng_state);
+    if (rc != NF_OK) return rc;
+    return spline_stack_tc_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true,
+                                  0, 0, (unsigned long long*)rng_state, stream);
 }
 
 extern "C" int64_t nf_coupling_stack_tc_block_words(int D) {
@@ -878,10 +906,10 @@ extern "C" int64_t nf_coupling_stack_tc_block_words_hidden(int D, int H) {  // h
 
 static int coupling_stack_tc_launch(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
                                     void* y, void* ld, int64_t B, int inverse, bool sample, uint64_t seed, uint64_t offset,
-                                    nf_stream_t stream) {
+                                    unsigned long long* rng_state, nf_stream_t stream) {
     if (B < 0 || (sample && B > (int64_t)0xFFFFFFFFLL)) return NF_ERR_BAD_SHAPE;
     NF_REQ(hdr_host);
-    if (B == 0) return NF_OK;
+    if (B == 0) return rng_state ? nf_rng_state_advance(rng_state, (cudaStream_t)stream) : NF_OK;
     NF_REQ(packed); NF_REQ(ld);
     if (!sample) NF_REQ(x);
     if (!(inverse & NF_STACK_SKIP_Y)) NF_REQ(y);
@@ -896,7 +924,8 @@ static int coupling_stack_tc_launch(const void* packed, const void* hdr_host, in
     cudaStream_t st = (cudaStream_t)stream;
     const int DMh = D <= 2 ? 2 : (D <= 3 ? 4 : 8);
     const int nbuf = HP == 64 ? 2 : 1, tmem_cols = HP == 64 ? 256 : 512;
-    const size_t smem = sizeof(float) * ((size_t)nbuf * NBW + (size_t)kTcSub * (2 * DMh + 1) * kTcThreads + NF_LAYER_HDR + 8);
+    const size_t smem = sizeof(float) * ((size_t)nbuf * NBW + (size_t)kTcSub * (2 * DMh + 1) * kTcThreads + NF_LAYER_HDR + 8 +
+                                         (rng_state ? 4 : 0));
     if (smem > 227 * 1024) return NF_ERR_UNSUPPORTED;
     // small batches: fewer sub-tiles per weight staging so that every SM gets rows (4 000 rows on eight 512-row tiles
     // left 140 SMs idle); from kTcSub sub-tiles per resident CTA on, the staging is shared by kTcSub sub-tiles
@@ -915,7 +944,7 @@ static int coupling_stack_tc_launch(const void* packed, const void* hdr_host, in
         const int64_t cap = (int64_t)kNumSMs * per_sm;                                                               \
         const int grid = (int)(ntiles < cap ? ntiles : cap);                                                         \
         kern<<<grid, kTcThreads, smem, st>>>((const float*)packed, (const float*)x, (float*)y, (float*)ld, B, inverse, nsub, \
-                                             seed, offset);                                                          \
+                                             seed, offset, rng_state);                                               \
     } while (0)
     if (HP == 64) { if (D <= 2) NF_CTC(2, 64); else if (D <= 3) NF_CTC(4, 64); else NF_CTC(8, 64); }
     else          { if (D <= 2) NF_CTC(2, 128); else if (D <= 3) NF_CTC(4, 128); else NF_CTC(8, 128); }
@@ -927,13 +956,21 @@ static int coupling_stack_tc_launch(const void* packed, const void* hdr_host, in
 
 extern "C" int nf_coupling_stack_tc_forward(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
                                             void* y, void* ld, int64_t B, int inverse, nf_stream_t stream) {
-    return coupling_stack_tc_launch(packed, hdr_host, packed_bytes, x, y, ld, B, inverse, false, 0, 0, stream);
+    return coupling_stack_tc_launch(packed, hdr_host, packed_bytes, x, y, ld, B, inverse, false, 0, 0, nullptr, stream);
 }
 
 extern "C" int nf_coupling_stack_tc_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, uint64_t seed,
                                            uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream) {
     return coupling_stack_tc_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true,
-                                    seed, offset, stream);
+                                    seed, offset, nullptr, stream);
+}
+
+extern "C" int nf_coupling_stack_tc_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes,
+                                                 void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream) {
+    const int rc = nf_rng_state_check(rng_state);
+    if (rc != NF_OK) return rc;
+    return coupling_stack_tc_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true,
+                                    0, 0, (unsigned long long*)rng_state, stream);
 }
 
 extern "C" int64_t nf_made_stack_tc_block_words(int D) {
@@ -943,10 +980,10 @@ extern "C" int64_t nf_made_stack_tc_block_words(int D) {
 
 static int made_stack_tc_launch(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x, void* y,
                                 void* ld, int64_t B, int flags, int mode, bool sample, uint64_t seed, uint64_t offset,
-                                nf_stream_t stream) {
+                                unsigned long long* rng_state, nf_stream_t stream) {
     if (B < 0 || (sample && B > (int64_t)0xFFFFFFFFLL)) return NF_ERR_BAD_SHAPE;
     NF_REQ(hdr_host);
-    if (B == 0) return NF_OK;
+    if (B == 0) return rng_state ? nf_rng_state_advance(rng_state, (cudaStream_t)stream) : NF_OK;
     NF_REQ(packed); NF_REQ(ld);
     if (!sample) NF_REQ(x);
     if (!(flags & NF_STACK_SKIP_Y)) NF_REQ(y);
@@ -961,7 +998,7 @@ static int made_stack_tc_launch(const void* packed, const void* hdr_host, int64_
     if (packed_bytes < (int64_t)sizeof(float) * (NF_STACK_HDR + (int64_t)L * NBW)) return NF_ERR_WORKSPACE;
     cudaStream_t st = (cudaStream_t)stream;
     const int DMh = D <= 2 ? 2 : (D <= 3 ? 4 : 8);
-    const size_t smem = sizeof(float) * ((size_t)NBW + (size_t)kTcSub * (DMh + 1) * kTcThreads + 8);
+    const size_t smem = sizeof(float) * ((size_t)NBW + (size_t)kTcSub * (DMh + 1) * kTcThreads + 8 + (rng_state ? 4 : 0));
     if (smem > 113 * 1024) return NF_ERR_UNSUPPORTED;             // two CTAs per SM
     const int res_ctas = kNumSMs * 2;
     int nsub = (int)cdiv(cdiv(B, kTcThreads), res_ctas);
@@ -974,7 +1011,7 @@ static int made_stack_tc_launch(const void* packed, const void* hdr_host, int64_
         NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                 \
         NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)); \
         kern<<<grid, kTcThreads, smem, st>>>((const float*)packed, (const float*)x, (float*)y, (float*)ld, B, flags, nsub, mode, \
-                                             seed, offset);                                                          \
+                                             seed, offset, rng_state);                                               \
     } while (0)
     if (D <= 2) NF_MTC(2); else if (D <= 3) NF_MTC(4); else NF_MTC(8);
 #undef NF_MTC
@@ -985,14 +1022,23 @@ static int made_stack_tc_launch(const void* packed, const void* hdr_host, int64_
 
 extern "C" int nf_made_stack_tc_forward(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
                                         void* y, void* ld, int64_t B, int flags, int mode, nf_stream_t stream) {
-    return made_stack_tc_launch(packed, hdr_host, packed_bytes, x, y, ld, B, flags, mode, false, 0, 0, stream);
+    return made_stack_tc_launch(packed, hdr_host, packed_bytes, x, y, ld, B, flags, mode, false, 0, 0, nullptr, stream);
 }
 
 extern "C" int nf_made_stack_tc_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, int mode, uint64_t seed,
                                        uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream) {
     if (mode != NF_AR_IAF_FORWARD && mode != NF_AR_MAF_FORWARD) return NF_ERR_UNSUPPORTED;     // the sampling directions
     return made_stack_tc_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, mode, true,
-                                seed, offset, stream);
+                                seed, offset, nullptr, stream);
+}
+
+extern "C" int nf_made_stack_tc_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes, int mode,
+                                             void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream) {
+    if (mode != NF_AR_IAF_FORWARD && mode != NF_AR_MAF_FORWARD) return NF_ERR_UNSUPPORTED;     // the sampling directions
+    const int rc = nf_rng_state_check(rng_state);
+    if (rc != NF_OK) return rc;
+    return made_stack_tc_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, mode, true,
+                                0, 0, (unsigned long long*)rng_state, stream);
 }
 
 // library options: key 7 = tensor-core passes per product of the dense-layer and weight-gradient kernels: 3 = 3xTF32

@@ -138,10 +138,88 @@ def _event_dim(flow):
     return d
 
 
+_U64 = (1 << 64) - 1
+
+
+class DeviceGenerator:
+    """Seed and offset of the on-device N(0, I) draw of sample_and_log_prob, kept in device memory so that the call can
+    be captured in a CUDA graph.
+
+    The state is an int64 [4] CUDA tensor {seed, offset, ticket, reserved} (include/nfb200.h, "device-resident generator
+    state").  The kernel that draws reads the key (seed, offset) there and moves the offset on by 4 in the same launch,
+    so every graph replay draws new samples, and manual_seed makes the replays reproducible.  A DeviceGenerator at
+    (s, o) draws the same bits as a torch.Generator with seed s at offset o.  seed=None takes the initial_seed() of
+    torch's default CUDA generator of `device`, so torch.manual_seed(s); DeviceGenerator() starts at (s, 0).
+
+    The state is stream-ordered: use one generator from one stream at a time.  manual_seed, get_offset and set_offset
+    copy between host and device and raise RuntimeError under stream capture; initial_seed reads a host copy."""
+
+    def __init__(self, device=None, seed=None):
+        device = torch.device(device if device is not None else "cuda")
+        if device.type != "cuda":
+            raise RuntimeError(f"DeviceGenerator keeps its state in CUDA memory; got device {device}")
+        torch.cuda.init()
+        if device.index is None:
+            device = torch.device("cuda", torch.cuda.current_device())
+        self._device = device
+        if seed is None:
+            seed = torch.cuda.default_generators[device.index].initial_seed()
+        self._state = torch.zeros(4, dtype=torch.int64, device=device)
+        self.manual_seed(seed)
+
+    @property
+    def device(self):
+        return self._device
+
+    @staticmethod
+    def _no_capture(what):
+        if torch.cuda.is_current_stream_capturing():
+            raise RuntimeError(f"DeviceGenerator.{what} copies between host and device and cannot run under CUDA-graph "
+                               "capture; call it before capturing or between replays")
+
+    @staticmethod
+    def _i64(v):
+        v = int(v) & _U64
+        return v - (1 << 64) if v >= (1 << 63) else v
+
+    def _write(self, words):
+        with torch.cuda.device(self._device):
+            self._state.copy_(torch.tensor([self._i64(w) for w in words], dtype=torch.int64))
+
+    def manual_seed(self, seed):
+        """State (seed, 0, 0, 0); returns self, like torch.Generator.manual_seed."""
+        self._no_capture("manual_seed")
+        self._seed = int(seed) & _U64
+        self._write((self._seed, 0, 0, 0))
+        return self
+
+    def initial_seed(self):
+        return self._seed
+
+    def get_offset(self):
+        """The offset of the next draw (waits for the draws queued on the current stream)."""
+        self._no_capture("get_offset")
+        with torch.cuda.device(self._device):
+            return int(self._state[1].item()) & _U64
+
+    def set_offset(self, offset):
+        offset = int(offset)
+        if offset < 0 or offset % 4:
+            raise ValueError(f"the offset must be a non-negative multiple of 4, got {offset}")
+        self._no_capture("set_offset")
+        self._write((self._seed, offset, 0, 0))
+
+    def __repr__(self):
+        return f"DeviceGenerator(device={self._device}, seed={self._seed})"
+
+
 def _draw_state(generator, device):
-    """(seed, offset) of one N(0, I) draw: the torch CUDA generator's seed and Philox offset, after which the offset
+    """Key of one N(0, I) draw.  A DeviceGenerator: its state tensor, which the drawing kernel reads and advances
+    (capturable).  Otherwise (seed, offset): the torch CUDA generator's seed and Philox offset, after which the offset
     moves on by 4 (torch keeps offsets a multiple of 4) -- torch.manual_seed makes a call reproducible, and consecutive
     calls draw new samples."""
+    if isinstance(generator, DeviceGenerator):
+        return generator._state
     if torch.cuda.is_current_stream_capturing():
         raise RuntimeError("sample_and_log_prob cannot be captured in a CUDA graph: the seed and offset of the draw are "
                            "read on the host, so every replay would repeat the same samples")
@@ -159,11 +237,13 @@ def flow_sample_and_log_prob(flow, num_samples, base_dist=None, device=None, gen
     as in Flow.log_prob), without materialising z where the route allows it.
 
     A standard-normal base (None, or any base is_std_normal accepts) is drawn on the device from the counter-based
-    stream of csrc/nf_rng.cuh, seeded from `generator` (default: torch's default CUDA generator of `device`); float64
+    stream of csrc/nf_rng.cuh, seeded from `generator` (default: torch's default CUDA generator of `device`; a
+    DeviceGenerator keeps seed and offset in device memory, which makes the call capturable in a CUDA graph); float64
     models widen its float32 normals.  A fused stack draws inside its one launch and evaluates log N(z) - log_det in the
     last layer's epilogue (`_sample_fused`); every other route draws z with nf_std_normal_draw, runs forward(z) -- with
     its autograd graph when parameters require grad, the reparameterised gradient -- and the log-q head kernel.  Any
-    other base is sampled by torch (rsample where it has one) and cannot take a generator."""
+    other base is sampled by torch (rsample where it has one) and cannot take a generator.  Every route draws once, so a
+    DeviceGenerator moves on by exactly 4 per call (a fused stack that refuses the call launches nothing)."""
     p = next(flow.parameters(), None)
     device = torch.device(device if device is not None else (p.device if p is not None else "cpu"))
     dtype = p.dtype if p is not None else torch.float32
@@ -178,16 +258,20 @@ def flow_sample_and_log_prob(flow, num_samples, base_dist=None, device=None, gen
         if log_p_z.dim() > 1:
             log_p_z = log_p_z.sum(dim=1)
         return x, log_p_z - log_det
+    if device.type == "cuda" and device.index is None:
+        device = torch.device("cuda", torch.cuda.current_device())
+    if isinstance(generator, DeviceGenerator) and generator.device != device:
+        raise ValueError(f"the DeviceGenerator lives on {generator.device} but the draw is on {device}")
     if device.type != "cuda":
         raise RuntimeError(L.NO_CPU_PATH)
     with torch.cuda.device(device):
-        seed, offset = _draw_state(generator, device)
+        draw = _draw_state(generator, device)
         fused = getattr(flow, "_sample_fused", None)
         if fused is not None and not wants_grad(flow):
-            out = fused(torch.empty((n, D), dtype=dtype, device=device), (seed, offset))
+            out = fused(torch.empty((n, D), dtype=dtype, device=device), draw)
             if out is not None:
                 return out
-        z = ops.std_normal_draw(seed, offset, n, D, dtype, device)
+        z = ops.std_normal_draw(*ops._draw_key(draw), n, D, dtype, device)
         x, log_det = flow.forward(z)
         return x, ops.std_normal_log_q(z, log_det)
 
@@ -738,7 +822,11 @@ class InverseAutoregressiveFlow(_AffineAutoregressive):
         f = self.conditioner.folded()
         if f is None or f.w[0].dtype != x.dtype:
             return None
-        return ops.made_chain_bf16(x, f, self._mode_parallel, draw=draw)
+        out = ops.made_chain_bf16(x, f, self._mode_parallel, draw=draw)
+        if isinstance(out, torch.Tensor):      # the chain refused after the draw: go on with that z, never draw twice
+            y, log_det = self.forward(out)
+            return y, ops.std_normal_log_q(out, log_det)
+        return out
 
 
 class ARQS(Flow):

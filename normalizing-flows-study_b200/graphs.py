@@ -9,6 +9,16 @@ because replays reuse the same addresses.
     step = GraphedTrainStep(model, optimizer, loss_fn, example_x)     # optimizer built with capturable=True
     for x in loader:
         loss = step(x)            # copies x into the static input, replays, returns the static loss tensor
+
+Reverse-KL / variational training draws its own samples: with a DeviceGenerator the draw reads and advances its seed
+and offset in device memory, so every replay takes fresh samples (and generator.manual_seed makes the replays
+reproducible); the example input is then only a placeholder.
+
+    g = nfb200.DeviceGenerator()
+    def loss_fn(m, _):
+        x, lq = m.sample_and_log_prob(n, generator=g)
+        return (lq - target_log_prob(x)).mean()
+    step = GraphedTrainStep(model, optimizer, loss_fn, torch.empty(1, device="cuda"))
 """
 from __future__ import annotations
 

@@ -686,10 +686,20 @@ def std_normal_log_prob(z, log_det=None):
 
 def std_normal_draw(seed, offset, B, D, dtype, device):
     """z [B, D] ~ N(0, I) from the counter-based stream of csrc/nf_rng.cuh at (seed, offset): the same bits as the
-    in-kernel draw of the fused stacks.  float64 widens the float32 normals."""
+    in-kernel draw of the fused stacks.  float64 widens the float32 normals.
+    seed may instead be the int64 [4] state tensor of a DeviceGenerator (offset None): the kernel reads the key from it
+    and advances it by 4 in the same launch (nf_std_normal_draw_state), so the call can be captured in a CUDA graph."""
     z = torch.empty((B, D), dtype=dtype, device=device)
-    call("nf_std_normal_draw", seed, offset, ptr(z), B, D, L.dtype_code(z), stream())
+    if isinstance(seed, torch.Tensor):
+        call("nf_std_normal_draw_state", ptr(seed), ptr(z), B, D, L.dtype_code(z), stream())
+    else:
+        call("nf_std_normal_draw", seed, offset, ptr(z), B, D, L.dtype_code(z), stream())
     return z
+
+
+def _draw_key(draw):
+    """The (seed, offset) argument pair of std_normal_draw for a `draw`: a host key (seed, offset) or a state tensor."""
+    return (draw, None) if isinstance(draw, torch.Tensor) else draw
 
 
 class _StdNormalLogQFn(Function):
@@ -735,11 +745,15 @@ def _stack_flags(inverse, head):
 def _stack(name, packed, hdr_host, x, inverse, head, sample, mode=()):
     """One fused-stack launch; returns None if the configuration is unsupported.  sample=(seed, offset): the `_sample`
     entry point instead -- x is the output buffer of the rows, drawn from N(0, I) in the kernel and run forward, and the
-    per-row output is log N(z) - log_det (sample_and_log_prob)."""
+    per-row output is log N(z) - log_det (sample_and_log_prob).  sample=<DeviceGenerator state tensor>: `_sample_state`,
+    the same draw with the key read from, and advanced in, device memory (a refused call leaves the state as it was)."""
     x = _c(x)
     B = x.shape[0]
     ld = torch.empty(B, dtype=x.dtype, device=x.device)
     hdr, nbytes = hdr_host.ctypes.data, packed.numel() * 4
+    if isinstance(sample, torch.Tensor):
+        ok = L.try_call(name + "_sample_state", ptr(packed), hdr, nbytes, *mode, ptr(sample), ptr(x), ptr(ld), B, stream())
+        return (x, ld) if ok else None
     if sample is not None:
         ok = L.try_call(name + "_sample", ptr(packed), hdr, nbytes, *mode, sample[0], sample[1], ptr(x), ptr(ld), B,
                         stream())
@@ -781,8 +795,10 @@ def made_chain_bf16(v, folded, mode, head=False, draw=None):
     """Whole parallel direction in ONE launch on bf16 tensor cores (csrc/made_chain_bf16.cu); None when the shape is
     outside the kernel's envelope (data_dim <= 64 and a multiple of 4, hidden_dim a multiple of 128 and <= 512).
     head=True: returns (None, log N(z;0,I) + log_det) without storing z.
-    draw=(seed, offset) (IAF.forward): v only gives the shape; the input is the N(0, I) draw at (seed, offset), made by
-    nf_std_normal_draw once the shape is known to fit, and the result is (x, log N(z) - log_det)."""
+    draw=(seed, offset) or a DeviceGenerator state tensor (IAF.forward): v only gives the shape; the input is the N(0, I)
+    draw of std_normal_draw, made once the shape is known to fit, and the result is (x, log N(z) - log_det).  Should the
+    chain refuse after the draw, the drawn z [B, D] is returned instead of None: the caller must go on with that z, since
+    drawing again would advance a device-resident state a second time."""
     from . import packing
     if v.dtype != torch.float32:
         return None
@@ -794,7 +810,7 @@ def made_chain_bf16(v, folded, mode, head=False, draw=None):
     B, D = v.shape
     flags = (STACK_LOG_PROB_HEAD | STACK_SKIP_Y) if head else 0
     if draw is not None:
-        v = std_normal_draw(draw[0], draw[1], B, D, v.dtype, v.device)
+        v = std_normal_draw(*_draw_key(draw), B, D, v.dtype, v.device)
         flags = STACK_SAMPLE_LOG_Q
     v = _c(v)
     out = None if head else torch.empty_like(v)
@@ -802,7 +818,9 @@ def made_chain_bf16(v, folded, mode, head=False, draw=None):
     ok = L.try_call("nf_made_chain_bf16_forward", ptr(v), ptr(pk.w[0]), ptr(pk.w[1]), ptr(pk.w[2]), ptr(pk.w[3]),
                     ptr(pk.b[0]), ptr(pk.b[1]), ptr(pk.b[2]), ptr(pk.b[3]), pk.kext16_host.ctypes.data, ptr(out), ptr(ld),
                     B, D, folded.H, mode, flags, stream())
-    return (out, ld) if ok else None
+    if ok:
+        return out, ld
+    return v if draw is not None else None
 
 
 def made_params_tc(v, folded):

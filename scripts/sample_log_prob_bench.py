@@ -1,12 +1,16 @@
 """Three ways to get samples and their log-density (x, log_q) from a flow, timed on the GPU:
   (a) model.sample_and_log_prob(n)                                   N(0, I) drawn on the device, fused where possible;
   (b) z = torch.randn; x, ld = model(z); base.log_prob(z).sum(1) - ld     the torch composition;
-  (c) x = model.sample(n); model.log_prob(x)                           both directions.
+  (c) x = model.sample(n); model.log_prob(x)                           both directions;
+  (d) model.sample_and_log_prob(n, generator=nfb200.DeviceGenerator())  (a) with the key read from and advanced in
+                                                                         device memory (the CUDA-graph-safe draw).
+(d) is timed in rounds alternated with (a) ("round" field), so that the difference can be read against the run-to-run
+spread of (a) itself.
 Per way: median / min / max ms per call over 7 timed regions of CUDA events (warmed up; the L2 cache is overwritten with
 a 256 MB buffer before each region, outside the timed window, since the outputs of a 2^20-row call fit in L2) and the
 library launch count of one call.  The card name and power limit are read in the same run.
 
-usage: sample_log_prob_bench.py [--out FILE.jsonl] [--regions 7] [--quick]"""
+usage: sample_log_prob_bench.py [--out FILE.jsonl] [--regions 7] [--rounds 3] [--quick]"""
 import argparse
 import json
 import math
@@ -23,6 +27,7 @@ import nfb200 as N
 ap = argparse.ArgumentParser()
 ap.add_argument("--out", default=None)
 ap.add_argument("--regions", type=int, default=7)
+ap.add_argument("--rounds", type=int, default=3, help="alternated (a) / (d) rounds per configuration")
 ap.add_argument("--quick", action="store_true", help="small sizes only (a rehearsal of the script, not a measurement)")
 a = ap.parse_args()
 if not torch.cuda.is_available():
@@ -115,9 +120,18 @@ def main():
                 x = model.sample(n, device=DEV)
                 return x, model.log_prob(x)
 
-            for way, fn in (("a", way_a), ("b", way_b), ("c", way_c)):
+            gen = N.DeviceGenerator(DEV)
+
+            def way_d():
+                return model.sample_and_log_prob(n, generator=gen)
+
+            timed = [(None, "a", way_a), (None, "b", way_b), (None, "c", way_c)]
+            timed += [(r, w, f) for r in range(a.rounds) for w, f in (("a", way_a), ("d", way_d))]
+            for rnd, way, fn in timed:
                 rec = dict(kind="timing", config=name, precision=prec, n=n, way=way, **time_way(fn),
                            gpu=info["gpu"], nvidia_smi=info["nvidia_smi"])
+                if rnd is not None:
+                    rec["round"] = rnd
                 lines.append(rec)
                 print(json.dumps(rec), flush=True)
     N.set_gemm_precision("fp32")

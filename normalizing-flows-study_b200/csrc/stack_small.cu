@@ -21,11 +21,6 @@ namespace nf {
 
 constexpr int kStackThreads = 128;
 
-struct StackHdr {
-    int D, H, HP, K, L, W1S, NO, layer_stride, bn_between;
-    float bound, min_w, min_h, min_d, scale_w, scale_h;
-};
-
 __device__ __forceinline__ StackHdr read_hdr(const float* __restrict__ p) {
     const int* q = reinterpret_cast<const int*>(p);
     StackHdr h;
@@ -384,33 +379,118 @@ coupling_stack_kernel(const float* __restrict__ packed, const float* __restrict_
 // ------------------------------------------------------------------------------------------------
 // host
 // ------------------------------------------------------------------------------------------------
+#define NF_REQ(p) do { if ((p) == nullptr) return NF_ERR_NULL; } while (0)
+
+// The checks every family shares, in this order, then the family's launcher.  The header lives in device memory; the
+// caller passes a host copy of its 16 words beside it (cheap, and keeps the library free of hidden device->host syncs).
+static int run_stack(const StackFamily& f, const StackCall& c) {
+    if (c.B < 0 || (c.sample && c.B > (int64_t)0xFFFFFFFFLL)) return NF_ERR_BAD_SHAPE;
+    NF_REQ(c.hdr_host);
+    if (c.B == 0) return c.rng_state ? nf_rng_state_advance(c.rng_state, c.st) : NF_OK;
+    NF_REQ(c.packed); NF_REQ(c.ld);
+    if (!c.sample) NF_REQ(c.x);
+    if (!(c.flags & NF_STACK_SKIP_Y)) NF_REQ(c.y);
+    if (!aligned16(c.packed)) return NF_ERR_MISALIGNED;
+    const StackHdr h = nf_stack_hdr(c.hdr_host);
+    if (h.magic != f.magic) return NF_ERR_BAD_SHAPE;
+    return f.launch(c, h);
+}
+
+int stack_forward(const StackFamily& f, const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
+                  void* y, void* ld, int64_t B, int flags, int mode, nf_stream_t stream) {
+    return run_stack(f, {packed, hdr_host, packed_bytes, x, y, ld, B, flags, mode, false, 0, 0, nullptr,
+                         (cudaStream_t)stream});
+}
+
+int stack_sample(const StackFamily& f, const void* packed, const void* hdr_host, int64_t packed_bytes, int mode,
+                 uint64_t seed, uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream) {
+    return run_stack(f, {packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, mode, true, seed,
+                         offset, nullptr, (cudaStream_t)stream});
+}
+
+int stack_sample_state(const StackFamily& f, const void* packed, const void* hdr_host, int64_t packed_bytes, int mode,
+                       void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream) {
+    const int rc = nf_rng_state_check(rng_state);
+    if (rc != NF_OK) return rc;
+    return run_stack(f, {packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, mode, true, 0, 0,
+                         (unsigned long long*)rng_state, (cudaStream_t)stream});
+}
+
 template <typename Kern>
-static int launch_stack(Kern kern, size_t smem_bytes, int rows_per_cta, const void* packed, const void* x, void* y,
-                        void* ld, int64_t B, int inverse, int extra, bool has_extra, bool sample, uint64_t seed,
-                        uint64_t offset, unsigned long long* rng_state, cudaStream_t st) {
+static int launch_stack(Kern kern, size_t smem_bytes, int rows_per_cta, const StackCall& c, int extra, bool has_extra) {
     // the SAMPLE twins hold the 16-byte key of nf_rng_state_take in static shared memory
-    if (smem_bytes + (sample ? 16 : 0) > 227 * 1024) return NF_ERR_UNSUPPORTED;
-    NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_bytes));
-    NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    if (smem_bytes + (c.sample ? 16 : 0) > 227 * 1024) return NF_ERR_UNSUPPORTED;
+    const int rc = stack_smem_attributes(kern, smem_bytes);
+    if (rc != NF_OK) return rc;
     int per_sm = 0;
     NF_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, kStackThreads, smem_bytes));
     if (per_sm < 1) return NF_ERR_UNSUPPORTED;
-    const int64_t ntiles = cdiv(B, rows_per_cta);
+    const int64_t ntiles = cdiv(c.B, rows_per_cta);
     const int64_t cap = (int64_t)kNumSMs * per_sm;
     const int grid = (int)(ntiles < cap ? ntiles : cap);
-    void* args_s[] = {(void*)&packed, (void*)&x, (void*)&y, (void*)&ld, (void*)&B, (void*)&inverse, (void*)&extra,
-                      (void*)&seed, (void*)&offset, (void*)&rng_state};
-    void* args_n[] = {(void*)&packed, (void*)&x, (void*)&y, (void*)&ld, (void*)&B, (void*)&inverse, (void*)&seed,
-                      (void*)&offset, (void*)&rng_state};
-    NF_CUDA(cudaLaunchKernel((const void*)kern, dim3(grid), dim3(kStackThreads), has_extra ? args_s : args_n, smem_bytes, st));
+    void* args_s[] = {(void*)&c.packed, (void*)&c.x, (void*)&c.y, (void*)&c.ld, (void*)&c.B, (void*)&c.flags, (void*)&extra,
+                      (void*)&c.seed, (void*)&c.offset, (void*)&c.rng_state};
+    void* args_n[] = {(void*)&c.packed, (void*)&c.x, (void*)&c.y, (void*)&c.ld, (void*)&c.B, (void*)&c.flags,
+                      (void*)&c.seed, (void*)&c.offset, (void*)&c.rng_state};
+    NF_CUDA(cudaLaunchKernel((const void*)kern, dim3(grid), dim3(kStackThreads), has_extra ? args_s : args_n, smem_bytes,
+                             c.st));
     count_launch();
     return NF_OK;
 }
 
+// the FP32-pipe layouts' header checks after the magic
+static int check_hdr(const StackHdr& h) {
+    if (h.D < 1 || h.D > NF_STACK_DMAX || h.L < 1) return NF_ERR_BAD_SHAPE;
+    if (h.HP != 64 && h.HP != 128) return NF_ERR_BAD_SHAPE;
+    if (h.layer_stride % 4 != 0) return NF_ERR_MISALIGNED;
+    return NF_OK;
+}
+
+static int spline_stack_launch(const StackCall& c, const StackHdr& h) {
+    const int rc = check_hdr(h);
+    if (rc != NF_OK) return rc;
+    const int D = h.D, HP = h.HP, K = h.K, NO = h.NO, stride = h.layer_stride;
+    if (K < 2 || K > 16 || NO % 4 != 0) return NF_ERR_BAD_SHAPE;
+    if (!c.holds(NF_STACK_HDR + (int64_t)h.L * stride)) return NF_ERR_WORKSPACE;
+    const int R = (HP == 64) ? 2 : 1;
+    const int rows = kStackThreads * R;
+    const size_t smem = sizeof(float) * ((size_t)stride + (size_t)NO * rows);
+#define NF_SS(HPv, Rv, DMv, KMv)                                                                                     \
+    return launch_stack(c.sample ? spline_stack_kernel<HPv, Rv, DMv, KMv, true> : spline_stack_kernel<HPv, Rv, DMv, KMv>, \
+                        smem, rows, c, stride, true)
+    if (HP == 64) {
+        if (D <= 3) { if (K <= 8) NF_SS(64, 2, 4, 8); else NF_SS(64, 2, 4, 16); }
+        else        { if (K <= 8) NF_SS(64, 2, 8, 8); else NF_SS(64, 2, 8, 16); }
+    } else {
+        if (D <= 3) { if (K <= 8) NF_SS(128, 1, 4, 8); else NF_SS(128, 1, 4, 16); }
+        else        { if (K <= 8) NF_SS(128, 1, 8, 8); else NF_SS(128, 1, 8, 16); }
+    }
+#undef NF_SS
+}
+
+static int coupling_stack_launch(const StackCall& c, const StackHdr& h) {
+    const int rc = check_hdr(h);
+    if (rc != NF_OK) return rc;
+    const int D = h.D, HP = h.HP, stride = h.layer_stride;
+    if (h.NO != (D <= 3 ? 4 : 8)) return NF_ERR_BAD_SHAPE;
+    if (!c.holds(NF_STACK_HDR + (int64_t)h.L * stride)) return NF_ERR_WORKSPACE;
+    const int R = (HP == 64) ? 2 : 1;
+    const int rows = kStackThreads * R;
+    const size_t smem = sizeof(float) * (size_t)stride;
+#define NF_CS(HPv, Rv, DMv)                                                                                          \
+    return launch_stack(c.sample ? coupling_stack_kernel<HPv, Rv, DMv, true> : coupling_stack_kernel<HPv, Rv, DMv>,   \
+                        smem, rows, c, 0, false)
+    if (HP == 64) { if (D <= 3) NF_CS(64, 2, 4); else NF_CS(64, 2, 8); }
+    else          { if (D <= 3) NF_CS(128, 1, 4); else NF_CS(128, 1, 8); }
+#undef NF_CS
+}
+
+static const StackFamily kSpline = {NF_STACK_MAGIC_SPLINE, spline_stack_launch};
+static const StackFamily kCoupling = {NF_STACK_MAGIC_AFFINE, coupling_stack_launch};
+
 }  // namespace nf
 
 using namespace nf;
-#define NF_REQ(p) do { if ((p) == nullptr) return NF_ERR_NULL; } while (0)
 
 extern "C" int64_t nf_spline_stack_packed_floats(int D, int H, int K, int L) {
     if (D < 1 || D > NF_STACK_DMAX || H < 1 || H > 128 || K < 2 || K > 16 || L < 1) return -1;
@@ -425,113 +505,33 @@ extern "C" int64_t nf_coupling_stack_packed_floats(int D, int H, int L) {
     return NF_STACK_HDR + (int64_t)L * (NF_LAYER_HDR + 2 * nf_stack_net_words(HP, W1S, NO));
 }
 
-// The header lives in device memory; the host side passes a host copy of the 16 header words in front of the
-// call (cheap, and keeps the library free of hidden device->host syncs): see nf_*_stack_forward's `hdr_host`.
-static int check_hdr(const int32_t* h, int magic) {
-    if (h[0] != magic) return NF_ERR_BAD_SHAPE;
-    if (h[1] < 1 || h[1] > NF_STACK_DMAX || h[5] < 1) return NF_ERR_BAD_SHAPE;
-    if (h[3] != 64 && h[3] != 128) return NF_ERR_BAD_SHAPE;
-    if (h[8] % 4 != 0) return NF_ERR_MISALIGNED;
-    return NF_OK;
-}
-
-// sample: the SAMPLE kernel draws the rows from (seed, offset); x is not read
-static int spline_stack_launch(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x, void* y,
-                               void* ld, int64_t B, int inverse, bool sample, uint64_t seed, uint64_t offset,
-                               unsigned long long* rng_state, nf_stream_t stream) {
-    if (B < 0 || (sample && B > (int64_t)0xFFFFFFFFLL)) return NF_ERR_BAD_SHAPE;
-    NF_REQ(hdr_host);
-    if (B == 0) return rng_state ? nf_rng_state_advance(rng_state, (cudaStream_t)stream) : NF_OK;
-    NF_REQ(packed); NF_REQ(ld);
-    if (!sample) NF_REQ(x);
-    if (!(inverse & NF_STACK_SKIP_Y)) NF_REQ(y);
-    if (!aligned16(packed)) return NF_ERR_MISALIGNED;
-    const int32_t* h = (const int32_t*)hdr_host;
-    int rc = check_hdr(h, NF_STACK_MAGIC_SPLINE);
-    if (rc != NF_OK) return rc;
-    const int D = h[1], HP = h[3], K = h[4], L = h[5], NO = h[7], stride = h[8];
-    if (K < 2 || K > 16 || NO % 4 != 0) return NF_ERR_BAD_SHAPE;
-    if (packed_bytes < (int64_t)sizeof(float) * (NF_STACK_HDR + (int64_t)L * stride)) return NF_ERR_WORKSPACE;
-    cudaStream_t st = (cudaStream_t)stream;
-    const int R = (HP == 64) ? 2 : 1;
-    const int rows = kStackThreads * R;
-    const size_t smem = sizeof(float) * ((size_t)stride + (size_t)NO * rows);
-#define NF_SS(HPv, Rv, DMv, KMv)                                                                                     \
-    return launch_stack(sample ? spline_stack_kernel<HPv, Rv, DMv, KMv, true> : spline_stack_kernel<HPv, Rv, DMv, KMv>,   \
-                        smem, rows, packed, x, y, ld, B, inverse, stride, true, sample, seed, offset, rng_state, st)
-    if (HP == 64) {
-        if (D <= 3) { if (K <= 8) NF_SS(64, 2, 4, 8); else NF_SS(64, 2, 4, 16); }
-        else        { if (K <= 8) NF_SS(64, 2, 8, 8); else NF_SS(64, 2, 8, 16); }
-    } else {
-        if (D <= 3) { if (K <= 8) NF_SS(128, 1, 4, 8); else NF_SS(128, 1, 4, 16); }
-        else        { if (K <= 8) NF_SS(128, 1, 8, 8); else NF_SS(128, 1, 8, 16); }
-    }
-#undef NF_SS
-}
-
 extern "C" int nf_spline_stack_forward(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
                                        void* y, void* ld, int64_t B, int inverse, nf_stream_t stream) {
-    return spline_stack_launch(packed, hdr_host, packed_bytes, x, y, ld, B, inverse, false, 0, 0, nullptr, stream);
+    return stack_forward(kSpline, packed, hdr_host, packed_bytes, x, y, ld, B, inverse, 0, stream);
 }
 
 extern "C" int nf_spline_stack_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, uint64_t seed,
                                       uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream) {
-    return spline_stack_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true, seed,
-                               offset, nullptr, stream);
+    return stack_sample(kSpline, packed, hdr_host, packed_bytes, 0, seed, offset, x, log_q, B, stream);
 }
 
 extern "C" int nf_spline_stack_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes,
                                             void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream) {
-    const int rc = nf_rng_state_check(rng_state);
-    if (rc != NF_OK) return rc;
-    return spline_stack_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true, 0, 0,
-                               (unsigned long long*)rng_state, stream);
-}
-
-static int coupling_stack_launch(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x, void* y,
-                                 void* ld, int64_t B, int inverse, bool sample, uint64_t seed, uint64_t offset,
-                                 unsigned long long* rng_state, nf_stream_t stream) {
-    if (B < 0 || (sample && B > (int64_t)0xFFFFFFFFLL)) return NF_ERR_BAD_SHAPE;
-    NF_REQ(hdr_host);
-    if (B == 0) return rng_state ? nf_rng_state_advance(rng_state, (cudaStream_t)stream) : NF_OK;
-    NF_REQ(packed); NF_REQ(ld);
-    if (!sample) NF_REQ(x);
-    if (!(inverse & NF_STACK_SKIP_Y)) NF_REQ(y);
-    if (!aligned16(packed)) return NF_ERR_MISALIGNED;
-    const int32_t* h = (const int32_t*)hdr_host;
-    int rc = check_hdr(h, NF_STACK_MAGIC_AFFINE);
-    if (rc != NF_OK) return rc;
-    const int D = h[1], HP = h[3], L = h[5], NO = h[7], stride = h[8];
-    if (NO != (D <= 3 ? 4 : 8)) return NF_ERR_BAD_SHAPE;
-    if (packed_bytes < (int64_t)sizeof(float) * (NF_STACK_HDR + (int64_t)L * stride)) return NF_ERR_WORKSPACE;
-    cudaStream_t st = (cudaStream_t)stream;
-    const int R = (HP == 64) ? 2 : 1;
-    const int rows = kStackThreads * R;
-    const size_t smem = sizeof(float) * (size_t)stride;
-#define NF_CS(HPv, Rv, DMv)                                                                                          \
-    return launch_stack(sample ? coupling_stack_kernel<HPv, Rv, DMv, true> : coupling_stack_kernel<HPv, Rv, DMv>, smem, \
-                        rows, packed, x, y, ld, B, inverse, 0, false, sample, seed, offset, rng_state, st)
-    if (HP == 64) { if (D <= 3) NF_CS(64, 2, 4); else NF_CS(64, 2, 8); }
-    else          { if (D <= 3) NF_CS(128, 1, 4); else NF_CS(128, 1, 8); }
-#undef NF_CS
+    return stack_sample_state(kSpline, packed, hdr_host, packed_bytes, 0, rng_state, x, log_q, B, stream);
 }
 
 extern "C" int nf_coupling_stack_forward(const void* packed, const void* hdr_host, int64_t packed_bytes,
                                          const void* x, void* y, void* ld, int64_t B, int inverse,
                                          nf_stream_t stream) {
-    return coupling_stack_launch(packed, hdr_host, packed_bytes, x, y, ld, B, inverse, false, 0, 0, nullptr, stream);
+    return stack_forward(kCoupling, packed, hdr_host, packed_bytes, x, y, ld, B, inverse, 0, stream);
 }
 
 extern "C" int nf_coupling_stack_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, uint64_t seed,
                                         uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream) {
-    return coupling_stack_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true, seed,
-                                 offset, nullptr, stream);
+    return stack_sample(kCoupling, packed, hdr_host, packed_bytes, 0, seed, offset, x, log_q, B, stream);
 }
 
 extern "C" int nf_coupling_stack_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes,
                                               void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream) {
-    const int rc = nf_rng_state_check(rng_state);
-    if (rc != NF_OK) return rc;
-    return coupling_stack_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true, 0, 0,
-                                 (unsigned long long*)rng_state, stream);
+    return stack_sample_state(kCoupling, packed, hdr_host, packed_bytes, 0, rng_state, x, log_q, B, stream);
 }

@@ -4,8 +4,9 @@
 //
 // All words are 32-bit; integers are stored as int32 bit patterns inside the float buffer.
 //
-//   header (NF_STACK_HDR words):
-//     [0] magic   [1] D   [2] H (true hidden_dim)   [3] HP (padded: 64 or 128)   [4] K (spline) / 0 (affine)
+//   header (NF_STACK_HDR words, read on the host through StackHdr below):
+//     [0] magic   [1] D   [2] H (true hidden_dim)   [3] HP (padded: 64 or 128; the tcgen05 layouts of stack_tc.cu
+//     store the number of conditioner nets per layer here instead: 1 spline / MADE, 2 affine)   [4] K (spline) / 0 (affine)
 //     [5] L       [6] W1S (words per hidden unit in W1k: 4 if D<=3 else 12)      [7] NO (padded #outputs of the head)
 //     [8] layer_stride (words)   [9] bn_between (0/1)   [10] bound   [11] min_w  [12] min_h  [13] min_d
 //     [14] scale_w = 1-min_w*K   [15] scale_h
@@ -21,6 +22,8 @@
 //   spline head outputs are ordered t*P + p for transformed dim t (P = 3K-1); affine head outputs are d.
 #pragma once
 #include <stdint.h>
+#include <string.h>
+#include "nf_common.cuh"
 
 #define NF_STACK_MAGIC_SPLINE 0x4e465331  /* 'NFS1' */
 #define NF_STACK_MAGIC_AFFINE 0x4e464131  /* 'NFA1' */
@@ -42,6 +45,20 @@
 #define NF_STACK_SKIP_Y 4
 #define NF_STACK_SAMPLE_LOG_Q 8
 
+// the 16 header words; HP is word 3 (nets per layer in the tcgen05 layouts)
+struct StackHdr {
+    int magic, D, H, HP, K, L, W1S, NO, layer_stride, bn_between;
+    float bound, min_w, min_h, min_d, scale_w, scale_h;
+};
+static_assert(sizeof(StackHdr) == 4 * NF_STACK_HDR, "StackHdr mirrors the 16 header words");
+
+// host copy of the header that the caller passes beside the device buffer (hdr_host of the entry points)
+static inline StackHdr nf_stack_hdr(const void* hdr_host) {
+    StackHdr h;
+    memcpy(&h, hdr_host, sizeof(int32_t) * NF_STACK_HDR);
+    return h;
+}
+
 static inline int nf_stack_hp(int H) { return H <= 64 ? 64 : 128; }
 static inline int nf_stack_w1s(int D) { return D <= 3 ? 4 : 12; }
 static inline int64_t nf_stack_net_words(int HP, int W1S, int NO) {
@@ -49,6 +66,43 @@ static inline int64_t nf_stack_net_words(int HP, int W1S, int NO) {
 }
 
 #ifdef __CUDACC__
+namespace nf {
+
+// One call of a fused-stack entry point.  sample: the SAMPLE kernel draws the rows from (seed, offset), or from the
+// device-resident state when rng_state is not NULL; x is not read.  mode: MADE only.
+struct StackCall {
+    const void* packed; const void* hdr_host; int64_t packed_bytes;
+    const void* x; void* y; void* ld; int64_t B; int flags; int mode;
+    bool sample; uint64_t seed, offset; unsigned long long* rng_state; cudaStream_t st;
+    bool holds(int64_t words) const { return packed_bytes >= (int64_t)sizeof(float) * words; }   // packed_bytes suffices
+};
+
+// A family's launcher: its envelope checks, shared-memory sizing and instantiation switch, called with the header
+// after the checks every family shares (stack_small.cu: run_stack).
+struct StackFamily {
+    int magic;
+    int (*launch)(const StackCall& c, const StackHdr& h);
+};
+
+// bodies of the nf_*_forward / nf_*_sample / nf_*_sample_state entry points
+int stack_forward(const StackFamily& f, const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
+                  void* y, void* ld, int64_t B, int flags, int mode, nf_stream_t stream);
+int stack_sample(const StackFamily& f, const void* packed, const void* hdr_host, int64_t packed_bytes, int mode,
+                 uint64_t seed, uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream);
+int stack_sample_state(const StackFamily& f, const void* packed, const void* hdr_host, int64_t packed_bytes, int mode,
+                       void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream);
+
+// dynamic shared memory beyond 48 KB, and the largest shared-memory carveout: with the default preference the driver
+// sizes the SM for ONE CTA of the kernel and a second co-resident CTA never arrives
+template <typename Kern>
+inline int stack_smem_attributes(Kern kern, size_t smem) {
+    NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    return NF_OK;
+}
+
+}  // namespace nf
+
 // log N(z; 0, I) + log_det for one row held in registers (same arithmetic as std_normal_log_prob_fwd_kernel)
 template <int DM>
 __device__ __forceinline__ float nf_stack_row_head(const float (&z)[DM], int D, float log_det) {

@@ -809,55 +809,40 @@ made_stack_tc_kernel(const float* __restrict__ packed, const float* __restrict__
     if (warp == 0) tc::tmem_dealloc(tb, kTmemCols);
 }
 
-}  // namespace nf
-
-using namespace nf;
-#define NF_REQ(p) do { if ((p) == nullptr) return NF_ERR_NULL; } while (0)
-
-extern "C" int64_t nf_spline_stack_tc_block_words(int D, int K, int max_dt) {
-    if (D < 1 || D > NF_STACK_DMAX || K < 2 || K > 10 || max_dt < 1 || max_dt > 2) return -1;
-    const int W1S = nf_stack_w1s(D), NO3 = 32 * max_dt;
-    return NF_LAYER_HDR + blk_offsets(W1S, NO3).net_words;
+// CTAs per SM that shared memory (1 KB reserved per CTA) and the SM's 512 TMEM columns allow, times the SMs; 0: none fits
+static int64_t tc_resident_ctas(size_t smem, int tmem_cols) {
+    int per_sm = (int)((227 * 1024) / (smem + 1024));
+    if (per_sm > 512 / tmem_cols) per_sm = 512 / tmem_cols;
+    return (int64_t)kNumSMs * per_sm;
 }
 
-// sample: the SAMPLE kernel draws the rows from (seed, offset); x is not read
-static int spline_stack_tc_launch(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x, void* y,
-                                  void* ld, int64_t B, int inverse, bool sample, uint64_t seed, uint64_t offset,
-                                  unsigned long long* rng_state, nf_stream_t stream) {
-    if (B < 0 || (sample && B > (int64_t)0xFFFFFFFFLL)) return NF_ERR_BAD_SHAPE;
-    NF_REQ(hdr_host);
-    if (B == 0) return rng_state ? nf_rng_state_advance(rng_state, (cudaStream_t)stream) : NF_OK;
-    NF_REQ(packed); NF_REQ(ld);
-    if (!sample) NF_REQ(x);
-    if (!(inverse & NF_STACK_SKIP_Y)) NF_REQ(y);
-    if (!aligned16(packed)) return NF_ERR_MISALIGNED;
-    const int32_t* h = (const int32_t*)hdr_host;
-    if (h[0] != NF_STACK_MAGIC_SPLINE_TC) return NF_ERR_BAD_SHAPE;
-    const int D = h[1], H = h[2], K = h[4], L = h[5], W1S = h[6], NO3 = h[7], BW = h[8];
-    if (D < 1 || D > NF_STACK_DMAX || H < 1 || H > 64 || L < 1 || K < 2 || K > 10) return NF_ERR_UNSUPPORTED;
+// small batches: fewer sub-tiles per weight staging so that every SM gets rows (4 000 rows on eight 512-row tiles left
+// 140 SMs idle); from kTcSub sub-tiles per resident CTA on, the staging is shared by kTcSub sub-tiles
+static int tc_nsub(int64_t B, int64_t res_ctas) {
+    const int nsub = (int)cdiv(cdiv(B, kTcThreads), res_ctas);
+    return nsub < 1 ? 1 : (nsub > kTcSub ? kTcSub : nsub);
+}
+
+static int spline_stack_tc_launch(const StackCall& c, const StackHdr& h) {
+    const int D = h.D, K = h.K, W1S = h.W1S, NO3 = h.NO, BW = h.layer_stride;
+    if (D < 1 || D > NF_STACK_DMAX || h.H < 1 || h.H > 64 || h.L < 1 || K < 2 || K > 10) return NF_ERR_UNSUPPORTED;
     if (NO3 != 32 && NO3 != 64) return NF_ERR_UNSUPPORTED;
     if (W1S != nf_stack_w1s(D) || BW != NF_LAYER_HDR + blk_offsets(W1S, NO3).net_words) return NF_ERR_BAD_SHAPE;
-    if (packed_bytes < (int64_t)sizeof(float) * (NF_STACK_HDR + (int64_t)L * BW)) return NF_ERR_WORKSPACE;
-    cudaStream_t st = (cudaStream_t)stream;
+    if (!c.holds(NF_STACK_HDR + (int64_t)h.L * BW)) return NF_ERR_WORKSPACE;
     const int DMh = D <= 2 ? 2 : (D <= 3 ? 4 : 8);
-    const size_t smem = sizeof(float) * ((size_t)2 * BW + (size_t)kTcSub * (DMh + 1) * kTcThreads + 12 + (rng_state ? 4 : 0));
+    const size_t smem = sizeof(float) * ((size_t)2 * BW + (size_t)kTcSub * (DMh + 1) * kTcThreads + 12 + (c.rng_state ? 4 : 0));
     if (smem > 227 * 1024) return NF_ERR_UNSUPPORTED;
-    const int rows = kTcThreads * kTcSub;
-    const int64_t ntiles = cdiv(B, rows);
-    int per_sm = (int)((227 * 1024) / (smem + 1024));
-    if (per_sm < 1) return NF_ERR_UNSUPPORTED;
-    if (per_sm > 512 / kTmemCols) per_sm = 512 / kTmemCols;   // TMEM: 512 columns per SM
-    const int64_t cap = (int64_t)kNumSMs * per_sm;
+    const int64_t ntiles = cdiv(c.B, kTcThreads * kTcSub);
+    const int64_t cap = tc_resident_ctas(smem, kTmemCols);
+    if (cap < 1) return NF_ERR_UNSUPPORTED;
     const int grid = (int)(ntiles < cap ? ntiles : cap);
 #define NF_TC(DMv, KMv, KSv)                                                                                         \
     do {                                                                                                             \
-        auto kern = sample ? spline_stack_tc2_kernel<DMv, KMv, KSv, true> : spline_stack_tc2_kernel<DMv, KMv, KSv>; \
-        NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                 \
-        /* ask for the largest shared-memory carveout: with the default preference the driver sizes the SM for ONE   \
-           CTA of this kernel and the second co-resident CTA (the latency hiding of this design) never arrives */    \
-        NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)); \
-        kern<<<grid, kTc2Threads, smem, st>>>((const float*)packed, (const float*)x, (float*)y, (float*)ld, B, inverse, \
-                                              seed, offset, rng_state);                                              \
+        auto kern = c.sample ? spline_stack_tc2_kernel<DMv, KMv, KSv, true> : spline_stack_tc2_kernel<DMv, KMv, KSv>; \
+        const int rc = stack_smem_attributes(kern, smem);                                                            \
+        if (rc != NF_OK) return rc;                                                                                  \
+        kern<<<grid, kTc2Threads, smem, c.st>>>((const float*)c.packed, (const float*)c.x, (float*)c.y, (float*)c.ld, \
+                                                c.B, c.flags, c.seed, c.offset, c.rng_state);                        \
     } while (0)
 #define NF_TC_K(DMv)                                      \
     do {                                                  \
@@ -876,23 +861,94 @@ static int spline_stack_tc_launch(const void* packed, const void* hdr_host, int6
     return NF_OK;
 }
 
+static int coupling_stack_tc_launch(const StackCall& c, const StackHdr& h) {
+    const int D = h.D, H = h.H, W1S = h.W1S, NO3 = h.NO, NBW = h.layer_stride;
+    if (D < 1 || D > NF_STACK_DMAX || H < 1 || H > 128 || h.L < 1 || NO3 != 16) return NF_ERR_UNSUPPORTED;
+    const int HP = H <= 64 ? 64 : 128;
+    if (W1S != nf_stack_w1s(D) || NBW != NF_LAYER_HDR + blk_offsets(W1S, NO3, HP).net_words) return NF_ERR_BAD_SHAPE;
+    if (!c.holds(NF_STACK_HDR + (int64_t)2 * h.L * NBW)) return NF_ERR_WORKSPACE;
+    const int DMh = D <= 2 ? 2 : (D <= 3 ? 4 : 8);
+    const int nbuf = HP == 64 ? 2 : 1, tmem_cols = HP == 64 ? 256 : 512;
+    const size_t smem = sizeof(float) * ((size_t)nbuf * NBW + (size_t)kTcSub * (2 * DMh + 1) * kTcThreads + NF_LAYER_HDR + 8 +
+                                         (c.rng_state ? 4 : 0));
+    if (smem > 227 * 1024) return NF_ERR_UNSUPPORTED;
+    const int nsub = tc_nsub(c.B, kNumSMs * (512 / tmem_cols));
+    const int64_t ntiles = cdiv(c.B, kTcThreads * nsub);
+    const int64_t cap = tc_resident_ctas(smem, tmem_cols);
+    if (cap < 1) return NF_ERR_UNSUPPORTED;
+    const int grid = (int)(ntiles < cap ? ntiles : cap);
+#define NF_CTC(DMv, HPv)                                                                                              \
+    do {                                                                                                             \
+        auto kern = c.sample ? coupling_stack_tc_kernel<DMv, HPv, true> : coupling_stack_tc_kernel<DMv, HPv>;          \
+        const int rc = stack_smem_attributes(kern, smem);                                                            \
+        if (rc != NF_OK) return rc;                                                                                  \
+        kern<<<grid, kTcThreads, smem, c.st>>>((const float*)c.packed, (const float*)c.x, (float*)c.y, (float*)c.ld,  \
+                                               c.B, c.flags, nsub, c.seed, c.offset, c.rng_state);                   \
+    } while (0)
+    if (HP == 64) { if (D <= 2) NF_CTC(2, 64); else if (D <= 3) NF_CTC(4, 64); else NF_CTC(8, 64); }
+    else          { if (D <= 2) NF_CTC(2, 128); else if (D <= 3) NF_CTC(4, 128); else NF_CTC(8, 128); }
+#undef NF_CTC
+    count_launch();
+    NF_LAUNCH_CHECK();
+    return NF_OK;
+}
+
+static int made_stack_tc_launch(const StackCall& c, const StackHdr& h) {
+    const int D = h.D, W1S = h.W1S, NBW = h.layer_stride, mode = c.mode;
+    if (D < 1 || D > NF_STACK_DMAX || h.H < 1 || h.H > 64 || h.L < 1) return NF_ERR_UNSUPPORTED;
+    if (mode < NF_AR_MAF_INVERSE || mode > NF_AR_IAF_INVERSE) return NF_ERR_UNSUPPORTED;
+    if ((mode == NF_AR_MAF_FORWARD || mode == NF_AR_IAF_INVERSE) && D != 2) return NF_ERR_UNSUPPORTED;   // sequential: 2-D only
+    if (W1S != nf_stack_w1s(D) || NBW != NF_LAYER_HDR + made_blk_offsets(W1S).words) return NF_ERR_BAD_SHAPE;
+    if (!c.holds(NF_STACK_HDR + (int64_t)h.L * NBW)) return NF_ERR_WORKSPACE;
+    const int DMh = D <= 2 ? 2 : (D <= 3 ? 4 : 8);
+    const size_t smem = sizeof(float) * ((size_t)NBW + (size_t)kTcSub * (DMh + 1) * kTcThreads + 8 + (c.rng_state ? 4 : 0));
+    if (smem > 113 * 1024) return NF_ERR_UNSUPPORTED;             // two CTAs per SM
+    const int res_ctas = kNumSMs * 2;
+    const int nsub = tc_nsub(c.B, res_ctas);
+    const int64_t ntiles = cdiv(c.B, kTcThreads * nsub);
+    const int grid = (int)(ntiles < res_ctas ? ntiles : res_ctas);
+#define NF_MTC(DMv)                                                                                                  \
+    do {                                                                                                             \
+        auto kern = c.sample ? made_stack_tc_kernel<DMv, true> : made_stack_tc_kernel<DMv>;                          \
+        const int rc = stack_smem_attributes(kern, smem);                                                            \
+        if (rc != NF_OK) return rc;                                                                                  \
+        kern<<<grid, kTcThreads, smem, c.st>>>((const float*)c.packed, (const float*)c.x, (float*)c.y, (float*)c.ld,  \
+                                               c.B, c.flags, nsub, mode, c.seed, c.offset, c.rng_state);             \
+    } while (0)
+    if (D <= 2) NF_MTC(2); else if (D <= 3) NF_MTC(4); else NF_MTC(8);
+#undef NF_MTC
+    count_launch();
+    NF_LAUNCH_CHECK();
+    return NF_OK;
+}
+
+static const StackFamily kSplineTc = {NF_STACK_MAGIC_SPLINE_TC, spline_stack_tc_launch};
+static const StackFamily kCouplingTc = {NF_STACK_MAGIC_AFFINE_TC, coupling_stack_tc_launch};
+static const StackFamily kMadeTc = {NF_STACK_MAGIC_MADE_TC, made_stack_tc_launch};
+
+}  // namespace nf
+
+using namespace nf;
+
+extern "C" int64_t nf_spline_stack_tc_block_words(int D, int K, int max_dt) {
+    if (D < 1 || D > NF_STACK_DMAX || K < 2 || K > 10 || max_dt < 1 || max_dt > 2) return -1;
+    const int W1S = nf_stack_w1s(D), NO3 = 32 * max_dt;
+    return NF_LAYER_HDR + blk_offsets(W1S, NO3).net_words;
+}
+
 extern "C" int nf_spline_stack_tc_forward(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
                                           void* y, void* ld, int64_t B, int inverse, nf_stream_t stream) {
-    return spline_stack_tc_launch(packed, hdr_host, packed_bytes, x, y, ld, B, inverse, false, 0, 0, nullptr, stream);
+    return stack_forward(kSplineTc, packed, hdr_host, packed_bytes, x, y, ld, B, inverse, 0, stream);
 }
 
 extern "C" int nf_spline_stack_tc_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, uint64_t seed,
                                          uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream) {
-    return spline_stack_tc_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true,
-                                  seed, offset, nullptr, stream);
+    return stack_sample(kSplineTc, packed, hdr_host, packed_bytes, 0, seed, offset, x, log_q, B, stream);
 }
 
 extern "C" int nf_spline_stack_tc_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes,
                                                void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream) {
-    const int rc = nf_rng_state_check(rng_state);
-    if (rc != NF_OK) return rc;
-    return spline_stack_tc_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true,
-                                  0, 0, (unsigned long long*)rng_state, stream);
+    return stack_sample_state(kSplineTc, packed, hdr_host, packed_bytes, 0, rng_state, x, log_q, B, stream);
 }
 
 extern "C" int64_t nf_coupling_stack_tc_block_words(int D) {
@@ -904,73 +960,19 @@ extern "C" int64_t nf_coupling_stack_tc_block_words_hidden(int D, int H) {  // h
     return NF_LAYER_HDR + blk_offsets(nf_stack_w1s(D), 16, H <= 64 ? 64 : 128).net_words;
 }
 
-static int coupling_stack_tc_launch(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
-                                    void* y, void* ld, int64_t B, int inverse, bool sample, uint64_t seed, uint64_t offset,
-                                    unsigned long long* rng_state, nf_stream_t stream) {
-    if (B < 0 || (sample && B > (int64_t)0xFFFFFFFFLL)) return NF_ERR_BAD_SHAPE;
-    NF_REQ(hdr_host);
-    if (B == 0) return rng_state ? nf_rng_state_advance(rng_state, (cudaStream_t)stream) : NF_OK;
-    NF_REQ(packed); NF_REQ(ld);
-    if (!sample) NF_REQ(x);
-    if (!(inverse & NF_STACK_SKIP_Y)) NF_REQ(y);
-    if (!aligned16(packed)) return NF_ERR_MISALIGNED;
-    const int32_t* h = (const int32_t*)hdr_host;
-    if (h[0] != NF_STACK_MAGIC_AFFINE_TC) return NF_ERR_BAD_SHAPE;
-    const int D = h[1], H = h[2], L = h[5], W1S = h[6], NO3 = h[7], NBW = h[8];
-    if (D < 1 || D > NF_STACK_DMAX || H < 1 || H > 128 || L < 1 || NO3 != 16) return NF_ERR_UNSUPPORTED;
-    const int HP = H <= 64 ? 64 : 128;
-    if (W1S != nf_stack_w1s(D) || NBW != NF_LAYER_HDR + blk_offsets(W1S, NO3, HP).net_words) return NF_ERR_BAD_SHAPE;
-    if (packed_bytes < (int64_t)sizeof(float) * (NF_STACK_HDR + (int64_t)2 * L * NBW)) return NF_ERR_WORKSPACE;
-    cudaStream_t st = (cudaStream_t)stream;
-    const int DMh = D <= 2 ? 2 : (D <= 3 ? 4 : 8);
-    const int nbuf = HP == 64 ? 2 : 1, tmem_cols = HP == 64 ? 256 : 512;
-    const size_t smem = sizeof(float) * ((size_t)nbuf * NBW + (size_t)kTcSub * (2 * DMh + 1) * kTcThreads + NF_LAYER_HDR + 8 +
-                                         (rng_state ? 4 : 0));
-    if (smem > 227 * 1024) return NF_ERR_UNSUPPORTED;
-    // small batches: fewer sub-tiles per weight staging so that every SM gets rows (4 000 rows on eight 512-row tiles
-    // left 140 SMs idle); from kTcSub sub-tiles per resident CTA on, the staging is shared by kTcSub sub-tiles
-    const int res_ctas = kNumSMs * (512 / tmem_cols);
-    int nsub = (int)cdiv(cdiv(B, kTcThreads), res_ctas);
-    nsub = nsub < 1 ? 1 : (nsub > kTcSub ? kTcSub : nsub);
-    const int64_t ntiles = cdiv(B, kTcThreads * nsub);
-#define NF_CTC(DMv, HPv)                                                                                                  \
-    do {                                                                                                             \
-        auto kern = sample ? coupling_stack_tc_kernel<DMv, HPv, true> : coupling_stack_tc_kernel<DMv, HPv>;            \
-        NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                 \
-        NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)); \
-        int per_sm = (int)((227 * 1024) / (smem + 1024));                                                            \
-        if (per_sm < 1) return NF_ERR_UNSUPPORTED;                                                                   \
-        if (per_sm > 512 / tmem_cols) per_sm = 512 / tmem_cols;                                                      \
-        const int64_t cap = (int64_t)kNumSMs * per_sm;                                                               \
-        const int grid = (int)(ntiles < cap ? ntiles : cap);                                                         \
-        kern<<<grid, kTcThreads, smem, st>>>((const float*)packed, (const float*)x, (float*)y, (float*)ld, B, inverse, nsub, \
-                                             seed, offset, rng_state);                                               \
-    } while (0)
-    if (HP == 64) { if (D <= 2) NF_CTC(2, 64); else if (D <= 3) NF_CTC(4, 64); else NF_CTC(8, 64); }
-    else          { if (D <= 2) NF_CTC(2, 128); else if (D <= 3) NF_CTC(4, 128); else NF_CTC(8, 128); }
-#undef NF_CTC
-    count_launch();
-    NF_LAUNCH_CHECK();
-    return NF_OK;
-}
-
 extern "C" int nf_coupling_stack_tc_forward(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
                                             void* y, void* ld, int64_t B, int inverse, nf_stream_t stream) {
-    return coupling_stack_tc_launch(packed, hdr_host, packed_bytes, x, y, ld, B, inverse, false, 0, 0, nullptr, stream);
+    return stack_forward(kCouplingTc, packed, hdr_host, packed_bytes, x, y, ld, B, inverse, 0, stream);
 }
 
 extern "C" int nf_coupling_stack_tc_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, uint64_t seed,
                                            uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream) {
-    return coupling_stack_tc_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true,
-                                    seed, offset, nullptr, stream);
+    return stack_sample(kCouplingTc, packed, hdr_host, packed_bytes, 0, seed, offset, x, log_q, B, stream);
 }
 
 extern "C" int nf_coupling_stack_tc_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes,
                                                  void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream) {
-    const int rc = nf_rng_state_check(rng_state);
-    if (rc != NF_OK) return rc;
-    return coupling_stack_tc_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, true,
-                                    0, 0, (unsigned long long*)rng_state, stream);
+    return stack_sample_state(kCouplingTc, packed, hdr_host, packed_bytes, 0, rng_state, x, log_q, B, stream);
 }
 
 extern "C" int64_t nf_made_stack_tc_block_words(int D) {
@@ -978,78 +980,22 @@ extern "C" int64_t nf_made_stack_tc_block_words(int D) {
     return NF_LAYER_HDR + made_blk_offsets(nf_stack_w1s(D)).words;           // words per layer block
 }
 
-static int made_stack_tc_launch(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x, void* y,
-                                void* ld, int64_t B, int flags, int mode, bool sample, uint64_t seed, uint64_t offset,
-                                unsigned long long* rng_state, nf_stream_t stream) {
-    if (B < 0 || (sample && B > (int64_t)0xFFFFFFFFLL)) return NF_ERR_BAD_SHAPE;
-    NF_REQ(hdr_host);
-    if (B == 0) return rng_state ? nf_rng_state_advance(rng_state, (cudaStream_t)stream) : NF_OK;
-    NF_REQ(packed); NF_REQ(ld);
-    if (!sample) NF_REQ(x);
-    if (!(flags & NF_STACK_SKIP_Y)) NF_REQ(y);
-    if (!aligned16(packed)) return NF_ERR_MISALIGNED;
-    const int32_t* h = (const int32_t*)hdr_host;
-    if (h[0] != NF_STACK_MAGIC_MADE_TC) return NF_ERR_BAD_SHAPE;
-    const int D = h[1], H = h[2], L = h[5], W1S = h[6], NBW = h[8];
-    if (D < 1 || D > NF_STACK_DMAX || H < 1 || H > 64 || L < 1) return NF_ERR_UNSUPPORTED;
-    if (mode < NF_AR_MAF_INVERSE || mode > NF_AR_IAF_INVERSE) return NF_ERR_UNSUPPORTED;
-    if ((mode == NF_AR_MAF_FORWARD || mode == NF_AR_IAF_INVERSE) && D != 2) return NF_ERR_UNSUPPORTED;   // sequential: 2-D only
-    if (W1S != nf_stack_w1s(D) || NBW != NF_LAYER_HDR + made_blk_offsets(W1S).words) return NF_ERR_BAD_SHAPE;
-    if (packed_bytes < (int64_t)sizeof(float) * (NF_STACK_HDR + (int64_t)L * NBW)) return NF_ERR_WORKSPACE;
-    cudaStream_t st = (cudaStream_t)stream;
-    const int DMh = D <= 2 ? 2 : (D <= 3 ? 4 : 8);
-    const size_t smem = sizeof(float) * ((size_t)NBW + (size_t)kTcSub * (DMh + 1) * kTcThreads + 8 + (rng_state ? 4 : 0));
-    if (smem > 113 * 1024) return NF_ERR_UNSUPPORTED;             // two CTAs per SM
-    const int res_ctas = kNumSMs * 2;
-    int nsub = (int)cdiv(cdiv(B, kTcThreads), res_ctas);
-    nsub = nsub < 1 ? 1 : (nsub > kTcSub ? kTcSub : nsub);
-    const int64_t ntiles = cdiv(B, kTcThreads * nsub);
-    const int grid = (int)(ntiles < res_ctas ? ntiles : res_ctas);
-#define NF_MTC(DMv)                                                                                                  \
-    do {                                                                                                             \
-        auto kern = sample ? made_stack_tc_kernel<DMv, true> : made_stack_tc_kernel<DMv>;                            \
-        NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));                 \
-        NF_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared)); \
-        kern<<<grid, kTcThreads, smem, st>>>((const float*)packed, (const float*)x, (float*)y, (float*)ld, B, flags, nsub, mode, \
-                                             seed, offset, rng_state);                                               \
-    } while (0)
-    if (D <= 2) NF_MTC(2); else if (D <= 3) NF_MTC(4); else NF_MTC(8);
-#undef NF_MTC
-    count_launch();
-    NF_LAUNCH_CHECK();
-    return NF_OK;
-}
-
 extern "C" int nf_made_stack_tc_forward(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
                                         void* y, void* ld, int64_t B, int flags, int mode, nf_stream_t stream) {
-    return made_stack_tc_launch(packed, hdr_host, packed_bytes, x, y, ld, B, flags, mode, false, 0, 0, nullptr, stream);
+    return stack_forward(kMadeTc, packed, hdr_host, packed_bytes, x, y, ld, B, flags, mode, stream);
 }
+
+// the sampling directions only: IAF.forward (parallel) and MAF.forward (sequential, data_dim 2)
+static bool made_samples(int mode) { return mode == NF_AR_IAF_FORWARD || mode == NF_AR_MAF_FORWARD; }
 
 extern "C" int nf_made_stack_tc_sample(const void* packed, const void* hdr_host, int64_t packed_bytes, int mode, uint64_t seed,
                                        uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream) {
-    if (mode != NF_AR_IAF_FORWARD && mode != NF_AR_MAF_FORWARD) return NF_ERR_UNSUPPORTED;     // the sampling directions
-    return made_stack_tc_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, mode, true,
-                                seed, offset, nullptr, stream);
+    if (!made_samples(mode)) return NF_ERR_UNSUPPORTED;
+    return stack_sample(kMadeTc, packed, hdr_host, packed_bytes, mode, seed, offset, x, log_q, B, stream);
 }
 
 extern "C" int nf_made_stack_tc_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes, int mode,
                                              void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream) {
-    if (mode != NF_AR_IAF_FORWARD && mode != NF_AR_MAF_FORWARD) return NF_ERR_UNSUPPORTED;     // the sampling directions
-    const int rc = nf_rng_state_check(rng_state);
-    if (rc != NF_OK) return rc;
-    return made_stack_tc_launch(packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, mode, true,
-                                0, 0, (unsigned long long*)rng_state, stream);
-}
-
-// library options: key 7 = tensor-core passes per product of the dense-layer and weight-gradient kernels: 3 = 3xTF32
-// (fp32 parity, default), 1 = one TF32 pass (reduced-precision mode, set_gemm_precision("tf32"));
-// key 10 = one-pass mode only: the dense layer reads its X operand straight from shared memory (SS form, gemm_tc2.cu;
-// set_gemm_precision("bf16") turns it on); key 11 = compact spline transform: 1 = TMA-staged kernels of spline_stream.cu
-// (default), 0 = first-version kernels (the bit-identical reference).  Any other key is refused.
-namespace nf { extern int g_tc_passes; extern int g_gemm_tc2_ss; extern int g_spline_stream; }
-extern "C" int nf_set_option(int key, int value) {
-    if (key == 7) { if (value != 1 && value != 3) return NF_ERR_BAD_SHAPE; nf::g_tc_passes = value; return NF_OK; }
-    if (key == 10) { nf::g_gemm_tc2_ss = value != 0; return NF_OK; }
-    if (key == 11) { nf::g_spline_stream = value != 0; return NF_OK; }
-    return NF_ERR_UNSUPPORTED;
+    if (!made_samples(mode)) return NF_ERR_UNSUPPORTED;
+    return stack_sample_state(kMadeTc, packed, hdr_host, packed_bytes, mode, rng_state, x, log_q, B, stream);
 }

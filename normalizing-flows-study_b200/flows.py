@@ -412,6 +412,25 @@ class SequentialFlow(Flow):
         return self._run(x, True)
 
 
+class _Coupling(Flow):
+    """Shared driver of CouplingLayer and SplineCouplingLayer: their one-launch route, which `_run` takes first when no
+    autograd graph is needed and `fusable` holds, and which draws the input in the kernel for sample_and_log_prob."""
+    _stack = None       # key of run_stack's family table
+
+    def _fused(self, v, inverse, sample=None):
+        return run_stack(self._stack, self._pack, self._pack.tensors_of([self]), [self], None, v, inverse, sample=sample)
+
+    def _sample_fused(self, x, draw):
+        """The layer's own fused route of forward (one launch), drawing its input in the kernel."""
+        return self._fused(x, False, draw) if self.fusable(x) else None
+
+    def forward(self, z):
+        return self._run(z, False)
+
+    def inverse(self, x):
+        return self._run(x, True)
+
+
 # ------------------------------------------------------------------------------------------------
 # affine coupling
 # ------------------------------------------------------------------------------------------------
@@ -422,13 +441,14 @@ def _coupling_net(data_dim, hidden_dim):
         nn.Linear(hidden_dim, data_dim))
 
 
-class CouplingLayer(Flow):
+class CouplingLayer(_Coupling):
     """RealNVP affine coupling layer (coupling_layer.py:5-111).
 
     s = clamp(s_net(x*mask), +-10), b = clamp(b_net(x*mask), +-10);
     forward  x = z*mask + (1-mask)*(z*exp(s)+b),     log_det =  sum((1-mask)*s)
     inverse  z = x*mask + (1-mask)*((x-b)*exp(-s)),  log_det = -sum((1-mask)*s);  NaN/Inf -> 0.
     """
+    _stack = "coupling"
 
     def __init__(self, data_dim, hidden_dim, mask):
         super().__init__()
@@ -471,7 +491,7 @@ class CouplingLayer(Flow):
     def _run(self, v, inverse):
         v = compute_input(v)
         if not wants_grad(self, v) and self.fusable(v):
-            out = run_coupling_stack(self._pack, self._pack.tensors_of([self]), [self], None, v, inverse)
+            out = self._fused(v, inverse)
             if out is not None:
                 return out
         if (not wants_grad(self, v) and not self.training and USE_TENSOR_CORES and ops.USE_TENSOR_CORE_GEMM and v.dtype == torch.float32
@@ -484,12 +504,6 @@ class CouplingLayer(Flow):
         b_raw = self._conditioner(self.b_net, v)
         return ops.affine_coupling(v, s_raw, b_raw, self.mask, inverse)
 
-    def _sample_fused(self, x, draw):
-        """The layer's own fused route of forward (one launch), drawing its input in the kernel."""
-        if self.fusable(x):
-            return run_coupling_stack(self._pack, self._pack.tensors_of([self]), [self], None, x, False, sample=draw)
-        return None
-
     def _fold_wide(self):
         with torch.no_grad():
             out = []
@@ -499,18 +513,13 @@ class CouplingLayer(Flow):
                 out.append([_tc_layer(W0, b0, True), _tc_layer(W1, b1, True), _tc_layer(net[6].weight, net[6].bias, False)])
             return out
 
-    def forward(self, z):
-        return self._run(z, False)
-
-    def inverse(self, x):
-        return self._run(x, True)
-
 
 # ------------------------------------------------------------------------------------------------
 # rational-quadratic spline coupling
 # ------------------------------------------------------------------------------------------------
-class SplineCouplingLayer(Flow):
+class SplineCouplingLayer(_Coupling):
     """Neural-spline coupling layer on [-bound, bound] with identity tails (spline_coupling_layer.py:6-323)."""
+    _stack = "spline"
 
     def __init__(self, data_dim, hidden_dim, mask, num_bins=10, bound=5.0, min_bin_width=1e-3, min_bin_height=1e-3,
                  min_derivative=1e-3, data_min=None, data_max=None):
@@ -565,7 +574,7 @@ class SplineCouplingLayer(Flow):
     def _run(self, v, inverse):
         v = compute_input(v)
         if not wants_grad(self, v) and self.fusable(v):
-            out = run_spline_stack(self._pack, self._pack.tensors_of([self]), [self], None, v, inverse)
+            out = self._fused(v, inverse)
             if out is not None:
                 return out
         tidx, rescale, tlist = self._aux_tensors(v)
@@ -587,11 +596,6 @@ class SplineCouplingLayer(Flow):
         return ops.spline_transform(v, params, self.mask, tidx, self.num_bins, inverse, self.bound, self._mins,
                                     rescale, compact=True)
 
-    def _sample_fused(self, x, draw):
-        if self.fusable(x):
-            return run_spline_stack(self._pack, self._pack.tensors_of([self]), [self], None, x, False, sample=draw)
-        return None
-
     def _fold_wide(self, tlist):
         """Mask-folded first Linear, compact head, TF32 splits: cached per weight version for the no-grad route."""
         with torch.no_grad():
@@ -610,12 +614,6 @@ class SplineCouplingLayer(Flow):
             return lin.weight[t[0] * P:(t[-1] + 1) * P], lin.bias[t[0] * P:(t[-1] + 1) * P]
         rows = torch.cat([torch.arange(d * P, (d + 1) * P, device=lin.weight.device) for d in t])
         return lin.weight.index_select(0, rows), lin.bias.index_select(0, rows)
-
-    def forward(self, z):
-        return self._run(z, False)
-
-    def inverse(self, x):
-        return self._run(x, True)
 
 
 def rational_quadratic_spline(inputs, widths, heights, derivatives, inverse=False, min_bin_width=1e-3,
@@ -880,40 +878,33 @@ class ARQS(Flow):
 USE_TENSOR_CORES = True      # tcgen05 stack kernels (3xTF32, fp32-accurate); False forces the FP32-pipe kernels
 
 
-def run_spline_stack(cache: _PackCache, tensors, flows, bns, v, inverse, head=False, sample=None):
-    """Spline-coupling stack in one launch: tcgen05 kernel when the configuration fits it, FP32-pipe kernel otherwise.
-    sample=(seed, offset): the in-kernel N(0, I) draw into v, returning (x, log_q) (see ops._stack)."""
+# family -> (tcgen05 packer, FP32-pipe packer, tcgen05 entry point, FP32-pipe entry point)
+_STACKS = {"spline": (packing.pack_spline_stack_tc, packing.pack_spline_stack, "nf_spline_stack_tc", "nf_spline_stack"),
+           "coupling": (packing.pack_coupling_stack_tc, packing.pack_coupling_stack, "nf_coupling_stack_tc",
+                        "nf_coupling_stack")}
+
+
+def run_stack(family, cache: _PackCache, tensors, flows, bns, v, inverse, head=False, sample=None):
+    """Spline-coupling or eval-mode affine coupling stack in one launch: the tcgen05 kernel when USE_TENSOR_CORES is set
+    and the configuration fits it (spline: hidden_dim <= 64; affine: hidden_dim <= 128), the FP32-pipe kernel otherwise
+    -- also when the tcgen05 launch refuses the configuration.  sample=(seed, offset): the in-kernel N(0, I) draw into v,
+    returning (x, log_q) (see ops.stack)."""
+    pack_tc, pack, entry_tc, entry = _STACKS[family]
+
     def build():
-        tcp = packing.pack_spline_stack_tc(flows, bns) if USE_TENSOR_CORES else None
-        return ("tc", tcp) if tcp is not None else ("simt", packing.pack_spline_stack(flows, bns))
+        tcp = pack_tc(flows, bns) if USE_TENSOR_CORES else None
+        return ("tc", tcp) if tcp is not None else ("simt", pack(flows, bns))
     kind, pk = cache.get(tensors, build, extra=(USE_TENSOR_CORES,))
     if pk is None:
         return None
     if kind == "tc":
-        out = ops.spline_stack_tc(pk[0], pk[1], v, inverse, head, sample)
+        out = ops.stack(entry_tc, pk[0], pk[1], v, inverse, head, sample)
         if out is not None:
             return out
-        pk = packing.pack_spline_stack(flows, bns)
-        return None if pk is None else ops.spline_stack(pk[0], pk[1], v, inverse, head, sample)
-    return ops.spline_stack(pk[0], pk[1], v, inverse, head, sample)
-
-
-def run_coupling_stack(cache: _PackCache, tensors, flows, bns, v, inverse, head=False, sample=None):
-    """Eval-mode affine coupling stack in one launch: the tcgen05 kernel (hidden_dim <= 128), or the FP32-pipe kernel
-    when USE_TENSOR_CORES is False."""
-    def build():
-        tcp = packing.pack_coupling_stack_tc(flows, bns) if USE_TENSOR_CORES else None
-        return ("tc", tcp) if tcp is not None else ("simt", packing.pack_coupling_stack(flows, bns))
-    kind, pk = cache.get(tensors, build, extra=(USE_TENSOR_CORES,))
-    if pk is None:
-        return None
-    if kind == "tc":
-        out = ops.coupling_stack_tc(pk[0], pk[1], v, inverse, head, sample)
-        if out is not None:
-            return out
-        pk = packing.pack_coupling_stack(flows, bns)
-        return None if pk is None else ops.coupling_stack(pk[0], pk[1], v, inverse, head, sample)
-    return ops.coupling_stack(pk[0], pk[1], v, inverse, head, sample)
+        pk = pack(flows, bns)
+        if pk is None:
+            return None
+    return ops.stack(entry, pk[0], pk[1], v, inverse, head, sample)
 
 
 # ------------------------------------------------------------------------------------------------
@@ -940,21 +931,19 @@ class ChainPlan:
         if bns is not None and training:          # train mode moves the running statistics layer by layer
             return None
         kind = type(flows[0])
-        if kind in (MaskedAutoregressiveFlow, InverseAutoregressiveFlow):
-            return self._run_made_stack(flows, bns, v, inverse, head, sample)
-        if kind not in (CouplingLayer, SplineCouplingLayer) or any(type(f) is not kind for f in flows):
-            return None
-        if not all(f.fusable(v) for f in flows):
+        made = kind in (MaskedAutoregressiveFlow, InverseAutoregressiveFlow)
+        if not made and (kind not in (CouplingLayer, SplineCouplingLayer) or any(type(f) is not kind for f in flows)
+                         or not all(f.fusable(v) for f in flows)):
             return None
         mods = flows + (list(bns) if bns is not None else [])
         tensors = self._pack.tensors_of(mods)
         if torch.is_grad_enabled() and (v.requires_grad or any(t.requires_grad for t in tensors)):
             return None
-        if kind is CouplingLayer:
-            return run_coupling_stack(self._pack, tensors, flows, bns, v, inverse, head, sample)
-        return run_spline_stack(self._pack, tensors, flows, bns, v, inverse, head, sample)
+        if made:
+            return self._run_made_stack(flows, bns, tensors, v, inverse, head, sample)
+        return run_stack(kind._stack, self._pack, tensors, flows, bns, v, inverse, head, sample)
 
-    def _run_made_stack(self, flows, bns, v, inverse, head, sample):
+    def _run_made_stack(self, flows, bns, tensors, v, inverse, head, sample):
         """Homogeneous MAF / IAF stack, hidden_dim <= 64, data_dim <= 8 (the sequential direction: data_dim == 2):
         one tcgen05 launch (made_stack_tc_kernel).  None -> the layers run one by one."""
         kind = type(flows[0])
@@ -972,12 +961,8 @@ class ChainPlan:
             return None
         if head and not inverse:
             return None
-        mods = flows + (list(bns) if bns is not None else [])
-        tensors = self._pack.tensors_of(mods)
-        if torch.is_grad_enabled() and (v.requires_grad or any(t.requires_grad for t in tensors)):
-            return None
         pk = self._pack.get(tensors, lambda: packing.pack_made_stack_tc(flows, bns), extra=("made_tc",))
         if pk is None:
             return None
         mode = f0._mode_parallel if parallel else f0._mode_sequential
-        return ops.made_stack_tc(pk[0], pk[1], v, inverse, mode, head, sample)
+        return ops.stack("nf_made_stack_tc", pk[0], pk[1], v, inverse, head, sample, (mode,))

@@ -134,11 +134,15 @@ def _half_masks(data_dim, n_layers):
     return [first.clone() if i % 2 == 0 else 1 - first for i in range(n_layers)]
 
 
-class RealNVP(_DensityAPI, nn.Module):
+class _HalfMaskStack(_DensityAPI, nn.Module):
+    """RealNVP / RealNVPSpline: n_layers coupling layers of class `_layer` on alternating half masks, wrapped in a
+    NormalizingFlowModel at `self.flow` (the reference's state_dict keys)."""
+    _layer = None
+
     def __init__(self, data_dim, n_layers, hidden_dim, batch_norm_between_layers=False):
         super().__init__()
         assert n_layers % 2 == 0, "Number of layers must be even to ensure all dimensions are transformed."
-        layers = [CouplingLayer(data_dim, hidden_dim, m) for m in _half_masks(data_dim, n_layers)]
+        layers = [self._layer(data_dim, hidden_dim, m) for m in _half_masks(data_dim, n_layers)]
         self.flow = NormalizingFlowModel(layers, batch_norm_between_layers)
 
     def _log_prob_fused(self, x):
@@ -154,21 +158,9 @@ class RealNVP(_DensityAPI, nn.Module):
         return self.flow.inverse(x)
 
 
-class RealNVPSpline(_DensityAPI, nn.Module):
-    def __init__(self, data_dim, n_layers, hidden_dim, batch_norm_between_layers=False):
-        super().__init__()
-        assert n_layers % 2 == 0, "Number of layers must be even to ensure all dimensions are transformed."
-        layers = [SplineCouplingLayer(data_dim, hidden_dim, m) for m in _half_masks(data_dim, n_layers)]
-        self.flow = NormalizingFlowModel(layers, batch_norm_between_layers)
+class RealNVP(_HalfMaskStack):
+    _layer = CouplingLayer
 
-    def _log_prob_fused(self, x):
-        return self.flow._log_prob_fused(x)
 
-    def _sample_fused(self, x, draw):
-        return self.flow._sample_fused(x, draw)
-
-    def forward(self, z):
-        return self.flow.forward(z)
-
-    def inverse(self, x):
-        return self.flow.inverse(x)
+class RealNVPSpline(_HalfMaskStack):
+    _layer = SplineCouplingLayer

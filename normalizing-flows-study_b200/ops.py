@@ -5,7 +5,7 @@ Two families:
       linear (F.linear incl. MaskedLinear's W*mask, masked_linear.py:14-18), batchnorm_relu
       (nn.BatchNorm1d+ReLU of coupling_layer.py:18-35), affine_coupling, spline_transform,
       affine_ar, rqs_unit;
-  * fused inference launches (no autograd): spline_stack, coupling_stack, made_affine,
+  * fused inference launches (no autograd): stack, made_affine,
     ar_sequential.
 Every op allocates its outputs with torch (device memory plumbing) and launches on the
 current CUDA stream.  Nothing here has a CPU implementation.
@@ -742,9 +742,10 @@ def _stack_flags(inverse, head):
     return (STACK_INVERSE if inverse else 0) | ((STACK_LOG_PROB_HEAD | STACK_SKIP_Y) if head else 0)
 
 
-def _stack(name, packed, hdr_host, x, inverse, head, sample, mode=()):
-    """One fused-stack launch; returns None if the configuration is unsupported.  sample=(seed, offset): the `_sample`
-    entry point instead -- x is the output buffer of the rows, drawn from N(0, I) in the kernel and run forward, and the
+def stack(entry, packed, hdr_host, x, inverse, head=False, sample=None, mode=()):
+    """One launch of the fused-stack entry point `entry` (nf_spline_stack, nf_spline_stack_tc, nf_coupling_stack,
+    nf_coupling_stack_tc; nf_made_stack_tc with mode=(mode,)) on the (packed, hdr_host) pair of its packer; returns None if
+    the configuration is unsupported.  sample=(seed, offset): the `_sample` entry point instead -- x is the output buffer of the rows, drawn from N(0, I) in the kernel and run forward, and the
     per-row output is log N(z) - log_det (sample_and_log_prob).  sample=<DeviceGenerator state tensor>: `_sample_state`,
     the same draw with the key read from, and advanced in, device memory (a refused call leaves the state as it was)."""
     x = _c(x)
@@ -752,40 +753,16 @@ def _stack(name, packed, hdr_host, x, inverse, head, sample, mode=()):
     ld = torch.empty(B, dtype=x.dtype, device=x.device)
     hdr, nbytes = hdr_host.ctypes.data, packed.numel() * 4
     if isinstance(sample, torch.Tensor):
-        ok = L.try_call(name + "_sample_state", ptr(packed), hdr, nbytes, *mode, ptr(sample), ptr(x), ptr(ld), B, stream())
+        ok = L.try_call(entry + "_sample_state", ptr(packed), hdr, nbytes, *mode, ptr(sample), ptr(x), ptr(ld), B, stream())
         return (x, ld) if ok else None
     if sample is not None:
-        ok = L.try_call(name + "_sample", ptr(packed), hdr, nbytes, *mode, sample[0], sample[1], ptr(x), ptr(ld), B,
+        ok = L.try_call(entry + "_sample", ptr(packed), hdr, nbytes, *mode, sample[0], sample[1], ptr(x), ptr(ld), B,
                         stream())
         return (x, ld) if ok else None
     y = None if head else torch.empty_like(x)
-    ok = L.try_call(name + "_forward", ptr(packed), hdr, nbytes, ptr(x), ptr(y), ptr(ld), B, _stack_flags(inverse, head),
+    ok = L.try_call(entry + "_forward", ptr(packed), hdr, nbytes, ptr(x), ptr(y), ptr(ld), B, _stack_flags(inverse, head),
                     *mode, stream())
     return (y, ld) if ok else None
-
-
-def spline_stack(packed, hdr_host, x, inverse, head=False, sample=None):
-    """Whole spline-coupling stack in one launch; returns None if the configuration is unsupported."""
-    return _stack("nf_spline_stack", packed, hdr_host, x, inverse, head, sample)
-
-
-def spline_stack_tc(packed, hdr_host, x, inverse, head=False, sample=None):
-    """Tensor-core (tcgen05) variant of spline_stack; returns None if the configuration is unsupported."""
-    return _stack("nf_spline_stack_tc", packed, hdr_host, x, inverse, head, sample)
-
-
-def coupling_stack_tc(packed, hdr_host, x, inverse, head=False, sample=None):
-    """Tensor-core (tcgen05) variant of coupling_stack; returns None if the configuration is unsupported."""
-    return _stack("nf_coupling_stack_tc", packed, hdr_host, x, inverse, head, sample)
-
-
-def made_stack_tc(packed, hdr_host, x, inverse, mode, head=False, sample=None):
-    """Whole MAF / IAF stack in one tcgen05 launch (csrc/stack_tc.cu: made_stack_tc_kernel); None if unsupported."""
-    return _stack("nf_made_stack_tc", packed, hdr_host, x, inverse, head, sample, (mode,))
-
-
-def coupling_stack(packed, hdr_host, x, inverse, head=False, sample=None):
-    return _stack("nf_coupling_stack", packed, hdr_host, x, inverse, head, sample)
 
 
 MADE_CHAIN_BF16 = False          # set by nfb200.set_gemm_precision("bf16"): the fused bf16 chain kernel for MAF / IAF

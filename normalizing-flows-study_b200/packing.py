@@ -114,34 +114,66 @@ def _bn_between_consts(bn: torch.nn.BatchNorm1d):
             _np(bn.bias, np.float32), float(ld))
 
 
-def _rescale_arrays(layer, D):
+def _rescale(layer, D):
+    """(a, lo, c) of the data_min / data_max rescale in float64 (spline_coupling_layer.py:101-102), or None."""
     if layer.data_min is None or layer.data_max is None:
         return None
     lo = np.broadcast_to(_np(torch.as_tensor(layer.data_min)), (D,)).astype(np.float64)
     hi = np.broadcast_to(_np(torch.as_tensor(layer.data_max)), (D,)).astype(np.float64)
-    return ((2 * layer.bound) / (hi - lo)).astype(np.float32), lo.astype(np.float32), \
-        ((hi - lo) / (2 * layer.bound)).astype(np.float32)
+    return (2 * layer.bound) / (hi - lo), lo, (hi - lo) / (2 * layer.bound)
+
+
+def _rescale_arrays(layer, D):
+    r = _rescale(layer, D)
+    return None if r is None else tuple(a.astype(np.float32) for a in r)
 
 
 def rescale_tensors(layer, D, dtype, device):
-    r = None
-    if layer.data_min is not None and layer.data_max is not None:
-        lo = np.broadcast_to(_np(torch.as_tensor(layer.data_min)), (D,)).astype(np.float64)
-        hi = np.broadcast_to(_np(torch.as_tensor(layer.data_max)), (D,)).astype(np.float64)
-        r = tuple(torch.tensor(a, dtype=dtype, device=device)
-                  for a in ((2 * layer.bound) / (hi - lo), lo, (hi - lo) / (2 * layer.bound)))
-    return r
+    r = _rescale(layer, D)
+    return None if r is None else tuple(torch.tensor(a, dtype=dtype, device=device) for a in r)
 
 
-def _stack_header(magic, D, H, HP, K, L_, W1S, NO, stride, bn, bound=0.0, mins=(0.0, 0.0, 0.0)):
+def _stack_header(magic, D, H, w3, K, L_, W1S, NO, stride, bns, spline=None, scales=False):
+    """The 16 header words (csrc/stack_small.cuh).  w3: HP in the FP32-pipe layouts, nets per layer in the tcgen05 ones.
+    spline: the layer whose bound, minimums and 1 - min * K fill words 10-15; zeros otherwise, except that
+    scales=True stores 1 - 0 * K = 1 in words 14 and 15 (the FP32-pipe affine layout)."""
     h = np.zeros(HDR, dtype=np.float32)
-    hi = h.view(np.int32)
-    hi[0:10] = [magic, D, H, HP, K, L_, W1S, NO, stride, int(bn)]
+    h.view(np.int32)[0:10] = [magic, D, H, w3, K, L_, W1S, NO, stride, int(bns is not None)]
+    bound, mins = (spline.bound, (spline.min_bin_width, spline.min_bin_height, spline.min_derivative)) \
+        if spline is not None else (0.0, (0.0, 0.0, 0.0))
     h[10] = bound
     h[11], h[12], h[13] = mins
-    h[14] = np.float32(1.0 - mins[0] * K)
-    h[15] = np.float32(1.0 - mins[1] * K)
+    if spline is not None or scales:
+        h[14] = np.float32(1.0 - mins[0] * K)
+        h[15] = np.float32(1.0 - mins[1] * K)
     return h
+
+
+def _between_bn(bns, i, n_layers):
+    """Constants of the BatchNorm between layer i and i + 1; None after the last layer or without BatchNorm."""
+    return _bn_between_consts(bns[i]) if (bns is not None and i < n_layers - 1) else None
+
+
+def _finish(words, n_words, device):
+    """(packed buffer on `device`, host copy of its header as int32 words)."""
+    flat = np.concatenate(words).astype(np.float32, copy=False)
+    assert flat.size == n_words, (flat.size, n_words)
+    return torch.from_numpy(flat).to(device), flat[:HDR].copy().view(np.int32)
+
+
+def _spline_key(l):
+    return (l.data_dim, l.param_net[0].out_features, l.num_bins, l.bound, l.min_bin_width, l.min_bin_height,
+            l.min_derivative)
+
+
+def _coupling_key(l):
+    return (l.data_dim, l.s_net[0].out_features)
+
+
+def _alike(layers, key):
+    """One fused launch takes one shape: every layer must have the first one's key."""
+    k0 = key(layers[0])
+    return all(key(l) == k0 for l in layers)
 
 
 def pack_spline_stack(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
@@ -150,11 +182,8 @@ def pack_spline_stack(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
     l0 = layers[0]
     D, K = l0.data_dim, l0.num_bins
     H = l0.param_net[0].out_features
-    key = (l0.num_bins, l0.bound, l0.min_bin_width, l0.min_bin_height, l0.min_derivative)
-    for l in layers:
-        if (l.data_dim != D or l.param_net[0].out_features != H
-                or (l.num_bins, l.bound, l.min_bin_width, l.min_bin_height, l.min_derivative) != key):
-            return None
+    if not _alike(layers, _spline_key):
+        return None
     if D > DMAX or H > 128 or K < 2 or K > 16 or l0.param_net[0].weight.dtype != torch.float32:
         return None
     if L.lib().nf_spline_stack_packed_floats(D, H, K, len(layers)) < 0:
@@ -167,20 +196,15 @@ def pack_spline_stack(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
     if NO == 0:
         return None
     stride = LAYER_HDR + _net_words(HP, W1S, NO)
-    words = [_stack_header(MAGIC_SPLINE, D, H, HP, K, len(layers), W1S, NO, stride, bns is not None, l0.bound,
-                           (l0.min_bin_width, l0.min_bin_height, l0.min_derivative))]
+    words = [_stack_header(MAGIC_SPLINE, D, H, HP, K, len(layers), W1S, NO, stride, bns, spline=l0)]
     for i, (l, m) in enumerate(zip(layers, masks)):
         tdims = [d for d in range(D) if m[d] == 0]
-        bn = _bn_between_consts(bns[i]) if (bns is not None and i < len(layers) - 1) else None
-        words.append(_layer_header(m.astype(np.float32), tdims, _rescale_arrays(l, D), bn))
+        words.append(_layer_header(m.astype(np.float32), tdims, _rescale_arrays(l, D), _between_bn(bns, i, len(layers))))
         net = l.param_net
         rows = [d * P + p for d in tdims for p in range(P)]
         words.append(_pack_net(_np(net[0].weight), _np(net[0].bias), _np(net[2].weight), _np(net[2].bias),
                                _np(net[4].weight), _np(net[4].bias), rows, D, H, HP, W1S, NO))
-    flat = np.concatenate(words)
-    assert flat.size == HDR + len(layers) * stride
-    dev = l0.param_net[0].weight.device
-    return torch.from_numpy(flat).to(dev), flat[:HDR].copy().view(np.int32)
+    return _finish(words, HDR + len(layers) * stride, l0.param_net[0].weight.device)
 
 
 def _fold_bn(W, b, bn: torch.nn.BatchNorm1d):
@@ -194,28 +218,24 @@ def pack_coupling_stack(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
     l0 = layers[0]
     D = l0.data_dim
     H = l0.s_net[0].out_features
-    for l in layers:
-        if l.data_dim != D or l.s_net[0].out_features != H:
-            return None
+    if not _alike(layers, _coupling_key):
+        return None
     if D > DMAX or H > 128 or l0.s_net[0].weight.dtype != torch.float32:
         return None
     HP, W1S = _hp(H), _w1s(D)
     NO = 4 if D <= 3 else 8
     stride = LAYER_HDR + 2 * _net_words(HP, W1S, NO)
-    words = [_stack_header(MAGIC_AFFINE, D, H, HP, 0, len(layers), W1S, NO, stride, bns is not None)]
+    words = [_stack_header(MAGIC_AFFINE, D, H, HP, 0, len(layers), W1S, NO, stride, bns, scales=True)]
     for i, l in enumerate(layers):
         m = _np(l.mask)
-        bn = _bn_between_consts(bns[i]) if (bns is not None and i < len(layers) - 1) else None
-        words.append(_layer_header(m.astype(np.float32), [d for d in range(D) if m[d] == 0], None, bn))
+        words.append(_layer_header(m.astype(np.float32), [d for d in range(D) if m[d] == 0], None,
+                                   _between_bn(bns, i, len(layers))))
         for net in (l.s_net, l.b_net):
             W1, b1 = _fold_bn(_np(net[0].weight), _np(net[0].bias), net[1])
             W2, b2 = _fold_bn(_np(net[3].weight), _np(net[3].bias), net[4])
             words.append(_pack_net(W1, b1, W2, b2, _np(net[6].weight), _np(net[6].bias), list(range(D)), D, H, HP,
                                    W1S, NO))
-    flat = np.concatenate(words)
-    assert flat.size == HDR + len(layers) * stride
-    dev = l0.s_net[0].weight.device
-    return torch.from_numpy(flat).to(dev), flat[:HDR].copy().view(np.int32)
+    return _finish(words, HDR + len(layers) * stride, l0.s_net[0].weight.device)
 
 
 @dataclass
@@ -452,18 +472,24 @@ def _pad256(n):
     return (n + 255) & ~255
 
 
+def _tc_w1k(W1, b1, D, H, W1S, HP=64):
+    """W1k[HP][W1S] of the tensor-core layouts: {W1[k][0..D-1], zero pad.., b1[k] at slot W1S-1}; for data_dim <= 3
+    (W1S == 4) the units are stored in PAIRS, [w0a w0b | w1a w1b | w2a w2b | ba bb] per pair (a = unit 2p, b = 2p+1), so
+    that the kernel's packed-fp32 FMAs (FFMA2) find both units' operands in adjacent registers."""
+    w1k = np.zeros((HP, W1S))
+    w1k[:H, :D] = W1
+    w1k[:H, W1S - 1] = b1
+    if W1S == 4:
+        w1k = w1k.reshape(HP // 2, 2, 4).transpose(0, 2, 1).reshape(HP, 4)
+    return w1k
+
+
 def _tc_net_block(W1, b1, W2, b2, W3rows, b3rows, D, H, W1S, NO3, lead_words, HP=64):
     """One conditioner block of the tensor-core stack layout (csrc/stack_tc.cu: blk_offsets):
     W1k[HP][W1S] (W1S == 4: pair-interleaved, see below) | b2[HP] | b3[NO3] | pad to a 256-word boundary (counting `lead_words` in front) |
     W2 hi image | W2 lo image | W3 hi image | W3 lo image.  W3rows/b3rows: [NO3, H] / [NO3] already in head-column order.
     HP: hidden units padded to 64, or 128 for the affine coupling stack with hidden_dim in (64, 128]."""
-    w1k = np.zeros((HP, W1S))
-    w1k[:H, :D] = W1
-    w1k[:H, W1S - 1] = b1
-    if W1S == 4:
-        # data_dim <= 3: units are stored in PAIRS, [w0a w0b | w1a w1b | w2a w2b | ba bb] per pair (a = unit 2p, b = 2p+1),
-        # so that the kernel's packed-fp32 FMAs (FFMA2) find both units' operands in adjacent registers
-        w1k = w1k.reshape(HP // 2, 2, 4).transpose(0, 2, 1).reshape(HP, 4)
+    w1k = _tc_w1k(W1, b1, D, H, W1S, HP)
     b2p = np.zeros(HP)
     b2p[:H] = b2
     small = np.concatenate([w1k.ravel(), b2p, b3rows]).astype(np.float32)
@@ -492,19 +518,12 @@ def pack_made_stack_tc(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
     if nbw < 0:
         return None
     W1S, NO = _w1s(D), 16
-    hdr = np.zeros(HDR, dtype=np.float32)
-    hdr.view(np.int32)[0:10] = [MAGIC_MADE_TC, D, H, 1, 0, len(layers), W1S, NO, nbw, int(bns is not None)]
-    words = [hdr]
+    words = [_stack_header(MAGIC_MADE_TC, D, H, 1, 0, len(layers), W1S, NO, nbw, bns)]
     for i, f in enumerate(folded):
-        bn = _bn_between_consts(bns[i]) if (bns is not None and i < len(layers) - 1) else None
-        lead = _layer_header(np.zeros(D, dtype=np.float32), [], None, bn)
+        lead = _layer_header(np.zeros(D, dtype=np.float32), [], None, _between_bn(bns, i, len(layers)))
         W = [_np(t) for t in f.w]
         b = [_np(t) for t in f.b]
-        w1k = np.zeros((64, W1S))
-        w1k[:H, :D] = W[0]
-        w1k[:H, W1S - 1] = b[0]
-        if W1S == 4:
-            w1k = w1k.reshape(32, 2, 4).transpose(0, 2, 1).reshape(64, 4)
+        w1k = _tc_w1k(W[0], b[0], D, H, W1S)
         b2p, b3p, b4p = np.zeros(64), np.zeros(64), np.zeros(NO)
         b2p[:H], b3p[:H], b4p[:2 * D] = b[1], b[2], b[3]
         small = np.concatenate([w1k.ravel(), b2p, b3p, b4p]).astype(np.float32)
@@ -513,10 +532,7 @@ def pack_made_stack_tc(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
         w3 = np.zeros((64, 64), dtype=np.float32); w3[:H, :H] = W[2]
         w4 = np.zeros((NO, 64), dtype=np.float32); w4[:2 * D, :H] = W[3]
         words += [lead, small, np.zeros(pad, dtype=np.float32), umma_sw128_images(w2), umma_sw128_images(w3), umma_sw128_images(w4)]
-    flat = np.concatenate(words).astype(np.float32)
-    assert flat.size == HDR + len(layers) * nbw, (flat.size, nbw)
-    dev = folded[0].w[0].device
-    return torch.from_numpy(flat).to(dev), flat[:HDR].copy().view(np.int32)
+    return _finish(words, HDR + len(layers) * nbw, folded[0].w[0].device)
 
 
 def pack_spline_stack_tc(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
@@ -525,11 +541,8 @@ def pack_spline_stack_tc(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
     l0 = layers[0]
     D, K = l0.data_dim, l0.num_bins
     H = l0.param_net[0].out_features
-    key = (l0.num_bins, l0.bound, l0.min_bin_width, l0.min_bin_height, l0.min_derivative)
-    for l in layers:
-        if (l.data_dim != D or l.param_net[0].out_features != H
-                or (l.num_bins, l.bound, l.min_bin_width, l.min_bin_height, l.min_derivative) != key):
-            return None
+    if not _alike(layers, _spline_key):
+        return None
     if D > DMAX or H > 64 or K < 2 or K > 10 or l0.param_net[0].weight.dtype != torch.float32:
         return None
     masks = [_np(l.mask) for l in layers]
@@ -542,18 +555,10 @@ def pack_spline_stack_tc(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
     P = 3 * K - 1
     GS = 8 if K <= 8 else 10                       # slots per parameter group inside a dim's 32 columns
     W1S, NO3 = _w1s(D), 32 * max_dt
-    hdr = np.zeros(HDR, dtype=np.float32)
-    hi = hdr.view(np.int32)
-    hi[0:10] = [MAGIC_SPLINE_TC, D, H, 1, K, len(layers), W1S, NO3, bw, int(bns is not None)]
-    hdr[10] = l0.bound
-    hdr[11], hdr[12], hdr[13] = l0.min_bin_width, l0.min_bin_height, l0.min_derivative
-    hdr[14] = np.float32(1.0 - l0.min_bin_width * K)
-    hdr[15] = np.float32(1.0 - l0.min_bin_height * K)
-    words = [hdr]
+    words = [_stack_header(MAGIC_SPLINE_TC, D, H, 1, K, len(layers), W1S, NO3, bw, bns, spline=l0)]
     for i, (l, m) in enumerate(zip(layers, masks)):
         tdims = [d for d in range(D) if m[d] == 0]
-        bn = _bn_between_consts(bns[i]) if (bns is not None and i < len(layers) - 1) else None
-        words.append(_layer_header(m.astype(np.float32), tdims, _rescale_arrays(l, D), bn))
+        words.append(_layer_header(m.astype(np.float32), tdims, _rescale_arrays(l, D), _between_bn(bns, i, len(layers))))
         net = l.param_net
         W3, b3 = _np(net[4].weight), _np(net[4].bias)
         W3rows = np.zeros((NO3, H))
@@ -565,10 +570,7 @@ def pack_spline_stack_tc(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
                     b3rows[t * 32 + g * GS + j] = b3[d * P + g * K + j]
         words.append(_tc_net_block(_np(net[0].weight), _np(net[0].bias), _np(net[2].weight), _np(net[2].bias),
                                    W3rows, b3rows, D, H, W1S, NO3, LAYER_HDR))
-    flat = np.concatenate(words).astype(np.float32)
-    assert flat.size == HDR + len(layers) * bw, (flat.size, bw)
-    dev = l0.param_net[0].weight.device
-    return torch.from_numpy(flat).to(dev), flat[:HDR].copy().view(np.int32)
+    return _finish(words, HDR + len(layers) * bw, l0.param_net[0].weight.device)
 
 
 def pack_coupling_stack_tc(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
@@ -578,23 +580,20 @@ def pack_coupling_stack_tc(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
     l0 = layers[0]
     D = l0.data_dim
     H = l0.s_net[0].out_features
-    for l in layers:
-        if l.data_dim != D or l.s_net[0].out_features != H:
-            return None
+    if not _alike(layers, _coupling_key):
+        return None
     if D > DMAX or H > 128 or l0.s_net[0].weight.dtype != torch.float32:
         return None
-    HP = 64 if H <= 64 else 128
+    HP = _hp(H)
     nbw = L.lib().nf_coupling_stack_tc_block_words_hidden(D, H)
     if nbw < 0:
         return None
     W1S, NO3 = _w1s(D), 16
-    hdr = np.zeros(HDR, dtype=np.float32)
-    hdr.view(np.int32)[0:10] = [MAGIC_AFFINE_TC, D, H, 2, 0, len(layers), W1S, NO3, nbw, int(bns is not None)]
-    words = [hdr]
+    words = [_stack_header(MAGIC_AFFINE_TC, D, H, 2, 0, len(layers), W1S, NO3, nbw, bns)]
     for i, l in enumerate(layers):
         m = _np(l.mask)
-        bn = _bn_between_consts(bns[i]) if (bns is not None and i < len(layers) - 1) else None
-        lead = [_layer_header(m.astype(np.float32), [d for d in range(D) if m[d] == 0], None, bn),
+        lead = [_layer_header(m.astype(np.float32), [d for d in range(D) if m[d] == 0], None,
+                              _between_bn(bns, i, len(layers))),
                 np.zeros(LAYER_HDR, dtype=np.float32)]
         for net, ld in zip((l.s_net, l.b_net), lead):
             W1, b1 = _fold_bn(_np(net[0].weight), _np(net[0].bias), net[1])
@@ -605,7 +604,4 @@ def pack_coupling_stack_tc(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
             b3rows[:D] = _np(net[6].bias)
             blk = _tc_net_block(W1, b1, W2, b2, W3rows, b3rows, D, H, W1S, NO3, LAYER_HDR, HP)
             words += [ld, blk]
-    flat = np.concatenate(words).astype(np.float32)
-    assert flat.size == HDR + 2 * len(layers) * nbw, (flat.size, nbw)
-    dev = l0.s_net[0].weight.device
-    return torch.from_numpy(flat).to(dev), flat[:HDR].copy().view(np.int32)
+    return _finish(words, HDR + 2 * len(layers) * nbw, l0.s_net[0].weight.device)

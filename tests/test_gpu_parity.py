@@ -155,7 +155,7 @@ def test_tensor_core_stack_is_taken_and_handles_ragged_batches():
     for B in (1, 127, 128, 129, 511, 512, 513, 5000):
         x = (torch.randn(B, 2, generator=gen) * 1.5)
         for inverse in (False, True):
-            out = N.ops.spline_stack_tc(pk[0], pk[1], x.to(_dev()), inverse)
+            out = N.ops.stack("nf_spline_stack_tc", pk[0], pk[1], x.to(_dev()), inverse)
             assert out is not None
             ry, rld = O.flow_model(g["sd"], "", [dict(kind="spline", num_bins=8)] * 8, x, inverse)
             sd64 = {k: (v.double() if v.is_floating_point() else v) for k, v in g["sd"].items()}

@@ -31,27 +31,32 @@ def stack_specs(g):
     raise ValueError(k)
 
 
-def oracle_eval(g, inverse):
-    """Run the oracle on golden case `g` in one direction; returns (y, ld)."""
+def oracle_eval(g, inverse, grad=False, training=False):
+    """Run the oracle on golden case `g` in one direction; returns (y, ld).  grad=True keeps the autograd graph (the
+    state_dict `g["sd"]` may hold leaves that require grad); training=True evaluates the conditioners' BatchNorms on
+    batch statistics without moving their running statistics (update=False)."""
+    with torch.set_grad_enabled(grad):
+        return _oracle_eval(g, inverse, training)
+
+
+def _oracle_eval(g, inverse, training):
     k = g["kind"]
     x = g["x"]
-    with torch.no_grad():
-        if k == "coupling":
-            return O.affine_coupling(g["sd"], "", x, inverse)
-        if k == "spline":
-            return O.spline_coupling(g["sd"], "", x, inverse, num_bins=g["K"], **g["extra"])
-        if k == "rqs_bounded":
-            return O.rqs_bounded(x, g["uw"], g["uh"], g["ud"], inverse, bound=g["bound"])
-        if k == "rqs_unit":
-            return O.rqs_unit(x, g["w"], g["h"], g["d"], inverse)
-        if k == "maf":
-            return O.maf_inverse(g["sd"], "", x) if inverse else O.maf_forward(g["sd"], "", x)
-        if k == "iaf":
-            return O.iaf_inverse(g["sd"], "", x) if inverse else O.iaf_forward(g["sd"], "", x)
-        if k == "arqs":
-            return O.arqs(g["sd"], "", x, inverse, num_bins=g["K"], **g["extra"])
-        if k == "sequential":
-            p, specs = stack_specs(g)
-            return O.sequential_flow(g["sd"], p, specs, x, inverse)
-        p, specs = stack_specs(g)
-        return O.flow_model(g["sd"], p, specs, x, inverse, bn_between=g.get("bn", False))
+    if k == "coupling":
+        return O.affine_coupling(g["sd"], "", x, inverse, training=training)
+    if k == "spline":
+        return O.spline_coupling(g["sd"], "", x, inverse, num_bins=g["K"], **g["extra"])
+    if k == "rqs_bounded":
+        return O.rqs_bounded(x, g["uw"], g["uh"], g["ud"], inverse, bound=g["bound"])
+    if k == "rqs_unit":
+        return O.rqs_unit(x, g["w"], g["h"], g["d"], inverse)
+    if k == "maf":
+        return O.maf_inverse(g["sd"], "", x, training=training) if inverse else O.maf_forward(g["sd"], "", x)
+    if k == "iaf":
+        return O.iaf_inverse(g["sd"], "", x) if inverse else O.iaf_forward(g["sd"], "", x, training=training)
+    if k == "arqs":
+        return O.arqs(g["sd"], "", x, inverse, num_bins=g["K"], **g["extra"])
+    p, specs = stack_specs(g)
+    if k == "sequential":
+        return O.sequential_flow(g["sd"], p, specs, x, inverse)
+    return O.flow_model(g["sd"], p, specs, x, inverse, bn_between=g.get("bn", False), training=training)

@@ -17,27 +17,8 @@ GRAD_CASES = ["coupling_eval_D4_H16_alt", "coupling_eval_D5_H8_alt", "spline_D4_
 
 
 def _oracle_loss(g, sd, x, inverse, wy, wl):
-    y, ld = _oracle_eval_grad(g, sd, x, inverse)
+    y, ld = G.oracle_eval(dict(g, sd=sd, x=x), inverse, grad=True)
     return (y * wy).sum() + (ld * wl).sum()
-
-
-def _oracle_eval_grad(g, sd, x, inverse):
-    """oracle evaluation with autograd enabled (golden_util.oracle_eval runs under no_grad)"""
-    k = g["kind"]
-    if k == "coupling":
-        return O.affine_coupling(sd, "", x, inverse)
-    if k == "spline":
-        return O.spline_coupling(sd, "", x, inverse, num_bins=g["K"], **g["extra"])
-    if k == "maf":
-        return O.maf_inverse(sd, "", x) if inverse else O.maf_forward(sd, "", x)
-    if k == "iaf":
-        return O.iaf_inverse(sd, "", x) if inverse else O.iaf_forward(sd, "", x)
-    if k == "arqs":
-        return O.arqs(sd, "", x, inverse, num_bins=g["K"], **g["extra"])
-    p, specs = G.stack_specs(g)
-    if k == "sequential":
-        return O.sequential_flow(sd, p, specs, x, inverse)
-    return O.flow_model(sd, p, specs, x, inverse, bn_between=g.get("bn", False))
 
 
 @pytest.mark.parametrize("name", GRAD_CASES)

@@ -397,23 +397,23 @@ static int run_stack(const StackFamily& f, const StackCall& c) {
 }
 
 int stack_forward(const StackFamily& f, const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
-                  void* y, void* ld, int64_t B, int flags, int mode, nf_stream_t stream) {
+                  void* y, void* ld, int64_t B, int flags, int mode, nf_stream_t stream, StackCtx cx) {
     return run_stack(f, {packed, hdr_host, packed_bytes, x, y, ld, B, flags, mode, false, 0, 0, nullptr,
-                         (cudaStream_t)stream});
+                         (cudaStream_t)stream, cx});
 }
 
 int stack_sample(const StackFamily& f, const void* packed, const void* hdr_host, int64_t packed_bytes, int mode,
-                 uint64_t seed, uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream) {
+                 uint64_t seed, uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream, StackCtx cx) {
     return run_stack(f, {packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, mode, true, seed,
-                         offset, nullptr, (cudaStream_t)stream});
+                         offset, nullptr, (cudaStream_t)stream, cx});
 }
 
 int stack_sample_state(const StackFamily& f, const void* packed, const void* hdr_host, int64_t packed_bytes, int mode,
-                       void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream) {
+                       void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream, StackCtx cx) {
     const int rc = nf_rng_state_check(rng_state);
     if (rc != NF_OK) return rc;
     return run_stack(f, {packed, hdr_host, packed_bytes, nullptr, x, log_q, B, x ? 0 : NF_STACK_SKIP_Y, mode, true, 0, 0,
-                         (unsigned long long*)rng_state, (cudaStream_t)stream});
+                         (unsigned long long*)rng_state, (cudaStream_t)stream, cx});
 }
 
 template <typename Kern>

@@ -6,7 +6,7 @@
 //
 //   header (NF_STACK_HDR words, read on the host through StackHdr below):
 //     [0] magic   [1] D   [2] H (true hidden_dim)   [3] HP (padded: 64 or 128; the tcgen05 layouts of stack_tc.cu
-//     store the number of conditioner nets per layer here instead: 1 spline / MADE, 2 affine)   [4] K (spline) / 0 (affine)
+//     store the number of conditioner nets per layer here instead: 1 spline / MADE, 2 affine; 'NFC2' the context width C)   [4] K (spline) / 0 (affine)
 //     [5] L       [6] W1S (words per hidden unit in W1k: 4 if D<=3 else 12)      [7] NO (padded #outputs of the head)
 //     [8] layer_stride (words)   [9] bn_between (0/1)   [10] bound   [11] min_w  [12] min_h  [13] min_d
 //     [14] scale_w = 1-min_w*K   [15] scale_h
@@ -20,6 +20,14 @@
 //       W3c [NO/4][HP][4]: W3c[c][j][q] = W3[out(c*4+q)][j]
 //       b3  [NO]
 //   spline head outputs are ordered t*P + p for transformed dim t (P = 3K-1); affine head outputs are d.
+//
+// The tcgen05 spline layout 'NFS2' (stack_tc.cu: blk_offsets, packing._tc_net_block) has per layer the 80-word header,
+// then W1k [64][W1S] | b2 [64] | b3 [NO] | pad to 256 words | W2 hi / lo images | W3 hi / lo images.  Its conditional
+// twin 'NFC2' (SplineCouplingLayer with context_dim = C, 1 <= C <= 8) stores C in header word [3] and inserts the
+// context columns of the first Linear after b3:
+//       Wc  [32][8][2]  : unit pairs (2p, 2p+1), 8 context slots each: Wc[p][c][e] = W1[2p+e][D+c], zero for c >= C
+// W1k keeps the x columns W1[k][0..D-1] exactly as in 'NFS2', so a pack whose context columns are zero computes what
+// the 'NFS2' pack of the remaining weights computes.
 #pragma once
 #include <stdint.h>
 #include <string.h>
@@ -30,6 +38,7 @@
 #define NF_STACK_MAGIC_SPLINE_TC 0x4e465332  /* 'NFS2': tensor-core layout, see stack_tc.cu */
 #define NF_STACK_MAGIC_AFFINE_TC 0x4e464132  /* 'NFA2' */
 #define NF_STACK_MAGIC_MADE_TC 0x4e464d32    /* 'NFM2': MADE / MAF / IAF stack on the tensor cores, see stack_tc.cu */
+#define NF_STACK_MAGIC_SPLINE_CTX_TC 0x4e464332  /* 'NFC2': conditional spline stack on the tensor cores, see below */
 #define NF_STACK_HDR 16
 #define NF_LAYER_HDR 80
 #define NF_STACK_DMAX 8
@@ -70,10 +79,15 @@ namespace nf {
 
 // One call of a fused-stack entry point.  sample: the SAMPLE kernel draws the rows from (seed, offset), or from the
 // device-resident state when rng_state is not NULL; x is not read.  mode: MADE only.
+// The context of a conditional stack: row r of the batch reads row r / div of ctx [rows][C] (div = 1: one context row
+// per row; div = B: one row broadcast; div = n: n samples per context row).  ctx == NULL in the unconditional families.
+struct StackCtx { const void* ctx = nullptr; int64_t rows = 0, div = 1; };
+
 struct StackCall {
     const void* packed; const void* hdr_host; int64_t packed_bytes;
     const void* x; void* y; void* ld; int64_t B; int flags; int mode;
     bool sample; uint64_t seed, offset; unsigned long long* rng_state; cudaStream_t st;
+    StackCtx cx = {};
     bool holds(int64_t words) const { return packed_bytes >= (int64_t)sizeof(float) * words; }   // packed_bytes suffices
 };
 
@@ -86,11 +100,11 @@ struct StackFamily {
 
 // bodies of the nf_*_forward / nf_*_sample / nf_*_sample_state entry points
 int stack_forward(const StackFamily& f, const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
-                  void* y, void* ld, int64_t B, int flags, int mode, nf_stream_t stream);
+                  void* y, void* ld, int64_t B, int flags, int mode, nf_stream_t stream, StackCtx cx = {});
 int stack_sample(const StackFamily& f, const void* packed, const void* hdr_host, int64_t packed_bytes, int mode,
-                 uint64_t seed, uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream);
+                 uint64_t seed, uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream, StackCtx cx = {});
 int stack_sample_state(const StackFamily& f, const void* packed, const void* hdr_host, int64_t packed_bytes, int mode,
-                       void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream);
+                       void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream, StackCtx cx = {});
 
 // dynamic shared memory beyond 48 KB, and the largest shared-memory carveout: with the default preference the driver
 // sizes the SM for ONE CTA of the kernel and a second co-resident CTA never arrives

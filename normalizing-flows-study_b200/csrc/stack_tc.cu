@@ -161,15 +161,17 @@ __device__ __forceinline__ void named_sync(int id, int nthreads) { asm volatile(
 __device__ __forceinline__ void named_arrive(int id, int nthreads) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
 
 // layout of one layer block in shared memory (words)
-struct BlkOff { int w1k, b2, b3, w2hi, w2lo, w3hi, w3lo, net_words; };
+struct BlkOff { int w1k, b2, b3, wc, w2hi, w2lo, w3hi, w3lo, net_words; };
 __host__ __device__ inline int pad256(int x) { return (x + 255) & ~255; }
 // nets conditioner blocks follow the 80-word layer header; every block is a multiple of 256 words so that the
 // weight images stay 1024-byte aligned
 // HP: hidden units padded to 64 (every kernel here) or 128 (the affine coupling stack with hidden_dim in (64, 128])
-__host__ __device__ inline BlkOff blk_offsets(int W1S, int NO3, int HP = 64) {
+// CW: context columns of the conditional spline layout ('NFC2': Wc[HP/2][CW][2] after b3), 0 in every other layout
+__host__ __device__ inline BlkOff blk_offsets(int W1S, int NO3, int HP = 64, int CW = 0) {
     BlkOff o;
     o.w1k = 0; o.b2 = HP * W1S; o.b3 = o.b2 + HP;
-    o.w2hi = pad256(NF_LAYER_HDR + o.b3 + NO3) - NF_LAYER_HDR;       // first net: header shares the leading pad
+    o.w2hi = pad256(NF_LAYER_HDR + o.b3 + NO3 + HP * CW) - NF_LAYER_HDR;   // first net: header shares the leading pad
+    o.wc = o.b3 + NO3;
     o.w2lo = o.w2hi + HP * HP; o.w3hi = o.w2lo + HP * HP; o.w3lo = o.w3hi + NO3 * HP;
     o.net_words = o.w3lo + NO3 * HP;
     return o;
@@ -212,6 +214,55 @@ __device__ __forceinline__ void layer1_chunk(const float* __restrict__ sW1k, int
     }
 }
 
+// Conditional twin of layer1_chunk: the same x FMAs in the same order, then the C context FMAs of each unit, in column
+// order, before the ReLU.  Wc holds the units in pairs, [c0a c0b | c1a c1b | ..] with CM column slots per pair
+// (packing._tc_wc), so every FFMA2 finds both units' weights in adjacent registers.  The loop runs column by column over
+// the chunk's 8 unit pairs, reading one context value (through L1) at a time: holding the row's CM values beside the
+// chunk's accumulators pushes the DM = 2 kernels into spills.  Columns at or beyond the runtime C are skipped, as
+// KS == 0 skips the bins beyond num_bins.
+template <int DM, int CM>
+__device__ __forceinline__ void layer1_chunk_ctx(const float* __restrict__ sW1k, int W1S, const float* __restrict__ sWc,
+                                                 const float (&xa)[DM], const float* __restrict__ crow, int C, int u0,
+                                                 uint32_t (&hi)[16], uint32_t (&lo)[16]) {
+    float2 t[8];
+#pragma unroll
+    for (int q = 0; q < 8; ++q) {
+        if constexpr (DM <= 4) {
+            const int p = (u0 >> 1) + q;
+            const float4 wa = *reinterpret_cast<const float4*>(sW1k + p * 8);
+            const float4 wb = *reinterpret_cast<const float4*>(sW1k + p * 8 + 4);
+            t[q] = make_float2(wb.z, wb.w);
+            t[q] = __ffma2_rn(make_float2(wa.x, wa.y), make_float2(xa[0], xa[0]), t[q]);
+            if constexpr (DM > 1) t[q] = __ffma2_rn(make_float2(wa.z, wa.w), make_float2(xa[1], xa[1]), t[q]);
+            if constexpr (DM > 2) t[q] = __ffma2_rn(make_float2(wb.x, wb.y), make_float2(xa[2], xa[2]), t[q]);
+        } else {
+            float u[2];
+#pragma unroll
+            for (int e = 0; e < 2; ++e) {
+                const float* w1 = sW1k + (u0 + 2 * q + e) * W1S;
+                const float4 v0 = *reinterpret_cast<const float4*>(w1);
+                const float4 v1 = *reinterpret_cast<const float4*>(w1 + 4);
+                float a = w1[W1S - 1];
+                a = fmaf(v0.x, xa[0], a); a = fmaf(v0.y, xa[1], a); a = fmaf(v0.z, xa[2], a); a = fmaf(v0.w, xa[3], a);
+                a = fmaf(v1.x, xa[4], a); a = fmaf(v1.y, xa[5], a); a = fmaf(v1.z, xa[6], a); a = fmaf(v1.w, xa[7], a);
+                u[e] = a;
+            }
+            t[q] = make_float2(u[0], u[1]);
+        }
+    }
+    const float* wc = sWc + (u0 >> 1) * (2 * CM);
+#pragma unroll 1
+    for (int c = 0; c < C; ++c) {
+        const float v = __ldg(crow + c);
+#pragma unroll
+        for (int q = 0; q < 8; ++q)
+            t[q] = __ffma2_rn(*reinterpret_cast<const float2*>(wc + q * 2 * CM + 2 * c), make_float2(v, v), t[q]);
+    }
+#pragma unroll
+    for (int q = 0; q < 8; ++q)
+        tc::split_tf32_x2(relu_keepnan(t[q].x), relu_keepnan(t[q].y), hi[2 * q], hi[2 * q + 1], lo[2 * q], lo[2 * q + 1]);
+}
+
 // 16 raw layer-2 accumulators + bias -> relu -> split
 __device__ __forceinline__ void hidden2_chunk(const uint32_t (&v)[16], const float* __restrict__ sb2, uint32_t (&hi)[16], uint32_t (&lo)[16]) {
 #pragma unroll
@@ -225,12 +276,16 @@ __device__ __forceinline__ void hidden2_chunk(const uint32_t (&v)[16], const flo
     }
 }
 
-// KS > 0: num_bins known at compile time (== KMAX), every per-bin guard folds away; KS == 0: runtime num_bins <= KMAX
-template <int DM, int KMAX, int KS, bool SAMPLE = false>
-__global__ void __launch_bounds__(kTc2Threads, 2)
-spline_stack_tc2_kernel(const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
-                        float* __restrict__ ld, int64_t B, int flags, uint64_t seed, uint64_t offset,
-                        unsigned long long* rng_state) {
+// KS > 0: num_bins known at compile time (== KMAX), every per-bin guard folds away; KS == 0: runtime num_bins <= KMAX.
+// CM > 0: the conditional layout ('NFC2'): layer 1 also reads C <= CM context columns of row r / ctx_div of `ctx`,
+// fetched through L1 at every layer (see DESIGN.md §3); CM == 0 is the unconditional kernel, the context arguments unused.
+// tid: threadIdx.x read in the __global__ wrapper, where the compiler knows its range from __launch_bounds__ (read here,
+// it would not, and the CM == 0 code would differ from the kernel's before the body moved here).
+template <int DM, int KMAX, int KS, bool SAMPLE, int CM>
+__device__ __forceinline__ void
+spline_stack_tc2_body(int tid, const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
+                      float* __restrict__ ld, int64_t B, int flags, uint64_t seed, uint64_t offset,
+                      unsigned long long* rng_state, const float* __restrict__ ctx, int64_t ctx_div, int C) {
     const int inverse = flags & NF_STACK_INVERSE;
     extern __shared__ __align__(1024) float sbuf[];
     const TcHdr hd = read_tc_hdr(packed);
@@ -240,13 +295,13 @@ spline_stack_tc2_kernel(const float* __restrict__ packed, const float* __restric
     uint64_t* mbar = bars;                                     // [2] MMA completion, one per warpgroup
     uint64_t* wbar = bars + 2;                                 // [2] weight-block arrival
     uint32_t& tmem_base_s = *reinterpret_cast<uint32_t*>(bars + 4);
-    const BlkOff off = blk_offsets(W1S, NO3);
+    const BlkOff off = blk_offsets(W1S, NO3, 64, CM);
 
     RqsCfg<float> cfg;
     cfg.lo = -hd.bound; cfg.hi = hd.bound; cfg.span = 2.0f * hd.bound; cfg.eps = 1e-8f;
     cfg.min_w = hd.min_w; cfg.min_h = hd.min_h; cfg.min_d = hd.min_d; cfg.scale_w = hd.scale_w; cfg.scale_h = hd.scale_h;
 
-    const int tid = threadIdx.x, warp = tid >> 5, wg = tid >> 7, wtid = tid & 127, wwarp = warp & 3;
+    const int warp = tid >> 5, wg = tid >> 7, wtid = tid & 127, wwarp = warp & 3;
     const int bar_local = 1 + wg;
     if (warp == 0) tc::tmem_alloc(&tmem_base_s, kTmemCols);
     unsigned long long* rng_key = reinterpret_cast<unsigned long long*>(bars + 5);   // SAMPLE + device state: every
@@ -325,10 +380,16 @@ spline_stack_tc2_kernel(const float* __restrict__ packed, const float* __restric
                     xa[d] = (d < D) ? v * mask[d] : 0.f;
                 }
                 uint32_t hi[16], lo[16];
+                uint32_t crow = 0;                              // the row's context row (conditional kernel)
+                if constexpr (CM > 0) {
+                    const int64_t r = tile * ROWS + s * kTcThreads + wtid;     // < 2^31, as ctx_div (the launcher)
+                    crow = r < B ? (uint32_t)r / (uint32_t)ctx_div : 0u;
+                }
                 // ---- layer 2, K half 1: hidden units 0..31 ----
 #pragma unroll
                 for (int c = 0; c < 2; ++c) {
-                    layer1_chunk<DM>(sW1k, W1S, xa, c * 16, hi, lo);
+                    if constexpr (CM > 0) layer1_chunk_ctx<DM, CM>(sW1k, W1S, net + off.wc, xa, ctx + (size_t)crow * C, C, c * 16, hi, lo);
+                    else layer1_chunk<DM>(sW1k, W1S, xa, c * 16, hi, lo);
                     tc::tmem_st16(lane_addr + kWgAhi + c * 16, hi);
                     tc::tmem_st16(lane_addr + kWgAlo + c * 16, lo);
                 }
@@ -338,8 +399,13 @@ spline_stack_tc2_kernel(const float* __restrict__ packed, const float* __restric
                 if (wwarp == 0) { tc::fence_after_sync(); tc::warp_issue_gemm_krange_3xtf32(tb, kWgD, kWgAhi, kWgAlo, w2hi, w2lo, 64u, 0, 4, 0u, mb); }
                 // ---- K half 2: hidden units 32..63, computed while half 1 multiplies ----
                 uint32_t hi2[16], lo2[16];
-                layer1_chunk<DM>(sW1k, W1S, xa, 32, hi, lo);
-                layer1_chunk<DM>(sW1k, W1S, xa, 48, hi2, lo2);
+                if constexpr (CM > 0) {
+                    layer1_chunk_ctx<DM, CM>(sW1k, W1S, net + off.wc, xa, ctx + (size_t)crow * C, C, 32, hi, lo);
+                    layer1_chunk_ctx<DM, CM>(sW1k, W1S, net + off.wc, xa, ctx + (size_t)crow * C, C, 48, hi2, lo2);
+                } else {
+                    layer1_chunk<DM>(sW1k, W1S, xa, 32, hi, lo);
+                    layer1_chunk<DM>(sW1k, W1S, xa, 48, hi2, lo2);
+                }
                 tc::mbar_wait(mb, phase); phase ^= 1;           // half-1 MMAs done: the A columns are free
                 tc::fence_after_sync();
                 tc::tmem_st16(lane_addr + kWgAhi, hi);   tc::tmem_st16(lane_addr + kWgAlo, lo);
@@ -451,6 +517,25 @@ spline_stack_tc2_kernel(const float* __restrict__ packed, const float* __restric
     tc::fence_before_sync();
     __syncthreads();
     if (warp == 0) tc::tmem_dealloc(tmem_base_s, kTmemCols);
+}
+
+template <int DM, int KMAX, int KS, bool SAMPLE = false>
+__global__ void __launch_bounds__(kTc2Threads, 2)
+spline_stack_tc2_kernel(const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
+                        float* __restrict__ ld, int64_t B, int flags, uint64_t seed, uint64_t offset,
+                        unsigned long long* rng_state) {
+    spline_stack_tc2_body<DM, KMAX, KS, SAMPLE, 0>(threadIdx.x, packed, x, y, ld, B, flags, seed, offset, rng_state, nullptr, 1, 0);
+}
+
+// conditional spline stack ('NFC2'): C <= kCtxMax context columns of row r / ctx_div enter every layer's first Linear
+constexpr int kCtxMax = 8;
+template <int DM, int KMAX, int KS, bool SAMPLE = false>
+__global__ void __launch_bounds__(kTc2Threads, 2)
+spline_stack_ctx_tc2_kernel(const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
+                            float* __restrict__ ld, int64_t B, int flags, uint64_t seed, uint64_t offset,
+                            unsigned long long* rng_state, const float* __restrict__ ctx, int64_t ctx_div, int C) {
+    spline_stack_tc2_body<DM, KMAX, KS, SAMPLE, kCtxMax>(threadIdx.x, packed, x, y, ld, B, flags, seed, offset, rng_state, ctx, ctx_div,
+                                                         C);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -823,11 +908,20 @@ static int tc_nsub(int64_t B, int64_t res_ctas) {
     return nsub < 1 ? 1 : (nsub > kTcSub ? kTcSub : nsub);
 }
 
+// CTX: the conditional layout ('NFC2'; header word 3 = context width C) and spline_stack_ctx_tc2_kernel
+template <bool CTX>
 static int spline_stack_tc_launch(const StackCall& c, const StackHdr& h) {
     const int D = h.D, K = h.K, W1S = h.W1S, NO3 = h.NO, BW = h.layer_stride;
+    if (CTX) {
+        if (c.cx.ctx == nullptr) return NF_ERR_NULL;
+        if (c.cx.div < 1 || c.cx.rows < cdiv(c.B, c.cx.div)) return NF_ERR_BAD_SHAPE;
+        if (h.HP < 1 || h.HP > kCtxMax) return NF_ERR_UNSUPPORTED;
+        if (c.B > 0x7FFFFFFF || c.cx.div > 0x7FFFFFFF) return NF_ERR_UNSUPPORTED;     // 32-bit row / context-row indices
+    }
     if (D < 1 || D > NF_STACK_DMAX || h.H < 1 || h.H > 64 || h.L < 1 || K < 2 || K > 10) return NF_ERR_UNSUPPORTED;
     if (NO3 != 32 && NO3 != 64) return NF_ERR_UNSUPPORTED;
-    if (W1S != nf_stack_w1s(D) || BW != NF_LAYER_HDR + blk_offsets(W1S, NO3).net_words) return NF_ERR_BAD_SHAPE;
+    if (W1S != nf_stack_w1s(D) || BW != NF_LAYER_HDR + blk_offsets(W1S, NO3, 64, CTX ? kCtxMax : 0).net_words)
+        return NF_ERR_BAD_SHAPE;
     if (!c.holds(NF_STACK_HDR + (int64_t)h.L * BW)) return NF_ERR_WORKSPACE;
     const int DMh = D <= 2 ? 2 : (D <= 3 ? 4 : 8);
     const size_t smem = sizeof(float) * ((size_t)2 * BW + (size_t)kTcSub * (DMh + 1) * kTcThreads + 12 + (c.rng_state ? 4 : 0));
@@ -838,11 +932,21 @@ static int spline_stack_tc_launch(const StackCall& c, const StackHdr& h) {
     const int grid = (int)(ntiles < cap ? ntiles : cap);
 #define NF_TC(DMv, KMv, KSv)                                                                                         \
     do {                                                                                                             \
-        auto kern = c.sample ? spline_stack_tc2_kernel<DMv, KMv, KSv, true> : spline_stack_tc2_kernel<DMv, KMv, KSv>; \
-        const int rc = stack_smem_attributes(kern, smem);                                                            \
-        if (rc != NF_OK) return rc;                                                                                  \
-        kern<<<grid, kTc2Threads, smem, c.st>>>((const float*)c.packed, (const float*)c.x, (float*)c.y, (float*)c.ld, \
-                                                c.B, c.flags, c.seed, c.offset, c.rng_state);                        \
+        if constexpr (CTX) {                                                                                         \
+            auto kern = c.sample ? spline_stack_ctx_tc2_kernel<DMv, KMv, KSv, true>                                  \
+                                 : spline_stack_ctx_tc2_kernel<DMv, KMv, KSv>;                                       \
+            const int rc = stack_smem_attributes(kern, smem);                                                        \
+            if (rc != NF_OK) return rc;                                                                              \
+            kern<<<grid, kTc2Threads, smem, c.st>>>((const float*)c.packed, (const float*)c.x, (float*)c.y,          \
+                                                    (float*)c.ld, c.B, c.flags, c.seed, c.offset, c.rng_state,       \
+                                                    (const float*)c.cx.ctx, c.cx.div, h.HP);                         \
+        } else {                                                                                                     \
+            auto kern = c.sample ? spline_stack_tc2_kernel<DMv, KMv, KSv, true> : spline_stack_tc2_kernel<DMv, KMv, KSv>; \
+            const int rc = stack_smem_attributes(kern, smem);                                                        \
+            if (rc != NF_OK) return rc;                                                                              \
+            kern<<<grid, kTc2Threads, smem, c.st>>>((const float*)c.packed, (const float*)c.x, (float*)c.y,          \
+                                                    (float*)c.ld, c.B, c.flags, c.seed, c.offset, c.rng_state);      \
+        }                                                                                                            \
     } while (0)
 #define NF_TC_K(DMv)                                      \
     do {                                                  \
@@ -922,7 +1026,8 @@ static int made_stack_tc_launch(const StackCall& c, const StackHdr& h) {
     return NF_OK;
 }
 
-static const StackFamily kSplineTc = {NF_STACK_MAGIC_SPLINE_TC, spline_stack_tc_launch};
+static const StackFamily kSplineTc = {NF_STACK_MAGIC_SPLINE_TC, spline_stack_tc_launch<false>};
+static const StackFamily kSplineCtxTc = {NF_STACK_MAGIC_SPLINE_CTX_TC, spline_stack_tc_launch<true>};
 static const StackFamily kCouplingTc = {NF_STACK_MAGIC_AFFINE_TC, coupling_stack_tc_launch};
 static const StackFamily kMadeTc = {NF_STACK_MAGIC_MADE_TC, made_stack_tc_launch};
 
@@ -949,6 +1054,27 @@ extern "C" int nf_spline_stack_tc_sample(const void* packed, const void* hdr_hos
 extern "C" int nf_spline_stack_tc_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes,
                                                void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream) {
     return stack_sample_state(kSplineTc, packed, hdr_host, packed_bytes, 0, rng_state, x, log_q, B, stream);
+}
+
+extern "C" int nf_spline_stack_ctx_tc_forward(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
+                                              const void* context, int64_t ctx_rows, int64_t ctx_div, void* y, void* ld,
+                                              int64_t B, int flags, nf_stream_t stream) {
+    return stack_forward(kSplineCtxTc, packed, hdr_host, packed_bytes, x, y, ld, B, flags, 0, stream,
+                         {context, ctx_rows, ctx_div});
+}
+
+extern "C" int nf_spline_stack_ctx_tc_sample(const void* packed, const void* hdr_host, int64_t packed_bytes,
+                                             const void* context, int64_t ctx_rows, int64_t ctx_div, uint64_t seed,
+                                             uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream) {
+    return stack_sample(kSplineCtxTc, packed, hdr_host, packed_bytes, 0, seed, offset, x, log_q, B, stream,
+                        {context, ctx_rows, ctx_div});
+}
+
+extern "C" int nf_spline_stack_ctx_tc_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes,
+                                                   const void* context, int64_t ctx_rows, int64_t ctx_div, void* rng_state,
+                                                   void* x, void* log_q, int64_t B, nf_stream_t stream) {
+    return stack_sample_state(kSplineCtxTc, packed, hdr_host, packed_bytes, 0, rng_state, x, log_q, B, stream,
+                              {context, ctx_rows, ctx_div});
 }
 
 extern "C" int64_t nf_coupling_stack_tc_block_words(int D) {

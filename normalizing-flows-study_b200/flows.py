@@ -19,6 +19,7 @@ There is no CPU route: tensors and modules must live on a CUDA device.
 """
 from __future__ import annotations
 
+
 import numpy as np
 import torch
 import torch.nn as nn
@@ -101,23 +102,93 @@ def is_std_normal(base_dist, D=None) -> bool:
     return ok
 
 
+class _Context:
+    """A validated context: row r of the batch is conditioned on t[r // div] (div = 1: one context row per row; the
+    batch size: one row for all; n: n samples per context row).  One object serves every layer of a call."""
+    __slots__ = ("t", "div", "_per_row")
+
+    def __init__(self, t, div):
+        self.t, self.div, self._per_row = t, div, None
+
+    def layered(self, B):
+        """(context rows, div) the layered first Linear reads: one row per row, or a single row for all.  n rows per
+        context row (the layered route of sampling) are expanded once per call, not once per layer."""
+        if self.div == 1 or self.t.shape[0] == 1:
+            return self.t, self.div
+        if self._per_row is None:
+            self._per_row = self.t.repeat_interleave(self.div, 0)[:B]
+        return self._per_row, 1
+
+
+def _context_dim(module) -> int:
+    """C of the conditional layers a flow or container holds (0: none); fixed when the module is built."""
+    return getattr(module, "context_dim", 0) or 0
+
+
+def _shared_context_dim(flows) -> int:
+    """The context width of a container: every conditional layer reads the one context, so they must agree."""
+    dims = {_context_dim(f) for f in flows} - {0}
+    if len(dims) > 1:
+        raise ValueError(f"the conditional layers of one model share one context; got context_dim values {sorted(dims)}")
+    return dims.pop() if dims else 0
+
+
+def _as_context(module, context, v, div=None, what="rows"):
+    """Validate `context` for a call of `module` on v [B, D] and return it as a _Context (None without one).  context:
+    [B, C] (one row per row), [1, C] (broadcast to every row) or, with div = n (sampling), [m, C] for m*n rows.  Raises
+    ValueError for a conditional model called without context, a context given to a model without conditional layer,
+    and a context of the wrong width, row count, dtype or device; a context is never dropped."""
+    C = _context_dim(module)
+    if context is None:
+        if C:
+            raise ValueError(f"{type(module).__name__} has conditional layers (context_dim={C}): pass context=")
+        return None
+    if not C:
+        raise ValueError(f"{type(module).__name__} has no conditional layer (context_dim=0) but a context was passed")
+    if isinstance(context, _Context):
+        return context
+    if not isinstance(context, torch.Tensor) or context.dim() != 2 or context.shape[1] != C:
+        shape = tuple(context.shape) if isinstance(context, torch.Tensor) else type(context).__name__
+        raise ValueError(f"context must be a [{what}, {C}] tensor (context_dim={C}); got {shape}")
+    context = compute_input(context)
+    dtype = compute_input(v).dtype if isinstance(v, torch.Tensor) else v[0]
+    device = v.device if isinstance(v, torch.Tensor) else v[1]
+    if context.dtype != dtype:
+        raise ValueError(f"context has dtype {context.dtype}, the flow computes in {dtype}")
+    if context.device != torch.device(device):
+        raise ValueError(f"context is on {context.device}, the flow's input on {device}")
+    if div is None:
+        B = v.shape[0]
+        if context.shape[0] == B:
+            div = 1
+        elif context.shape[0] == 1:
+            div = max(B, 1)
+        else:
+            raise ValueError(f"context has {context.shape[0]} rows; expected {B} (one per row) or 1 (broadcast)")
+    elif context.shape[0] < 1:
+        raise ValueError("context has no rows")
+    return _Context(context.contiguous(), int(div))
+
+
 def _default_base(D, device, dtype=torch.float32):
     from torch import distributions as td
     return td.Normal(torch.zeros(D, device=device, dtype=dtype), torch.ones(D, device=device, dtype=dtype))
 
 
-def flow_log_prob(flow, x, base_dist, fused_head=None):
+def flow_log_prob(flow, x, base_dist, fused_head=None, context=None):
     """Flow.log_prob (flow.py:56-73).  For a standard-normal base the head log N(z; 0, I) + log_det is one kernel
     (nf_std_normal_log_prob_*, with a backward), or -- `fused_head`, no autograd graph needed -- part of the last
-    layer's epilogue of the fused stack launch; any other base goes through the torch distribution on the returned z."""
+    layer's epilogue of the fused stack launch; any other base goes through the torch distribution on the returned z.
+    context: the conditional layers' context, [B, C] or [1, C] (see _as_context)."""
+    ctx = _as_context(flow, context, x)
     D = x.shape[-1] if x.dim() == 2 else None
     std = x.is_cuda and x.dim() == 2 and is_std_normal(base_dist, D)
     if std and fused_head is not None:
         with torch.cuda.device(x.device):
-            lp = fused_head(x)
+            lp = fused_head(x) if ctx is None else fused_head(x, ctx)
         if lp is not None:
             return lp
-    z, log_det_inv = flow.inverse(x)
+    z, log_det_inv = flow.inverse(x) if ctx is None else flow.inverse(x, ctx)
     if std and z.dtype in (torch.float32, torch.float64):
         return ops.std_normal_log_prob(z, log_det_inv)
     log_p_z = base_dist.log_prob(z)
@@ -232,7 +303,7 @@ def _draw_state(generator, device):
     return seed, offset
 
 
-def flow_sample_and_log_prob(flow, num_samples, base_dist=None, device=None, generator=None):
+def flow_sample_and_log_prob(flow, num_samples, base_dist=None, device=None, generator=None, context=None):
     """(x, log_q): z ~ base, (x, log_det) = flow.forward(z), log_q = log p_base(z) - log_det (summed over the event axis
     as in Flow.log_prob), without materialising z where the route allows it.
 
@@ -243,23 +314,31 @@ def flow_sample_and_log_prob(flow, num_samples, base_dist=None, device=None, gen
     last layer's epilogue (`_sample_fused`); every other route draws z with nf_std_normal_draw, runs forward(z) -- with
     its autograd graph when parameters require grad, the reparameterised gradient -- and the log-q head kernel.  Any
     other base is sampled by torch (rsample where it has one) and cannot take a generator.  Every route draws once, so a
-    DeviceGenerator moves on by exactly 4 per call (a fused stack that refuses the call launches nothing)."""
+    DeviceGenerator moves on by exactly 4 per call (a fused stack that refuses the call launches nothing).
+    context [m, C] (conditional models): num_samples rows per context row, context-major -- row r of the flat [m*n, D]
+    draw is conditioned on context row r // n, and the draw itself does not depend on the context; x is returned as
+    [m, n, D] and log_q as [m, n]."""
     p = next(flow.parameters(), None)
     device = torch.device(device if device is not None else (p.device if p is not None else "cpu"))
     dtype = p.dtype if p is not None else torch.float32
     D = _event_dim(flow)
     n = int(num_samples)
+    if device.type == "cuda" and device.index is None:
+        device = torch.device("cuda", torch.cuda.current_device())
+    ctx = _as_context(flow, context, (dtype, device), div=max(n, 1), what="m")
+    rows = n if ctx is None else ctx.t.shape[0] * n
+    shaped = (lambda x, lq: (x, lq)) if ctx is None else \
+        (lambda x, lq: (x.view(ctx.t.shape[0], n, D), lq.view(ctx.t.shape[0], n)))
+    fwd = flow.forward if ctx is None else (lambda z: flow.forward(z, ctx))
     if base_dist is not None and not is_std_normal(base_dist, D):
         if generator is not None:
             raise ValueError("generator= seeds the on-device N(0, I) draw only; torch distributions cannot take a generator")
-        z = (base_dist.rsample if base_dist.has_rsample else base_dist.sample)((n,)).to(device)
-        x, log_det = flow.forward(z)
+        z = (base_dist.rsample if base_dist.has_rsample else base_dist.sample)((rows,)).to(device)
+        x, log_det = fwd(z)
         log_p_z = base_dist.log_prob(z)
         if log_p_z.dim() > 1:
             log_p_z = log_p_z.sum(dim=1)
-        return x, log_p_z - log_det
-    if device.type == "cuda" and device.index is None:
-        device = torch.device("cuda", torch.cuda.current_device())
+        return shaped(x, log_p_z - log_det)
     if isinstance(generator, DeviceGenerator) and generator.device != device:
         raise ValueError(f"the DeviceGenerator lives on {generator.device} but the draw is on {device}")
     if device.type != "cuda":
@@ -267,13 +346,14 @@ def flow_sample_and_log_prob(flow, num_samples, base_dist=None, device=None, gen
     with torch.cuda.device(device):
         draw = _draw_state(generator, device)
         fused = getattr(flow, "_sample_fused", None)
-        if fused is not None and not wants_grad(flow):
-            out = fused(torch.empty((n, D), dtype=dtype, device=device), draw)
+        if fused is not None and not wants_grad(flow, None if ctx is None else ctx.t):
+            buf = torch.empty((rows, D), dtype=dtype, device=device)
+            out = fused(buf, draw) if ctx is None else fused(buf, draw, ctx)
             if out is not None:
-                return out
-        z = ops.std_normal_draw(*ops._draw_key(draw), n, D, dtype, device)
-        x, log_det = flow.forward(z)
-        return x, ops.std_normal_log_q(z, log_det)
+                return shaped(*out)
+        z = ops.std_normal_draw(*ops._draw_key(draw), rows, D, dtype, device)
+        x, log_det = fwd(z)
+        return shaped(x, ops.std_normal_log_q(z, log_det))
 
 
 def _module_tensors(module: nn.Module):
@@ -348,6 +428,7 @@ class Flow(nn.Module):
     def __init__(self):
         super().__init__()
         self.data_dim = None
+        self.context_dim = 0          # > 0: a conditional layer (or a container holding some), see _as_context
 
     def forward(self, z):
         raise NotImplementedError
@@ -355,26 +436,53 @@ class Flow(nn.Module):
     def inverse(self, x):
         raise NotImplementedError
 
-    def sample(self, num_samples, base_dist=None, device="cpu"):
-        """flow.py:40-54 (base_dist=None: standard normal over data_dim / dim)."""
-        if base_dist is None:
-            base_dist = _default_base(self.data_dim, device)
-        z = base_dist.sample((num_samples,)).to(device)
-        x, _ = self.forward(z)
-        return x
+    def sample(self, num_samples, base_dist=None, device="cpu", context=None):
+        """flow.py:40-54 (base_dist=None: standard normal over data_dim / dim).  context [m, C] (conditional flows):
+        num_samples rows per context row, returned as [m, n, D]."""
+        return sample_from(self, self.data_dim, num_samples, base_dist, device, context)
 
-    def log_prob(self, x, base_dist=None):
+    def log_prob(self, x, base_dist=None, context=None):
         """flow.py:56-73: log p(z) (summed over the event axis if the base is factorised) + log|det J_inv|.
-        A standard-normal base is detected (is_std_normal) and evaluated by the fused head kernels."""
-        return flow_log_prob(self, x, base_dist, getattr(self, "_log_prob_fused", None))
+        A standard-normal base is detected (is_std_normal) and evaluated by the fused head kernels.  context: [B, C]
+        or [1, C] for a conditional flow."""
+        return flow_log_prob(self, x, base_dist, getattr(self, "_log_prob_fused", None), context)
 
-    def sample_and_log_prob(self, num_samples, base_dist=None, device=None, generator=None):
+    def sample_and_log_prob(self, num_samples, base_dist=None, device=None, generator=None, context=None):
         """Samples and their log-density in one pass: z ~ base, (x, log_det) = forward(z), log_q = log p_base(z) - log_det.
         device=None: the parameters' device; dtype: the parameters'.  A standard-normal base (None or N(0, I)) is drawn on
         the GPU from `generator` (torch.Generator on that device; None = torch's default CUDA generator, so
         torch.manual_seed makes the call reproducible); float64 models widen the float32 draw.  Raises RuntimeError under
-        CUDA-graph capture, ValueError for a generator with any other base.  See flow_sample_and_log_prob."""
-        return flow_sample_and_log_prob(self, num_samples, base_dist, device, generator)
+        CUDA-graph capture, ValueError for a generator with any other base.  context [m, C] (conditional flows): x
+        [m, n, D] and log_q [m, n].  See flow_sample_and_log_prob."""
+        return flow_sample_and_log_prob(self, num_samples, base_dist, device, generator, context)
+
+
+def sample_from(flow, D, num_samples, base_dist, device, context):
+    """Flow.sample: z ~ base (a torch distribution), x = forward(z); with context [m, C], m * num_samples rows,
+    context-major, returned as [m, n, D]."""
+    if base_dist is None:
+        base_dist = _default_base(D, device)
+    if context is None:
+        z = base_dist.sample((num_samples,)).to(device)
+        x, _ = flow.forward(z)
+        return x
+    p = next(flow.parameters(), None)
+    device = torch.device(device)
+    if device.type == "cuda" and device.index is None:           # as flow_sample_and_log_prob: 'cuda' is the current one
+        device = torch.device("cuda", torch.cuda.current_device())
+    ctx = _as_context(flow, context, (p.dtype if p is not None else torch.float32, device),
+                      div=max(int(num_samples), 1), what="m")
+    m = ctx.t.shape[0]
+    z = base_dist.sample((m * num_samples,)).to(device)
+    x, _ = flow.forward(z, ctx)
+    return x.view(m, num_samples, -1)
+
+
+def _apply_layer(flow, v, inverse, ctx):
+    """One layer of a container: conditional layers get the container's context, the others are called as before."""
+    if ctx is not None and _context_dim(flow):
+        return flow._run(v, inverse, ctx)
+    return flow.inverse(v) if inverse else flow.forward(v)
 
 
 class SequentialFlow(Flow):
@@ -385,31 +493,32 @@ class SequentialFlow(Flow):
         if not isinstance(flows, (list, nn.ModuleList)):
             raise ValueError("flows must be a list or nn.ModuleList")
         self.flows = nn.ModuleList(flows)
+        self.context_dim = _shared_context_dim(self.flows)
         self._chain = ChainPlan()
 
-    def _log_prob_fused(self, x):
-        out = self._chain.run(self.flows, None, self.training, x, True, head=True)
+    def _log_prob_fused(self, x, ctx=None):
+        out = self._chain.run(self.flows, None, self.training, x, True, head=True, ctx=ctx)
         return None if out is None else out[1]
 
-    def _sample_fused(self, x, draw):
-        return self._chain.run(self.flows, None, self.training, x, False, sample=draw)
+    def _sample_fused(self, x, draw, ctx=None):
+        return self._chain.run(self.flows, None, self.training, x, False, sample=draw, ctx=ctx)
 
     @on_input_device
-    def _run(self, v, inverse):
-        fused = self._chain.run(self.flows, None, self.training, v, inverse)
+    def _run(self, v, inverse, ctx=None):
+        fused = self._chain.run(self.flows, None, self.training, v, inverse, ctx=ctx)
         if fused is not None:
             return fused
         total = torch.zeros(v.size(0), device=v.device)         # float32 accumulator, as the reference
         for flow in (reversed(self.flows) if inverse else self.flows):
-            v, ld = flow.inverse(v) if inverse else flow.forward(v)
+            v, ld = _apply_layer(flow, v, inverse, ctx)
             total += ld
         return v, total
 
-    def forward(self, z):
-        return self._run(z, False)
+    def forward(self, z, context=None):
+        return self._run(z, False, _as_context(self, context, z))
 
-    def inverse(self, x):
-        return self._run(x, True)
+    def inverse(self, x, context=None):
+        return self._run(x, True, _as_context(self, context, x))
 
 
 class _Coupling(Flow):
@@ -417,18 +526,19 @@ class _Coupling(Flow):
     autograd graph is needed and `fusable` holds, and which draws the input in the kernel for sample_and_log_prob."""
     _stack = None       # key of run_stack's family table
 
-    def _fused(self, v, inverse, sample=None):
-        return run_stack(self._stack, self._pack, self._pack.tensors_of([self]), [self], None, v, inverse, sample=sample)
+    def _fused(self, v, inverse, sample=None, ctx=None):
+        return run_stack(self._stack, self._pack, self._pack.tensors_of([self]), [self], None, v, inverse, sample=sample,
+                         ctx=ctx)
 
-    def _sample_fused(self, x, draw):
+    def _sample_fused(self, x, draw, ctx=None):
         """The layer's own fused route of forward (one launch), drawing its input in the kernel."""
-        return self._fused(x, False, draw) if self.fusable(x) else None
+        return self._fused(x, False, draw, ctx) if self.fusable(x) else None
 
-    def forward(self, z):
-        return self._run(z, False)
+    def forward(self, z, context=None):
+        return self._run(z, False, _as_context(self, context, z))
 
-    def inverse(self, x):
-        return self._run(x, True)
+    def inverse(self, x, context=None):
+        return self._run(x, True, _as_context(self, context, x))
 
 
 # ------------------------------------------------------------------------------------------------
@@ -488,7 +598,7 @@ class CouplingLayer(_Coupling):
                 and self.data_dim <= packing.DMAX and H <= 128)
 
     @on_input_device
-    def _run(self, v, inverse):
+    def _run(self, v, inverse, ctx=None):
         v = compute_input(v)
         if not wants_grad(self, v) and self.fusable(v):
             out = self._fused(v, inverse)
@@ -518,12 +628,18 @@ class CouplingLayer(_Coupling):
 # rational-quadratic spline coupling
 # ------------------------------------------------------------------------------------------------
 class SplineCouplingLayer(_Coupling):
-    """Neural-spline coupling layer on [-bound, bound] with identity tails (spline_coupling_layer.py:6-323)."""
-    _stack = "spline"
+    """Neural-spline coupling layer on [-bound, bound] with identity tails (spline_coupling_layer.py:6-323).
+
+    context_dim = C > 0 makes it conditional, p(x | c): the conditioner's input is [x_rescaled * mask, c] (context
+    columns last, as in nflows), so param_net[0] is Linear(data_dim + C, hidden_dim); the context is neither rescaled
+    nor masked.  forward / inverse then take context= [B, C] or [1, C] (broadcast)."""
 
     def __init__(self, data_dim, hidden_dim, mask, num_bins=10, bound=5.0, min_bin_width=1e-3, min_bin_height=1e-3,
-                 min_derivative=1e-3, data_min=None, data_max=None):
+                 min_derivative=1e-3, data_min=None, data_max=None, context_dim=0):
         super().__init__()
+        if int(context_dim) != context_dim or context_dim < 0:
+            raise ValueError(f"context_dim must be a non-negative integer, got {context_dim!r}")
+        self.context_dim = int(context_dim)
         self.data_dim = data_dim
         self.num_bins = num_bins
         self.bound = bound
@@ -534,7 +650,7 @@ class SplineCouplingLayer(_Coupling):
         self.data_max = data_max
         self.register_buffer("mask", mask)
         self.param_net = nn.Sequential(
-            nn.Linear(data_dim, hidden_dim), nn.ReLU(),
+            nn.Linear(data_dim + self.context_dim, hidden_dim), nn.ReLU(),
             nn.Linear(hidden_dim, hidden_dim), nn.ReLU(),
             nn.Linear(hidden_dim, data_dim * (3 * num_bins - 1)))
         self._initialize_weights()
@@ -550,6 +666,10 @@ class SplineCouplingLayer(_Coupling):
                 nn.init.zeros_(layer.bias)
         nn.init.zeros_(self.param_net[-1].weight)
         nn.init.zeros_(self.param_net[-1].bias)
+
+    @property
+    def _stack(self):             # key of run_stack's family table
+        return "spline_ctx" if self.context_dim else "spline"
 
     @property
     def _mins(self):
@@ -571,10 +691,11 @@ class SplineCouplingLayer(_Coupling):
                 and self.data_dim <= packing.DMAX and H <= 128 and 2 <= self.num_bins <= 16)
 
     @on_input_device
-    def _run(self, v, inverse):
+    def _run(self, v, inverse, ctx=None):
         v = compute_input(v)
-        if not wants_grad(self, v) and self.fusable(v):
-            out = self._fused(v, inverse)
+        ct = None if ctx is None else ctx.t
+        if not wants_grad(self, v, ct) and self.fusable(v):
+            out = self._fused(v, inverse, ctx=ctx)
             if out is not None:
                 return out
         tidx, rescale, tlist = self._aux_tensors(v)
@@ -582,12 +703,16 @@ class SplineCouplingLayer(_Coupling):
         vin = v
         if rescale is not None:                       # conditioner sees the rescaled input (:101-102)
             vin = ops.feature_affine(v, rescale[1], None, rescale[0], -float(self.bound))
-        if (not wants_grad(self, v) and USE_TENSOR_CORES and ops.USE_TENSOR_CORE_GEMM and v.dtype == torch.float32 and net[0].weight.dtype == torch.float32
+        if ctx is not None:                           # [x_rescaled * mask, c] -> first Linear, without concatenating
+            c, div = ctx.layered(v.shape[0])
+            h = ops.linear_ctx(vin, c, net[0].weight, net[0].bias, self.mask, div)
+        elif (not wants_grad(self, v) and USE_TENSOR_CORES and ops.USE_TENSOR_CORE_GEMM and v.dtype == torch.float32 and net[0].weight.dtype == torch.float32
                 and v.shape[0] >= WIDE_TC_MIN_ROWS and tlist):
             layers = self._wide.get(self._wide.tensors_of([self]), lambda: self._fold_wide(tlist))
             return ops.spline_transform(v, _tc_mlp(vin, layers), self.mask, tidx, self.num_bins, inverse, self.bound,
                                         self._mins, rescale, compact=True)
-        h = ops.linear(vin, net[0].weight, net[0].bias, mask=self.mask, relu=True)
+        else:
+            h = ops.linear(vin, net[0].weight, net[0].bias, mask=self.mask, relu=True)
         h = ops.linear(h, net[2].weight, net[2].bias, relu=True)
         # head restricted to the transformed dims: the reference evaluates all D*(3K-1) outputs and discards the rows
         # of the conditioning dims (SURVEY D9); no used value changes
@@ -881,25 +1006,28 @@ USE_TENSOR_CORES = True      # tcgen05 stack kernels (3xTF32, fp32-accurate); Fa
 # family -> (tcgen05 packer, FP32-pipe packer, tcgen05 entry point, FP32-pipe entry point)
 _STACKS = {"spline": (packing.pack_spline_stack_tc, packing.pack_spline_stack, "nf_spline_stack_tc", "nf_spline_stack"),
            "coupling": (packing.pack_coupling_stack_tc, packing.pack_coupling_stack, "nf_coupling_stack_tc",
-                        "nf_coupling_stack")}
+                        "nf_coupling_stack"),
+           # conditional spline layers: tcgen05 only, outside its envelope the layered route
+           "spline_ctx": (packing.pack_spline_stack_ctx_tc, None, "nf_spline_stack_ctx_tc", None)}
 
 
-def run_stack(family, cache: _PackCache, tensors, flows, bns, v, inverse, head=False, sample=None):
+def run_stack(family, cache: _PackCache, tensors, flows, bns, v, inverse, head=False, sample=None, ctx=None):
     """Spline-coupling or eval-mode affine coupling stack in one launch: the tcgen05 kernel when USE_TENSOR_CORES is set
     and the configuration fits it (spline: hidden_dim <= 64; affine: hidden_dim <= 128), the FP32-pipe kernel otherwise
     -- also when the tcgen05 launch refuses the configuration.  sample=(seed, offset): the in-kernel N(0, I) draw into v,
-    returning (x, log_q) (see ops.stack)."""
+    returning (x, log_q) (see ops.stack).  ctx: the _Context of the conditional family "spline_ctx"."""
     pack_tc, pack, entry_tc, entry = _STACKS[family]
 
     def build():
         tcp = pack_tc(flows, bns) if USE_TENSOR_CORES else None
-        return ("tc", tcp) if tcp is not None else ("simt", pack(flows, bns))
+        return ("tc", tcp) if tcp is not None else ("simt", pack(flows, bns) if pack is not None else None)
     kind, pk = cache.get(tensors, build, extra=(USE_TENSOR_CORES,))
     if pk is None:
         return None
     if kind == "tc":
-        out = ops.stack(entry_tc, pk[0], pk[1], v, inverse, head, sample)
-        if out is not None:
+        out = ops.stack(entry_tc, pk[0], pk[1], v, inverse, head, sample,
+                        context=None if ctx is None else (ctx.t, ctx.div))
+        if out is not None or pack is None:
             return out
         pk = pack(flows, bns)
         if pk is None:
@@ -918,12 +1046,13 @@ class ChainPlan:
     def __init__(self):
         self._pack = _PackCache()
 
-    def run(self, flows, bns, training, v, inverse, head=False, sample=None):
+    def run(self, flows, bns, training, v, inverse, head=False, sample=None, ctx=None):
         """(y, log_det) from one fused launch, or None when the chain must be walked layer by layer.
         head=True (inverse only): (None, log_prob) with the standard-normal Flow.log_prob head evaluated in the last
         layer's epilogue -- z is never written.
         sample=(seed, offset) (forward only): the sampling twin of the head -- v is the [n, D] output buffer, the rows are
-        the N(0, I) draw of csrc/nf_rng.cuh made in the kernel, and the result is (x, log N(z) - log_det)."""
+        the N(0, I) draw of csrc/nf_rng.cuh made in the kernel, and the result is (x, log N(z) - log_det).
+        ctx (a _Context): every layer must be a SplineCouplingLayer with that context width, float32 context included."""
         flows = list(flows)
         v = compute_input(v)
         if not flows or not v.is_cuda or v.dim() != 2:
@@ -935,13 +1064,17 @@ class ChainPlan:
         if not made and (kind not in (CouplingLayer, SplineCouplingLayer) or any(type(f) is not kind for f in flows)
                          or not all(f.fusable(v) for f in flows)):
             return None
+        if ctx is not None and (kind is not SplineCouplingLayer or ctx.t.dtype != torch.float32
+                                or any(f.context_dim != ctx.t.shape[1] for f in flows)):
+            return None
         mods = flows + (list(bns) if bns is not None else [])
         tensors = self._pack.tensors_of(mods)
-        if torch.is_grad_enabled() and (v.requires_grad or any(t.requires_grad for t in tensors)):
+        if torch.is_grad_enabled() and (v.requires_grad or any(t.requires_grad for t in tensors)
+                                        or (ctx is not None and ctx.t.requires_grad)):
             return None
         if made:
             return self._run_made_stack(flows, bns, tensors, v, inverse, head, sample)
-        return run_stack(kind._stack, self._pack, tensors, flows, bns, v, inverse, head, sample)
+        return run_stack(flows[0]._stack, self._pack, tensors, flows, bns, v, inverse, head, sample, ctx)
 
     def _run_made_stack(self, flows, bns, tensors, v, inverse, head, sample):
         """Homogeneous MAF / IAF stack, hidden_dim <= 64, data_dim <= 8 (the sequential direction: data_dim == 2):

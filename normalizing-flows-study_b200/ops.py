@@ -245,6 +245,74 @@ def linear(x, weight, bias=None, mask=None, relu=False):
     return _LinearFn.apply(x, weight, bias, mask, relu)
 
 
+def _product(a, w):
+    """a [M, K] @ w[N, K]^T without bias, on the route _LinearFn takes for that shape: tcgen05 (3xTF32) for float32 with
+    >= 256 rows and K % 4 == 0, the FP32 / FP64-pipe nf_gemm otherwise."""
+    M, K = a.shape
+    N = w.shape[0]
+    if _tc_ok(a, K):
+        hi, lo = split_tf32(w)
+        y = linear_tc(a, hi, lo)
+        if y is not None:
+            return y
+    return gemm(a, w, M, N, K, K, 1, 1, K)
+
+
+def _wgrad(g, a):
+    """dW[N, K] = g[B, N]^T a[B, K], on the route _LinearFn.backward takes."""
+    B, N = g.shape
+    K = a.shape[1]
+    gw = linear_wgrad_tc(g, a) if _tc_ok(g, K) else None
+    return gw if gw is not None else gemm(g, a, N, K, B, 1, N, K, 1)
+
+
+class _LinearCtxFn(Function):
+    """relu(W[:, :D] (x*mask) + W[:, D:] c + b): the first Linear of a conditional spline conditioner, whose input is
+    [x*mask, c] (context columns last), without concatenating x and c.  Two products into one output: the context one
+    without bias, then the masked x one with bias and ReLU accumulated onto it (nf_gemm computes relu(acc + bias + C_old)
+    on every path).  `div`: row r of x uses context row r // div; 1 (one context row per row) or, with a single context
+    row, anything (that row is read with row stride 0)."""
+
+    @staticmethod
+    def forward(ctx, x, c, weight, bias, mask, div):
+        x, c = _c(x), _c(c)
+        B, D = x.shape
+        H, C = weight.shape[0], c.shape[1]
+        wx = mul_rows(_c(weight[:, :D]), mask)                      # x*mask folded into the x columns, as linear()
+        wc = _c(weight[:, D:])
+        per_row = c.shape[0] == B and div == 1
+        y = _product(c, wc) if per_row else gemm(c, wc, B, H, C, 0, 1, 1, C)
+        gemm(x, wx, B, H, D, D, 1, 1, D, bias=_c(bias), relu=True, out=y, accumulate=True)
+        ctx.per_row = per_row
+        ctx.save_for_backward(x, c, wx, wc, mask, y)
+        return y
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, gy):
+        x, c, wx, wc, mask, y = ctx.saved_tensors
+        B, D = x.shape
+        H, C = wc.shape
+        g, gb = relu_backward_colsum(y, _c(gy))                     # the bias gradient comes out of the same pass
+        gx = gc = gw = None
+        if ctx.needs_input_grad[0]:
+            gx = _product(g, _c(wx.t()))                            # dX = dY Wx
+        if ctx.needs_input_grad[1]:                                 # one shared row: (column sums of dY) Wc
+            gc = _product(g, _c(wc.t())) if ctx.per_row else gemm(gb.view(1, H), wc, 1, C, H, H, 1, C, 1)
+        if ctx.needs_input_grad[2]:
+            gw = torch.empty((H, D + C), dtype=g.dtype, device=g.device)
+            gw[:, :D] = mul_rows(_wgrad(g, x), mask)
+            gw[:, D:] = _wgrad(g, c) if ctx.per_row else gemm(gb.view(H, 1), c, H, C, 1, 1, 1, C, 1)
+        return gx, gc, gw, (gb if ctx.needs_input_grad[3] else None), None, None
+
+
+def linear_ctx(x, c, weight, bias, mask, div):
+    """relu(F.linear(cat([x*mask, c[r // div]]), weight, bias)) with x [B, D], c [rows, C], weight [H, D+C] (see
+    _LinearCtxFn)."""
+    weight, bias, mask, c = _same_dtype(x, weight, bias, mask, c)
+    return _LinearCtxFn.apply(x, c, weight, bias, mask, int(div))
+
+
 # --------------------------------------------------------------------------------------------
 # BatchNorm1d (+ReLU)
 # --------------------------------------------------------------------------------------------
@@ -742,26 +810,29 @@ def _stack_flags(inverse, head):
     return (STACK_INVERSE if inverse else 0) | ((STACK_LOG_PROB_HEAD | STACK_SKIP_Y) if head else 0)
 
 
-def stack(entry, packed, hdr_host, x, inverse, head=False, sample=None, mode=()):
+def stack(entry, packed, hdr_host, x, inverse, head=False, sample=None, mode=(), context=None):
     """One launch of the fused-stack entry point `entry` (nf_spline_stack, nf_spline_stack_tc, nf_coupling_stack,
     nf_coupling_stack_tc; nf_made_stack_tc with mode=(mode,)) on the (packed, hdr_host) pair of its packer; returns None if
     the configuration is unsupported.  sample=(seed, offset): the `_sample` entry point instead -- x is the output buffer of the rows, drawn from N(0, I) in the kernel and run forward, and the
     per-row output is log N(z) - log_det (sample_and_log_prob).  sample=<DeviceGenerator state tensor>: `_sample_state`,
-    the same draw with the key read from, and advanced in, device memory (a refused call leaves the state as it was)."""
+    the same draw with the key read from, and advanced in, device memory (a refused call leaves the state as it was).
+    context=(c, div) (nf_spline_stack_ctx_tc): the float32 [rows, C] context, row r of the batch reading row r // div."""
     x = _c(x)
     B = x.shape[0]
     ld = torch.empty(B, dtype=x.dtype, device=x.device)
     hdr, nbytes = hdr_host.ctypes.data, packed.numel() * 4
+    cargs = () if context is None else (ptr(_c(context[0])), context[0].shape[0], int(context[1]))
     if isinstance(sample, torch.Tensor):
-        ok = L.try_call(entry + "_sample_state", ptr(packed), hdr, nbytes, *mode, ptr(sample), ptr(x), ptr(ld), B, stream())
-        return (x, ld) if ok else None
-    if sample is not None:
-        ok = L.try_call(entry + "_sample", ptr(packed), hdr, nbytes, *mode, sample[0], sample[1], ptr(x), ptr(ld), B,
+        ok = L.try_call(entry + "_sample_state", ptr(packed), hdr, nbytes, *mode, *cargs, ptr(sample), ptr(x), ptr(ld), B,
                         stream())
         return (x, ld) if ok else None
+    if sample is not None:
+        ok = L.try_call(entry + "_sample", ptr(packed), hdr, nbytes, *mode, *cargs, sample[0], sample[1], ptr(x), ptr(ld),
+                        B, stream())
+        return (x, ld) if ok else None
     y = None if head else torch.empty_like(x)
-    ok = L.try_call(entry + "_forward", ptr(packed), hdr, nbytes, ptr(x), ptr(y), ptr(ld), B, _stack_flags(inverse, head),
-                    *mode, stream())
+    ok = L.try_call(entry + "_forward", ptr(packed), hdr, nbytes, ptr(x), *cargs, ptr(y), ptr(ld), B,
+                    _stack_flags(inverse, head), *mode, stream())
     return (y, ld) if ok else None
 
 

@@ -21,6 +21,8 @@ MAGIC_AFFINE = 0x4E464131
 MAGIC_SPLINE_TC = 0x4E465332
 MAGIC_AFFINE_TC = 0x4E464132
 MAGIC_MADE_TC = 0x4E464D32
+MAGIC_SPLINE_CTX_TC = 0x4E464332
+CTX_MAX = 8                     # context columns of the conditional tcgen05 spline layout ('NFC2'; csrc/stack_small.cuh)
 HDR, LAYER_HDR, DMAX = 16, 80, 8
 
 
@@ -163,7 +165,7 @@ def _finish(words, n_words, device):
 
 def _spline_key(l):
     return (l.data_dim, l.param_net[0].out_features, l.num_bins, l.bound, l.min_bin_width, l.min_bin_height,
-            l.min_derivative)
+            l.min_derivative, l.context_dim)
 
 
 def _coupling_key(l):
@@ -182,7 +184,7 @@ def pack_spline_stack(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
     l0 = layers[0]
     D, K = l0.data_dim, l0.num_bins
     H = l0.param_net[0].out_features
-    if not _alike(layers, _spline_key):
+    if not _alike(layers, _spline_key) or l0.context_dim:
         return None
     if D > DMAX or H > 128 or K < 2 or K > 16 or l0.param_net[0].weight.dtype != torch.float32:
         return None
@@ -484,15 +486,25 @@ def _tc_w1k(W1, b1, D, H, W1S, HP=64):
     return w1k
 
 
-def _tc_net_block(W1, b1, W2, b2, W3rows, b3rows, D, H, W1S, NO3, lead_words, HP=64):
+def _tc_wc(Wc, H, HP=64):
+    """Wc[HP/2][CTX_MAX][2] of the conditional layout: context column c of units 2p and 2p+1 at [p][c][0..1], zero beyond
+    the C columns of Wc [H, C] and the H units."""
+    wc = np.zeros((HP, CTX_MAX))
+    wc[:H, :Wc.shape[1]] = Wc
+    return wc.reshape(HP // 2, 2, CTX_MAX).transpose(0, 2, 1)
+
+
+def _tc_net_block(W1, b1, W2, b2, W3rows, b3rows, D, H, W1S, NO3, lead_words, HP=64, Wc=None):
     """One conditioner block of the tensor-core stack layout (csrc/stack_tc.cu: blk_offsets):
     W1k[HP][W1S] (W1S == 4: pair-interleaved, see below) | b2[HP] | b3[NO3] | pad to a 256-word boundary (counting `lead_words` in front) |
     W2 hi image | W2 lo image | W3 hi image | W3 lo image.  W3rows/b3rows: [NO3, H] / [NO3] already in head-column order.
-    HP: hidden units padded to 64, or 128 for the affine coupling stack with hidden_dim in (64, 128]."""
+    HP: hidden units padded to 64, or 128 for the affine coupling stack with hidden_dim in (64, 128].
+    Wc [H, C]: the context columns of the first Linear (conditional layout), stored by _tc_wc after b3."""
     w1k = _tc_w1k(W1, b1, D, H, W1S, HP)
     b2p = np.zeros(HP)
     b2p[:H] = b2
-    small = np.concatenate([w1k.ravel(), b2p, b3rows]).astype(np.float32)
+    parts = [w1k.ravel(), b2p, b3rows] + ([] if Wc is None else [_tc_wc(Wc, H, HP).ravel()])
+    small = np.concatenate(parts).astype(np.float32)
     pad = _pad256(lead_words + small.size) - lead_words - small.size
     w2 = np.zeros((HP, HP), dtype=np.float32)
     w2[:H, :H] = W2
@@ -538,6 +550,21 @@ def pack_made_stack_tc(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
 def pack_spline_stack_tc(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
     """Tensor-core layout of a spline-coupling stack; None when the configuration is outside the kernel's envelope
     (hidden_dim <= 64, num_bins <= 10, <= 2 transformed dims per layer, data_dim <= 8)."""
+    if layers[0].context_dim:
+        return None
+    return _pack_spline_tc(layers, bns, 0)
+
+
+def pack_spline_stack_ctx_tc(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
+    """Conditional twin of pack_spline_stack_tc ('NFC2', csrc/stack_small.cuh): the same envelope for layers that share
+    one context_dim in 1..CTX_MAX; header word 3 holds it and every block gains the Wc section."""
+    C = layers[0].context_dim
+    if C < 1 or C > CTX_MAX:
+        return None
+    return _pack_spline_tc(layers, bns, C)
+
+
+def _pack_spline_tc(layers, bns, C):
     l0 = layers[0]
     D, K = l0.data_dim, l0.num_bins
     H = l0.param_net[0].out_features
@@ -555,7 +582,11 @@ def pack_spline_stack_tc(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
     P = 3 * K - 1
     GS = 8 if K <= 8 else 10                       # slots per parameter group inside a dim's 32 columns
     W1S, NO3 = _w1s(D), 32 * max_dt
-    words = [_stack_header(MAGIC_SPLINE_TC, D, H, 1, K, len(layers), W1S, NO3, bw, bns, spline=l0)]
+    if C:                                          # the Wc section moves the weight images by whole 256-word steps
+        small = LAYER_HDR + 64 * W1S + 64 + NO3
+        bw += _pad256(small + 64 * CTX_MAX) - _pad256(small)
+    magic, w3 = (MAGIC_SPLINE_CTX_TC, C) if C else (MAGIC_SPLINE_TC, 1)
+    words = [_stack_header(magic, D, H, w3, K, len(layers), W1S, NO3, bw, bns, spline=l0)]
     for i, (l, m) in enumerate(zip(layers, masks)):
         tdims = [d for d in range(D) if m[d] == 0]
         words.append(_layer_header(m.astype(np.float32), tdims, _rescale_arrays(l, D), _between_bn(bns, i, len(layers))))
@@ -568,8 +599,9 @@ def pack_spline_stack_tc(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
                 for j in range(cnt):
                     W3rows[t * 32 + g * GS + j] = W3[d * P + g * K + j]
                     b3rows[t * 32 + g * GS + j] = b3[d * P + g * K + j]
-        words.append(_tc_net_block(_np(net[0].weight), _np(net[0].bias), _np(net[2].weight), _np(net[2].bias),
-                                   W3rows, b3rows, D, H, W1S, NO3, LAYER_HDR))
+        W1 = _np(net[0].weight)
+        words.append(_tc_net_block(W1[:, :D], _np(net[0].bias), _np(net[2].weight), _np(net[2].bias),
+                                   W3rows, b3rows, D, H, W1S, NO3, LAYER_HDR, Wc=W1[:, D:] if C else None))
     return _finish(words, HDR + len(layers) * bw, l0.param_net[0].weight.device)
 
 

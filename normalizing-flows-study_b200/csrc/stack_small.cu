@@ -21,15 +21,6 @@ namespace nf {
 
 constexpr int kStackThreads = 128;
 
-__device__ __forceinline__ StackHdr read_hdr(const float* __restrict__ p) {
-    const int* q = reinterpret_cast<const int*>(p);
-    StackHdr h;
-    h.D = q[1]; h.H = q[2]; h.HP = q[3]; h.K = q[4]; h.L = q[5]; h.W1S = q[6]; h.NO = q[7];
-    h.layer_stride = q[8]; h.bn_between = q[9];
-    h.bound = p[10]; h.min_w = p[11]; h.min_h = p[12]; h.min_d = p[13]; h.scale_w = p[14]; h.scale_h = p[15];
-    return h;
-}
-
 // cooperative global->shared copy of n words (n % 4 == 0, both 16B aligned)
 __device__ __forceinline__ void stage_words(float* dst, const float* __restrict__ src, int n) {
     for (int i = threadIdx.x * 4; i < n; i += kStackThreads * 4) cp_async16(dst + i, src + i);
@@ -118,21 +109,11 @@ __device__ __forceinline__ void head_chunk(const float* __restrict__ sW3c, const
     for (int i = 0; i < R; ++i) { o[i][0] = o01[i].x; o[i][1] = o01[i].y; o[i][2] = o23[i].x; o[i][3] = o23[i].y; }
 }
 
-// between-layer BatchNorm as an invertible affine on running stats (normalizing_flow_model.py:67-128)
+// R rows of one thread through the between-layer BatchNorm
 template <int R, int DM>
-__device__ __forceinline__ void bn_between(const float* __restrict__ sL, int D, bool inverse, float (&xv)[R][DM],
-                                           float (&tot)[R]) {
-    const float* mean = sL + 48; const float* sd = sL + 56; const float* gm = sL + 64; const float* bt = sL + 72;
-    const float bn_ld = sL[16 + 3];
+__device__ __forceinline__ void bn_between(LayerHdr lh, int D, bool inverse, float (&xv)[R][DM], float (&tot)[R]) {
 #pragma unroll
-    for (int i = 0; i < R; ++i) {
-#pragma unroll
-        for (int d = 0; d < DM; ++d) if (d < D) {
-            if (!inverse) xv[i][d] = (xv[i][d] - mean[d]) / sd[d] * gm[d] + bt[d];
-            else          xv[i][d] = (xv[i][d] - bt[d]) / gm[d] * sd[d] + mean[d];
-        }
-        tot[i] = inverse ? tot[i] - bn_ld : tot[i] + bn_ld;
-    }
+    for (int i = 0; i < R; ++i) nf_stack_bn_between<DM>(lh, D, inverse, xv[i], tot[i]);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -149,7 +130,7 @@ spline_stack_kernel(const float* __restrict__ packed, const float* __restrict__ 
                     unsigned long long* rng_state) {
     const int inverse = flags & NF_STACK_INVERSE;
     extern __shared__ __align__(16) float smem[];
-    const StackHdr hd = read_hdr(packed);
+    const StackHdr hd = nf_stack_hdr_device(packed);
     const int D = hd.D, K = hd.K, L = hd.L, W1S = hd.W1S, NO = hd.NO, P = 3 * hd.K - 1;
     constexpr int ROWS = kStackThreads * R;
     float* sL = smem;                          // staged layer block
@@ -195,10 +176,10 @@ spline_stack_kernel(const float* __restrict__ packed, const float* __restrict__ 
             cp_async_commit();
             cp_async_wait<0>();
             __syncthreads();
-            const int* meta = reinterpret_cast<const int*>(sL + 16);
-            const bool rescale = meta[1] != 0, bn_on = meta[2] != 0;
-            const float* mask = sL;
-            if (inverse && bn_on) bn_between<R, DM>(sL, D, true, xv, tot);
+            const LayerHdr lh{sL};
+            const bool rescale = lh.rescale(), bn_on = lh.bn_on();
+            const float* mask = lh.mask();
+            if (inverse && bn_on) bn_between<R, DM>(lh, D, true, xv, tot);
 
             float xs[R][DM];                                  // value in spline coordinates
             {
@@ -208,7 +189,7 @@ spline_stack_kernel(const float* __restrict__ packed, const float* __restrict__ 
 #pragma unroll
                     for (int d = 0; d < DM; ++d) {
                         float v = xv[i][d];
-                        if (rescale && d < D) v = sL[24 + d] * (v - sL[32 + d]) - hd.bound;
+                        if (rescale && d < D) v = lh.to_spline(v, d, hd.bound);
                         xs[i][d] = v;
                         xa[i][d] = (d < D) ? v * mask[d] : 0.f;
                     }
@@ -243,7 +224,7 @@ spline_stack_kernel(const float* __restrict__ packed, const float* __restrict__ 
                         }
                         float out, lad;
                         rqs_eval<float, KMAX, true>(xs[i][d], uw, uh, ud, K, inverse != 0, cfg, out, lad);
-                        if (rescale) out = (out + hd.bound) * sL[40 + d] + sL[32 + d];
+                        if (rescale) out = lh.from_spline(out, d, hd.bound);
                         xv[i][d] = out;
                         lsum[i] += lad;
                     }
@@ -256,18 +237,11 @@ spline_stack_kernel(const float* __restrict__ packed, const float* __restrict__ 
                 for (int d = 0; d < DM; ++d) xv[i][d] = scrub0(xv[i][d]);      // layer-level scrub (:130-135)
                 tot[i] += scrub0(lsum[i]);
             }
-            if (!inverse && bn_on) bn_between<R, DM>(sL, D, false, xv, tot);
+            if (!inverse && bn_on) bn_between<R, DM>(lh, D, false, xv, tot);
         }
 #pragma unroll
-        for (int i = 0; i < R; ++i) {
-            if (row[i] < B) {
-                if (!(flags & NF_STACK_SKIP_Y)) {
-#pragma unroll
-                    for (int d = 0; d < DM; ++d) if (d < D) st_stream(y + row[i] * D + d, xv[i][d]);
-                }
-                st_stream(ld + row[i], SAMPLE ? -tot[i] : (flags & NF_STACK_LOG_PROB_HEAD) ? nf_stack_row_head<DM>(xv[i], D, tot[i]) : tot[i]);
-            }
-        }
+        for (int i = 0; i < R; ++i)
+            if (row[i] < B) nf_stack_row_store<DM, SAMPLE>(y, ld, row[i], D, flags, xv[i], tot[i]);
     }
 }
 
@@ -281,7 +255,7 @@ coupling_stack_kernel(const float* __restrict__ packed, const float* __restrict_
                       unsigned long long* rng_state) {
     const int inverse = flags & NF_STACK_INVERSE;
     extern __shared__ __align__(16) float smem[];
-    const StackHdr hd = read_hdr(packed);
+    const StackHdr hd = nf_stack_hdr_device(packed);
     const int D = hd.D, L = hd.L, W1S = hd.W1S;
     constexpr int NO = DM;                      // head outputs padded to DM (4 or 8)
     constexpr int ROWS = kStackThreads * R;
@@ -319,10 +293,10 @@ coupling_stack_kernel(const float* __restrict__ packed, const float* __restrict_
             cp_async_commit();
             cp_async_wait<0>();
             __syncthreads();
-            const int* meta = reinterpret_cast<const int*>(sL + 16);
-            const bool bn_on = meta[2] != 0;
-            const float* mask = sL;
-            if (inverse && bn_on) bn_between<R, DM>(sL, D, true, xv, tot);
+            const LayerHdr lh{sL};
+            const bool bn_on = lh.bn_on();
+            const float* mask = lh.mask();
+            if (inverse && bn_on) bn_between<R, DM>(lh, D, true, xv, tot);
 
             float xa[R][DM];
 #pragma unroll
@@ -361,18 +335,11 @@ coupling_stack_kernel(const float* __restrict__ packed, const float* __restrict_
                 }
                 tot[i] += scrub0(lsum);
             }
-            if (!inverse && bn_on) bn_between<R, DM>(sL, D, false, xv, tot);
+            if (!inverse && bn_on) bn_between<R, DM>(lh, D, false, xv, tot);
         }
 #pragma unroll
-        for (int i = 0; i < R; ++i) {
-            if (row[i] < B) {
-                if (!(flags & NF_STACK_SKIP_Y)) {
-#pragma unroll
-                    for (int d = 0; d < DM; ++d) if (d < D) st_stream(y + row[i] * D + d, xv[i][d]);
-                }
-                st_stream(ld + row[i], SAMPLE ? -tot[i] : (flags & NF_STACK_LOG_PROB_HEAD) ? nf_stack_row_head<DM>(xv[i], D, tot[i]) : tot[i]);
-            }
-        }
+        for (int i = 0; i < R; ++i)
+            if (row[i] < B) nf_stack_row_store<DM, SAMPLE>(y, ld, row[i], D, flags, xv[i], tot[i]);
     }
 }
 

@@ -11,8 +11,7 @@
 //     [8] layer_stride (words)   [9] bn_between (0/1)   [10] bound   [11] min_w  [12] min_h  [13] min_d
 //     [14] scale_w = 1-min_w*K   [15] scale_h
 //   per layer (layer_stride words, 16-byte aligned sections):
-//     mask[8] | tdim[8] (int) | meta[8]: {Dt, rescale, bn_on, bn_ld(float), 0..} | r_in[8] | r_lo[8] | r_out[8]
-//     | bn_mean[8] | bn_sd[8] | bn_gamma[8] | bn_beta[8]                      (NF_LAYER_HDR = 80 words)
+//     the 80-word layer header (NF_LAYER_HDR, see LayerHdr below)
 //     then `nets` conditioner blocks (1 for spline: param_net; 2 for affine: s_net, b_net), each:
 //       W1k [HP][W1S]   : {W1[k][0..D-1], zero pad.., b1[k] at slot W1S-1}
 //       W2t [HP][HP]    : W2t[k][j] = W2[j][k]
@@ -68,6 +67,18 @@ static inline StackHdr nf_stack_hdr(const void* hdr_host) {
     return h;
 }
 
+#ifdef __CUDACC__
+// the kernels' read of the same words at the start of the packed buffer
+__device__ __forceinline__ StackHdr nf_stack_hdr_device(const float* __restrict__ p) {
+    const int* q = reinterpret_cast<const int*>(p);
+    StackHdr h;
+    h.magic = q[0]; h.D = q[1]; h.H = q[2]; h.HP = q[3]; h.K = q[4]; h.L = q[5]; h.W1S = q[6]; h.NO = q[7];
+    h.layer_stride = q[8]; h.bn_between = q[9];
+    h.bound = p[10]; h.min_w = p[11]; h.min_h = p[12]; h.min_d = p[13]; h.scale_w = p[14]; h.scale_h = p[15];
+    return h;
+}
+#endif
+
 static inline int nf_stack_hp(int H) { return H <= 64 ? 64 : 128; }
 static inline int nf_stack_w1s(int D) { return D <= 3 ? 4 : 12; }
 static inline int64_t nf_stack_net_words(int HP, int W1S, int NO) {
@@ -115,7 +126,42 @@ inline int stack_smem_attributes(Kern kern, size_t smem) {
     return NF_OK;
 }
 
-}  // namespace nf
+// The 80-word header at the start of every layer block, as packing._layer_header writes it (ints as int32 bit
+// patterns, one 8-word section per field):
+//   mask | tdim (int) | meta: {Dt, rescale, bn_on (int), bn_ld (float)} | r_in | r_lo | r_out | bn_mean | bn_sd | bn_gamma
+//   | bn_beta
+// A view of it in shared memory.
+struct LayerHdr {
+    enum : int { kMask = 0, kTdim = 8, kMeta = 16, kRin = 24, kRlo = 32, kRout = 40,
+                 kBnMean = 48, kBnSd = 56, kBnGamma = 64, kBnBeta = 72 };
+    const float* p;
+    __device__ __forceinline__ const float* mask() const { return p + kMask; }
+    __device__ __forceinline__ bool rescale() const { return reinterpret_cast<const int*>(p + kMeta)[1] != 0; }
+    __device__ __forceinline__ bool bn_on() const { return reinterpret_cast<const int*>(p + kMeta)[2] != 0; }
+    // data_min / data_max rescale of a spline layer (spline_coupling_layer.py:101-102): dim d into spline coordinates
+    // [-bound, bound] and back
+    __device__ __forceinline__ float to_spline(float v, int d, float bound) const {
+        return p[kRin + d] * (v - p[kRlo + d]) - bound;
+    }
+    __device__ __forceinline__ float from_spline(float v, int d, float bound) const {
+        return (v + bound) * p[kRout + d] + p[kRlo + d];
+    }
+};
+static_assert(LayerHdr::kBnBeta + 8 == NF_LAYER_HDR, "LayerHdr covers the layer header");
+
+// between-layer BatchNorm as an invertible affine on running stats (normalizing_flow_model.py:67-128), one row
+template <int DM>
+__device__ __forceinline__ void nf_stack_bn_between(LayerHdr lh, int D, bool inverse, float (&xv)[DM], float& tot) {
+    const float* mean = lh.p + LayerHdr::kBnMean; const float* sd = lh.p + LayerHdr::kBnSd;
+    const float* gm = lh.p + LayerHdr::kBnGamma; const float* bt = lh.p + LayerHdr::kBnBeta;
+    const float bn_ld = lh.p[LayerHdr::kMeta + 3];
+#pragma unroll
+    for (int d = 0; d < DM; ++d) if (d < D) {
+        if (!inverse) xv[d] = (xv[d] - mean[d]) / sd[d] * gm[d] + bt[d];
+        else          xv[d] = (xv[d] - bt[d]) / gm[d] * sd[d] + mean[d];
+    }
+    tot = inverse ? tot - bn_ld : tot + bn_ld;
+}
 
 // log N(z; 0, I) + log_det for one row held in registers (same arithmetic as std_normal_log_prob_fwd_kernel)
 template <int DM>
@@ -125,4 +171,18 @@ __device__ __forceinline__ float nf_stack_row_head(const float (&z)[DM], int D, 
     for (int d = 0; d < DM; ++d) if (d < D) acc += -0.5f * z[d] * z[d];
     return acc - (float)(0.5 * (double)D * 1.8378770664093453) + log_det;
 }
+
+// Row epilogue (r < B): the row into y unless NF_STACK_SKIP_Y, then the per-row value into ld:
+// -tot when sampling, the log-prob head under NF_STACK_LOG_PROB_HEAD, tot otherwise
+template <int DM, bool SAMPLE>
+__device__ __forceinline__ void nf_stack_row_store(float* __restrict__ y, float* __restrict__ ld, int64_t r, int D, int flags,
+                                                   const float (&z)[DM], float tot) {
+    if (!(flags & NF_STACK_SKIP_Y)) {
+#pragma unroll
+        for (int d = 0; d < DM; ++d) if (d < D) st_stream(y + r * D + d, z[d]);
+    }
+    st_stream(ld + r, SAMPLE ? -tot : (flags & NF_STACK_LOG_PROB_HEAD) ? nf_stack_row_head<DM>(z, D, tot) : tot);
+}
+
+}  // namespace nf
 #endif

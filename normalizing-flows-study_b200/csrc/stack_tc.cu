@@ -29,25 +29,26 @@ constexpr int kTcSub = 4;            // sub-tiles (of 128 rows) per weight stagi
 constexpr int kColAhi = 0, kColAlo = 64, kColD2 = 128, kColD3 = 192;
 constexpr int kTmemCols = 256;
 
-struct TcHdr {
-    int D, H, K, L, W1S, NO3, blk_words, bn_between, nets, aux_words;
-    float bound, min_w, min_h, min_d, scale_w, scale_h;
-};
-
-__device__ __forceinline__ TcHdr read_tc_hdr(const float* __restrict__ p) {
-    const int* q = reinterpret_cast<const int*>(p);
-    TcHdr h;
-    h.D = q[1]; h.H = q[2]; h.nets = q[3]; h.K = q[4]; h.L = q[5]; h.W1S = q[6]; h.NO3 = q[7];
-    h.blk_words = q[8]; h.bn_between = q[9];
-    h.bound = p[10]; h.min_w = p[11]; h.min_h = p[12]; h.min_d = p[13]; h.scale_w = p[14]; h.scale_h = p[15];
-    h.aux_words = 0;
-    return h;
-}
-
 __device__ __forceinline__ float relu_keepnan(float x) {      // torch.relu: NaN stays NaN
     float r;
     asm("max.NaN.f32 %0, %1, 0f00000000;" : "=f"(r) : "f"(x));
     return r;
+}
+
+// Row state of a tile in shared memory, sx [kTcSub][DM+1][128]: thread t of sub-tile s keeps its row's DM values and
+// then its log-det slot, from the row load through every layer to the row store.
+template <int DM>
+__device__ __forceinline__ float slab_load(const float* sx, int s, int t, float (&xv)[DM]) {
+#pragma unroll
+    for (int d = 0; d < DM; ++d) xv[d] = sx[(s * (DM + 1) + d) * kTcThreads + t];
+    return sx[(s * (DM + 1) + DM) * kTcThreads + t];
+}
+
+template <int DM>
+__device__ __forceinline__ void slab_store(float* sx, int s, int t, const float (&xv)[DM], float tot) {
+#pragma unroll
+    for (int d = 0; d < DM; ++d) sx[(s * (DM + 1) + d) * kTcThreads + t] = xv[d];
+    sx[(s * (DM + 1) + DM) * kTcThreads + t] = tot;
 }
 
 // SAMPLE variants of the stack kernels (nf_*_sample): the row is the N(0, I) draw of nf_rng.cuh instead of a load, and
@@ -69,17 +70,16 @@ __device__ __forceinline__ void draw_row_tc(float* srow, int64_t r, int64_t B, i
     srow[DM * kTcThreads] = -lz;
 }
 
-// between-layer BatchNorm as an invertible affine on running stats (normalizing_flow_model.py:67-128)
-template <int DM>
-__device__ __forceinline__ void bn_between_tc(const float* __restrict__ sL, int D, bool inverse, float (&xv)[DM], float& tot) {
-    const float* mean = sL + 48; const float* sd = sL + 56; const float* gm = sL + 64; const float* bt = sL + 72;
-    const float bn_ld = sL[16 + 3];
-#pragma unroll
-    for (int d = 0; d < DM; ++d) if (d < D) {
-        if (!inverse) xv[d] = (xv[d] - mean[d]) / sd[d] * gm[d] + bt[d];
-        else          xv[d] = (xv[d] - bt[d]) / gm[d] * sd[d] + mean[d];
-    }
-    tot = inverse ? tot - bn_ld : tot + bn_ld;
+// One CTA-wide round of the coupling and MADE kernels: every thread's TMEM stores are done, warp 0 issues the MMAs
+// (`issue`, completing on `bar`), and every thread waits for them.
+template <typename Issue>
+__device__ __forceinline__ void cta_mma_round(int warp, uint64_t* bar, uint32_t& phase, Issue issue) {
+    tc::wait_st();
+    tc::fence_before_sync();
+    __syncthreads();
+    if (warp == 0) { tc::fence_after_sync(); issue(); }
+    tc::mbar_wait(bar, phase); phase ^= 1;
+    tc::fence_after_sync();
 }
 
 // Layer 1 for data_dim <= 3 (W1S == 4), two hidden units per packed-fp32 FMA.  The host stores the units in pairs:
@@ -288,8 +288,8 @@ spline_stack_tc2_body(int tid, const float* __restrict__ packed, const float* __
                       unsigned long long* rng_state, const float* __restrict__ ctx, int64_t ctx_div, int C) {
     const int inverse = flags & NF_STACK_INVERSE;
     extern __shared__ __align__(1024) float sbuf[];
-    const TcHdr hd = read_tc_hdr(packed);
-    const int D = hd.D, K = (KS > 0) ? KS : hd.K, L = hd.L, W1S = hd.W1S, NO3 = hd.NO3, BW = hd.blk_words;
+    const StackHdr hd = nf_stack_hdr_device(packed);
+    const int D = hd.D, K = (KS > 0) ? KS : hd.K, L = hd.L, W1S = hd.W1S, NO3 = hd.NO, BW = hd.layer_stride;
     float* sx = sbuf + (size_t)2 * BW;                         // [kTcSub][DM+1][128] row state
     uint64_t* bars = reinterpret_cast<uint64_t*>(sx + kTcSub * (DM + 1) * kTcThreads);
     uint64_t* mbar = bars;                                     // [2] MMA completion, one per warpgroup
@@ -356,9 +356,9 @@ spline_stack_tc2_body(int tid, const float* __restrict__ packed, const float* __
             wphase ^= (1u << buf);
             const float* sL = sbuf + (size_t)buf * BW;
             const float* net = sL + NF_LAYER_HDR;
-            const int* meta = reinterpret_cast<const int*>(sL + 16);
-            const bool rescale = meta[1] != 0, bn_on = meta[2] != 0;
-            const float* mask = sL;
+            const LayerHdr lh{sL};
+            const bool rescale = lh.rescale(), bn_on = lh.bn_on();
+            const float* mask = lh.mask();
             const uint32_t w2hi = tc::smem_u32(net + off.w2hi), w2lo = tc::smem_u32(net + off.w2lo);
             const uint32_t w3hi = tc::smem_u32(net + off.w3hi), w3lo = tc::smem_u32(net + off.w3lo);
             const float* sW1k = net + off.w1k;
@@ -366,16 +366,14 @@ spline_stack_tc2_body(int tid, const float* __restrict__ packed, const float* __
 
 #pragma unroll 1
             for (int s = wg; s < kTcSub; s += 2) {
-                float xv[DM], tot;
-#pragma unroll
-                for (int d = 0; d < DM; ++d) xv[d] = sx[(s * (DM + 1) + d) * kTcThreads + wtid];
-                tot = sx[(s * (DM + 1) + DM) * kTcThreads + wtid];
-                if (inverse && bn_on) bn_between_tc<DM>(sL, D, true, xv, tot);
+                float xv[DM];
+                float tot = slab_load<DM>(sx, s, wtid, xv);
+                if (inverse && bn_on) nf_stack_bn_between<DM>(lh, D, true, xv, tot);
                 float xs[DM], xa[DM];
 #pragma unroll
                 for (int d = 0; d < DM; ++d) {
                     float v = xv[d];
-                    if (rescale && d < D) v = sL[24 + d] * (v - sL[32 + d]) - hd.bound;
+                    if (rescale && d < D) v = lh.to_spline(v, d, hd.bound);
                     xs[d] = v;
                     xa[d] = (d < D) ? v * mask[d] : 0.f;
                 }
@@ -482,7 +480,7 @@ spline_stack_tc2_body(int tid, const float* __restrict__ packed, const float* __
                         }
                         float out, lad;
                         rqs_eval<float, KMAX, true>(xs[d], uw, uh, ud, K, inverse != 0, cfg, out, lad);
-                        if (rescale) out = (out + hd.bound) * sL[40 + d] + sL[32 + d];
+                        if (rescale) out = lh.from_spline(out, d, hd.bound);
                         xv[d] = out;
                         lsum += lad;
                         ++t;
@@ -492,10 +490,8 @@ spline_stack_tc2_body(int tid, const float* __restrict__ packed, const float* __
 #pragma unroll
                 for (int d = 0; d < DM; ++d) xv[d] = scrub0(xv[d]);
                 tot += scrub0(lsum);
-                if (!inverse && bn_on) bn_between_tc<DM>(sL, D, false, xv, tot);
-#pragma unroll
-                for (int d = 0; d < DM; ++d) sx[(s * (DM + 1) + d) * kTcThreads + wtid] = xv[d];
-                sx[(s * (DM + 1) + DM) * kTcThreads + wtid] = tot;
+                if (!inverse && bn_on) nf_stack_bn_between<DM>(lh, D, false, xv, tot);
+                slab_store<DM>(sx, s, wtid, xv, tot);
             }
             buf ^= 1;
         }
@@ -558,8 +554,8 @@ coupling_stack_tc_kernel(const float* __restrict__ packed, const float* __restri
     constexpr int kTmemCols = (HP == 64) ? 256 : 512;
     const int inverse = flags & NF_STACK_INVERSE;
     extern __shared__ __align__(1024) float sbuf[];
-    const TcHdr hd = read_tc_hdr(packed);
-    const int D = hd.D, L = hd.L, W1S = hd.W1S, NO3 = hd.NO3, NBW = hd.blk_words;       // NBW: words per net block
+    const StackHdr hd = nf_stack_hdr_device(packed);
+    const int D = hd.D, L = hd.L, W1S = hd.W1S, NO3 = hd.NO, NBW = hd.layer_stride;     // NBW: words per net block
     float* sx = sbuf + (size_t)NBUF * NBW;                       // [kTcSub][DM+1][128] row state
     float* sraw = sx + kTcSub * (DM + 1) * kTcThreads;           // [kTcSub][DM][128] raw s_net outputs
     float* shdr = sraw + kTcSub * DM * kTcThreads;               // [80] layer header (outlives the net-s buffer)
@@ -627,48 +623,32 @@ coupling_stack_tc_kernel(const float* __restrict__ packed, const float* __restri
                 __syncthreads();
             }
             const float* nb = sN + NF_LAYER_HDR;
-            const int* meta = reinterpret_cast<const int*>(shdr + 16);
-            const bool bn_on = meta[2] != 0;
-            const float* mask = shdr;
+            const LayerHdr lh{shdr};
+            const bool bn_on = lh.bn_on();
+            const float* mask = lh.mask();
             const uint32_t w2hi = tc::smem_u32(nb + off.w2hi), w2lo = tc::smem_u32(nb + off.w2lo);
             const uint32_t w3hi = tc::smem_u32(nb + off.w3hi), w3lo = tc::smem_u32(nb + off.w3lo);
 #pragma unroll 1
             for (int s = 0; s < nsub; ++s) {
-                float xv[DM], tot;
-#pragma unroll
-                for (int d = 0; d < DM; ++d) xv[d] = sx[(s * (DM + 1) + d) * kTcThreads + tid];
-                tot = sx[(s * (DM + 1) + DM) * kTcThreads + tid];
+                float xv[DM];
+                float tot = slab_load<DM>(sx, s, tid, xv);
                 if (net == 0 && inverse && bn_on) {
-                    bn_between_tc<DM>(shdr, D, true, xv, tot);
-#pragma unroll
-                    for (int d = 0; d < DM; ++d) sx[(s * (DM + 1) + d) * kTcThreads + tid] = xv[d];
-                    sx[(s * (DM + 1) + DM) * kTcThreads + tid] = tot;
+                    nf_stack_bn_between<DM>(lh, D, true, xv, tot);
+                    slab_store<DM>(sx, s, tid, xv, tot);
                 }
                 float xa[DM];
 #pragma unroll
                 for (int d = 0; d < DM; ++d) xa[d] = (d < D) ? xv[d] * mask[d] : 0.f;
                 layer1_to_tmem<DM, HP>(nb + off.w1k, W1S, xa, lane_addr);
-                tc::wait_st();
-                tc::fence_before_sync();
-                __syncthreads();
-                if (warp == 0) {
-                    tc::fence_after_sync();
+                cta_mma_round(warp, &bar, phase, [&] {
                     if (HP == 64) tc::warp_issue_gemm_k64_3xtf32(tb, kColD2, kColAhi, kColAlo, w2hi, w2lo, 64u, &bar);
                     else tc::warp_issue_gemm_krange_3xtf32(tb, kColD2, kColAhi, kColAlo, w2hi, w2lo, (uint32_t)HP, 0, HP / 8, 0u, &bar);
-                }
-                tc::mbar_wait(&bar, phase); phase ^= 1;
-                tc::fence_after_sync();
+                });
                 hidden2_to_tmem<HP>(nb + off.b2, lane_addr);
-                tc::wait_st();
-                tc::fence_before_sync();
-                __syncthreads();
-                if (warp == 0) {
-                    tc::fence_after_sync();
+                cta_mma_round(warp, &bar, phase, [&] {
                     if (HP == 64) tc::warp_issue_gemm_k64_3xtf32(tb, kColD3, kColAhi, kColAlo, w3hi, w3lo, (uint32_t)NO3, &bar);
                     else tc::warp_issue_gemm_krange_3xtf32(tb, kColD3, kColAhi, kColAlo, w3hi, w3lo, (uint32_t)NO3, 0, HP / 8, 0u, &bar);
-                }
-                tc::mbar_wait(&bar, phase); phase ^= 1;
-                tc::fence_after_sync();
+                });
                 uint32_t p[8];
                 tc::tmem_ld8(lane_addr + kColD3, p);
                 tc::wait_ld();
@@ -688,10 +668,8 @@ coupling_stack_tc_kernel(const float* __restrict__ packed, const float* __restri
                         lsum += t;
                     }
                     tot += scrub0(lsum);
-                    if (!inverse && bn_on) bn_between_tc<DM>(shdr, D, false, xv, tot);
-#pragma unroll
-                    for (int d = 0; d < DM; ++d) sx[(s * (DM + 1) + d) * kTcThreads + tid] = xv[d];
-                    sx[(s * (DM + 1) + DM) * kTcThreads + tid] = tot;
+                    if (!inverse && bn_on) nf_stack_bn_between<DM>(lh, D, false, xv, tot);
+                    slab_store<DM>(sx, s, tid, xv, tot);
                 }
             }
             if (NBUF == 2) buf ^= 1;
@@ -747,8 +725,8 @@ made_stack_tc_kernel(const float* __restrict__ packed, const float* __restrict__
                      unsigned long long* rng_state) {
     const int inverse = flags & NF_STACK_INVERSE;
     extern __shared__ __align__(1024) float sbuf[];
-    const TcHdr hd = read_tc_hdr(packed);
-    const int D = hd.D, L = hd.L, W1S = hd.W1S, NBW = hd.blk_words;
+    const StackHdr hd = nf_stack_hdr_device(packed);
+    const int D = hd.D, L = hd.L, W1S = hd.W1S, NBW = hd.layer_stride;
     float* sx = sbuf + (size_t)NBW;                              // [kTcSub][DM+1][128] row state
     uint64_t* bars = reinterpret_cast<uint64_t*>(sx + kTcSub * (DM + 1) * kTcThreads);
     uint64_t& bar = bars[0];
@@ -794,21 +772,18 @@ made_stack_tc_kernel(const float* __restrict__ packed, const float* __restrict__
                 tc::bulk_g2s(sbuf, blocks + (size_t)layer * NBW, (uint32_t)NBW * 4u, &wbar);
             }
             tc::mbar_wait(&wbar, wphase); wphase ^= 1u;
-            const float* shdr = sbuf;
+            const LayerHdr lh{sbuf};
             const float* nb = sbuf + NF_LAYER_HDR;
-            const int* meta = reinterpret_cast<const int*>(shdr + 16);
-            const bool bn_on = meta[2] != 0;
+            const bool bn_on = lh.bn_on();
             const uint32_t w2hi = tc::smem_u32(nb + off.w2hi), w2lo = tc::smem_u32(nb + off.w2lo);
             const uint32_t w3hi = tc::smem_u32(nb + off.w3hi), w3lo = tc::smem_u32(nb + off.w3lo);
             const uint32_t w4hi = tc::smem_u32(nb + off.w4hi), w4lo = tc::smem_u32(nb + off.w4lo);
             const float* b4 = nb + off.b4;
 #pragma unroll 1
             for (int s = 0; s < nsub; ++s) {
-                float xv[DM], tot;
-#pragma unroll
-                for (int d = 0; d < DM; ++d) xv[d] = sx[(s * (DM + 1) + d) * kTcThreads + tid];
-                tot = sx[(s * (DM + 1) + DM) * kTcThreads + tid];
-                if (inverse && bn_on) bn_between_tc<DM>(shdr, D, true, xv, tot);
+                float xv[DM];
+                float tot = slab_load<DM>(sx, s, tid, xv);
+                if (inverse && bn_on) nf_stack_bn_between<DM>(lh, D, true, xv, tot);
                 // conditioner input: the row itself (parallel), or (out_0, 0) with out_0 from the output biases (sequential, D == 2)
                 float xa[DM], c0 = 0.f, t0 = 0.f;
 #pragma unroll
@@ -820,26 +795,11 @@ made_stack_tc_kernel(const float* __restrict__ packed, const float* __restrict__
                     xa[0] = c0;
                 }
                 layer1_to_tmem<DM, 64>(nb + off.w1k, W1S, xa, lane_addr);
-                tc::wait_st();
-                tc::fence_before_sync();
-                __syncthreads();
-                if (warp == 0) { tc::fence_after_sync(); tc::warp_issue_gemm_k64_3xtf32(tb, kColD2, kColAhi, kColAlo, w2hi, w2lo, 64u, &bar); }
-                tc::mbar_wait(&bar, phase); phase ^= 1;
-                tc::fence_after_sync();
+                cta_mma_round(warp, &bar, phase, [&] { tc::warp_issue_gemm_k64_3xtf32(tb, kColD2, kColAhi, kColAlo, w2hi, w2lo, 64u, &bar); });
                 hidden2_to_tmem<64>(nb + off.b2, lane_addr);
-                tc::wait_st();
-                tc::fence_before_sync();
-                __syncthreads();
-                if (warp == 0) { tc::fence_after_sync(); tc::warp_issue_gemm_k64_3xtf32(tb, kColD2, kColAhi, kColAlo, w3hi, w3lo, 64u, &bar); }
-                tc::mbar_wait(&bar, phase); phase ^= 1;
-                tc::fence_after_sync();
+                cta_mma_round(warp, &bar, phase, [&] { tc::warp_issue_gemm_k64_3xtf32(tb, kColD2, kColAhi, kColAlo, w3hi, w3lo, 64u, &bar); });
                 hidden2_to_tmem<64>(nb + off.b3, lane_addr);
-                tc::wait_st();
-                tc::fence_before_sync();
-                __syncthreads();
-                if (warp == 0) { tc::fence_after_sync(); tc::warp_issue_gemm_k64_3xtf32(tb, kColD3, kColAhi, kColAlo, w4hi, w4lo, 16u, &bar); }
-                tc::mbar_wait(&bar, phase); phase ^= 1;
-                tc::fence_after_sync();
+                cta_mma_round(warp, &bar, phase, [&] { tc::warp_issue_gemm_k64_3xtf32(tb, kColD3, kColAhi, kColAlo, w4hi, w4lo, 16u, &bar); });
                 uint32_t p[16];
                 tc::tmem_ld16(lane_addr + kColD3, p);
                 tc::wait_ld();
@@ -868,10 +828,8 @@ made_stack_tc_kernel(const float* __restrict__ packed, const float* __restrict__
                     xv[1] = is_finite(c1) ? c1 : (iaf ? xv[1] : 0.f);
                 }
                 tot += clamp_mm(scrub0(lsum), -lim, lim);
-                if (!inverse && bn_on) bn_between_tc<DM>(shdr, D, false, xv, tot);
-#pragma unroll
-                for (int d = 0; d < DM; ++d) sx[(s * (DM + 1) + d) * kTcThreads + tid] = xv[d];
-                sx[(s * (DM + 1) + DM) * kTcThreads + tid] = tot;
+                if (!inverse && bn_on) nf_stack_bn_between<DM>(lh, D, false, xv, tot);
+                slab_store<DM>(sx, s, tid, xv, tot);
             }
         }
         for (int s = 0; s < nsub; ++s) {

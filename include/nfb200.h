@@ -344,6 +344,28 @@ NF_API int nf_spline_stack_ctx_tc_sample(const void* packed, const void* hdr_hos
 NF_API int nf_spline_stack_ctx_tc_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes,
                                                const void* context, int64_t ctx_rows, int64_t ctx_div, void* rng_state,
                                                void* x, void* log_q, int64_t B, nf_stream_t stream);
+/* ---- conditional affine coupling stack on the tensor cores: L x CouplingLayer with context_dim = C (1 <= C <= 8), whose
+ * s_net and b_net both read [x * mask, c] in their first Linear.  Same contract, flags and envelope as
+ * nf_coupling_stack_tc_forward / _sample / _sample_state, with `packed` in the conditional layout (magic 'NFD2', header
+ * word 3 = C; csrc/stack_small.cuh).
+ * context: float32 [ctx_rows][C], row-major; row r of the batch reads context row r / ctx_div (ctx_div = 1: one context
+ * row per row; ctx_div = B: one row broadcast to all; ctx_div = n: n consecutive sampled rows per context row).
+ * Refused before any CUDA call, after the checks of the other stacks (B == 0 returns first, advancing a device state):
+ * context == NULL -> NF_ERR_NULL; ctx_div < 1 or ctx_rows < ceil(B / ctx_div) -> NF_ERR_BAD_SHAPE; C outside 1..8, or B
+ * or ctx_div beyond 2^31 - 1 -> NF_ERR_UNSUPPORTED.  An unconditional pack has another magic (NF_ERR_BAD_SHAPE), and so
+ * has an 'NFD2' pack passed to the unconditional entry points.  The context does not enter the N(0, I) draw: the same
+ * (seed, offset) draws the same rows as nf_coupling_stack_tc_sample. */
+NF_API int nf_coupling_stack_ctx_tc_forward(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
+                                            const void* context, int64_t ctx_rows, int64_t ctx_div, void* y, void* ld,
+                                            int64_t B, int flags, nf_stream_t stream);
+NF_API int nf_coupling_stack_ctx_tc_sample(const void* packed, const void* hdr_host, int64_t packed_bytes,
+                                           const void* context, int64_t ctx_rows, int64_t ctx_div, uint64_t seed,
+                                           uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream);
+NF_API int nf_coupling_stack_ctx_tc_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes,
+                                                 const void* context, int64_t ctx_rows, int64_t ctx_div, void* rng_state,
+                                                 void* x, void* log_q, int64_t B, nf_stream_t stream);
+/* words per NET block of the 'NFD2' layout for data_dim D and hidden_dim H (<= 128); -1 = unsupported */
+NF_API int64_t nf_coupling_stack_ctx_tc_block_words_hidden(int D, int H);
 
 /* ---- a8/a10 and the conditioner MLPs on the tensor cores: y[M,N] = relu?(x[M,K] * W[N,K]^T + bias) ---------
  * fp32 in / fp32 out, 3xTF32 on tcgen05 (fp32-accurate), TMA-fed, accumulators in TMEM (csrc/gemm_tc2.cu).

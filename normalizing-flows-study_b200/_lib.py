@@ -94,6 +94,10 @@ _SIGNATURES = {
     "nf_spline_stack_ctx_tc_forward": [_P, _P, _L, _P, _P, _L, _L, _P, _P, _L, _I, _P],
     "nf_spline_stack_ctx_tc_sample": [_P, _P, _L, _P, _L, _L, _U, _U, _P, _P, _L, _P],
     "nf_spline_stack_ctx_tc_sample_state": [_P, _P, _L, _P, _L, _L, _P, _P, _P, _L, _P],
+    "nf_coupling_stack_ctx_tc_forward": [_P, _P, _L, _P, _P, _L, _L, _P, _P, _L, _I, _P],
+    "nf_coupling_stack_ctx_tc_sample": [_P, _P, _L, _P, _L, _L, _U, _U, _P, _P, _L, _P],
+    "nf_coupling_stack_ctx_tc_sample_state": [_P, _P, _L, _P, _L, _L, _P, _P, _P, _L, _P],
+    "nf_coupling_stack_ctx_tc_block_words_hidden": [_I, _I],
     "nf_made_chain_bf16_forward": [_P] * 9 + [_P, _P, _P, _L, _I, _I, _I, _I, _P],
     "nf_batchnorm_forward_staged": [_P] * 9 + [_L, _I, _D, _D, _I, _I, _L, _I, _P],
     "nf_batchnorm_backward_staged": [_P] * 10 + [_L, _I, _I, _I, _L, _I, _P, _P],
@@ -108,6 +112,7 @@ _RESTYPES = {
     "nf_ar_blocked_workspace_floats": _L,
     "nf_coupling_stack_tc_block_words": _L,
     "nf_coupling_stack_tc_block_words_hidden": _L,
+    "nf_coupling_stack_ctx_tc_block_words_hidden": _L,
     "nf_made_stack_tc_block_words": _L,
     "nf_linear_wgrad_tc_workspace": _L,
 }

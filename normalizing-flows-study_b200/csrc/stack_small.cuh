@@ -6,7 +6,7 @@
 //
 //   header (NF_STACK_HDR words, read on the host through StackHdr below):
 //     [0] magic   [1] D   [2] H (true hidden_dim)   [3] HP (padded: 64 or 128; the tcgen05 layouts of stack_tc.cu
-//     store the number of conditioner nets per layer here instead: 1 spline / MADE, 2 affine; 'NFC2' the context width C)   [4] K (spline) / 0 (affine)
+//     store the number of conditioner nets per layer here instead: 1 spline / MADE, 2 affine; 'NFC2' / 'NFD2' the context width C)   [4] K (spline) / 0 (affine)
 //     [5] L       [6] W1S (words per hidden unit in W1k: 4 if D<=3 else 12)      [7] NO (padded #outputs of the head)
 //     [8] layer_stride (words)   [9] bn_between (0/1)   [10] bound   [11] min_w  [12] min_h  [13] min_d
 //     [14] scale_w = 1-min_w*K   [15] scale_h
@@ -27,6 +27,11 @@
 //       Wc  [32][8][2]  : unit pairs (2p, 2p+1), 8 context slots each: Wc[p][c][e] = W1[2p+e][D+c], zero for c >= C
 // W1k keeps the x columns W1[k][0..D-1] exactly as in 'NFS2', so a pack whose context columns are zero computes what
 // the 'NFS2' pack of the remaining weights computes.
+// The tcgen05 affine layout 'NFA2' has two such net blocks per layer (s_net, b_net; HP = 64 or 128 hidden units, each
+// block led by 80 words: the layer header for s_net, zeros for b_net).  Its conditional twin 'NFD2' (CouplingLayer with
+// context_dim = C, 1 <= C <= 8) stores C in header word [3] and gives EACH net block a Wc [HP/2][8][2] section after b3,
+// laid out as above, from the first Linear with its BatchNorm folded in: the fold scales whole rows of the [H, D + C]
+// weight, context columns included, before they are split into W1k and Wc.
 #pragma once
 #include <stdint.h>
 #include <string.h>
@@ -38,6 +43,7 @@
 #define NF_STACK_MAGIC_AFFINE_TC 0x4e464132  /* 'NFA2' */
 #define NF_STACK_MAGIC_MADE_TC 0x4e464d32    /* 'NFM2': MADE / MAF / IAF stack on the tensor cores, see stack_tc.cu */
 #define NF_STACK_MAGIC_SPLINE_CTX_TC 0x4e464332  /* 'NFC2': conditional spline stack on the tensor cores, see below */
+#define NF_STACK_MAGIC_AFFINE_CTX_TC 0x4e464432  /* 'NFD2': conditional affine coupling stack on the tensor cores */
 #define NF_STACK_HDR 16
 #define NF_LAYER_HDR 80
 #define NF_STACK_DMAX 8

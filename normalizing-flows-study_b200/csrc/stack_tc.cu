@@ -96,39 +96,6 @@ __device__ __forceinline__ float2 layer1_pair(const float* __restrict__ sW1k, in
     return make_float2(relu_keepnan(t.x), relu_keepnan(t.y));
 }
 
-// (a): hidden layer 1 of one conditioner for this thread's row -> TMEM A operand (hi at kColAhi, lo at kColAlo)
-template <int DM, int HP = 64>
-__device__ __forceinline__ void layer1_to_tmem(const float* __restrict__ sW1k, int W1S, const float (&xa)[DM], uint32_t lane_addr) {
-    constexpr int kColAhi = 0, kColAlo = HP;        // TMEM columns of an HP-wide conditioner: A hi | A lo | D2 | D3
-#pragma unroll
-    for (int c = 0; c < HP / 16; ++c) {
-        uint32_t hi[16], lo[16];
-        if constexpr (DM <= 4) {
-#pragma unroll
-            for (int j = 0; j < 16; j += 2) {
-                const float2 t = layer1_pair<DM>(sW1k, (c * 16 + j) >> 1, xa);
-                tc::split_tf32_x2(t.x, t.y, hi[j], hi[j + 1], lo[j], lo[j + 1]);
-            }
-        } else {
-            float t16[16];
-#pragma unroll
-            for (int j = 0; j < 16; ++j) {
-                const float* w1 = sW1k + (c * 16 + j) * W1S;
-                const float4 v0 = *reinterpret_cast<const float4*>(w1);
-                const float4 v1 = *reinterpret_cast<const float4*>(w1 + 4);
-                float t = w1[W1S - 1];
-                t = fmaf(v0.x, xa[0], t); t = fmaf(v0.y, xa[1], t); t = fmaf(v0.z, xa[2], t); t = fmaf(v0.w, xa[3], t);
-                t = fmaf(v1.x, xa[4], t); t = fmaf(v1.y, xa[5], t); t = fmaf(v1.z, xa[6], t); t = fmaf(v1.w, xa[7], t);
-                t16[j] = relu_keepnan(t);
-            }
-#pragma unroll
-            for (int j = 0; j < 16; j += 2) tc::split_tf32_x2(t16[j], t16[j + 1], hi[j], hi[j + 1], lo[j], lo[j + 1]);
-        }
-        tc::tmem_st16(lane_addr + kColAhi + c * 16, hi);
-        tc::tmem_st16(lane_addr + kColAlo + c * 16, lo);
-    }
-}
-
 // (c): D2 + b2 -> ReLU -> split -> A operand.  Four 16-column loads are issued before each wait (64 columns at a time).
 template <int HP = 64>
 __device__ __forceinline__ void hidden2_to_tmem(const float* __restrict__ sb2, uint32_t lane_addr) {
@@ -166,7 +133,8 @@ __host__ __device__ inline int pad256(int x) { return (x + 255) & ~255; }
 // nets conditioner blocks follow the 80-word layer header; every block is a multiple of 256 words so that the
 // weight images stay 1024-byte aligned
 // HP: hidden units padded to 64 (every kernel here) or 128 (the affine coupling stack with hidden_dim in (64, 128])
-// CW: context columns of the conditional spline layout ('NFC2': Wc[HP/2][CW][2] after b3), 0 in every other layout
+// CW: context columns of the conditional layouts ('NFC2' spline, 'NFD2' affine: Wc[HP/2][CW][2] after b3), 0 in every other
+// layout
 __host__ __device__ inline BlkOff blk_offsets(int W1S, int NO3, int HP = 64, int CW = 0) {
     BlkOff o;
     o.w1k = 0; o.b2 = HP * W1S; o.b3 = o.b2 + HP;
@@ -261,6 +229,45 @@ __device__ __forceinline__ void layer1_chunk_ctx(const float* __restrict__ sW1k,
 #pragma unroll
     for (int q = 0; q < 8; ++q)
         tc::split_tf32_x2(relu_keepnan(t[q].x), relu_keepnan(t[q].y), hi[2 * q], hi[2 * q + 1], lo[2 * q], lo[2 * q + 1]);
+}
+
+// (a): hidden layer 1 of one conditioner for this thread's row -> TMEM A operand (hi at kColAhi, lo at kColAlo).
+// CM > 0 (the conditional affine layout 'NFD2'): each 16-unit chunk goes through layer1_chunk_ctx, which adds the C
+// context columns of row `crow` (Wc at sWc) after the x FMAs of every unit, before the ReLU.
+template <int DM, int HP = 64, int CM = 0>
+__device__ __forceinline__ void layer1_to_tmem(const float* __restrict__ sW1k, int W1S, const float (&xa)[DM], uint32_t lane_addr,
+                                               const float* __restrict__ sWc = nullptr, const float* __restrict__ crow = nullptr,
+                                               int C = 0) {
+    constexpr int kColAhi = 0, kColAlo = HP;        // TMEM columns of an HP-wide conditioner: A hi | A lo | D2 | D3
+#pragma unroll
+    for (int c = 0; c < HP / 16; ++c) {
+        uint32_t hi[16], lo[16];
+        if constexpr (CM > 0) {
+            layer1_chunk_ctx<DM, CM>(sW1k, W1S, sWc, xa, crow, C, c * 16, hi, lo);
+        } else if constexpr (DM <= 4) {
+#pragma unroll
+            for (int j = 0; j < 16; j += 2) {
+                const float2 t = layer1_pair<DM>(sW1k, (c * 16 + j) >> 1, xa);
+                tc::split_tf32_x2(t.x, t.y, hi[j], hi[j + 1], lo[j], lo[j + 1]);
+            }
+        } else {
+            float t16[16];
+#pragma unroll
+            for (int j = 0; j < 16; ++j) {
+                const float* w1 = sW1k + (c * 16 + j) * W1S;
+                const float4 v0 = *reinterpret_cast<const float4*>(w1);
+                const float4 v1 = *reinterpret_cast<const float4*>(w1 + 4);
+                float t = w1[W1S - 1];
+                t = fmaf(v0.x, xa[0], t); t = fmaf(v0.y, xa[1], t); t = fmaf(v0.z, xa[2], t); t = fmaf(v0.w, xa[3], t);
+                t = fmaf(v1.x, xa[4], t); t = fmaf(v1.y, xa[5], t); t = fmaf(v1.z, xa[6], t); t = fmaf(v1.w, xa[7], t);
+                t16[j] = relu_keepnan(t);
+            }
+#pragma unroll
+            for (int j = 0; j < 16; j += 2) tc::split_tf32_x2(t16[j], t16[j + 1], hi[j], hi[j + 1], lo[j], lo[j + 1]);
+        }
+        tc::tmem_st16(lane_addr + kColAhi + c * 16, hi);
+        tc::tmem_st16(lane_addr + kColAlo + c * 16, lo);
+    }
 }
 
 // 16 raw layer-2 accumulators + bias -> relu -> split
@@ -544,11 +551,14 @@ spline_stack_ctx_tc2_kernel(const float* __restrict__ packed, const float* __res
 //   D2 128, D3 16 = all 512 columns of the SM, so ONE CTA per SM; a net block is ~151 KB (W2 hi / lo images alone 128 KB)
 //   and is single buffered -- the next block is requested when every thread is done with the current one (~1 us of a
 //   ~16 us net pass per tile).  Same code otherwise: K = 128 is 16 k-steps per pass, the head reads 4 K atoms.
-template <int DM, int HP, bool SAMPLE = false>
-__global__ void __launch_bounds__(kTcThreads, HP == 64 ? 2 : 1)
-coupling_stack_tc_kernel(const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
-                         float* __restrict__ ld, int64_t B, int flags, int nsub, uint64_t seed, uint64_t offset,
-                         unsigned long long* rng_state) {     // nsub <= kTcSub sub-tiles per weight staging
+// CM > 0: the conditional layout ('NFD2'): layer 1 of both nets also reads C <= CM context columns of row r / ctx_div
+// of `ctx`, through L1 at every use, as the conditional spline kernel; CM == 0 is the unconditional kernel.  tid: see
+// spline_stack_tc2_body.
+template <int DM, int HP, bool SAMPLE, int CM>
+__device__ __forceinline__ void
+coupling_stack_tc_body(int tid, const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
+                       float* __restrict__ ld, int64_t B, int flags, int nsub, uint64_t seed, uint64_t offset,
+                       unsigned long long* rng_state, const float* __restrict__ ctx, int64_t ctx_div, int C) {
     constexpr int NBUF = (HP == 64) ? 2 : 1;
     constexpr int kColAhi = 0, kColAlo = HP, kColD2 = 2 * HP, kColD3 = 3 * HP;
     constexpr int kTmemCols = (HP == 64) ? 256 : 512;
@@ -563,9 +573,9 @@ coupling_stack_tc_kernel(const float* __restrict__ packed, const float* __restri
     uint64_t& bar = bars[0];
     uint64_t* wbar = bars + 1;
     uint32_t& tmem_base_s = *reinterpret_cast<uint32_t*>(bars + 3);
-    const BlkOff off = blk_offsets(W1S, NO3, HP);
+    const BlkOff off = blk_offsets(W1S, NO3, HP, CM);
 
-    const int tid = threadIdx.x, warp = tid >> 5;
+    const int warp = tid >> 5;
     if (warp == 0) tc::tmem_alloc(&tmem_base_s, kTmemCols);
     unsigned long long* rng_key = reinterpret_cast<unsigned long long*>(bars + 4);   // SAMPLE + device state: every
     if constexpr (SAMPLE) if (rng_state) nf_rng_state_take(rng_state, rng_key);   // CTA, before the role split / tiles
@@ -639,7 +649,13 @@ coupling_stack_tc_kernel(const float* __restrict__ packed, const float* __restri
                 float xa[DM];
 #pragma unroll
                 for (int d = 0; d < DM; ++d) xa[d] = (d < D) ? xv[d] * mask[d] : 0.f;
-                layer1_to_tmem<DM, HP>(nb + off.w1k, W1S, xa, lane_addr);
+                if constexpr (CM > 0) {
+                    const int64_t r = tile * ROWS + s * kTcThreads + tid;     // < 2^31, as ctx_div (the launcher)
+                    const uint32_t crow = r < B ? (uint32_t)r / (uint32_t)ctx_div : 0u;
+                    layer1_to_tmem<DM, HP, CM>(nb + off.w1k, W1S, xa, lane_addr, nb + off.wc, ctx + (size_t)crow * C, C);
+                } else {
+                    layer1_to_tmem<DM, HP>(nb + off.w1k, W1S, xa, lane_addr);
+                }
                 cta_mma_round(warp, &bar, phase, [&] {
                     if (HP == 64) tc::warp_issue_gemm_k64_3xtf32(tb, kColD2, kColAhi, kColAlo, w2hi, w2lo, 64u, &bar);
                     else tc::warp_issue_gemm_krange_3xtf32(tb, kColD2, kColAhi, kColAlo, w2hi, w2lo, (uint32_t)HP, 0, HP / 8, 0u, &bar);
@@ -692,6 +708,25 @@ coupling_stack_tc_kernel(const float* __restrict__ packed, const float* __restri
     tc::fence_before_sync();
     __syncthreads();
     if (warp == 0) tc::tmem_dealloc(tb, kTmemCols);
+}
+
+template <int DM, int HP, bool SAMPLE = false>
+__global__ void __launch_bounds__(kTcThreads, HP == 64 ? 2 : 1)
+coupling_stack_tc_kernel(const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
+                         float* __restrict__ ld, int64_t B, int flags, int nsub, uint64_t seed, uint64_t offset,
+                         unsigned long long* rng_state) {     // nsub <= kTcSub sub-tiles per weight staging
+    coupling_stack_tc_body<DM, HP, SAMPLE, 0>(threadIdx.x, packed, x, y, ld, B, flags, nsub, seed, offset, rng_state, nullptr, 1, 0);
+}
+
+// conditional affine coupling stack ('NFD2'): C <= kCtxMax context columns of row r / ctx_div enter the first Linear of
+// both conditioner nets of every layer
+template <int DM, int HP, bool SAMPLE = false>
+__global__ void __launch_bounds__(kTcThreads, HP == 64 ? 2 : 1)
+coupling_stack_ctx_tc_kernel(const float* __restrict__ packed, const float* __restrict__ x, float* __restrict__ y,
+                             float* __restrict__ ld, int64_t B, int flags, int nsub, uint64_t seed, uint64_t offset,
+                             unsigned long long* rng_state, const float* __restrict__ ctx, int64_t ctx_div, int C) {
+    coupling_stack_tc_body<DM, HP, SAMPLE, kCtxMax>(threadIdx.x, packed, x, y, ld, B, flags, nsub, seed, offset, rng_state, ctx,
+                                                    ctx_div, C);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -923,11 +958,21 @@ static int spline_stack_tc_launch(const StackCall& c, const StackHdr& h) {
     return NF_OK;
 }
 
+// CTX: the conditional layout ('NFD2'; header word 3 = context width C) and coupling_stack_ctx_tc_kernel, with the
+// refusals of spline_stack_tc_launch<true>
+template <bool CTX>
 static int coupling_stack_tc_launch(const StackCall& c, const StackHdr& h) {
     const int D = h.D, H = h.H, W1S = h.W1S, NO3 = h.NO, NBW = h.layer_stride;
+    if (CTX) {
+        if (c.cx.ctx == nullptr) return NF_ERR_NULL;
+        if (c.cx.div < 1 || c.cx.rows < cdiv(c.B, c.cx.div)) return NF_ERR_BAD_SHAPE;
+        if (h.HP < 1 || h.HP > kCtxMax) return NF_ERR_UNSUPPORTED;
+        if (c.B > 0x7FFFFFFF || c.cx.div > 0x7FFFFFFF) return NF_ERR_UNSUPPORTED;     // 32-bit row / context-row indices
+    }
     if (D < 1 || D > NF_STACK_DMAX || H < 1 || H > 128 || h.L < 1 || NO3 != 16) return NF_ERR_UNSUPPORTED;
     const int HP = H <= 64 ? 64 : 128;
-    if (W1S != nf_stack_w1s(D) || NBW != NF_LAYER_HDR + blk_offsets(W1S, NO3, HP).net_words) return NF_ERR_BAD_SHAPE;
+    if (W1S != nf_stack_w1s(D) || NBW != NF_LAYER_HDR + blk_offsets(W1S, NO3, HP, CTX ? kCtxMax : 0).net_words)
+        return NF_ERR_BAD_SHAPE;
     if (!c.holds(NF_STACK_HDR + (int64_t)2 * h.L * NBW)) return NF_ERR_WORKSPACE;
     const int DMh = D <= 2 ? 2 : (D <= 3 ? 4 : 8);
     const int nbuf = HP == 64 ? 2 : 1, tmem_cols = HP == 64 ? 256 : 512;
@@ -941,11 +986,20 @@ static int coupling_stack_tc_launch(const StackCall& c, const StackHdr& h) {
     const int grid = (int)(ntiles < cap ? ntiles : cap);
 #define NF_CTC(DMv, HPv)                                                                                              \
     do {                                                                                                             \
-        auto kern = c.sample ? coupling_stack_tc_kernel<DMv, HPv, true> : coupling_stack_tc_kernel<DMv, HPv>;          \
-        const int rc = stack_smem_attributes(kern, smem);                                                            \
-        if (rc != NF_OK) return rc;                                                                                  \
-        kern<<<grid, kTcThreads, smem, c.st>>>((const float*)c.packed, (const float*)c.x, (float*)c.y, (float*)c.ld,  \
-                                               c.B, c.flags, nsub, c.seed, c.offset, c.rng_state);                   \
+        if constexpr (CTX) {                                                                                         \
+            auto kern = c.sample ? coupling_stack_ctx_tc_kernel<DMv, HPv, true> : coupling_stack_ctx_tc_kernel<DMv, HPv>; \
+            const int rc = stack_smem_attributes(kern, smem);                                                        \
+            if (rc != NF_OK) return rc;                                                                              \
+            kern<<<grid, kTcThreads, smem, c.st>>>((const float*)c.packed, (const float*)c.x, (float*)c.y,           \
+                                                   (float*)c.ld, c.B, c.flags, nsub, c.seed, c.offset, c.rng_state,  \
+                                                   (const float*)c.cx.ctx, c.cx.div, h.HP);                          \
+        } else {                                                                                                     \
+            auto kern = c.sample ? coupling_stack_tc_kernel<DMv, HPv, true> : coupling_stack_tc_kernel<DMv, HPv>;      \
+            const int rc = stack_smem_attributes(kern, smem);                                                        \
+            if (rc != NF_OK) return rc;                                                                              \
+            kern<<<grid, kTcThreads, smem, c.st>>>((const float*)c.packed, (const float*)c.x, (float*)c.y,           \
+                                                   (float*)c.ld, c.B, c.flags, nsub, c.seed, c.offset, c.rng_state); \
+        }                                                                                                            \
     } while (0)
     if (HP == 64) { if (D <= 2) NF_CTC(2, 64); else if (D <= 3) NF_CTC(4, 64); else NF_CTC(8, 64); }
     else          { if (D <= 2) NF_CTC(2, 128); else if (D <= 3) NF_CTC(4, 128); else NF_CTC(8, 128); }
@@ -986,7 +1040,8 @@ static int made_stack_tc_launch(const StackCall& c, const StackHdr& h) {
 
 static const StackFamily kSplineTc = {NF_STACK_MAGIC_SPLINE_TC, spline_stack_tc_launch<false>};
 static const StackFamily kSplineCtxTc = {NF_STACK_MAGIC_SPLINE_CTX_TC, spline_stack_tc_launch<true>};
-static const StackFamily kCouplingTc = {NF_STACK_MAGIC_AFFINE_TC, coupling_stack_tc_launch};
+static const StackFamily kCouplingTc = {NF_STACK_MAGIC_AFFINE_TC, coupling_stack_tc_launch<false>};
+static const StackFamily kCouplingCtxTc = {NF_STACK_MAGIC_AFFINE_CTX_TC, coupling_stack_tc_launch<true>};
 static const StackFamily kMadeTc = {NF_STACK_MAGIC_MADE_TC, made_stack_tc_launch};
 
 }  // namespace nf
@@ -1057,6 +1112,32 @@ extern "C" int nf_coupling_stack_tc_sample(const void* packed, const void* hdr_h
 extern "C" int nf_coupling_stack_tc_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes,
                                                  void* rng_state, void* x, void* log_q, int64_t B, nf_stream_t stream) {
     return stack_sample_state(kCouplingTc, packed, hdr_host, packed_bytes, 0, rng_state, x, log_q, B, stream);
+}
+
+extern "C" int64_t nf_coupling_stack_ctx_tc_block_words_hidden(int D, int H) {   // 'NFD2': with the Wc section
+    if (D < 1 || D > NF_STACK_DMAX || H < 1 || H > 128) return -1;
+    return NF_LAYER_HDR + blk_offsets(nf_stack_w1s(D), 16, H <= 64 ? 64 : 128, kCtxMax).net_words;
+}
+
+extern "C" int nf_coupling_stack_ctx_tc_forward(const void* packed, const void* hdr_host, int64_t packed_bytes, const void* x,
+                                                const void* context, int64_t ctx_rows, int64_t ctx_div, void* y, void* ld,
+                                                int64_t B, int flags, nf_stream_t stream) {
+    return stack_forward(kCouplingCtxTc, packed, hdr_host, packed_bytes, x, y, ld, B, flags, 0, stream,
+                         {context, ctx_rows, ctx_div});
+}
+
+extern "C" int nf_coupling_stack_ctx_tc_sample(const void* packed, const void* hdr_host, int64_t packed_bytes,
+                                               const void* context, int64_t ctx_rows, int64_t ctx_div, uint64_t seed,
+                                               uint64_t offset, void* x, void* log_q, int64_t B, nf_stream_t stream) {
+    return stack_sample(kCouplingCtxTc, packed, hdr_host, packed_bytes, 0, seed, offset, x, log_q, B, stream,
+                        {context, ctx_rows, ctx_div});
+}
+
+extern "C" int nf_coupling_stack_ctx_tc_sample_state(const void* packed, const void* hdr_host, int64_t packed_bytes,
+                                                     const void* context, int64_t ctx_rows, int64_t ctx_div, void* rng_state,
+                                                     void* x, void* log_q, int64_t B, nf_stream_t stream) {
+    return stack_sample_state(kCouplingCtxTc, packed, hdr_host, packed_bytes, 0, rng_state, x, log_q, B, stream,
+                              {context, ctx_rows, ctx_div});
 }
 
 extern "C" int64_t nf_made_stack_tc_block_words(int D) {

@@ -544,9 +544,9 @@ class _Coupling(Flow):
 # ------------------------------------------------------------------------------------------------
 # affine coupling
 # ------------------------------------------------------------------------------------------------
-def _coupling_net(data_dim, hidden_dim):
+def _coupling_net(data_dim, hidden_dim, context_dim=0):
     return nn.Sequential(
-        nn.Linear(data_dim, hidden_dim), nn.BatchNorm1d(hidden_dim), nn.ReLU(),
+        nn.Linear(data_dim + context_dim, hidden_dim), nn.BatchNorm1d(hidden_dim), nn.ReLU(),
         nn.Linear(hidden_dim, hidden_dim), nn.BatchNorm1d(hidden_dim), nn.ReLU(),
         nn.Linear(hidden_dim, data_dim))
 
@@ -557,15 +557,21 @@ class CouplingLayer(_Coupling):
     s = clamp(s_net(x*mask), +-10), b = clamp(b_net(x*mask), +-10);
     forward  x = z*mask + (1-mask)*(z*exp(s)+b),     log_det =  sum((1-mask)*s)
     inverse  z = x*mask + (1-mask)*((x-b)*exp(-s)),  log_det = -sum((1-mask)*s);  NaN/Inf -> 0.
-    """
-    _stack = "coupling"
 
-    def __init__(self, data_dim, hidden_dim, mask):
+    context_dim = C > 0 makes it conditional, p(x | c): both conditioners read [x * mask, c] (context columns last, as in
+    nflows), so s_net[0] and b_net[0] are Linear(data_dim + C, hidden_dim); the context is not masked.  forward /
+    inverse then take context= [B, C] or [1, C] (broadcast).
+    """
+
+    def __init__(self, data_dim, hidden_dim, mask, context_dim=0):
         super().__init__()
+        if int(context_dim) != context_dim or context_dim < 0:
+            raise ValueError(f"context_dim must be a non-negative integer, got {context_dim!r}")
+        self.context_dim = int(context_dim)
         self.data_dim = data_dim
         self.register_buffer("mask", mask)
-        self.s_net = _coupling_net(data_dim, hidden_dim)
-        self.b_net = _coupling_net(data_dim, hidden_dim)
+        self.s_net = _coupling_net(data_dim, hidden_dim, self.context_dim)
+        self.b_net = _coupling_net(data_dim, hidden_dim, self.context_dim)
         self._initialize_weights()
         self._pack = _PackCache()
         self._wide = _PackCache()
@@ -581,10 +587,20 @@ class CouplingLayer(_Coupling):
             nn.init.zeros_(net[-1].weight)
             nn.init.zeros_(net[-1].bias)
 
+    @property
+    def _stack(self):             # key of run_stack's family table
+        return "coupling_ctx" if self.context_dim else "coupling"
+
     # -- layered route -------------------------------------------------------------------------
-    def _conditioner(self, net, v):
-        # x*mask is folded into the first weight's columns (same zero/NaN propagation as the product x*mask)
-        h = ops.linear(v, net[0].weight, net[0].bias, mask=self.mask)
+    def _conditioner(self, net, v, ctx=None):
+        # x*mask is folded into the first weight's columns (same zero/NaN propagation as the product x*mask); the
+        # context columns [x*mask, c] go through linear_ctx without its ReLU, so that a train-mode BatchNorm normalises
+        # the full pre-activation, context included, as after a concatenated input
+        if ctx is not None:
+            c, div = ctx.layered(v.shape[0])
+            h = ops.linear_ctx(v, c, net[0].weight, net[0].bias, self.mask, div, relu=False)
+        else:
+            h = ops.linear(v, net[0].weight, net[0].bias, mask=self.mask)
         h = ops.batchnorm_relu(h, net[1])
         h = ops.linear(h, net[3].weight, net[3].bias)
         h = ops.batchnorm_relu(h, net[4])
@@ -600,18 +616,19 @@ class CouplingLayer(_Coupling):
     @on_input_device
     def _run(self, v, inverse, ctx=None):
         v = compute_input(v)
-        if not wants_grad(self, v) and self.fusable(v):
-            out = self._fused(v, inverse)
+        ct = None if ctx is None else ctx.t
+        if not wants_grad(self, v, ct) and self.fusable(v):
+            out = self._fused(v, inverse, ctx=ctx)
             if out is not None:
                 return out
-        if (not wants_grad(self, v) and not self.training and USE_TENSOR_CORES and ops.USE_TENSOR_CORE_GEMM and v.dtype == torch.float32
-                and self.s_net[0].weight.dtype == torch.float32 and v.shape[0] >= WIDE_TC_MIN_ROWS):
+        if (ctx is None and not wants_grad(self, v) and not self.training and USE_TENSOR_CORES and ops.USE_TENSOR_CORE_GEMM
+                and v.dtype == torch.float32 and self.s_net[0].weight.dtype == torch.float32 and v.shape[0] >= WIDE_TC_MIN_ROWS):
             # wide eval route: mask and eval-mode BatchNorm folded into the Linears once per weight version, TF32 splits
             # cached, three tensor-core GEMMs per net (the layered route re-folds and re-splits on every call)
             nets = self._wide.get(self._wide.tensors_of([self]), self._fold_wide)
             return ops.affine_coupling(v, _tc_mlp(v, nets[0]), _tc_mlp(v, nets[1]), self.mask, inverse)
-        s_raw = self._conditioner(self.s_net, v)
-        b_raw = self._conditioner(self.b_net, v)
+        s_raw = self._conditioner(self.s_net, v, ctx)
+        b_raw = self._conditioner(self.b_net, v, ctx)
         return ops.affine_coupling(v, s_raw, b_raw, self.mask, inverse)
 
     def _fold_wide(self):
@@ -1007,15 +1024,17 @@ USE_TENSOR_CORES = True      # tcgen05 stack kernels (3xTF32, fp32-accurate); Fa
 _STACKS = {"spline": (packing.pack_spline_stack_tc, packing.pack_spline_stack, "nf_spline_stack_tc", "nf_spline_stack"),
            "coupling": (packing.pack_coupling_stack_tc, packing.pack_coupling_stack, "nf_coupling_stack_tc",
                         "nf_coupling_stack"),
-           # conditional spline layers: tcgen05 only, outside its envelope the layered route
-           "spline_ctx": (packing.pack_spline_stack_ctx_tc, None, "nf_spline_stack_ctx_tc", None)}
+           # conditional layers: tcgen05 only, outside its envelope the layered route
+           "spline_ctx": (packing.pack_spline_stack_ctx_tc, None, "nf_spline_stack_ctx_tc", None),
+           "coupling_ctx": (packing.pack_coupling_stack_ctx_tc, None, "nf_coupling_stack_ctx_tc", None)}
 
 
 def run_stack(family, cache: _PackCache, tensors, flows, bns, v, inverse, head=False, sample=None, ctx=None):
     """Spline-coupling or eval-mode affine coupling stack in one launch: the tcgen05 kernel when USE_TENSOR_CORES is set
     and the configuration fits it (spline: hidden_dim <= 64; affine: hidden_dim <= 128), the FP32-pipe kernel otherwise
     -- also when the tcgen05 launch refuses the configuration.  sample=(seed, offset): the in-kernel N(0, I) draw into v,
-    returning (x, log_q) (see ops.stack).  ctx: the _Context of the conditional family "spline_ctx"."""
+    returning (x, log_q) (see ops.stack).  ctx: the _Context of the conditional families "spline_ctx" and
+    "coupling_ctx"."""
     pack_tc, pack, entry_tc, entry = _STACKS[family]
 
     def build():
@@ -1052,7 +1071,8 @@ class ChainPlan:
         layer's epilogue -- z is never written.
         sample=(seed, offset) (forward only): the sampling twin of the head -- v is the [n, D] output buffer, the rows are
         the N(0, I) draw of csrc/nf_rng.cuh made in the kernel, and the result is (x, log N(z) - log_det).
-        ctx (a _Context): every layer must be a SplineCouplingLayer with that context width, float32 context included."""
+        ctx (a _Context): every layer must be a SplineCouplingLayer or CouplingLayer with that context width, float32
+        context included."""
         flows = list(flows)
         v = compute_input(v)
         if not flows or not v.is_cuda or v.dim() != 2:
@@ -1064,7 +1084,7 @@ class ChainPlan:
         if not made and (kind not in (CouplingLayer, SplineCouplingLayer) or any(type(f) is not kind for f in flows)
                          or not all(f.fusable(v) for f in flows)):
             return None
-        if ctx is not None and (kind is not SplineCouplingLayer or ctx.t.dtype != torch.float32
+        if ctx is not None and (made or ctx.t.dtype != torch.float32
                                 or any(f.context_dim != ctx.t.shape[1] for f in flows)):
             return None
         mods = flows + (list(bns) if bns is not None else [])

@@ -161,7 +161,11 @@ class _HalfMaskStack(_DensityAPI, nn.Module):
 
 
 class RealNVP(_HalfMaskStack):
+    """context_dim = C > 0: every layer is a conditional CouplingLayer reading the one context."""
     _layer = CouplingLayer
+
+    def __init__(self, data_dim, n_layers, hidden_dim, batch_norm_between_layers=False, context_dim=0):
+        super().__init__(data_dim, n_layers, hidden_dim, batch_norm_between_layers, context_dim=context_dim)
 
 
 class RealNVPSpline(_HalfMaskStack):

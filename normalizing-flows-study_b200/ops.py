@@ -267,14 +267,15 @@ def _wgrad(g, a):
 
 
 class _LinearCtxFn(Function):
-    """relu(W[:, :D] (x*mask) + W[:, D:] c + b): the first Linear of a conditional spline conditioner, whose input is
+    """relu(W[:, :D] (x*mask) + W[:, D:] c + b): the first Linear of a conditional coupling conditioner, whose input is
     [x*mask, c] (context columns last), without concatenating x and c.  Two products into one output: the context one
     without bias, then the masked x one with bias and ReLU accumulated onto it (nf_gemm computes relu(acc + bias + C_old)
     on every path).  `div`: row r of x uses context row r // div; 1 (one context row per row) or, with a single context
-    row, anything (that row is read with row stride 0)."""
+    row, anything (that row is read with row stride 0).  relu=False (the affine conditioner, whose BatchNorm follows the
+    Linear): the same products without the ReLU."""
 
     @staticmethod
-    def forward(ctx, x, c, weight, bias, mask, div):
+    def forward(ctx, x, c, weight, bias, mask, div, relu=True):
         x, c = _c(x), _c(c)
         B, D = x.shape
         H, C = weight.shape[0], c.shape[1]
@@ -282,8 +283,8 @@ class _LinearCtxFn(Function):
         wc = _c(weight[:, D:])
         per_row = c.shape[0] == B and div == 1
         y = _product(c, wc) if per_row else gemm(c, wc, B, H, C, 0, 1, 1, C)
-        gemm(x, wx, B, H, D, D, 1, 1, D, bias=_c(bias), relu=True, out=y, accumulate=True)
-        ctx.per_row = per_row
+        gemm(x, wx, B, H, D, D, 1, 1, D, bias=_c(bias), relu=relu, out=y, accumulate=True)
+        ctx.per_row, ctx.relu = per_row, relu
         ctx.save_for_backward(x, c, wx, wc, mask, y)
         return y
 
@@ -293,7 +294,11 @@ class _LinearCtxFn(Function):
         x, c, wx, wc, mask, y = ctx.saved_tensors
         B, D = x.shape
         H, C = wc.shape
-        g, gb = relu_backward_colsum(y, _c(gy))                     # the bias gradient comes out of the same pass
+        if ctx.relu:
+            g, gb = relu_backward_colsum(y, _c(gy))                 # the bias gradient comes out of the same pass
+        else:
+            g = _c(gy)
+            gb = col_sum(g)
         gx = gc = gw = None
         if ctx.needs_input_grad[0]:
             gx = _product(g, _c(wx.t()))                            # dX = dY Wx
@@ -303,14 +308,14 @@ class _LinearCtxFn(Function):
             gw = torch.empty((H, D + C), dtype=g.dtype, device=g.device)
             gw[:, :D] = mul_rows(_wgrad(g, x), mask)
             gw[:, D:] = _wgrad(g, c) if ctx.per_row else gemm(gb.view(H, 1), c, H, C, 1, 1, 1, C, 1)
-        return gx, gc, gw, (gb if ctx.needs_input_grad[3] else None), None, None
+        return gx, gc, gw, (gb if ctx.needs_input_grad[3] else None), None, None, None
 
 
-def linear_ctx(x, c, weight, bias, mask, div):
+def linear_ctx(x, c, weight, bias, mask, div, relu=True):
     """relu(F.linear(cat([x*mask, c[r // div]]), weight, bias)) with x [B, D], c [rows, C], weight [H, D+C] (see
-    _LinearCtxFn)."""
+    _LinearCtxFn); relu=False: without the ReLU."""
     weight, bias, mask, c = _same_dtype(x, weight, bias, mask, c)
-    return _LinearCtxFn.apply(x, c, weight, bias, mask, int(div))
+    return _LinearCtxFn.apply(x, c, weight, bias, mask, int(div), bool(relu))
 
 
 # --------------------------------------------------------------------------------------------
@@ -816,7 +821,8 @@ def stack(entry, packed, hdr_host, x, inverse, head=False, sample=None, mode=(),
     the configuration is unsupported.  sample=(seed, offset): the `_sample` entry point instead -- x is the output buffer of the rows, drawn from N(0, I) in the kernel and run forward, and the
     per-row output is log N(z) - log_det (sample_and_log_prob).  sample=<DeviceGenerator state tensor>: `_sample_state`,
     the same draw with the key read from, and advanced in, device memory (a refused call leaves the state as it was).
-    context=(c, div) (nf_spline_stack_ctx_tc): the float32 [rows, C] context, row r of the batch reading row r // div."""
+    context=(c, div) (nf_spline_stack_ctx_tc, nf_coupling_stack_ctx_tc): the float32 [rows, C] context, row r of the
+    batch reading row r // div."""
     x = _c(x)
     B = x.shape[0]
     ld = torch.empty(B, dtype=x.dtype, device=x.device)

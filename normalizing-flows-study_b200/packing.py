@@ -22,7 +22,8 @@ MAGIC_SPLINE_TC = 0x4E465332
 MAGIC_AFFINE_TC = 0x4E464132
 MAGIC_MADE_TC = 0x4E464D32
 MAGIC_SPLINE_CTX_TC = 0x4E464332
-CTX_MAX = 8                     # context columns of the conditional tcgen05 spline layout ('NFC2'; csrc/stack_small.cuh)
+MAGIC_AFFINE_CTX_TC = 0x4E464432
+CTX_MAX = 8                     # context columns of the conditional tcgen05 layouts ('NFC2', 'NFD2'; csrc/stack_small.cuh)
 HDR, LAYER_HDR, DMAX = 16, 80, 8
 
 
@@ -169,7 +170,7 @@ def _spline_key(l):
 
 
 def _coupling_key(l):
-    return (l.data_dim, l.s_net[0].out_features)
+    return (l.data_dim, l.s_net[0].out_features, l.context_dim)
 
 
 def _alike(layers, key):
@@ -220,7 +221,7 @@ def pack_coupling_stack(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
     l0 = layers[0]
     D = l0.data_dim
     H = l0.s_net[0].out_features
-    if not _alike(layers, _coupling_key):
+    if not _alike(layers, _coupling_key) or l0.context_dim:
         return None
     if D > DMAX or H > 128 or l0.s_net[0].weight.dtype != torch.float32:
         return None
@@ -609,6 +610,23 @@ def pack_coupling_stack_tc(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
     """Tensor-core layout of an eval-mode affine coupling stack (hidden_dim <= 128, padded to 64 or 128; data_dim <= 8):
     per layer two net blocks (s_net then b_net), each `lead (80 words: the layer header for s_net, zeros for b_net) |
     W1k | b2 | b3 | pad | W2 hi/lo images | W3 hi/lo images`, conditioner BatchNorm folded into the Linears."""
+    if layers[0].context_dim:
+        return None
+    return _pack_coupling_tc(layers, bns, 0)
+
+
+def pack_coupling_stack_ctx_tc(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
+    """Conditional twin of pack_coupling_stack_tc ('NFD2', csrc/stack_small.cuh): the same envelope for layers that share
+    one context_dim in 1..CTX_MAX; header word 3 holds it and every net block gains the Wc section after b3.  The
+    conditioner BatchNorm is folded into the whole [H, D + C] first weight -- it scales rows, context columns included --
+    before the weight is split into its x columns (W1k) and context columns (Wc)."""
+    C = layers[0].context_dim
+    if C < 1 or C > CTX_MAX:
+        return None
+    return _pack_coupling_tc(layers, bns, C)
+
+
+def _pack_coupling_tc(layers, bns, C):
     l0 = layers[0]
     D = l0.data_dim
     H = l0.s_net[0].out_features
@@ -617,11 +635,12 @@ def pack_coupling_stack_tc(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
     if D > DMAX or H > 128 or l0.s_net[0].weight.dtype != torch.float32:
         return None
     HP = _hp(H)
-    nbw = L.lib().nf_coupling_stack_tc_block_words_hidden(D, H)
+    nbw = (L.lib().nf_coupling_stack_ctx_tc_block_words_hidden if C else L.lib().nf_coupling_stack_tc_block_words_hidden)(D, H)
     if nbw < 0:
         return None
     W1S, NO3 = _w1s(D), 16
-    words = [_stack_header(MAGIC_AFFINE_TC, D, H, 2, 0, len(layers), W1S, NO3, nbw, bns)]
+    magic, w3 = (MAGIC_AFFINE_CTX_TC, C) if C else (MAGIC_AFFINE_TC, 2)
+    words = [_stack_header(magic, D, H, w3, 0, len(layers), W1S, NO3, nbw, bns)]
     for i, l in enumerate(layers):
         m = _np(l.mask)
         lead = [_layer_header(m.astype(np.float32), [d for d in range(D) if m[d] == 0], None,
@@ -634,6 +653,7 @@ def pack_coupling_stack_tc(layers, bns: Optional[List[torch.nn.BatchNorm1d]]):
             b3rows = np.zeros(NO3)
             W3rows[:D] = _np(net[6].weight)
             b3rows[:D] = _np(net[6].bias)
-            blk = _tc_net_block(W1, b1, W2, b2, W3rows, b3rows, D, H, W1S, NO3, LAYER_HDR, HP)
+            blk = _tc_net_block(W1[:, :D], b1, W2, b2, W3rows, b3rows, D, H, W1S, NO3, LAYER_HDR, HP,
+                                Wc=W1[:, D:] if C else None)
             words += [ld, blk]
     return _finish(words, HDR + 2 * len(layers) * nbw, l0.s_net[0].weight.device)
